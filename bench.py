@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                 # this repo's CUDA path; headline = configs[1]
     python bench.py --impl reference --gpus N --steps K ...       # reference arm: the reference's CPU path, host cores
     python bench.py --workload full_step --gpus N ...             # configs[2]: reference backbone + fused losses under DDP
+    python bench.py --gpus 1 --steps K --dump-outputs DIR         # + the last timed step's outputs as DIR/<name>.npy
 
 Headline workload (one "step" = one fused forward+backward pass over one batch): B=64 images of 256x256 pixel
 embeddings, D=512, bf16, K=256 text rows (63 ground-truth labels + 193 curriculum distractors), sampling weights as in
@@ -391,6 +392,26 @@ def section(fn):
         return {"error": repr(e)[:300]}
 
 
+DUMP_PIXELS = 8192
+
+
+def dump_outputs(out_dir, dx, lse, acc):
+    """Write what the headline step returns to its caller, from its last timed run, as DIR/<name>.npy: the loss and
+    weight sums and dlogtau (float64), the log-sum-exp of every pixel row (float32), and dX (float32) at DUMP_PIXELS
+    pixels drawn with a fixed seed, all D channels each (dx_sample[i] is pixel dx_sample_pixels[i] = b * HW + p).
+    About 34 MB at the headline shape, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    B, D, HW = dx.shape
+    pix = np.sort(np.random.default_rng(0).choice(B * HW, size=min(DUMP_PIXELS, B * HW), replace=False))
+    pix_d = torch.from_numpy(pix).to(dx.device)
+    out = {"loss_sum": acc[0], "w_sum": acc[1], "dlogtau": acc[2], "lse": lse,
+           "dx_sample": dx[pix_d // HW, :, pix_d % HW].float(), "dx_sample_pixels": pix.astype(np.float64)}
+    for name, v in out.items():
+        if isinstance(v, torch.Tensor):
+            v = v.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def run_gpu(args):
     import torch.distributed as dist
     from rangeclip_b200 import _lib, ops
@@ -486,6 +507,8 @@ def run_gpu(args):
     ms = float(tmax)
     loss = float(acc[0] / acc[1])
     value = world * M * args.steps / (ms * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:      # before the sections below reuse dx / lse / acc
+        dump_outputs(args.dump_outputs, dx, lse, acc)
 
     # ---- dominant kernel: average launch duration from the CUDA events recorded inside the timed region
     k_ms = sum(e0.elapsed_time(e1) for e0, e1 in kernel_events) / max(1, len(kernel_events))
@@ -938,7 +961,13 @@ def main():
     ap.add_argument("--phase", default="step", choices=["step", "backbone", "nosync"], help="full_step: what is timed")
     ap.add_argument("--builder", default="device", choices=["device", "reference"],
                     help="full_step: contrast-set builder of compute_loss (device = sync-free, SURVEY 8f-2; reference = host RNG parity)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "infonce" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the headline workload (--workload infonce --impl ours)")
     if args.workload == "full_step":
         from tools.full_step import run_full_step
         run_full_step(args)

@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench as BN
 from rangeclip_b200 import ops, losses
 dev = torch.device("cuda:0")
