@@ -97,10 +97,14 @@ int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t ld_b,
  *                           round 2 = backward launches with both flags: dx and dlogtau of each block add up to the full gradient */
 #define RC_INFONCE_KEEP_WEIGHT 2
 #define RC_INFONCE_LSE_GIVEN 4
-/* RC_INFONCE_TS_KERNEL: backward launches (dx given, no dt) of D = 256 / 512 run the kernel whose softmax tile is a
- * tensor-memory operand of the dX GEMM (TS-mode tcgen05.mma, csrc/infonce_ts.cu) instead of the kernel with both operands
- * in shared memory (csrc/infonce_umma2.cu).  Same results bit for bit; which one is faster is recorded in DESIGN.md. */
+/* Backward launches (dx given, no dt) of D = 256 / 512 with K and log tau given by the host (rc_infonce_bf16, _rep4 and the
+ * K-blocked rounds) run the kernel whose softmax tile is a tensor-memory operand of the dX GEMM (TS-mode tcgen05.mma,
+ * csrc/infonce_ts.cu).  Forward-only launches, launches with dt and rc_infonce_bf16_dyn run the kernel with both operands in
+ * shared memory (SS, csrc/infonce_umma2.cu).  Both give the same results bit for bit; DESIGN.md records their speed.
+ *   RC_INFONCE_SS_KERNEL  run the SS kernel for a backward launch too (A/B measurements)
+ *   RC_INFONCE_TS_KERNEL  the default for the launches above; kept so that callers that asked for TS keep working */
 #define RC_INFONCE_TS_KERNEL 8
+#define RC_INFONCE_SS_KERNEL 32
 /* RC_INFONCE_ACCUMULATE_DX: dx += this launch's gradient instead of dx = (TMA reduce-add stores, bf16 accumulation).  The
  * backward launches of the K-blocked scheme after the first one: the per-block gradients add up in ONE bf16 tensor. */
 #define RC_INFONCE_ACCUMULATE_DX 16

@@ -12,9 +12,9 @@
 //                   B = own 32 rows of T^T [D][Kp] (K-major, shared memory: 32 B/clk of operand reads); two 64-column fp32
 //                   accumulators in the remaining 128 columns of the slot
 // Tensor memory holds TWO slots (2 x 256 columns); tile pairs alternate between them.  MMA issue order
-//   S(0) S(1) | dX(0) S(2) | dX(1) S(3) | dX(2) S(4) | ...
-// so the exp pass of pair j+1 runs while the tensor pipe works on dX(j) and S(j+2) of the OTHER slot: no role waits for a
-// hand-off it has just produced.  Pixels stay on the TMEM lanes for both GEMMs, so a CTA's softmax and dX epilogue work on
+//   S(0) | dX(0)[0,2) S(1) dX(0)[2,n) | dX(1)[0,2) S(2) dX(1)[2,n) | ...      ([a,b): 64-channel blocks of dX)
+// so the exp pass of pair j+1 runs while the tensor pipe works on dX(j) of the OTHER slot, and the dX epilogue drains the
+// first two blocks of dX(j) while S(j+1) is computed: no role waits for a hand-off it has just produced.  Pixels stay on the TMEM lanes for both GEMMs, so a CTA's softmax and dX epilogue work on
 // its own tile only (no row-scale exchange between the CTAs).  The dX epilogue thread owns a pixel: 32 channels per step
 // come out of TMEM, the x values of the same [32 ch][32 px] box arrive by TMA in a small per-warp ring (the box doubles as
 // the staging tile of the TMA store), dx = acc - cs x is formed in place and the box goes back with one TMA store.
@@ -29,8 +29,32 @@ using namespace umma;
 
 namespace ts {
 
+// L2 policy of the two reads of a tile of X.  The dX epilogue reads the tile again two pair iterations after the S GEMM did;
+// in between, the L2 sees about 2 x 74 clusters x 256 KB of other X and as much dX written.  1: the S GEMM's loads mark
+// the lines evict_last and the epilogue's (last) load marks them evict_first, so that kept lines are released as soon as
+// they have been consumed.  0: no hints (A/B: make variant VSRC=infonce_ts NAME=.. DEFS=-DRC_TS_X_HINT=0).
 #ifndef RC_TS_X_HINT
-#define RC_TS_X_HINT 0      // A/B: evict_last on the X loads of the S GEMM
+#define RC_TS_X_HINT 1
+#endif
+
+#ifdef RC_TIMING
+__device__ __forceinline__ unsigned long long globaltimer_ns() {     // one clock for both CTAs of the pair
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+// per-role wait cycles (tools/timing_ts.py): wt[tag] += cycles spent in the wait with that tag, wt[0] = lifetime
+#define RC_T0(name) const long long name = clock64()
+#define RC_TACC(idx, name) wt[idx] += clock64() - name
+#define RC_WAIT(fn, bar, par, tag) do { const long long t0_ = clock64(); fn(bar, par, tag); wt[tag] += clock64() - t0_; } while (0)
+// event trace of cluster 0: %globaltimer of event `id` of tile-pair iteration `iter` in [40, 44)
+#define RC_EV(iter, id) do { if (prm.dbg != nullptr && blockIdx.x < 2 && lane == 0 && (iter) >= 40u && (iter) < 44u) \
+    prm.dbg[256 + blockIdx.x * 192 + ((iter) - 40u) * 48 + (id)] = (long long)globaltimer_ns(); } while (0)
+#else
+#define RC_T0(name)
+#define RC_TACC(idx, name)
+#define RC_WAIT(fn, bar, par, tag) fn(bar, par, tag)
+#define RC_EV(iter, id)
 #endif
 
 constexpr int kTilePx = 128;
@@ -44,6 +68,7 @@ constexpr int kEpiBufBytes = 2048;
 constexpr int kTmemCols = 512;
 constexpr int kSlotCols = 256;         // one slot: S [0,256) -> P [0,128) + two dX accumulators [128,192), [192,256)
 constexpr int kColAcc = 128, kAccCols = 64;
+constexpr int kDxLead = 2;             // dX blocks of pair l issued before S(l+1): one per accumulator of the slot
 constexpr int kRegsCtl = 48, kRegsSoftmax = 120;     // epilogue warps keep the entry allocation (96); 48 + 2*120 + 2*96 = 5*96
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
@@ -65,11 +90,14 @@ constexpr int kOffEpi = kOffT + kTStages * kStageBytes;
 constexpr int kOffScale = kOffEpi + 8 * kEpiBufs * kEpiBufBytes;      // -cs per pixel: [kScaleBufs][128] float
 constexpr int kOffXch = kOffScale + kScaleBufs * 128 * 4;
 constexpr int kOffPart = kOffXch + 2 * 4 * 2 * 128 * 4;               // exchange: [2 tile parities][max, sum, sez, sy][2 halves][128]
-constexpr int kOffBars = kOffPart + 8 * 128 * 4;                      // row-norm partial sums of squares [8 softmax warps][128 px]
+constexpr int kOffAcc = kOffPart + 8 * 128 * 4;                       // row-norm partial sums of squares [8 softmax warps][128 px]
+constexpr int kOffBars = kOffAcc + 3 * 128 * 4;                       // per-pixel-row loss / weight / dlogtau sums [3][128]
 constexpr int kSmemBytes = kOffBars + (int)sizeof(Bars);
 static_assert(kSmemBytes <= 232448, "shared-memory budget of one SM (227 KB)");
 
 struct Params {
+  long long* dbg;           // timing build: per-role wait cycles and the event trace (tools/timing_ts.py)
+  int ablate;               // bring-up only (RANGECLIP_B200_ABLATE): 1 no epilogue x loads, 2 no dX stores, 256 no text reloads
   int B, D, K, Kp;
   int64_t HW;
   int tiles_per_img, n_tiles, n_pairs;
@@ -166,6 +194,12 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
   cluster_sync();            // both CTAs' barriers are initialised before any remote arrive / 2-SM TMA credit
   tc_fence_after();
   const uint32_t tmem = bars->tmem_base;
+#ifdef RC_TIMING
+  long long wt[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) wt[i] = 0;
+  const long long t_start = clock64();
+#endif
   const uint32_t idesc_s = make_idesc_bf16(256, prm.Kp, /*A MN-major*/ 1, /*B K-major*/ 0);
   const uint32_t idesc_d = make_idesc_bf16(256, kAccCols, 0, 0);
   auto arrive_leader = [&](uint64_t* bar) {
@@ -184,22 +218,30 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsCtl));
     if (warp == 0 && lane == 0) {
       // =============================== text producer (both CTAs) ===============================
-      // ring order == MMA issue order: S(0) S(1) | dX(0) S(2) | dX(1) S(3) | ...
+      // ring order == MMA issue order: S(0) | dX(0)[0,2) S(1) dX(0)[2,n) | dX(1)[0,2) S(2) dX(1)[2,n) | ...
       uint32_t it = 0;
       auto load_s = [&](int l) {
         const int koff = koff_of(pair_of(l));
         for (int c = 0; c < n_dchunks; ++c, ++it) {   // own half (Nh rows) of text chunk c
           const int st = it % kTStages;
-          mbar_wait(&bars->tempty[st], ((it / kTStages) & 1) ^ 1, 1);
+          RC_WAIT(mbar_wait, &bars->tempty[st], ((it / kTStages) & 1) ^ 1, 1);
+          if ((prm.ablate & 256) && it >= (uint32_t)kTStages) {      // bring-up: no text traffic after the first ring pass (stale operands)
+            if (leader_cta) mbar_arrive(&bars->tfull[st]);
+            continue;
+          }
           if (leader_cta) mbar_arrive_expect_tx(&bars->tfull[st], 2 * Nh * 128);
           tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_t, &bars->tfull[st], c * 64, koff + (int)rank * Nh);
         }
       };
-      auto load_dx = [&](int l) {          // per 64-channel block: own 32 rows of T^T, all Kp columns (4 KB per 64 k)
+      auto load_dx = [&](int l, int b0, int b1) {     // per 64-channel block: own 32 rows of T^T, all Kp columns (4 KB per 64 k)
         const int koff = koff_of(pair_of(l));
-        for (int blk = 0; blk < n_blk; ++blk, ++it) {
+        for (int blk = b0; blk < b1; ++blk, ++it) {
           const int st = it % kTStages;
-          mbar_wait(&bars->tempty[st], ((it / kTStages) & 1) ^ 1, 2);
+          RC_WAIT(mbar_wait, &bars->tempty[st], ((it / kTStages) & 1) ^ 1, 2);
+          if ((prm.ablate & 256) && it >= (uint32_t)kTStages) {
+            if (leader_cta) mbar_arrive(&bars->tfull[st]);
+            continue;
+          }
           if (leader_cta) mbar_arrive_expect_tx(&bars->tfull[st], 2 * n_kchunks * 4096);
           for (int kc = 0; kc < n_kchunks; ++kc)
             tma_load_2d_2sm(smem + kOffT + st * kStageBytes + kc * 4096, &map_tt, &bars->tfull[st], koff + kc * 64,
@@ -207,10 +249,10 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
         }
       };
       if (my_pairs > 0) load_s(0);
-      if (my_pairs > 1) load_s(1);
       for (int l = 0; l < my_pairs; ++l) {
-        load_dx(l);
-        if (l + 2 < my_pairs) load_s(l + 2);
+        load_dx(l, 0, kDxLead);
+        if (l + 1 < my_pairs) load_s(l + 1);
+        load_dx(l, kDxLead, n_blk);
       }
     } else if (warp == 3 && lane == 0) {
       // =============================== X producer (both CTAs) ===============================
@@ -221,11 +263,11 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
         tile_coords(prm, 2 * pair_of(l) + (int)rank, b, px0);
         for (int c = 0; c < n_dchunks; ++c, ++xit) {
           const int st = xit % kXStages;
-          mbar_wait(&bars->xempty[st], ((xit / kXStages) & 1) ^ 1, 3);
+          RC_WAIT(mbar_wait, &bars->xempty[st], ((xit / kXStages) & 1) ^ 1, 3);
           uint8_t* sb = smem + st * kStageBytes;
           mbar_arrive_expect_tx(&bars->xf[st], 2 * 8192);          // CTA-local: the row-norm warp reads the chunk too
           const int bx = (kKB && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;      // kb mode: the one image of X (1 = out of bounds)
-          if (RC_TS_X_HINT) {       // the tile is read again by the dX epilogue two iterations later: keep it in the L2
+          if (RC_TS_X_HINT) {
             tma_load_3d_hint(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx, pol_keep);
             tma_load_3d_hint(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx, pol_keep);
           } else {
@@ -238,26 +280,27 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       // =============================== MMA issuer (leader CTA) ================================
       // whole warp converged (addresses / descriptors in uniform registers), one elected lane issues
       uint32_t it = 0, xit = 0;
-      uint32_t acc_uses[2][2] = {{0, 0}, {0, 0}};      // per slot, per accumulator: launches so far
+      uint32_t acc_par = 0;      // bit 2 * slot + accumulator: parity of that accumulator's launches so far (no local array)
       const uint32_t smem_base = smem_u32(smem);
       const uint64_t dsc_x = desc_mnmajor_sw128(0, 8192);
       const uint64_t dsc_k = desc_kmajor_sw128(0);
       // the slot's accumulators have been drained by the epilogue warps (all launches so far)
-      auto wait_acc_free = [&](int sl, int ab) {
-        mbar_wait(&bars->acc_empty[sl][ab], (acc_uses[sl][ab] & 1u) ^ 1u, 7);
+      auto wait_acc_free = [&](int sl, int ab, int tag) {
+        RC_WAIT(mbar_wait, &bars->acc_empty[sl][ab], ((acc_par >> (2 * sl + ab)) & 1u) ^ 1u, tag);
       };
       auto issue_s = [&](int l) {
         const int sl = l & 1;
         const uint32_t s_tmem = tmem + sl * kSlotCols;
         // S overwrites the slot: its P has been consumed (the dX MMAs were issued before, the pipe runs in order) and
         // both dX accumulators must have been read out
-        wait_acc_free(sl, 0);
-        wait_acc_free(sl, 1);
+        wait_acc_free(sl, 0, 7);
+        wait_acc_free(sl, 1, 7);
         tc_fence_after();
+        RC_EV(l, 0);               // S(l) issue starts (slot free)
         for (int c = 0; c < n_dchunks; ++c, ++it, ++xit) {
           const int sa = xit % kXStages, sb_ = it % kTStages;
-          mbar_wait(&bars->xfull[sa], (xit / kXStages) & 1, 5);
-          mbar_wait(&bars->tfull[sb_], (it / kTStages) & 1, 6);
+          RC_WAIT(mbar_wait, &bars->xfull[sa], (xit / kXStages) & 1, 5);
+          RC_WAIT(mbar_wait, &bars->tfull[sb_], (it / kTStages) & 1, 6);
           tc_fence_after();
           const uint64_t xa = dsc_x + ((smem_base + sa * kStageBytes) >> 4);
           const uint64_t tb = dsc_k + ((smem_base + kOffT + sb_ * kStageBytes) >> 4);
@@ -271,17 +314,22 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
           }
           __syncwarp();
         }
+        RC_EV(l, 1);               // S(l) issued
       };
-      auto issue_dx = [&](int l) {
+      auto issue_dx = [&](int l, int b0, int b1) {      // blocks [b0, b1) of dX(l)
         const int sl = l & 1;
         const uint32_t base = tmem + sl * kSlotCols;
-        mbar_wait(&bars->p_full[sl], (l >> 1) & 1, 9);           // P(l) is in tensor memory
-        tc_fence_after();
-        for (int blk = 0; blk < n_blk; ++blk, ++it) {
+        if (b0 == 0) {
+          RC_WAIT(mbar_wait, &bars->p_full[sl], (l >> 1) & 1, 9);         // P(l) is in tensor memory
+          tc_fence_after();
+          RC_EV(l, 2);             // dX(l) issue starts (P(l) in tensor memory)
+        }
+        for (int blk = b0; blk < b1; ++blk, ++it) {
           const int ab = blk & 1;
-          wait_acc_free(sl, ab);
+          wait_acc_free(sl, ab, 4);
+          if (blk < 8) RC_EV(l, 3 + blk);     // block's accumulator free
           const int st = it % kTStages;
-          mbar_wait(&bars->tfull[st], (it / kTStages) & 1, 8);
+          RC_WAIT(mbar_wait, &bars->tfull[st], (it / kTStages) & 1, 8);
           tc_fence_after();
           const uint64_t sb = dsc_k + ((smem_base + kOffT + st * kStageBytes) >> 4);
           const uint32_t dcol = base + kColAcc + ab * kAccCols;
@@ -295,14 +343,17 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
             mma_commit_2sm(&bars->acc_full[sl][ab]);
           }
           __syncwarp();
-          ++acc_uses[sl][ab];
+          acc_par ^= 1u << (2 * sl + ab);
         }
+        if (b1 == n_blk) RC_EV(l, 11);      // dX(l) issued
       };
+      // S(l+1) goes between the first kDxLead blocks of dX(l) and the rest: the epilogue drains those blocks while the
+      // tensor pipe computes S(l+1), instead of idling through every S GEMM
       if (my_pairs > 0) issue_s(0);
-      if (my_pairs > 1) issue_s(1);
       for (int l = 0; l < my_pairs; ++l) {
-        issue_dx(l);
-        if (l + 2 < my_pairs) issue_s(l + 2);
+        issue_dx(l, 0, kDxLead);
+        if (l + 1 < my_pairs) issue_s(l + 1);
+        issue_dx(l, kDxLead, n_blk);
       }
     } else if (warp == 2 && lane == 0) {
       // ========== relay (both CTAs): "own X chunk has landed" (CTA-local xf) -> the leader's full barrier ==========
@@ -323,12 +374,14 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     const int cb = half * Kh;
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     float* xch_base = reinterpret_cast<float*>(smem + kOffXch);
-    float loss_acc = 0.f, w_acc = 0.f, dlt_acc = 0.f;
-    float inv_wsum = 0.f, gscale = 1.f;
+    // the running loss / weight / dlogtau sums of a row live in shared memory: in registers they are spilled across the exp
+    // pass (96 registers at compile time)
+    float* acc_s = reinterpret_cast<float*>(smem + kOffAcc) + row;
+    if (half == 0) acc_s[0] = acc_s[128] = acc_s[256] = 0.f;
+    float coefb;               // d loss / d (mean) = grad_scale / sum of weights
     {
       const double ws = prm.w_sum_in[0];
-      inv_wsum = ws > 0.0 ? (float)(1.0 / ws) : 0.f;
-      if (prm.grad_scale) gscale = prm.grad_scale[0];
+      coefb = (prm.grad_scale ? prm.grad_scale[0] : 1.f) * (ws > 0.0 ? (float)(1.0 / ws) : 0.f);
     }
     float nx_ok = 0.f, nx_w = 0.f;
     int nx_y = -1;
@@ -366,7 +419,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       for (int j = 0; j < 8; ++j) ss[j] = 0.f;
       for (int c = 0; c < n_dchunks; ++c, ++nit) {
         const int st = nit % kXStages;
-        mbar_wait(&bars->xf[st], (nit / kXStages) & 1, 11);
+        RC_WAIT(mbar_wait, &bars->xf[st], (nit / kXStages) & 1, 11);
         const uint8_t* base = smem + st * kStageBytes + (ng >> 3) * 8192 + nr * 128;
         const int ch = ng & 7;
 #pragma unroll
@@ -414,12 +467,17 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       load_pixel_scalars(l + 1);
       float* xch = xch_base + (l & 1) * (4 * 2 * 128);
       const uint32_t trow = lane_base + sl * kSlotCols + cb;
+      RC_T0(tnorm);
       const float inv_n_tile = norm_tile();
+      RC_TACC(1, tnorm);
+      if (warp == 4) RC_EV(l, 12);      // row norms of the tile done
       const float inv_n = px_ok ? inv_n_tile : 0.f;
       const float zs = inv_n * prm.inv_tau;
       const float zl = zs * kLog2e;
-      mbar_wait(&bars->s_full[sl], (l >> 1) & 1, 12);
+      RC_WAIT(mbar_wait, &bars->s_full[sl], (l >> 1) & 1, 12);
       tc_fence_after();
+      if (warp == 4) RC_EV(l, 13);      // S(l) complete (seen by the softmax warps)
+      RC_T0(texp);
       float ml = ml_bound;
       if (!use_bound) {
         float mx = -FLT_MAX;
@@ -511,9 +569,14 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       xch[(3 * 2 + half) * 128 + row] = tz;
       // every softmax warp has read its S columns (tcgen05.wait::ld above): after this barrier the slot's columns may be
       // overwritten with P
+      RC_TACC(2, texp);
+      if (warp == 4) RC_EV(l, 14);      // exp pass done
       tc_fence_before();
+      RC_T0(txch);
       named_bar_sync(2, 256);
+      RC_TACC(13, txch);
       tc_fence_after();
+      RC_T0(tpst);
       sum += xch[(1 * 2 + (half ^ 1)) * 128 + row];
       sez += xch[(2 * 2 + (half ^ 1)) * 128 + row];
       tz += xch[(3 * 2 + (half ^ 1)) * 128 + row];
@@ -521,10 +584,9 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       float lse = 0.f;
       if (half == 0) {
         lse = (ml + __log2f(sum)) * kLn2;
-        loss_acc += wtot * lse - tz * zs;
-        w_acc += wtot;
+        acc_s[0] += wtot * lse - tz * zs;
+        acc_s[128] += wtot;
       }
-      const float coefb = gscale * inv_wsum;
       const float coef = coefb * wtot;
       const float inv_sum = 1.f / sum;
       // P is stored pre-scaled: G[p][k] = rs_p (e_pk - sum_p [k = y_p]) = d loss / d(xhat_p . that_k) / |x_p|
@@ -532,7 +594,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       if (half == 0) {
         const float cj = coef * sez * zs * inv_sum - coefb * tz * zs;
         sc_s[(l & (kScaleBufs - 1)) * 128 + row] = -(inv_n * inv_n * cj);      // dx = acc + (-cs) x
-        dlt_acc -= cj;
+        acc_s[256] -= cj;
         __syncwarp();
         if (lane == 0) mbar_arrive(&bars->sc_full[l & (kScaleBufs - 1)]);
       }
@@ -584,10 +646,12 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
         tc_fence_before();
         arrive_leader_warp(&bars->p_full[sl]);
       }
+      RC_TACC(3, tpst);
+      if (warp == 4) RC_EV(l, 15);      // P(l) stored
       if (half == 0 && valid && prm.lse && !(kKB && prm.lse_in != nullptr)) prm.lse[m] = lse;
     }
     if (half == 0) {
-      loss_acc = warp_sum(loss_acc); w_acc = warp_sum(w_acc); dlt_acc = warp_sum(dlt_acc);
+      const float loss_acc = warp_sum(acc_s[0]), w_acc = warp_sum(acc_s[128]), dlt_acc = warp_sum(acc_s[256]);
       if (lane == 0) {
         if (prm.loss_sum) atomicAdd(prm.loss_sum, (double)loss_acc);
         if (prm.w_sum) atomicAdd(prm.w_sum, (double)w_acc);
@@ -621,8 +685,14 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     int s_req = 0;
     auto request_x = [&]() {                         // lane 0: the x box of step s_req
       const int bi = s_req % kEpiBufs;
+      if (prm.ablate & 1) {           // bring-up: no x traffic (the box keeps stale data)
+        mbar_arrive(&ebar[bi]);
+        return;
+      }
       mbar_arrive_expect_tx(&ebar[bi], kEpiBufBytes);
-      tma_load_3d(ebuf + bi * kEpiBufBytes, &map_xe, &ebar[bi], cr.px, cr.u * 64 + h * 32, cr.bx);
+      // the tile's last read: release the lines the S GEMM's loads kept in the L2
+      if (RC_TS_X_HINT) tma_load_3d_hint(ebuf + bi * kEpiBufBytes, &map_xe, &ebar[bi], cr.px, cr.u * 64 + h * 32, cr.bx, pol_first);
+      else tma_load_3d(ebuf + bi * kEpiBufBytes, &map_xe, &ebar[bi], cr.px, cr.u * 64 + h * 32, cr.bx);
     };
     for (; s_req < kEpiAhead && s_req < total; ++s_req) {
       if (lane == 0) request_x();
@@ -635,10 +705,10 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     // thread t addresses row (channel) 8g + (t & 7) of pixel block t >> 3
     const uint32_t moff = (uint32_t)((lane & 7) * 64 + ((((lane >> 3) ^ ((lane >> 1) & 3)) & 3) << 4));
     int s = 0;
-    uint32_t acc_seen[2][2] = {{0, 0}, {0, 0}};
+    uint32_t acc_par = 0;      // bit 2 * slot + accumulator: parity of the completions seen so far
     for (int l = 0; l < my_pairs; ++l) {
       const int sl = l & 1;
-      mbar_wait(&bars->sc_full[l & (kScaleBufs - 1)], (l >> 2) & 1, 14);
+      RC_WAIT(mbar_wait, &bars->sc_full[l & (kScaleBufs - 1)], (l >> 2) & 1, 14);
       uint32_t ncs2[4];                                // -cs of the thread's pixel in each of the four pixel blocks
 #pragma unroll
       for (int pb = 0; pb < 4; ++pb) {
@@ -648,9 +718,11 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       const uint32_t tacc = tmem + ((uint32_t)(q * 32) << 16) + sl * kSlotCols + kColAcc + h * 32;
       for (int blk = 0; blk < n_blk; ++blk, ++s) {
         const int ab = blk & 1;
-        mbar_wait(&bars->acc_full[sl][ab], acc_seen[sl][ab] & 1u, 15);
-        ++acc_seen[sl][ab];
+        RC_WAIT(mbar_wait, &bars->acc_full[sl][ab], (acc_par >> (2 * sl + ab)) & 1u, 15);
+        acc_par ^= 1u << (2 * sl + ab);
         tc_fence_after();
+        if (warp == 12 && blk < 8) RC_EV(l, 20 + 2 * blk);      // block's accumulator complete
+        RC_T0(tld);
         // accumulators of pixels [0,16) and [16,32) of the warp's lane quarter, 32 channel columns each, rounded to packed
         // bf16 channel pairs; the accumulator is handed back before any of it is processed
         uint32_t pa[4][4];                             // [g][pb]
@@ -673,8 +745,10 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
         }
         tc_fence_before();
         arrive_leader_warp(&bars->acc_empty[sl][ab]);
+        RC_TACC(3, tld);
         const int bi = s % kEpiBufs;
-        mbar_wait(&ebar[bi], (s / kEpiBufs) & 1, 16);
+        RC_WAIT(mbar_wait, &ebar[bi], (s / kEpiBufs) & 1, 4);
+        RC_T0(tmath);
         // dx = acc - cs x in place on the box (same rounding as infonce_umma2.cu: the accumulator is rounded to bf16, then
         // one fused multiply-add on packed pairs)
         const uint32_t bx0 = smem_u32(ebuf + bi * kEpiBufBytes) + moff;
@@ -689,23 +763,38 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
         }
         fence_proxy_async_smem();
         __syncwarp();
+        RC_TACC(2, tmath);
         if (lane == 0) {
-          if (kKB && prm.acc_dx) tma_reduce_add_3d(&map_dx, ebuf + bi * kEpiBufBytes, cs.px, cs.u * 64 + h * 32, cs.bo);
-          else tma_store_3d_hint(&map_dx, ebuf + bi * kEpiBufBytes, cs.px, cs.u * 64 + h * 32, cs.bo, pol_first);
-          tma_store_commit();
+          if (!(prm.ablate & 2)) {
+            if (kKB && prm.acc_dx) tma_reduce_add_3d(&map_dx, ebuf + bi * kEpiBufBytes, cs.px, cs.u * 64 + h * 32, cs.bo);
+            else tma_store_3d_hint(&map_dx, ebuf + bi * kEpiBufBytes, cs.px, cs.u * 64 + h * 32, cs.bo, pol_first);
+            tma_store_commit();
+          }
           if (s_req < total) {
             // the box to refill was stored kEpiBufs - kEpiAhead steps ago: that store must have read it
+            RC_T0(tsw);
             asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(kEpiBufs - kEpiAhead) : "memory");
+            RC_TACC(5, tsw);
             request_x();
           }
         }
         cursor_next(cs);
         if (s_req < total) { cursor_next(cr); ++s_req; }
         __syncwarp();
+        if (warp == 12 && blk < 8) RC_EV(l, 21 + 2 * blk);      // block drained, its store issued
       }
     }
     if (lane == 0) tma_store_wait_all0();       // shared memory must stay valid until the last bulk store has read it
   }
+#ifdef RC_TIMING
+  // roles: 0 text producer, 1 MMA issuer, 2 softmax (warp 4), 3 dX epilogue (warp 12), 4 X producer
+  if (prm.dbg != nullptr && blockIdx.x < 2 && lane == 0 && (warp <= 1 || warp == 3 || warp == 4 || warp == 12)) {
+    wt[0] = clock64() - t_start;
+    const int role = warp == 0 ? 0 : (warp == 1 ? 1 : (warp == 4 ? 2 : (warp == 12 ? 3 : 4)));
+#pragma unroll
+    for (int i = 0; i < 16; ++i) prm.dbg[(blockIdx.x * 5 + role) * 16 + i] = wt[i];
+  }
+#endif
   tc_fence_before();
   cluster_sync();            // no CTA leaves while its peer may still touch its barriers / shared memory
   if (warp == 2) {
@@ -743,6 +832,11 @@ int launch_infonce_ts(const void* xsrc, void* dx, const void* t_bf16, const void
     if ((rcode = make_tmap_bf16(&m_tt, tt_bf16, 2, ttdims, ttstr, ttbox, "ts map_tt"))) return rcode;
   }
   Params prm;
+  prm.dbg = debug_timing_buffer();
+  prm.ablate = 0;
+#ifdef RC_BRINGUP      // ablation switches of the bring-up build (tools/timing_ts.py ablate); the shipped library has no environment knobs
+  { const char* ab = getenv("RANGECLIP_B200_ABLATE"); prm.ablate = ab ? atoi(ab) : 0; }
+#endif
   prm.B = B; prm.D = D; prm.K = K; prm.Kp = Kp; prm.HW = HW;
   prm.tiles_per_img = (int)((HW + kTilePx - 1) / kTilePx);
   if ((int64_t)B * prm.tiles_per_img > 0x3fffffff) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: too many tiles");

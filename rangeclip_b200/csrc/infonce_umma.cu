@@ -995,8 +995,8 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
     return launch_infonce_dt(g, xsrc, B, D, HW, K, dt, s);
   }
   if (use_pair) {
-    // RC_INFONCE_TS_KERNEL: backward launches with the softmax tile as a tensor-memory operand of the dX GEMM (infonce_ts.cu)
-    if (bwd && (flags & RC_INFONCE_TS_KERNEL) && k_dev == nullptr && log_tau_dev == nullptr)
+    // backward launches: the softmax tile as a tensor-memory operand of the dX GEMM (infonce_ts.cu) unless RC_INFONCE_SS_KERNEL
+    if (bwd && !(flags & RC_INFONCE_SS_KERNEL) && k_dev == nullptr && log_tau_dev == nullptr)
       return launch_infonce_ts(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, y, w, inv_tau, grad_scale, w_sum_in, lse, loss_sum, w_sum,
                                dlogtau, rep, keep_w, lse_in, 0, acc_dx, s);
     return launch_infonce_pair(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
@@ -1092,7 +1092,7 @@ extern "C" int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, i
   if ((rcode = infonce_prepass_impl(x, x_dtype, 1, D, HW, workspace, workspace_bytes, skip_prepass ? (cudaStream_t)-1 : s, &inv_norm, &xb))) return rcode;
   const void* xsrc = (x_dtype == RC_F32) ? (const void*)xb : x;
   const float* lse_in = (flags & RC_INFONCE_LSE_GIVEN) ? lse : nullptr;
-  if (bwd && (flags & RC_INFONCE_TS_KERNEL))
+  if (bwd && !(flags & RC_INFONCE_SS_KERNEL))
     return launch_infonce_ts(xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, y_rel, w_rep, inv_tau, grad_scale, w_sum_in,
                              lse, loss_sum, w_sum, dlogtau, 1, 1, lse_in, n_blocks, 0, s);
   return launch_infonce_pair(xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, inv_norm, y_rel, w_rep, inv_tau, grad_scale,

@@ -186,7 +186,7 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
     rep = 4: every row of x is the embedding shared by a 2x2 block of pixels (decoder.py:113, Q8);
     y / w are [rows, 4] and dx is the gradient w.r.t. the shared row (tensor-core path only).
     keep_bf16: leave the tensor-core path's dx in bf16 whatever x's dtype (the autograd wrappers widen and scale it
-    in one pass at backward time); flags: extra RC_INFONCE_* bits for rc_infonce_bf16 (e.g. RC_INFONCE_TS_KERNEL).
+    in one pass at backward time); flags: extra RC_INFONCE_* bits for rc_infonce_bf16 (e.g. RC_INFONCE_SS_KERNEL).
     k_dev / log_tau_dev (device int32[>=1] / float[1]): the sync-free form (rc_infonce_bf16_dyn) -- the number of valid rows of
     t_norm and log(tau) are read by the kernel from device memory; ``inv_tau`` is ignored; CTA-pair kernel shapes only.
     fuse_tv: the caller also wants tv_sums(x); where the launch has a pre-pass over x anyway (fp32 NCHW x on the tensor-core
@@ -297,6 +297,7 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
 
 
 RC_INFONCE_PREPASS_DONE, RC_INFONCE_KEEP_WEIGHT, RC_INFONCE_LSE_GIVEN, RC_INFONCE_TS_KERNEL, RC_INFONCE_ACCUMULATE_DX = 1, 2, 4, 8, 16
+RC_INFONCE_SS_KERNEL = 32
 
 
 def kblocked_supported(D: int, HW: int) -> bool:

@@ -1,6 +1,7 @@
 """Sensitivity of the CTA-pair InfoNCE kernel to its memory traffic classes (bring-up build, RANGECLIP_B200_ABLATE bits; results
 are garbage under ablation, only the time counts): 1 no epilogue x loads, 2 no dX stores, 64 no row-norm reads, 256 no text
-reloads after the first ring pass.   python tools/ablate_pair.py"""
+reloads after the first ring pass.   python tools/ablate_pair.py
+RC_AB_FLAGS: rc_infonce_bf16 flags (default 32 = RC_INFONCE_SS_KERNEL, the pair kernel; 0 = the default TS kernel)."""
 import json, os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if len(sys.argv) > 1 and sys.argv[1] == "child":
@@ -27,7 +28,7 @@ if len(sys.argv) > 1 and sys.argv[1] == "child":
     def run():
         _lib.check(L.rc_infonce_bf16(x.data_ptr(), _lib.RC_BF16, B, D, HW, tb.data_ptr(), ttb.data_ptr(), K, y.data_ptr(), w.data_ptr(), 1 / 0.07,
                                      lse.data_ptr(), acc[0:].data_ptr(), acc[1:].data_ptr(), acc[3:].data_ptr(), None, dx.data_ptr(), None,
-                                     acc[2:].data_ptr(), ws.data_ptr(), wsb, int(os.environ.get('RC_AB_FLAGS', 0)), st), "infonce")
+                                     acc[2:].data_ptr(), ws.data_ptr(), wsb, int(os.environ.get('RC_AB_FLAGS', 32)), st), "infonce")
     for _ in range(3): run()
     torch.cuda.synchronize()
     ts = []

@@ -17,7 +17,7 @@ buf = torch.zeros(1024, device=dev, dtype=torch.int64)
 for rep in range(2):
     buf.zero_()
     _lib.lib().rc_debug_set_timing_buffer(buf.data_ptr())
-    ops.infonce_raw(x, t, y, w, 1 / 0.07, True, False, "bf16")
+    ops.infonce_raw(x, t, y, w, 1 / 0.07, True, False, "bf16", flags=ops.RC_INFONCE_SS_KERNEL)
     torch.cuda.synchronize()
 _lib.lib().rc_debug_set_timing_buffer(None)
 ev = buf[256:256 + 2 * 4 * 48].view(2, 4, 48).tolist()

@@ -20,7 +20,7 @@ names = {0: {1: "empty(S)", 2: "empty(dX)"}, 1: {3: "s_empty", 4: "xfull(S)", 12
 roles = ["producer", "mma", "softmax", "epilogue"]
 for rep in range(2):
     _lib.lib().rc_debug_set_timing_buffer(buf[rep].data_ptr())
-    ops.infonce_raw(x, t, y, w, 1 / 0.07, True, False, "bf16")
+    ops.infonce_raw(x, t, y, w, 1 / 0.07, True, False, "bf16", flags=ops.RC_INFONCE_SS_KERNEL)
     torch.cuda.synchronize()
 _lib.lib().rc_debug_set_timing_buffer(None)
 pairs = (B * H * W // 128 // 2 + 73) // 74
