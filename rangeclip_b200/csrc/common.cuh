@@ -44,10 +44,24 @@ inline int num_sms() {
   return n;
 }
 
-// fp32 -> bf16 copy + inverse row norms (defined in infonce_umma.cu, shared with eval_topk_umma.cu)
+// the tensor-core kernels need an sm_100 device
+inline int check_sm100(const char* what) {
+  int dev = 0, major = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return fail(RC_ERR_NO_DEVICE, "%s: no CUDA device", what);
+  cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev);
+  if (major != 10) return fail(RC_ERR_NO_DEVICE, "%s: needs an sm_100 device (compute capability %d.x found)", what, major);
+  return RC_OK;
+}
+
+// fp32 -> bf16 copy + inverse row norms (defined in infonce.cu, shared with eval_topk_umma.cu)
 int launch_rownorm_f32(const float* x, int B, int D, int64_t HW, __nv_bfloat16* xb, float* inv_norm, cudaStream_t s);
 
 long long* debug_timing_buffer();   // bring-up instrumentation target (rc_debug_set_timing_buffer)
+// The fused InfoNCE kernels; infonce.cu validates the arguments, runs the pre-pass and picks one of them.
+// single-CTA version (infonce_umma.cu): D = 128 / 384, and the A/B baseline of the bring-up build
+int launch_infonce_1cta(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
+                        const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
+                        const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, cudaStream_t s);
 // CTA-pair (cta_group::2) version of the fused InfoNCE kernel (infonce_umma2.cu)
 bool infonce_pair_supported(int D);
 int launch_infonce_pair(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,

@@ -181,13 +181,8 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
   const int n_units = kPair ? (prm.n_tiles + 1) / 2 : prm.n_tiles;
   auto tile_of = [&](int u) -> int { return kPair ? 2 * u + (int)rank : u; };
   // the candidate set may have been built on the device (rc_contrast_build): its size is read here, by every role alike
-#if RC_TOPK_STATIC_K       // A/B only (tools/ab_topk.py): the set size as a launch parameter, as before rc_eval_topk_dyn_bf16 existed
-  const int Kv = prm.K;
-  const int n_blocks = prm.n_blocks;
-#else
   const int Kv = prm.k_dev != nullptr ? max(1, min(__ldg(prm.k_dev), prm.K)) : prm.K;
   const int n_blocks = prm.k_dev != nullptr ? (Kv + kNB - 1) / kNB : prm.n_blocks;
-#endif
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&map_x); tma_prefetch_desc(&map_t);
     for (int i = 0; i < kMaxStages; ++i) { mbar_init(&bars->full[i], 1); mbar_init(&bars->empty[i], 1); }
@@ -540,13 +535,10 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   RC_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(t_bf16) & 15) == 0,
              "%s: x and t must be 16-byte aligned", who);
   if (B == 0 || HW == 0) return RC_OK;
-  int dev = 0, major = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev);
-  if (major != 10) return fail(RC_ERR_NO_DEVICE, "%s: needs an sm_100 device", who);
+  int rcode = check_sm100(who);
+  if (rcode) return rcode;
   cudaStream_t s = (cudaStream_t)stream;
   const void* xsrc = x;
-  int rcode;
   if (x_dtype == RC_F32) {
     const int64_t M = (int64_t)B * HW;
     RC_REQUIRE(workspace && workspace_bytes >= rc_infonce_workspace_bytes(B, D, HW, K, RC_F32), "%s: workspace too small for the bf16 copy", who);

@@ -21,6 +21,7 @@
 // The row norms 1/|x_p| (model.py:272 F.normalize) are computed by the relay warp from the X chunks in the operand ring.
 #include "common.cuh"
 #include "umma.cuh"
+#include "infonce_device.cuh"
 #include <float.h>
 #include <stdlib.h>
 
@@ -28,34 +29,6 @@ namespace rc {
 using namespace umma;
 
 namespace ts {
-
-// L2 policy of the two reads of a tile of X.  The dX epilogue reads the tile again two pair iterations after the S GEMM did;
-// in between, the L2 sees about 2 x 74 clusters x 256 KB of other X and as much dX written.  1: the S GEMM's loads mark
-// the lines evict_last and the epilogue's (last) load marks them evict_first, so that kept lines are released as soon as
-// they have been consumed.  0: no hints (A/B: make variant VSRC=infonce_ts NAME=.. DEFS=-DRC_TS_X_HINT=0).
-#ifndef RC_TS_X_HINT
-#define RC_TS_X_HINT 1
-#endif
-
-#ifdef RC_TIMING
-__device__ __forceinline__ unsigned long long globaltimer_ns() {     // one clock for both CTAs of the pair
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-// per-role wait cycles (tools/timing_ts.py): wt[tag] += cycles spent in the wait with that tag, wt[0] = lifetime
-#define RC_T0(name) const long long name = clock64()
-#define RC_TACC(idx, name) wt[idx] += clock64() - name
-#define RC_WAIT(fn, bar, par, tag) do { const long long t0_ = clock64(); fn(bar, par, tag); wt[tag] += clock64() - t0_; } while (0)
-// event trace of cluster 0: %globaltimer of event `id` of tile-pair iteration `iter` in [40, 44)
-#define RC_EV(iter, id) do { if (prm.dbg != nullptr && blockIdx.x < 2 && lane == 0 && (iter) >= 40u && (iter) < 44u) \
-    prm.dbg[256 + blockIdx.x * 192 + ((iter) - 40u) * 48 + (id)] = (long long)globaltimer_ns(); } while (0)
-#else
-#define RC_T0(name)
-#define RC_TACC(idx, name)
-#define RC_WAIT(fn, bar, par, tag) fn(bar, par, tag)
-#define RC_EV(iter, id)
-#endif
 
 constexpr int kTilePx = 128;
 constexpr int kThreads = 640;          // warps: 0 text TMA, 1 MMA (leader CTA), 2 relay + row norms + TMEM alloc, 3 X TMA, 4-11 softmax, 12-19 dX epilogue
@@ -70,8 +43,6 @@ constexpr int kSlotCols = 256;         // one slot: S [0,256) -> P [0,128) + two
 constexpr int kColAcc = 128, kAccCols = 64;
 constexpr int kDxLead = 2;             // dX blocks of pair l issued before S(l+1): one per accumulator of the slot
 constexpr int kRegsCtl = 48, kRegsSoftmax = 120;     // epilogue warps keep the entry allocation (96); 48 + 2*120 + 2*96 = 5*96
-constexpr float kLog2e = 1.4426950408889634f;
-constexpr float kLn2 = 0.6931471805599453f;
 
 struct __align__(8) Bars {
   uint64_t xf[kXStages];        // own X chunk has landed (CTA-local; relayed to the leader's xfull)
@@ -121,23 +92,6 @@ __device__ __forceinline__ int div_tiles(const Params& prm, int tile) {
   int q = (int)__umulhi((uint32_t)tile, prm.tpi_magic);
   if (tile - q * prm.tiles_per_img >= prm.tiles_per_img) ++q;
   return q;
-}
-
-__device__ __forceinline__ float fast_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
-__device__ __forceinline__ float select16(const uint32_t (&r)[16], int i) {
-  float a[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) a[j] = __uint_as_float((i & 1) ? r[2 * j + 1] : r[2 * j]);
-#pragma unroll
-  for (int j = 0; j < 4; ++j) a[j] = (i & 2) ? a[2 * j + 1] : a[2 * j];
-#pragma unroll
-  for (int j = 0; j < 2; ++j) a[j] = (i & 4) ? a[2 * j + 1] : a[2 * j];
-  return (i & 8) ? a[1] : a[0];
 }
 
 // tile -> (image, first pixel); tiles past the end map to image index B (out of bounds for every tensor map)
@@ -257,7 +211,10 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     } else if (warp == 3 && lane == 0) {
       // =============================== X producer (both CTAs) ===============================
       uint32_t xit = 0;
-      const uint64_t pol_keep = RC_TS_X_HINT ? l2_policy_evict_last() : 0;
+      // L2 policy of the two reads of a tile of X: the dX epilogue reads the tile again two pair iterations later, and in
+      // between the L2 sees about 2 x 74 clusters x 256 KB of other X and as much dX written.  These loads mark the lines
+      // evict_last and the epilogue's (last) load marks them evict_first, so that kept lines are released once consumed.
+      const uint64_t pol_keep = l2_policy_evict_last();
       for (int l = 0; l < my_pairs; ++l) {
         int b, px0;
         tile_coords(prm, 2 * pair_of(l) + (int)rank, b, px0);
@@ -267,13 +224,8 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
           uint8_t* sb = smem + st * kStageBytes;
           mbar_arrive_expect_tx(&bars->xf[st], 2 * 8192);          // CTA-local: the row-norm warp reads the chunk too
           const int bx = (kKB && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;      // kb mode: the one image of X (1 = out of bounds)
-          if (RC_TS_X_HINT) {
-            tma_load_3d_hint(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx, pol_keep);
-            tma_load_3d_hint(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx, pol_keep);
-          } else {
-            tma_load_3d(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx);
-            tma_load_3d(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx);
-          }
+          tma_load_3d_hint(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx, pol_keep);
+          tma_load_3d_hint(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx, pol_keep);
         }
       }
     } else if (warp == 1 && leader_cta) {
@@ -691,8 +643,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       }
       mbar_arrive_expect_tx(&ebar[bi], kEpiBufBytes);
       // the tile's last read: release the lines the S GEMM's loads kept in the L2
-      if (RC_TS_X_HINT) tma_load_3d_hint(ebuf + bi * kEpiBufBytes, &map_xe, &ebar[bi], cr.px, cr.u * 64 + h * 32, cr.bx, pol_first);
-      else tma_load_3d(ebuf + bi * kEpiBufBytes, &map_xe, &ebar[bi], cr.px, cr.u * 64 + h * 32, cr.bx);
+      tma_load_3d_hint(ebuf + bi * kEpiBufBytes, &map_xe, &ebar[bi], cr.px, cr.u * 64 + h * 32, cr.bx, pol_first);
     };
     for (; s_req < kEpiAhead && s_req < total; ++s_req) {
       if (lane == 0) request_x();
@@ -805,7 +756,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
 
 }  // namespace ts
 
-// launch helper used by rc_infonce_bf16 for backward launches without dText (infonce_umma.cu owns argument checking)
+// launch helper used by rc_infonce_bf16 for backward launches without dText (infonce.cu owns argument checking)
 int launch_infonce_ts(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
                       const int32_t* y, const float* w, float inv_tau, const float* grad_scale, const double* w_sum_in,
                       float* lse, double* loss_sum, double* w_sum, double* dlogtau, int rep, int keep_w, const float* lse_in,
@@ -862,94 +813,3 @@ int launch_infonce_ts(const void* xsrc, void* dx, const void* t_bf16, const void
 }
 
 }  // namespace rc
-
-// ------------------------------------------------------------------------------------------------
-// bring-up kernel for the TS-mode building blocks: C[256][N] = A[256][Kd] B[N][Kd]^T with A written to tensor memory by
-// the threads (tcgen05.st, packed bf16 pairs) and B rows split N/2 / N/2 over the two CTAs' shared memory
-// ------------------------------------------------------------------------------------------------
-namespace rc {
-
-struct __align__(8) DebugTsBars { uint64_t full, done; uint32_t tmem_base, pad; };
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1)
-debug_umma_gemm_ts_2sm_kernel(const __grid_constant__ CUtensorMap map_b, const __nv_bfloat16* __restrict__ a, int N, int Kd,
-                              float* __restrict__ c) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sbm = smem;              // Kd/64 chunks of own N/2 rows of B (<= 4 x 16 KB)
-  DebugTsBars* bars = reinterpret_cast<DebugTsBars*>(smem + 65536);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int nh = N / 2;
-  if (threadIdx.x == 0) {
-    mbar_init(&bars->full, 1);
-    mbar_init(&bars->done, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc_2sm<512>(&bars->tmem_base);
-  tc_fence_before();
-  cluster_sync();
-  tc_fence_after();
-  const uint32_t tmem = bars->tmem_base;
-  const int row = warp * 32 + lane;
-  {
-    // own row of A as packed pairs: column 256 + j holds k = 2j (low half), 2j + 1 (high half)
-    const uint32_t* src = reinterpret_cast<const uint32_t*>(a + ((int64_t)rank * 128 + row) * Kd);
-    for (int cc = 0; cc < Kd / 32; ++cc) {
-      uint32_t v[16];
-      for (int i = 0; i < 16; ++i) v[i] = src[cc * 16 + i];
-      tmem_st_32x16(tmem + ((uint32_t)(warp * 32) << 16) + 256 + cc * 16, v);
-    }
-    tmem_st_wait();
-  }
-  tc_fence_before();
-  cluster_sync();
-  tc_fence_after();
-  if (threadIdx.x == 0) {
-    const int nck = Kd / 64;
-    if (rank == 0) mbar_arrive_expect_tx(&bars->full, 2 * nck * nh * 128);
-    for (int ck = 0; ck < nck; ++ck) tma_load_2d_2sm(sbm + ck * nh * 128, &map_b, &bars->full, ck * 64, (int)rank * nh);
-    if (rank == 0) {
-      const uint32_t idesc = make_idesc_bf16(256, N, 0, 0);
-      mbar_wait(&bars->full, 0, 210);
-      tc_fence_after();
-      for (int ck = 0; ck < nck; ++ck)
-        for (int ks = 0; ks < 4; ++ks)
-          mma_bf16_ts_2sm(tmem, tmem + 256 + (ck * 4 + ks) * 8, desc_kmajor_sw128(smem_u32(sbm) + ck * nh * 128 + ks * 32), idesc,
-                          (ck | ks) != 0);
-      mma_commit_2sm(&bars->done);
-    }
-    mbar_wait(&bars->done, 0, 211);
-  }
-  __syncthreads();
-  tc_fence_after();
-  for (int cc = 0; cc < N / 32; ++cc) {
-    uint32_t r[32];
-    tmem_ld_32x32(tmem + ((uint32_t)(warp * 32) << 16) + cc * 32, r);
-    tmem_ld_wait();
-    for (int i = 0; i < 32; ++i) c[((int64_t)rank * 128 + row) * N + cc * 32 + i] = __uint_as_float(r[i]);
-  }
-  tc_fence_before();
-  cluster_sync();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc_2sm<512>(tmem); }
-}
-
-}  // namespace rc
-
-#ifdef RC_BRINGUP
-extern "C" int rc_debug_umma_gemm_ts_2sm(const void* a_bf16, const void* b_bf16, int N, int Kd, float* c, void* stream) {
-  RC_REQUIRE(a_bf16 && b_bf16 && c, "rc_debug_umma_gemm_ts_2sm: null pointer");
-  RC_REQUIRE(N >= 64 && N <= 256 && N % 64 == 0 && Kd >= 64 && Kd <= 256 && Kd % 64 == 0, "rc_debug_umma_gemm_ts_2sm: bad shape N=%d Kd=%d", N, Kd);
-  CUtensorMap mb;
-  int rcode;
-  {
-    const uint64_t bdims[2] = {(uint64_t)Kd, (uint64_t)N}, str[2] = {2, (uint64_t)Kd * 2};
-    const uint32_t bbox[2] = {64, (uint32_t)(N / 2)};
-    if ((rcode = rc::make_tmap_bf16(&mb, b_bf16, 2, bdims, str, bbox, "debug ts B"))) return rcode;
-  }
-  const int smem = 65536 + 64;
-  cudaError_t e = cudaFuncSetAttribute(rc::debug_umma_gemm_ts_2sm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return rc::fail(RC_ERR_CUDA, "rc_debug_umma_gemm_ts_2sm: smem opt-in: %s", cudaGetErrorString(e));
-  rc::debug_umma_gemm_ts_2sm_kernel<<<2, 128, smem, (cudaStream_t)stream>>>(mb, (const __nv_bfloat16*)a_bf16, N, Kd, c);
-  return rc::check_launch("rc_debug_umma_gemm_ts_2sm");
-}
-#endif  // RC_BRINGUP

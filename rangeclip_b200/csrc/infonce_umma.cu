@@ -1,244 +1,27 @@
-// K1/K2: fused pixel-text InfoNCE forward + backward on the 5th-gen tensor cores (sm_100a).
+// K1/K2, single-CTA version: the fused pixel-text InfoNCE forward + backward on the 5th-gen tensor cores (sm_100a).
+// rc_infonce_bf16 runs it for D = 128 / 384 (the CTA-pair kernels in infonce_umma2.cu / infonce_ts.cu need D = 256 or 512);
+// the bring-up build also takes it as the A/B baseline (RANGECLIP_B200_INFONCE=1cta).
 //
 // Replaces model.py:272-291 (normalize, [N,512]@[512,K], /tau, cross_entropy) and its autograd
-// (CE backward, two matmuls, normalize backward, index_put/scatter_add) with
-//   * rownorm_kernel      one pass over X: 1/|x_p| (and the bf16 copy when X is fp32)
-//   * infonce_umma_kernel persistent, warp-specialised: per 128-pixel tile
-//        S  = X^T T^T           tcgen05.mma, A = X tile straight from NCHW (MN-major via TMA),
-//                               B = text rows (K-major via TMA), fp32 accumulators in TMEM
-//        softmax/CE epilogue    one thread per pixel reads its S row from TMEM: logsumexp, loss,
-//                               dlogtau, and P = exp(z-m) - sum*onehot written as bf16 to smem
-//        dX^T = T^T P^T          tcgen05.mma per 128-channel block, accumulators in TMEM
-//        dX epilogue            row scale + normalize-backward projection, TMA store to NCHW
-//     The [B*HW, K] logits never leave the SM.
-//   * infonce_dt_umma_kernel  dText = P^T Xhat, text rows sliced across CTAs, S recomputed
-//                             slice-wise from the saved logsumexp (TMEM cannot hold S, dX and the
-//                             256x512 fp32 dText at once).
+// (CE backward, two matmuls, normalize backward, index_put/scatter_add).  Needs the pre-pass (rownorm_kernel,
+// infonce.cu: 1/|x_p| and the bf16 copy of an fp32 X).  infonce_umma_kernel is persistent and warp-specialised; per
+// 128-pixel tile
+//   S  = X^T T^T           tcgen05.mma, A = X tile straight from NCHW (MN-major via TMA),
+//                          B = text rows (K-major via TMA), fp32 accumulators in TMEM
+//   softmax/CE epilogue    one thread per pixel reads its S row from TMEM: logsumexp, loss,
+//                          dlogtau, and P = exp(z-m) - sum*onehot written as bf16 to smem
+//   dX^T = T^T P^T         tcgen05.mma per 128-channel block, accumulators in TMEM
+//   dX epilogue            row scale + normalize-backward projection, TMA store to NCHW
+// The [B*HW, K] logits never leave the SM.
 #include "common.cuh"
 #include "umma.cuh"
+#include "infonce_device.cuh"
 #include <float.h>
-#include <stdlib.h>
 
 namespace rc {
 
 using namespace umma;
 
-// ------------------------------------------------------------------------------------------------
-// host: driver entry point + tensor maps
-// ------------------------------------------------------------------------------------------------
-PFN_encodeTiled get_encode_tiled() {
-  static PFN_encodeTiled fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
-  return fn;
-}
-
-int make_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                   const uint32_t* box, const char* what) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  if (!enc) return fail(RC_ERR_NO_DEVICE, "%s: cuTensorMapEncodeTiled entry point unavailable", what);
-  cuuint64_t gdim[3];
-  cuuint64_t gstr[2];
-  cuuint32_t bx[3];
-  cuuint32_t es[3] = {1, 1, 1};
-  for (int i = 0; i < rank; ++i) { gdim[i] = dims[i]; bx[i] = box[i]; }
-  for (int i = 0; i + 1 < rank; ++i) gstr[i] = strides_bytes[i + 1];
-  const CUtensorMapSwizzle sw = (box[0] * 2 >= 128) ? CU_TENSOR_MAP_SWIZZLE_128B
-                                : (box[0] * 2 == 64) ? CU_TENSOR_MAP_SWIZZLE_64B
-                                                     : CU_TENSOR_MAP_SWIZZLE_32B;
-  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gdim, gstr, bx, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(RC_ERR_CUDA, "%s: cuTensorMapEncodeTiled failed (%d)", what, (int)r);
-  return RC_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// pre-pass: inverse row norms of the bf16-rounded rows (+ bf16 copy of an fp32 input)
-// ------------------------------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(256)
-rownorm_kernel(const T* __restrict__ x, int B, int D, int64_t HW, __nv_bfloat16* __restrict__ xb,
-               float* __restrict__ inv_norm) {
-  const int64_t groups_per_img = HW / 8;
-  const int64_t n = (int64_t)B * groups_per_img;
-  for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t b = g / groups_per_img;
-    const int64_t p0 = (g - b * groups_per_img) * 8;
-    const T* src = x + b * (int64_t)D * HW + p0;
-    __nv_bfloat16* dst = xb ? xb + b * (int64_t)D * HW + p0 : nullptr;
-    float ss[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) ss[j] = 0.f;
-    if (sizeof(T) == 2) {          // bf16 rows: nothing to round or copy, squares straight from the packed words
-#pragma unroll 8
-      for (int d = 0; d < D; ++d) {
-        const uint4 w = __ldg(reinterpret_cast<const uint4*>(src + (int64_t)d * HW));
-        const uint32_t u[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          ss[2 * j] = sqacc_bf16x2_lo(ss[2 * j], u[j]);
-          ss[2 * j + 1] = sqacc_bf16x2_hi(ss[2 * j + 1], u[j]);
-        }
-      }
-    } else
-#pragma unroll 4
-    for (int d = 0; d < D; ++d) {
-      float v[8];
-      load8(src + (int64_t)d * HW, v);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        v[j] = __bfloat162float(__float2bfloat16_rn(v[j]));   // the tensor cores see the rounded value
-        ss[j] = fmaf(v[j], v[j], ss[j]);
-      }
-      if (dst) store8(dst + (int64_t)d * HW, v);
-    }
-    float o[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) o[j] = 1.f / fmaxf(sqrtf(ss[j]), 1e-12f);
-    store8(inv_norm + b * HW + p0, o);
-  }
-}
-
-// fp32 X: the same pre-pass AND the smoothness sums (tv.cu: sums[0] = sum |x[h][w+1] - x[h][w]|, sums[1] = sum |x[h+1][w] - x[h][w]|)
-// from ONE read of X.  A thread owns a strip of R rows x 8 pixels and walks the channels; per channel it loads its R rows plus the
-// row below (the only re-read: (R+1)/R of X, mostly L2 hits), takes the right-hand neighbour from the next lane (consecutive
-// lanes = consecutive 8-pixel groups of the same rows), rounds to bf16 for the copy and the norms, and keeps the TV terms on
-// the unrounded fp32 values as rc_tv_fwd does.  kCodes: the signs of those differences are kept as well -- 4 bits per element,
-// one 32-bit word per 8-pixel group: pixel j at bits 4j..4j+3, low pair sgn(x[h][w] - x[h][w+1]), high pair
-// sgn(x[h][w] - x[h+1][w]), each a 2-bit two's-complement -1 / 0 / +1 (0 past the last column / row) -- which is all the
-// smoothness BACKWARD needs (rc_tv_bwd_codes: 0.5 bytes per element read instead of x again).
-#ifndef RC_PREPASS_TV_UNROLL
-#define RC_PREPASS_TV_UNROLL 1
-#endif
-#ifndef RC_PREPASS_TV_THREADS
-#define RC_PREPASS_TV_THREADS 128
-#endif
-#ifndef RC_PREPASS_TV_BLOCKS
-#define RC_PREPASS_TV_BLOCKS 4
-#endif
-constexpr int kPrepassTvUnroll = RC_PREPASS_TV_UNROLL;
-constexpr int kPrepassTvThreads = RC_PREPASS_TV_THREADS;
-// acc + (sgn(d) + 1) * unit in FLOAT arithmetic, three FMA-pipe instructions per difference: d * 2^64 is normal for every
-// non-zero d (an overflow to +-inf keeps its sign), so sat(d * 2^64 * 2^100 + 0.5) is exactly 0, 0.5 or 1 = (sgn(d) + 1) / 2.
-// Four pixels x (horizontal, vertical) codes = 16 bits per accumulator: exact in a float.  (Packed bf16 compares of the
-// differences -- set.gt/lt.bf16x2, two results per instruction --, integer selects and a two's-complement code from two
-// saturating multiplies were measured too: 2.7-2.8 ms each, the pass is bound by its instruction count.)
-__device__ __forceinline__ float add_sgn_code(float acc, float d, float unit) {
-  const float q = __saturatef(fmaf(d * 18446744073709551616.f, 1.2676506002282294e30f, 0.5f));
-  return fmaf(q, 2.f * unit, acc);
-}
-
-template <int R, bool kCodes>
-__global__ void __launch_bounds__(kPrepassTvThreads, RC_PREPASS_TV_BLOCKS)
-rownorm_tv_kernel(const float* __restrict__ x, int B, int D, int H, int W, __nv_bfloat16* __restrict__ xb,
-                  float* __restrict__ inv_norm, double* __restrict__ tv_sums, uint32_t* __restrict__ codes) {
-  const int gpr = W >> 3;                                   // 8-pixel groups per row
-  const int strips = (H + R - 1) / R;
-  const int64_t HW = (int64_t)H * W;
-  const int64_t n = (int64_t)B * strips * gpr;
-  const int lane = threadIdx.x & 31;
-  double acc_h = 0.0, acc_v = 0.0;
-  for (int64_t u0 = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); u0 < n; u0 += (int64_t)gridDim.x * blockDim.x) {
-    const bool live = u0 + lane < n;                        // warp-uniform trip count: dead lanes shadow the last unit, store nothing
-    const int64_t u = live ? u0 + lane : n - 1;
-    const int gi = (int)(u % gpr);
-    const int64_t bs = u / gpr;
-    const int strip = (int)(bs % strips);
-    const int64_t b = bs / strips;
-    const int h0 = strip * R;
-    const int rows = min(R, H - h0);
-    const bool has_below = h0 + rows < H;
-    const bool has_right = gi + 1 < gpr;
-    const bool right_shfl = has_right && lane < 31;         // lane + 1 then holds group gi + 1 of the same rows
-    const int64_t off = b * (int64_t)D * HW + (int64_t)h0 * W + gi * 8;
-    const float* src = x + off;
-    __nv_bfloat16* dst = xb + off;
-    uint32_t* cdst = kCodes ? codes + (b * (int64_t)D * H + h0) * gpr + gi : nullptr;
-    float ss[R][8];
-#pragma unroll
-    for (int r = 0; r < R; ++r)
-#pragma unroll
-      for (int j = 0; j < 8; ++j) ss[r][j] = 0.f;
-#pragma unroll kPrepassTvUnroll
-    for (int d = 0; d < D; ++d) {
-      const float* p = src + (int64_t)d * HW;
-      float v[R + 1][8];
-#pragma unroll
-      for (int r = 0; r <= R; ++r)
-        if (r < rows || (r == rows && has_below)) load8(p + (int64_t)r * W, v[r]);
-      float sh = 0.f, sv = 0.f;
-#pragma unroll
-      for (int r = 0; r < R; ++r) {
-        float right = __shfl_down_sync(0xffffffffu, v[r][0], 1);
-        if (r < rows) {
-          // a missing neighbour is replaced by the value itself: difference 0, sign code 0
-          if (!right_shfl) right = has_right ? __ldg(p + (int64_t)r * W + 8) : v[r][7];
-          const bool below = r + 1 < rows || has_below;
-          uint32_t pk[4];
-          float dh[8], dv[8];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            pk[i] = pack_bf16x2(v[r][2 * i], v[r][2 * i + 1]);                 // the tensor cores see the rounded value
-            ss[r][2 * i] = sqacc_bf16x2_lo(ss[r][2 * i], pk[i]);
-            ss[r][2 * i + 1] = sqacc_bf16x2_hi(ss[r][2 * i + 1], pk[i]);
-          }
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            dh[j] = v[r][j] - (j < 7 ? v[r][j + 1] : right);
-            dv[j] = below ? v[r][j] - v[r + 1][j] : 0.f;
-            sh += fabsf(dh[j]);
-            sv += fabsf(dv[j]);
-          }
-          if (live) *reinterpret_cast<uint4*>(dst + (int64_t)d * HW + (int64_t)r * W) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-          if (kCodes) {
-            // word layout: pixel j at bits 4j..4j+3; +0 horizontal, +2 vertical
-            float lo = 0.f, hi = 0.f;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              lo = add_sgn_code(add_sgn_code(lo, dh[j], (float)(1 << (4 * j))), dv[j], (float)(4 << (4 * j)));
-              hi = add_sgn_code(add_sgn_code(hi, dh[j + 4], (float)(1 << (4 * j))), dv[j + 4], (float)(4 << (4 * j)));
-            }
-            if (live) cdst[((int64_t)d * H + r) * gpr] = __float2uint_rz(lo) | (__float2uint_rz(hi) << 16);
-          }
-        }
-      }
-      if (live) { acc_h += (double)sh; acc_v += (double)sv; }
-    }
-    if (live) {
-#pragma unroll
-      for (int r = 0; r < R; ++r)
-        if (r < rows) {
-          float o[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) o[j] = 1.f / fmaxf(sqrtf(ss[r][j]), 1e-12f);
-          store8(inv_norm + b * HW + (int64_t)(h0 + r) * W + gi * 8, o);
-        }
-    }
-  }
-  acc_h = warp_sum(acc_h);
-  acc_v = warp_sum(acc_v);
-  __shared__ double red[2][kPrepassTvThreads / 32];
-  if (lane == 0) { red[0][threadIdx.x >> 5] = acc_h; red[1][threadIdx.x >> 5] = acc_v; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double a = 0, c = 0;
-    for (int i = 0; i < kPrepassTvThreads / 32; ++i) { a += red[0][i]; c += red[1][i]; }
-    atomicAdd(&tv_sums[0], a);
-    atomicAdd(&tv_sums[1], c);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// main kernel
-// ------------------------------------------------------------------------------------------------
 constexpr int kTilePx = 128;
 constexpr int kThreads = 384;          // 12 warps: 0 TMA, 1 MMA, 2 TMEM alloc, 3 spare, 4-11 compute (softmax, then dX epilogue)
 constexpr int kStages = 4;             // ring of 32 KB slots, each with its own full/empty barrier
@@ -248,8 +31,6 @@ constexpr int kStgBufs = 3;             // dX staging buffers; X for the epilogu
 constexpr int kStgPx = 32;             // pixels per dX staging step
 constexpr int kStgBytes = 128 * kStgPx * 2;   // [128 d][32 px] bf16 = 8 KB
 constexpr int kTmemCols = 512;
-constexpr float kLog2e = 1.4426950408889634f;
-constexpr float kLn2 = 0.6931471805599453f;
 
 struct __align__(8) UmmaBars {
   uint64_t full[kStages], empty[kStages];
@@ -268,24 +49,14 @@ constexpr int kOffXch = kOffScale + 2 * kScaleBufs * 128 * 4;   // softmax half<
 constexpr int kOffBars = kOffXch + 4 * 2 * 128 * 4;
 constexpr int kSmemBytes = kOffBars + (int)sizeof(UmmaBars) + 1024;   // + alignment slack
 
-__device__ __forceinline__ float fast_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
 // mbar_wait that also accumulates the cycles spent waiting (per role, reported for CTA 0)
 #ifdef RC_TIMING
-#define RC_T0(name) const long long name = clock64()
-#define RC_TACC(idx, name) wt[idx] += clock64() - name
 __device__ __forceinline__ void mbar_wait_t(uint64_t* bar, uint32_t parity, int tag, long long* acc) {
   const long long t0 = clock64();
   mbar_wait(bar, parity, tag);
   acc[tag] += clock64() - t0;
 }
 #else
-#define RC_T0(name)
-#define RC_TACC(idx, name)
 __device__ __forceinline__ void mbar_wait_t(uint64_t* bar, uint32_t parity, int tag, long long*) {
   mbar_wait(bar, parity, tag);
 }
@@ -741,267 +512,12 @@ infonce_umma_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][H
   }
 }
 
-}  // namespace rc
-
-// ------------------------------------------------------------------------------------------------
-// bring-up kernel: one 128 x N x Kd GEMM tile through the same TMA / descriptor / tcgen05 / TMEM path
-// ------------------------------------------------------------------------------------------------
-namespace rc {
-
-struct __align__(8) DebugBars { uint64_t full, done; uint32_t tmem_base, pad; };
-
-__global__ void __launch_bounds__(128, 1)
-debug_umma_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, int N, int Kd,
-                       int variant, float* __restrict__ c) {
-  // 1024-byte alignment (128B-swizzle atoms) comes from the declaration, so that the compiler keeps the
-  // shared address space (LDS/STS instead of generic LD/ST) for every access derived from `smem`.
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sa = smem;               // 16 KB
-  uint8_t* sbm = smem + 16384;      // <= 32 KB
-  DebugBars* bars = reinterpret_cast<DebugBars*>(smem + 49152);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    mbar_init(&bars->full, 1);
-    mbar_init(&bars->done, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc<256>(&bars->tmem_base);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = bars->tmem_base;
-  if (threadIdx.x == 0) {
-    const uint32_t idesc = make_idesc_bf16(128, N, variant == 0 ? 0 : 1, 0);
-    for (int ck = 0; ck < Kd / 64; ++ck) {
-      mbar_arrive_expect_tx(&bars->full, 16384 + N * 128);
-      if (variant == 0) {
-        tma_load_2d(sa, &map_a, &bars->full, ck * 64, 0);             // A [128][Kd]: box (64 k, 128 rows)
-      } else {
-        tma_load_2d(sa, &map_a, &bars->full, 0, ck * 64);             // A^T [Kd][128]: box (64 m, 64 k) x 2
-        tma_load_2d(sa + 8192, &map_a, &bars->full, 64, ck * 64);
-      }
-      tma_load_2d(sbm, &map_b, &bars->full, ck * 64, 0);              // B [N][Kd]: box (64 k, N rows)
-      mbar_wait(&bars->full, ck & 1, 100);
-      tc_fence_after();
-      for (int ks = 0; ks < 4; ++ks) {
-        uint64_t a;
-        if (variant == 0) a = desc_kmajor_sw128(smem_u32(sa) + ks * 32);
-        else if (variant == 1) a = desc_mnmajor_sw128(smem_u32(sa) + ks * 2048, 8192);
-        else a = make_smem_desc_sw128(smem_u32(sa) + ks * 2048, 1024, 8192);   // hypothesis: LBO/SBO roles swapped
-        const uint64_t b = desc_kmajor_sw128(smem_u32(sbm) + ks * 32);
-        mma_bf16_ss(tmem, a, b, idesc, (ck | ks) != 0);
-      }
-      mma_commit(&bars->done);
-      mbar_wait(&bars->done, ck & 1, 101);
-    }
-  }
-  __syncthreads();
-  tc_fence_after();
-  const int row = warp * 32 + lane;
-  for (int cc = 0; cc < N / 32; ++cc) {
-    uint32_t r[32];
-    tmem_ld_32x32(tmem + ((uint32_t)(warp * 32) << 16) + cc * 32, r);
-    tmem_ld_wait();
-    for (int i = 0; i < 32; ++i) c[(int64_t)row * N + cc * 32 + i] = __uint_as_float(r[i]);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc<256>(tmem); }
-}
-
-static int check_sm100(const char* what) {
-  int dev = 0, major = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return fail(RC_ERR_NO_DEVICE, "%s: no CUDA device", what);
-  cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev);
-  if (major != 10) return fail(RC_ERR_NO_DEVICE, "%s: needs an sm_100 device (compute capability %d.x found)", what, major);
-  return RC_OK;
-}
-
-}  // namespace rc
-
-#ifdef RC_BRINGUP
-extern "C" int rc_debug_umma_gemm(const void* a_bf16, const void* b_bf16, int N, int Kd, int variant, float* c, void* stream) {
-  RC_REQUIRE(a_bf16 && b_bf16 && c, "rc_debug_umma_gemm: null pointer");
-  RC_REQUIRE(N >= 32 && N <= 256 && N % 32 == 0 && Kd >= 64 && Kd % 64 == 0 && variant >= 0 && variant <= 2,
-             "rc_debug_umma_gemm: bad shape N=%d Kd=%d variant=%d", N, Kd, variant);
-  int rcode = rc::check_sm100("rc_debug_umma_gemm");
-  if (rcode) return rcode;
-  CUtensorMap ma, mb;
-  if (variant == 0) {
-    const uint64_t dims[2] = {(uint64_t)Kd, 128}, str[2] = {2, (uint64_t)Kd * 2};
-    const uint32_t box[2] = {64, 128};
-    if ((rcode = rc::make_tmap_bf16(&ma, a_bf16, 2, dims, str, box, "debug A"))) return rcode;
-  } else {
-    const uint64_t dims[2] = {128, (uint64_t)Kd}, str[2] = {2, 256};
-    const uint32_t box[2] = {64, 64};
-    if ((rcode = rc::make_tmap_bf16(&ma, a_bf16, 2, dims, str, box, "debug A^T"))) return rcode;
-  }
-  {
-    const uint64_t dims[2] = {(uint64_t)Kd, (uint64_t)N}, str[2] = {2, (uint64_t)Kd * 2};
-    const uint32_t box[2] = {64, (uint32_t)N};
-    if ((rcode = rc::make_tmap_bf16(&mb, b_bf16, 2, dims, str, box, "debug B"))) return rcode;
-  }
-  const int smem = 49152 + 64 + 1024;
-  cudaError_t e = cudaFuncSetAttribute(rc::debug_umma_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return rc::fail(RC_ERR_CUDA, "rc_debug_umma_gemm: smem opt-in: %s", cudaGetErrorString(e));
-  rc::debug_umma_gemm_kernel<<<1, 128, smem, (cudaStream_t)stream>>>(ma, mb, N, Kd, variant, c);
-  return rc::check_launch("rc_debug_umma_gemm");
-}
-#endif  // RC_BRINGUP
-
-extern "C" int64_t rc_infonce_workspace_bytes(int B, int D, int64_t HW, int K, rc_dtype x_dtype) {
-  (void)K;
-  const int64_t M = (int64_t)B * HW;
-  int64_t bytes = ((M * 4 + 255) / 256) * 256;                                   // inv_norm
-  if (x_dtype == RC_F32) bytes += (((int64_t)B * D * HW * 2 + 255) / 256) * 256;   // bf16 copy of X
-  return bytes + 256;
-}
-
-extern "C" int64_t rc_infonce_workspace_bytes_dt(int B, int D, int64_t HW, int K, rc_dtype x_dtype) {
-  const int64_t Kp = (K + 63) / 64 * 64;
-  const int64_t base = (rc_infonce_workspace_bytes(B, D, HW, K, x_dtype) + 255) / 256 * 256;
-  return base + (int64_t)B * HW * Kp * 2 + 512;       // + G, bf16 [B][HW][Kp]
-}
-
-namespace rc {
-int launch_rownorm_f32(const float* x, int B, int D, int64_t HW, __nv_bfloat16* xb, float* inv_norm, cudaStream_t s) {
-  const int64_t blocks = ((int64_t)B * HW / 8 + 255) / 256;
-  const int grid = (int)(blocks < (int64_t)num_sms() * 8 ? blocks : (int64_t)num_sms() * 8);
-  rownorm_kernel<float><<<grid, 256, 0, s>>>(x, B, D, HW, xb, inv_norm);
-  return check_launch("rownorm(f32 -> bf16)");
-}
-static int infonce_prepass_impl(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, void* workspace,
-                                int64_t workspace_bytes, cudaStream_t s, float** inv_norm_out, __nv_bfloat16** xb_out) {
-  RC_REQUIRE(x && workspace, "rc_infonce_prepass: null pointer");
-  if (HW % 8 != 0) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: HW=%lld must be a multiple of 8", (long long)HW);
-  RC_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0, "rc_infonce_bf16: x must be 16-byte aligned");
-  RC_REQUIRE(workspace_bytes >= rc_infonce_workspace_bytes(B, D, HW, 0, x_dtype), "rc_infonce_bf16: workspace too small");
-  const int64_t M = (int64_t)B * HW;
-  uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
-  *inv_norm_out = reinterpret_cast<float*>(ws);
-  *xb_out = (x_dtype == RC_F32) ? reinterpret_cast<__nv_bfloat16*>(ws + ((M * 4 + 255) / 256) * 256) : nullptr;
-  if (s == (cudaStream_t)-1 || M == 0) return RC_OK;   // pointers only
-  const int64_t groups = M / 8;
-  const int64_t blocks = (groups + 255) / 256;
-  const int grid = (int)(blocks < (int64_t)num_sms() * 8 ? blocks : (int64_t)num_sms() * 8);
-  if (x_dtype == RC_F32) rownorm_kernel<float><<<grid, 256, 0, s>>>((const float*)x, B, D, HW, *xb_out, *inv_norm_out);
-  else rownorm_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>((const __nv_bfloat16*)x, B, D, HW, nullptr, *inv_norm_out);
-  return check_launch("rc_infonce_prepass");
-}
-}  // namespace rc
-
-namespace rc { static long long* g_dbg_buf = nullptr; long long* debug_timing_buffer() { return g_dbg_buf; } }
-#if defined(RC_BRINGUP) || defined(RC_TIMING)
-extern "C" int rc_debug_set_timing_buffer(int64_t* dev_buf) { rc::g_dbg_buf = (long long*)dev_buf; return RC_OK; }
-#endif
-
-extern "C" int rc_infonce_prepass(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, void* workspace,
-                                  int64_t workspace_bytes, void* stream) {
-  float* inv_norm; __nv_bfloat16* xb;
-  int rcode = rc::check_sm100("rc_infonce_prepass");
-  if (rcode) return rcode;
-  return rc::infonce_prepass_impl(x, x_dtype, B, D, HW, workspace, workspace_bytes, (cudaStream_t)stream, &inv_norm, &xb);
-}
-
-#ifndef RC_PREPASS_TV_ROWS
-#define RC_PREPASS_TV_ROWS 4
-#endif
-// fp32 x [B][D][H][W], W % 8 == 0: the pre-pass of rc_infonce_bf16 (bf16 copy + 1/|x_p| into workspace, to be followed by
-// RC_INFONCE_PREPASS_DONE) and the smoothness sums of rc_tv_fwd (ADDED to tv_sums[0..1]) from a single read of x; tv_codes
-// (nullable, [B][D][H][W/8] words): the difference signs for rc_tv_bwd_codes.
-extern "C" int rc_infonce_prepass_tv(const float* x, int B, int D, int H, int W, void* workspace, int64_t workspace_bytes,
-                                     double* tv_sums, uint32_t* tv_codes, void* stream) {
-  using namespace rc;
-  RC_REQUIRE(x && workspace && tv_sums, "rc_infonce_prepass_tv: null pointer");
-  RC_REQUIRE(B >= 0 && D >= 1 && H >= 0 && W >= 0, "rc_infonce_prepass_tv: bad shape");
-  if (W % 8 != 0) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_prepass_tv: W=%d must be a multiple of 8", W);
-  int rcode = check_sm100("rc_infonce_prepass_tv");
-  if (rcode) return rcode;
-  const int64_t HW = (int64_t)H * W;
-  float* inv_norm; __nv_bfloat16* xb;
-  if ((rcode = infonce_prepass_impl(x, RC_F32, B, D, HW, workspace, workspace_bytes, (cudaStream_t)-1, &inv_norm, &xb))) return rcode;
-  if (B == 0 || HW == 0) return RC_OK;
-  constexpr int R = RC_PREPASS_TV_ROWS;
-  const int64_t units = (int64_t)B * ((H + R - 1) / R) * (W / 8);
-  constexpr int T = kPrepassTvThreads;
-  const int64_t blocks = (units + T - 1) / T;
-  const int grid = (int)(blocks < (int64_t)num_sms() * 16 ? blocks : (int64_t)num_sms() * 16);
-  if (tv_codes != nullptr) rownorm_tv_kernel<R, true><<<grid, T, 0, (cudaStream_t)stream>>>(x, B, D, H, W, xb, inv_norm, tv_sums, tv_codes);
-  else rownorm_tv_kernel<R, false><<<grid, T, 0, (cudaStream_t)stream>>>(x, B, D, H, W, xb, inv_norm, tv_sums, nullptr);
-  return check_launch("rc_infonce_prepass_tv");
-}
-
-// rep = 1: rc_infonce_bf16; rep = 4: rc_infonce_bf16_rep4 (y, w are [B*HW][4])
-static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16,
-                             const void* tt_bf16, int K, const int32_t* y, const float* w, float inv_tau, float* lse,
-                             double* loss_sum, double* w_sum, const double* w_sum_in, const float* grad_scale, void* dx,
-                             float* dt, double* dlogtau, void* workspace, int64_t workspace_bytes, int flags, int rep,
-                             void* stream, const int32_t* k_dev = nullptr, const float* log_tau_dev = nullptr) {
-  using namespace rc;
-  RC_REQUIRE(x && t_bf16 && y && w && workspace, "rc_infonce_bf16: null pointer");
-  RC_REQUIRE(B >= 0 && HW >= 0, "rc_infonce_bf16: bad shape");
-  if (K < 1 || K > 256) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: K=%d outside [1,256] (use rc_infonce_f32)", K);
-  if (D < 128 || D > 512 || D % 128 != 0) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: D=%d must be 128, 256, 384 or 512", D);
-  RC_REQUIRE((reinterpret_cast<uintptr_t>(t_bf16) & 15) == 0, "rc_infonce_bf16: t must be 16-byte aligned");
+// launch helper used by rc_infonce_bf16 (infonce.cu owns argument checking and the pre-pass)
+int launch_infonce_1cta(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
+                        const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
+                        const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, cudaStream_t s) {
   const bool bwd = dx != nullptr;
-  if (bwd) RC_REQUIRE(tt_bf16 && w_sum_in && (reinterpret_cast<uintptr_t>(dx) & 15) == 0, "rc_infonce_bf16: backward needs tt_bf16, w_sum_in and aligned dx");
-  if (dlogtau && !bwd) return fail(RC_ERR_INVALID, "rc_infonce_bf16: dlogtau needs dx");
-  if (B == 0 || HW == 0) return RC_OK;
-  int rcode = check_sm100("rc_infonce_bf16");
-  if (rcode) return rcode;
-  if ((k_dev != nullptr || log_tau_dev != nullptr) && !infonce_pair_supported(D))
-    return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn: device-side K / log tau need D = 256 or 512 (CTA-pair kernel)");
-  cudaStream_t s = (cudaStream_t)stream;
-  float* inv_norm; __nv_bfloat16* xb;
-  // CTA-pair kernel (cta_group::2) when the channel count allows it; RANGECLIP_B200_INFONCE=1cta forces the
-  // single-CTA kernel (kept for D = 128 / 384 and as the A/B baseline).  The pair kernel computes 1/|x_p| itself
-  // from the operand tiles in shared memory, so a bf16 input needs no pre-pass at all (an fp32 input still needs
-  // its bf16 copy).
-#ifdef RC_BRINGUP
-  const char* impl = getenv("RANGECLIP_B200_INFONCE");     // bring-up A/B switch; never compiled into the shipped library
-#else
-  const char* impl = nullptr;
-#endif
-  const bool use_pair = (rep != 1 || !(impl != nullptr && impl[0] == '1')) && infonce_pair_supported(D);
-  const int keep_w = (flags & RC_INFONCE_KEEP_WEIGHT) ? 1 : 0;
-  const int acc_dx = (flags & RC_INFONCE_ACCUMULATE_DX) ? 1 : 0;
-  const float* lse_in = (flags & RC_INFONCE_LSE_GIVEN) ? lse : nullptr;
-  if (acc_dx) RC_REQUIRE(bwd, "rc_infonce_bf16: RC_INFONCE_ACCUMULATE_DX needs dx");
-  if (keep_w || lse_in || acc_dx) {
-    if (!use_pair || rep != 1 || dt != nullptr)
-      return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: the K-blocked flags need D = 256 or 512, one target per row and no dText");
-    RC_REQUIRE(!(flags & RC_INFONCE_LSE_GIVEN) || lse != nullptr, "rc_infonce_bf16: RC_INFONCE_LSE_GIVEN needs lse");
-  }
-  if (rep != 1) {
-    if (!use_pair) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_rep4: D=%d must be 256 or 512", D);
-    RC_REQUIRE((reinterpret_cast<uintptr_t>(y) & 15) == 0 && (reinterpret_cast<uintptr_t>(w) & 15) == 0,
-               "rc_infonce_bf16_rep4: y and w must be 16-byte aligned");
-  }
-  const bool skip_prepass = (flags & RC_INFONCE_PREPASS_DONE) || (use_pair && x_dtype == RC_BF16);
-  if ((rcode = infonce_prepass_impl(x, x_dtype, B, D, HW, workspace, workspace_bytes, skip_prepass ? (cudaStream_t)-1 : s,
-                                    &inv_norm, &xb))) return rcode;
-  const void* xsrc = (x_dtype == RC_F32) ? (const void*)xb : x;
-  if (dt != nullptr) {
-    // dText: the pair kernel also writes G = rs (P - sum onehot) (bf16 [B][HW][Kp]) into the workspace, then one
-    // split-K GEMM over the pixels (infonce_dt_umma.cu) adds G^T X to dt.
-    if (!use_pair || !bwd)
-      return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: dText needs dx and D = 256 or 512 (use rc_infonce_f32 otherwise)");
-    const int64_t base = rc_infonce_workspace_bytes(B, D, HW, K, x_dtype);
-    RC_REQUIRE(workspace_bytes >= rc_infonce_workspace_bytes_dt(B, D, HW, K, x_dtype), "rc_infonce_bf16: workspace too small for dText");
-    uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
-    void* g = ws + ((base + 255) / 256) * 256;
-    if ((rcode = launch_infonce_pair(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
-                                     loss_sum, w_sum, dlogtau, g, rep, 0, nullptr, 0, 0, k_dev, log_tau_dev, s))) return rcode;
-    return launch_infonce_dt(g, xsrc, B, D, HW, K, dt, s);
-  }
-  if (use_pair) {
-    // backward launches: the softmax tile as a tensor-memory operand of the dX GEMM (infonce_ts.cu) unless RC_INFONCE_SS_KERNEL
-    if (bwd && !(flags & RC_INFONCE_SS_KERNEL) && k_dev == nullptr && log_tau_dev == nullptr)
-      return launch_infonce_ts(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, y, w, inv_tau, grad_scale, w_sum_in, lse, loss_sum, w_sum,
-                               dlogtau, rep, keep_w, lse_in, 0, acc_dx, s);
-    return launch_infonce_pair(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
-                               loss_sum, w_sum, dlogtau, nullptr, rep, keep_w, lse_in, 0, acc_dx, k_dev, log_tau_dev, s);
-  }
+  int rcode;
   const int Kp = (K + 63) / 64 * 64;
   CUtensorMap m_xs, m_t, m_tt, m_xe, m_dx;
   {
@@ -1025,7 +541,7 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   if ((int64_t)B * prm.tiles_per_img > 0x7fffffff) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: too many tiles");
   prm.n_tiles = B * prm.tiles_per_img;
   prm.inv_norm = inv_norm; prm.y = y; prm.w = w; prm.inv_tau = inv_tau; prm.grad_scale = grad_scale;
-  prm.w_sum_in = w_sum_in; prm.lse = lse; prm.loss_sum = loss_sum; prm.w_sum = w_sum; prm.dlogtau = dlogtau; prm.dbg = g_dbg_buf;
+  prm.w_sum_in = w_sum_in; prm.lse = lse; prm.loss_sum = loss_sum; prm.w_sum = w_sum; prm.dlogtau = dlogtau; prm.dbg = debug_timing_buffer();
   const int grid = prm.n_tiles < num_sms() ? prm.n_tiles : num_sms();
   cudaError_t e;
   if (bwd) {
@@ -1040,143 +556,4 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   return check_launch("rc_infonce_bf16");
 }
 
-extern "C" int rc_infonce_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16,
-                               const void* tt_bf16, int K, const int32_t* y, const float* w, float inv_tau, float* lse,
-                               double* loss_sum, double* w_sum, const double* w_sum_in, const float* grad_scale, void* dx,
-                               float* dt, double* dlogtau, void* workspace, int64_t workspace_bytes, int flags, void* stream) {
-  return infonce_bf16_impl(x, x_dtype, B, D, HW, t_bf16, tt_bf16, K, y, w, inv_tau, lse, loss_sum, w_sum, w_sum_in, grad_scale,
-                           dx, dt, dlogtau, workspace, workspace_bytes, flags, 1, stream);
-}
-
-extern "C" int rc_infonce_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16,
-                                    const void* tt_bf16, int K, const int32_t* y4, const float* w4, float inv_tau, float* lse,
-                                    double* loss_sum, double* w_sum, const double* w_sum_in, const float* grad_scale,
-                                    void* dx, float* dt, double* dlogtau, void* workspace, int64_t workspace_bytes,
-                                    int flags, void* stream) {
-  return infonce_bf16_impl(x, x_dtype, B, D, HW, t_bf16, tt_bf16, K, y4, w4, inv_tau, lse, loss_sum, w_sum, w_sum_in,
-                           grad_scale, dx, dt, dlogtau, workspace, workspace_bytes, flags, 4, stream);
-}
-
-// rep = 1 or 4; the number of valid candidate rows (<= K, the rest are zero pad rows) and log(tau) come from device memory
-extern "C" int rc_infonce_bf16_dyn(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16,
-                                   const void* tt_bf16, int K, const int32_t* k_dev, const int32_t* y, const float* w,
-                                   const float* log_tau_dev, int rep, float* lse, double* loss_sum, double* w_sum,
-                                   const double* w_sum_in, const float* grad_scale, void* dx, double* dlogtau,
-                                   void* workspace, int64_t workspace_bytes, int flags, void* stream) {
-  RC_REQUIRE(log_tau_dev != nullptr, "rc_infonce_bf16_dyn: log_tau_dev is required");
-  RC_REQUIRE(rep == 1 || rep == 4, "rc_infonce_bf16_dyn: rep must be 1 or 4");
-  RC_REQUIRE(!(flags & (RC_INFONCE_KEEP_WEIGHT | RC_INFONCE_LSE_GIVEN | RC_INFONCE_ACCUMULATE_DX)), "rc_infonce_bf16_dyn: K-blocked flags are not supported");
-  return infonce_bf16_impl(x, x_dtype, B, D, HW, t_bf16, tt_bf16, K, y, w, 0.f, lse, loss_sum, w_sum, w_sum_in, grad_scale, dx,
-                           nullptr, dlogtau, workspace, workspace_bytes, flags, rep, stream, k_dev, log_tau_dev);
-}
-
-extern "C" int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, int64_t HW, const void* t_bf16_all,
-                                       const void* tt_bf16_all, int K, int n_blocks, const int32_t* y_rel, const float* w_rep,
-                                       float inv_tau, float* lse, double* loss_sum, double* w_sum, const double* w_sum_in,
-                                       const float* grad_scale, void* dx_blocks, double* dlogtau, void* workspace,
-                                       int64_t workspace_bytes, int flags, void* stream) {
-  using namespace rc;
-  RC_REQUIRE(x && t_bf16_all && y_rel && w_rep && workspace && lse, "rc_infonce_bf16_kblocks: null pointer");
-  RC_REQUIRE(HW >= 0 && K >= 1 && n_blocks >= 1 && n_blocks == (K + 255) / 256, "rc_infonce_bf16_kblocks: n_blocks must be ceil(K / 256)");
-  if (!infonce_pair_supported(D)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: D=%d must be 256 or 512", D);
-  if (HW % 256 != 0) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: HW=%lld must be a multiple of 256", (long long)HW);
-  RC_REQUIRE((reinterpret_cast<uintptr_t>(t_bf16_all) & 15) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0, "rc_infonce_bf16_kblocks: alignment");
-  const bool bwd = dx_blocks != nullptr;
-  if (bwd) RC_REQUIRE(tt_bf16_all && w_sum_in && (flags & RC_INFONCE_LSE_GIVEN), "rc_infonce_bf16_kblocks: the backward needs tt_bf16_all, w_sum_in and RC_INFONCE_LSE_GIVEN");
-  if (HW == 0) return RC_OK;
-  int rcode = check_sm100("rc_infonce_bf16_kblocks");
-  if (rcode) return rcode;
-  cudaStream_t s = (cudaStream_t)stream;
-  float* inv_norm; __nv_bfloat16* xb;
-  const bool skip_prepass = (flags & RC_INFONCE_PREPASS_DONE) || x_dtype == RC_BF16;
-  if ((rcode = infonce_prepass_impl(x, x_dtype, 1, D, HW, workspace, workspace_bytes, skip_prepass ? (cudaStream_t)-1 : s, &inv_norm, &xb))) return rcode;
-  const void* xsrc = (x_dtype == RC_F32) ? (const void*)xb : x;
-  const float* lse_in = (flags & RC_INFONCE_LSE_GIVEN) ? lse : nullptr;
-  if (bwd && !(flags & RC_INFONCE_SS_KERNEL))
-    return launch_infonce_ts(xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, y_rel, w_rep, inv_tau, grad_scale, w_sum_in,
-                             lse, loss_sum, w_sum, dlogtau, 1, 1, lse_in, n_blocks, 0, s);
-  return launch_infonce_pair(xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, inv_norm, y_rel, w_rep, inv_tau, grad_scale,
-                             w_sum_in, lse, loss_sum, w_sum, dlogtau, nullptr, 1, 1, lse_in, n_blocks, 0, nullptr, nullptr, s);
-}
-
-// ------------------------------------------------------------------------------------------------
-// bring-up kernel for the CTA-pair (cta_group::2) building blocks: C[256][N] = A[256][Kd] B[N][Kd]^T
-// with A rows split 128/128 over the two CTAs and B rows split N/2 / N/2.
-// ------------------------------------------------------------------------------------------------
-namespace rc {
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1)
-debug_umma_gemm_2sm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, int N, int Kd,
-                           float* __restrict__ c) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sa = smem;               // 16 KB: own 128 rows of A, one 64-wide K chunk
-  uint8_t* sbm = smem + 16384;      // <= 16 KB: own N/2 rows of B
-  DebugBars* bars = reinterpret_cast<DebugBars*>(smem + 32768);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  if (threadIdx.x == 0) {
-    mbar_init(&bars->full, 1);
-    mbar_init(&bars->done, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc_2sm<256>(&bars->tmem_base);
-  tc_fence_before();
-  cluster_sync();
-  tc_fence_after();
-  const uint32_t tmem = bars->tmem_base;
-  if (threadIdx.x == 0) {
-    const uint32_t idesc = make_idesc_bf16(256, N, 0, 0);
-    const int nh = N / 2;
-    for (int ck = 0; ck < Kd / 64; ++ck) {
-      if (rank == 0) mbar_arrive_expect_tx(&bars->full, 2 * (16384 + nh * 128));
-      tma_load_2d_2sm(sa, &map_a, &bars->full, ck * 64, (int)rank * 128);
-      tma_load_2d_2sm(sbm, &map_b, &bars->full, ck * 64, (int)rank * nh);
-      if (rank == 0) {
-        mbar_wait_cluster(&bars->full, ck & 1, 200);
-        tc_fence_after();
-        for (int ks = 0; ks < 4; ++ks)
-          mma_bf16_ss_2sm(tmem, desc_kmajor_sw128(smem_u32(sa) + ks * 32), desc_kmajor_sw128(smem_u32(sbm) + ks * 32), idesc,
-                          (ck | ks) != 0);
-        mma_commit_2sm(&bars->done);
-      }
-      mbar_wait_cluster(&bars->done, ck & 1, 201);   // both CTAs: smem may be refilled, TMEM is current
-    }
-  }
-  __syncthreads();
-  tc_fence_after();
-  const int row = warp * 32 + lane;
-  for (int cc = 0; cc < N / 32; ++cc) {
-    uint32_t r[32];
-    tmem_ld_32x32(tmem + ((uint32_t)(warp * 32) << 16) + cc * 32, r);
-    tmem_ld_wait();
-    for (int i = 0; i < 32; ++i) c[((int64_t)rank * 128 + row) * N + cc * 32 + i] = __uint_as_float(r[i]);
-  }
-  tc_fence_before();
-  cluster_sync();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc_2sm<256>(tmem); }
-}
-
 }  // namespace rc
-
-#ifdef RC_BRINGUP
-extern "C" int rc_debug_umma_gemm_2sm(const void* a_bf16, const void* b_bf16, int N, int Kd, float* c, void* stream) {
-  RC_REQUIRE(a_bf16 && b_bf16 && c, "rc_debug_umma_gemm_2sm: null pointer");
-  RC_REQUIRE(N >= 64 && N <= 256 && N % 64 == 0 && Kd >= 64 && Kd % 64 == 0, "rc_debug_umma_gemm_2sm: bad shape N=%d Kd=%d", N, Kd);
-  int rcode = rc::check_sm100("rc_debug_umma_gemm_2sm");
-  if (rcode) return rcode;
-  CUtensorMap ma, mb;
-  {
-    const uint64_t dims[2] = {(uint64_t)Kd, 256}, str[2] = {2, (uint64_t)Kd * 2};
-    const uint32_t box[2] = {64, 128};
-    if ((rcode = rc::make_tmap_bf16(&ma, a_bf16, 2, dims, str, box, "debug2 A"))) return rcode;
-    const uint64_t bdims[2] = {(uint64_t)Kd, (uint64_t)N};
-    const uint32_t bbox[2] = {64, (uint32_t)(N / 2)};
-    if ((rcode = rc::make_tmap_bf16(&mb, b_bf16, 2, bdims, str, bbox, "debug2 B"))) return rcode;
-  }
-  const int smem = 32768 + 64;
-  cudaError_t e = cudaFuncSetAttribute(rc::debug_umma_gemm_2sm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return rc::fail(RC_ERR_CUDA, "rc_debug_umma_gemm_2sm: smem opt-in: %s", cudaGetErrorString(e));
-  rc::debug_umma_gemm_2sm_kernel<<<2, 128, smem, (cudaStream_t)stream>>>(ma, mb, N, Kd, c);
-  return rc::check_launch("rc_debug_umma_gemm_2sm");
-}
-#endif  // RC_BRINGUP

@@ -16,7 +16,8 @@
 //                 single shared-memory P buffer as soon as the dX(i-1) MMAs have finished reading P(i-1)
 //   dX epilogue : own 128 channel rows x 64 contiguous pixels per accumulator: x is read straight from
 //                 global memory (L2-resident: the S GEMM just streamed it) with 256-bit loads, prefetched one
-//                 accumulator ahead, and dX goes back with 256-bit stores -- no shared-memory staging.
+//                 accumulator ahead; each warp stages its [32 d][32 px] dX box in shared memory and writes it
+//                 with its own TMA store.
 // Register budget by role (setmaxnreg; the sum over the five warpgroups must stay within the 5 x 96 the CTA is
 // launched with): control warps 48, softmax warps 120, epilogue warps 96.
 // Only the leader CTA (cluster rank 0) issues MMAs; completion is multicast to the mbarriers of both CTAs,
@@ -25,9 +26,9 @@
 // pixels of both tiles).
 #include "common.cuh"
 #include "umma.cuh"
+#include "infonce_device.cuh"
 #include <float.h>
 #include <stdlib.h>
-#include <stdio.h>
 
 namespace rc {
 using namespace umma;
@@ -35,74 +36,14 @@ using namespace umma;
 namespace pair {
 
 constexpr int kTilePx = 128;
-constexpr int kThreads = 640;          // warps: 0 TMA, 1 MMA (leader CTA only), 2 TMEM alloc, 3 idle, 4-11 softmax, 12-19 dX epilogue
-// RC_PAIR_STG2: two dX staging buffers per epilogue warp (a chunk's TMA store reads its buffer while the next chunk is staged)
-// paid for with one X-ring stage (shared memory is full).  Measured, not adopted: 2.83 ms against 2.41 ms -- the X ring is the
-// first-touch HBM path and three stages starve the S GEMM (with the dX stores ablated: 2.51 against 2.13 ms).
-#ifndef RC_PAIR_STG2
-#define RC_PAIR_STG2 0
-#endif
-// RC_PAIR_NORM_WARP: the row norms 1/|x_p| are taken by the relay warp (warp 2, otherwise one busy lane) as soon as a chunk
-// lands, instead of by the eight softmax warps between their hand-offs: an X-ring slot is then released by the MMA commit and
-// ONE early reader (was: eight readers that get to it only after their exp pass), and the softmax warps lose the pass.
-// Measured, not adopted: 2.54 ms against 2.41 ms -- one warp's 64 dependent-latency LDS rounds per chunk release the slot
-// later than eight warps' four, and warp 2 issues last on its scheduler.
-// A/B knobs (tools/ablate_pair.py ab ...): L2 eviction hint of the text operand loads (0 none, 1 evict_last) and of the epilogue's
-// x loads (1 evict_first, 0 none)
-#ifndef RC_PAIR_TEXT_HINT
-#define RC_PAIR_TEXT_HINT 0
-#endif
-#ifndef RC_PAIR_X_HINT
-#define RC_PAIR_X_HINT 0      // evict_last on the X tile loads of the S GEMM (kBwd launches)
-#endif
-#ifndef RC_EPI_X_HINT
-#define RC_EPI_X_HINT 1
-#endif
-// RC_PAIR_SMX_UNIT: the dX epilogue is the role that paces the launch (four accumulator units per tile pair, one after the other
-// on eight warps), while the softmax warps idle between their P hand-off and the next S.  With this switch the softmax warps
-// drain ONE of the four units (unit 1: channel block 0, pixels [64,128) of both tiles) in that window -- TMEM load, projection,
-// direct 256-bit global stores (they have no staging tile) -- and the epilogue warps skip it.  Measured, not adopted (same box,
-// base 2.43 ms): after the row norms (1) 3.18 ms, before them (2) 2.90 ms.  The softmax warps' wait for the next S is not slack:
-// they sit on the S -> exp -> P -> dX dependency cycle, and whatever they do in between delays the exp pass of the next tile.
-#ifndef RC_PAIR_SMX_UNIT
-#define RC_PAIR_SMX_UNIT 0
-#endif
-#ifndef RC_EPI_FETCH_EARLY
-#define RC_EPI_FETCH_EARLY 0      // measured (same box): early 2.50 ms, late 2.45 ms
-#endif
-#ifndef RC_PAIR_NORM_WARP
-#define RC_PAIR_NORM_WARP 0
-#endif
-// RC_PAIR_CTL_HIGH: the four control warps (text TMA, MMA issuer, relay, X TMA) are the HIGHEST warp ids of the CTA.  The
-// schedulers pick the highest eligible warp id first; as warps 0-3 the producers and the MMA issuer issue after the four busy
-// softmax / epilogue warps that share their scheduler.
-// Measured: 2.64 ms against 2.41 ms -- the control warps' barrier polling then takes issue slots from the workers.
-// RC_PAIR_CTL_HIGH == 2: control warps stay lowest, but the SOFTMAX warps (the exp pass is on the S -> P -> dX dependency cycle)
-// get the highest warp ids and the epilogue warps the middle ones: 2.56 ms.  The shipped order (control < softmax < epilogue)
-// is the best of the three: the epilogue is the role with the least slack.
-#ifndef RC_PAIR_CTL_HIGH
-#define RC_PAIR_CTL_HIGH 0
-#endif
-constexpr int kXStages = RC_PAIR_STG2 ? 3 : 4;   // X ring: own X chunks [64 d][128 px] (first touch: HBM latency; also read by the row norms)
-constexpr int kStgBufs = RC_PAIR_STG2 ? 2 : 1;
+constexpr int kThreads = 640;          // warps: 0 text TMA, 1 MMA (leader CTA only), 2 relay + TMEM alloc, 3 X TMA, 4-11 softmax, 12-19 dX epilogue
+constexpr int kXStages = 4;            // X ring: own X chunks [64 d][128 px] (first touch: HBM latency; also read by the row norms)
 constexpr int kTStages = 4;            // text ring: text half-chunks [Kp/2][64 d] for S, own T^T rows [128 d][64 k] for dX (L2 hits)
 constexpr int kStageBytes = 16 * 1024;
 static_assert(kTStages >= 4, "a dX block keeps Kp/64 <= 4 slots of the text ring at once");
 constexpr int kPBytes = 64 * 1024;
 constexpr int kTmemCols = 512;
-// Measured, not adopted: TMEM load of softmax step c+1 in flight while step c is computed (needs 128 softmax registers,
-// taken from the control warps): 2.62 ms against 2.49 ms; forward-only launches, which have the registers without
-// spilling, also lose (1.61 ms against 1.47 ms) -- the exposed TMEM latency is not what bounds the exp pass.
-#ifndef RC_SMX_DOUBLE_BUFFER
-#define RC_SMX_DOUBLE_BUFFER 0
-#endif
-#if RC_SMX_DOUBLE_BUFFER
-constexpr int kRegsCtl = 32, kRegsSoftmax = 128;     // epilogue warps keep the entry allocation (96); 32 + 2*128 + 2*96 = 5*96
-#else
 constexpr int kRegsCtl = 48, kRegsSoftmax = 120;     // epilogue warps keep the entry allocation (96); 48 + 2*120 + 2*96 = 5*96
-#endif
-constexpr float kLog2e = 1.4426950408889634f;
-constexpr float kLn2 = 0.6931471805599453f;
 
 struct __align__(8) Bars {
   uint64_t xf[kXStages];        // own X chunk has landed (CTA-local; relayed to the leader's xfull)
@@ -111,7 +52,6 @@ struct __align__(8) Bars {
   uint64_t s_full[2], s_empty[2], p_full, p_empty;   // S: one TMEM buffer with a backward, two (columns 0 / 256) forward-only
   uint64_t acc_full[2], acc_empty[2];
   uint64_t sc_full[2];
-  uint64_t n_full[2], n_empty[2];   // row norms of a tile are in shared memory / have been read (RC_PAIR_NORM_WARP; by tile parity)
   uint32_t tmem_base, pad;
 };
 
@@ -122,48 +62,10 @@ constexpr int kOffScale = kOffP + kPBytes;                  // {rs, -cs} bf16x2 
 constexpr int kOffXch = kOffScale + 2 * kScaleBufs * 2 * 128 * 4;
 constexpr int kOffStg = kOffXch + 2 * 4 * 2 * 128 * 4;      // exchange: [2 tile parities][max, sum, sez, sy][2 halves][128]
 constexpr int kStgBytes = 32 * 32 * 2;                      // dX staging of one epilogue warp: [32 d][32 px] bf16, 64-byte swizzle
-constexpr int kOffPart = kOffStg + 8 * kStgBufs * kStgBytes;           // kStgBufs staging buffers per epilogue warp
+constexpr int kOffPart = kOffStg + 8 * kStgBytes;
 constexpr int kOffBars = kOffPart + 8 * 128 * 4;            // row-norm partial sums of squares [8 softmax warps][128 px]
 constexpr int kSmemBytes = kOffBars + (int)sizeof(Bars);
 static_assert(kSmemBytes <= 232448, "shared-memory budget of one SM (227 KB)");
-
-#ifdef RC_TIMING
-__device__ __forceinline__ unsigned long long globaltimer_ns() {     // one clock for both CTAs of the pair
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define RC_T0(name) const long long name = clock64()
-#define RC_TACC(idx, name) wt[idx] += clock64() - name
-#define RC_WAIT(fn, bar, par, tag) do { const long long t0_ = clock64(); fn(bar, par, tag); wt[tag] += clock64() - t0_; } while (0)
-// event trace of CTA 0 (tools/timeline_pair.py): clock of event `id` of tile-pair iteration `iter` in [40, 44)
-#define RC_EV(iter, id) do { if (prm.dbg != nullptr && blockIdx.x < 2 && lane == 0 && (iter) >= 40u && (iter) < 44u) \
-    prm.dbg[256 + blockIdx.x * 192 + ((iter) - 40u) * 48 + (id)] = (long long)globaltimer_ns(); } while (0)
-#else
-#define RC_T0(name)
-#define RC_TACC(idx, name)
-#define RC_WAIT(fn, bar, par, tag) fn(bar, par, tag)
-#define RC_EV(iter, id)
-#endif
-
-// Measured, not adopted (RC_ROLE_WAIT): a whole role (eight warps) waits for one mbarrier phase with ONE polling warp and
-// the others blocked in a named barrier.  A polling warp spends ~12 issue slots per probe and the epilogue's probes are
-// a quarter of all instructions the SM issues (ncu source view), yet coupling the epilogue warps costs more than the
-// probes (2.65 ms against 2.52 ms) and coupling the softmax warps is within noise (2.49 against 2.52 ms).
-#ifndef RC_ROLE_WAIT
-#define RC_ROLE_WAIT 0      // bit 0: epilogue warps, bit 1: softmax warps
-#endif
-#define ROLE_WAIT_ON(poller, bar, par, tag, bar_id) do { if (poller) RC_WAIT(mbar_wait, bar, par, tag); named_bar_sync(bar_id, 256); } while (0)
-#if RC_ROLE_WAIT & 1
-#define ROLE_WAIT_EPI ROLE_WAIT_ON
-#else
-#define ROLE_WAIT_EPI(poller, bar, par, tag, bar_id) RC_WAIT(mbar_wait, bar, par, tag)
-#endif
-#if RC_ROLE_WAIT & 2
-#define ROLE_WAIT_SMX ROLE_WAIT_ON
-#else
-#define ROLE_WAIT_SMX(poller, bar, par, tag, bar_id) RC_WAIT(mbar_wait, bar, par, tag)
-#endif
 
 struct Params {
   long long* dbg;
@@ -174,7 +76,6 @@ struct Params {
   int ablate;               // bring-up only (RANGECLIP_B200_ABLATE): 1 no epilogue x loads, 2 no dX stores, 64 no row-norm reads, 128 no dX staging, 256 no text reloads
   int store_g;              // 1: also write G = rs (P - sum onehot) (bf16 [B][HW][Kp]) for the dText GEMM
   int wide;                 // 1: rows of X / dX are 32-byte aligned (256-bit global accesses allowed)
-  int split_c, split_b;     // bring-up (RANGECLIP_B200_SPLIT="c,b"): S chunks / dX blocks issued in the first half of an iteration; -1 = default
   const __nv_bfloat16* x;
   __nv_bfloat16* dx;
   const float* inv_norm;
@@ -211,29 +112,9 @@ __device__ __forceinline__ int div_tiles(const Params& prm, int tile) {
   return q;
 }
 
-__device__ __forceinline__ float fast_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
-// r[i] for a per-thread dynamic i (registers cannot be indexed dynamically): binary select tree
-__device__ __forceinline__ float select32(const uint32_t (&r)[32], int i) {
-  float a[16];
-#pragma unroll
-  for (int j = 0; j < 16; ++j) a[j] = __uint_as_float((i & 1) ? r[2 * j + 1] : r[2 * j]);
-#pragma unroll
-  for (int j = 0; j < 8; ++j) a[j] = (i & 2) ? a[2 * j + 1] : a[2 * j];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) a[j] = (i & 4) ? a[2 * j + 1] : a[2 * j];
-#pragma unroll
-  for (int j = 0; j < 2; ++j) a[j] = (i & 8) ? a[2 * j + 1] : a[2 * j];
-  return (i & 16) ? a[1] : a[0];
-}
-
-// 16 pixels (32 bytes) of one channel row, straight from / to global memory.  `n8` = number of valid
+// 16 pixels (32 bytes) of one channel row, straight from global memory.  `n8` = number of valid
 // 8-pixel groups (0, 1 or 2); the 256-bit form needs 32-byte alignment (`wide`).
-__device__ __forceinline__ void ldg_px16(const __nv_bfloat16* p, bool wide, int n8, uint32_t* r, uint64_t pol = 0) {
+__device__ __forceinline__ void ldg_px16(const __nv_bfloat16* p, bool wide, int n8, uint32_t* r, uint64_t pol) {
   if (wide && n8 == 2 && pol != 0) {
     asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8], %9;"
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
@@ -251,29 +132,6 @@ __device__ __forceinline__ void ldg_px16(const __nv_bfloat16* p, bool wide, int 
     }
   }
 }
-__device__ __forceinline__ void stg_px16(__nv_bfloat16* p, bool wide, int n8, const uint32_t* r) {
-  if (wide && n8 == 2) {
-    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]),
-                 "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-                 : "memory");
-  } else {
-#pragma unroll
-    for (int g = 0; g < 2; ++g)
-      if (g < n8) reinterpret_cast<uint4*>(p)[g] = make_uint4(r[g * 4], r[g * 4 + 1], r[g * 4 + 2], r[g * 4 + 3]);
-  }
-}
-
-__device__ __forceinline__ float select16(const uint32_t (&r)[16], int i) {
-  float a[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) a[j] = __uint_as_float((i & 1) ? r[2 * j + 1] : r[2 * j]);
-#pragma unroll
-  for (int j = 0; j < 4; ++j) a[j] = (i & 2) ? a[2 * j + 1] : a[2 * j];
-#pragma unroll
-  for (int j = 0; j < 2; ++j) a[j] = (i & 4) ? a[2 * j + 1] : a[2 * j];
-  return (i & 8) ? a[1] : a[0];
-}
-
 // tile -> (image, first pixel); tiles past the end map to image index B, which is out of bounds for every
 // tensor map (TMA loads return zeros)
 __device__ __forceinline__ void tile_coords(const Params& prm, int tile, int& b, int& px0) {
@@ -301,13 +159,8 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
   extern __shared__ __align__(1024) uint8_t smem[];
   Bars* bars = reinterpret_cast<Bars*>(smem + kOffBars);
   uint32_t* sc_s = reinterpret_cast<uint32_t*>(smem + kOffScale);   // -cs as bf16x2 of a pixel PAIR: [kScaleBufs tiles][2 owner CTAs][64 pairs]
-  // `warp` is the ROLE index (0-3 control, 4-11 softmax, 12-19 epilogue); with RC_PAIR_CTL_HIGH the control roles run on the
-  // hardware warps 16-19 (the TMEM lane quarter of a softmax / epilogue warp, warp & 3, is the same either way)
   const int lane = threadIdx.x & 31;
-  const int pwarp = (int)(threadIdx.x >> 5);
-  const int warp = RC_PAIR_CTL_HIGH == 1 ? (pwarp + 4) % (kThreads / 32)
-                 : RC_PAIR_CTL_HIGH == 2 ? (pwarp < 4 ? pwarp : (pwarp < 12 ? pwarp + 8 : pwarp - 8)) : pwarp;
-  const int rtid = warp * 32 + lane;          // thread index in role order
+  const int warp = (int)(threadIdx.x >> 5);
   const uint32_t rank = cluster_ctarank();
   const bool leader_cta = rank == 0;
   const int n_dchunks = prm.D / 64;      // 64-channel chunks of the S GEMM
@@ -315,8 +168,8 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
   const int n_kchunks = prm.Kp / 64;
   // MMA issue order per tile pair: the S GEMM of the next pair is split in two and wrapped around the dX blocks of
   // this pair, so that the dX epilogue drains accumulators while the tensor pipe works on S
-  const int c_half = prm.split_c >= 0 ? min(prm.split_c, n_dchunks) : n_dchunks / 2;
-  const int b_half = prm.split_b >= 0 ? min(prm.split_b, n_blk) : (n_blk + 1) / 2;
+  const int c_half = n_dchunks / 2;
+  const int b_half = (n_blk + 1) / 2;
   const int Nh = prm.Kp / 2;             // text rows staged by each CTA
   const int n_clusters = gridDim.x / 2;
   const int cluster_id = blockIdx.x / 2;
@@ -326,8 +179,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
     if (kBwd) { tma_prefetch_desc(&map_tt); tma_prefetch_desc(&map_dx); }
     // X ring: xfull = the relays of both CTAs, xempty = MMA commit + the eight softmax warps (row norms);
     // text ring: tfull = the leader's expect_tx (bytes of both CTAs), tempty = MMA commit
-    for (int i = 0; i < kXStages; ++i) { mbar_init(&bars->xf[i], 1); mbar_init(&bars->xfull[i], 2); mbar_init(&bars->xempty[i], RC_PAIR_NORM_WARP ? 2 : 9); }
-    mbar_init(&bars->n_full[0], 1); mbar_init(&bars->n_full[1], 1); mbar_init(&bars->n_empty[0], 8); mbar_init(&bars->n_empty[1], 8);
+    for (int i = 0; i < kXStages; ++i) { mbar_init(&bars->xf[i], 1); mbar_init(&bars->xfull[i], 2); mbar_init(&bars->xempty[i], 9); }
     for (int i = 0; i < kTStages; ++i) { mbar_init(&bars->tfull[i], 1); mbar_init(&bars->tempty[i], 1); }
     // consumer releases are ONE arrival per warp (after __syncwarp), not one per thread: an mbarrier arrive is a
     // shared-memory atomic, and 512 of them per hand-off (half of them remote) cost the leader's shared-memory pipe
@@ -374,7 +226,6 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       // text ring, in MMA issue order: S(first), then per tile pair
       //   [S(next) first half] [dX(this) first blocks] [S(next) second half] [dX(this) remaining blocks]
       uint32_t it = 0;
-      const uint64_t pol_text = RC_PAIR_TEXT_HINT ? l2_policy_evict_last() : 0;
       // first candidate row of the pair's block (kb mode: both tiles of a pair lie in one block, tiles_per_img is even)
       auto koff_of = [&](int pj) -> int { return (kKB && prm.kb > 0) ? div_tiles(prm, 2 * pj) * 256 : 0; };
       auto load_s = [&](int c_begin, int c_end, int koff) {
@@ -386,8 +237,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
             continue;
           }
           if (leader_cta) mbar_arrive_expect_tx(&bars->tfull[st], 2 * Nh * 128);
-          if (RC_PAIR_TEXT_HINT) tma_load_2d_2sm_hint(smem + kOffT + st * kStageBytes, &map_t, &bars->tfull[st], c * 64, koff + (int)rank * Nh, pol_text);
-          else tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_t, &bars->tfull[st], c * 64, koff + (int)rank * Nh);
+          tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_t, &bars->tfull[st], c * 64, koff + (int)rank * Nh);
         }
       };
       auto load_dx = [&](int b_begin, int b_end, int koff) {
@@ -400,8 +250,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
               continue;
             }
             if (leader_cta) mbar_arrive_expect_tx(&bars->tfull[st], 2 * 16384);
-            if (RC_PAIR_TEXT_HINT) tma_load_2d_2sm_hint(smem + kOffT + st * kStageBytes, &map_tt, &bars->tfull[st], koff + kc * 64, blk * 256 + (int)rank * 128, pol_text);
-            else tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_tt, &bars->tfull[st], koff + kc * 64, blk * 256 + (int)rank * 128);
+            tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_tt, &bars->tfull[st], koff + kc * 64, blk * 256 + (int)rank * 128);
           }
       };
       if (cluster_id < prm.n_pairs) load_s(0, n_dchunks, koff_of(cluster_id));
@@ -418,7 +267,6 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       // own X chunks of every tile, as far ahead as the X ring allows (the next tile's first chunks are in flight
       // while the dX GEMM of the previous pair runs)
       uint32_t xit = 0;
-      const uint64_t pol_keep = RC_PAIR_X_HINT ? l2_policy_evict_last() : 0;
       for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters) {
         int b, px0;
         tile_coords(prm, 2 * pj + (int)rank, b, px0);
@@ -428,13 +276,8 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
           uint8_t* sb = smem + st * kStageBytes;
           mbar_arrive_expect_tx(&bars->xf[st], 2 * 8192);          // CTA-local: the softmax warps read the chunk too
           const int bx = (kKB && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;      // kb mode: the one image of X (1 = out of bounds)
-          if (RC_PAIR_X_HINT) {       // the dX epilogue reads the tile again about one and a half iterations later
-            tma_load_3d_hint(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx, pol_keep);
-            tma_load_3d_hint(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx, pol_keep);
-          } else {
-            tma_load_3d(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx);
-            tma_load_3d(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx);
-          }
+          tma_load_3d(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx);
+          tma_load_3d(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx);
         }
       }
     } else if (warp == 1 && leader_cta) {
@@ -530,44 +373,14 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
         }
       }
     }
-    else if (warp == 2 && (RC_PAIR_NORM_WARP || lane == 0)) {
+    else if (warp == 2 && lane == 0) {
       // ========== relay (both CTAs): "own X chunk has landed" (CTA-local xf) -> the leader's full barrier ==========
-      // + (RC_PAIR_NORM_WARP) the row norms 1/|x_p| (model.py:272 F.normalize) of the tile, read from the chunk where it sits in
-      // the operand ring ([64 d][2 x 64 px], 128-byte swizzle): lane = 4 consecutive pixels (8 bytes of every channel row),
-      // channel rows and chunks summed in a fixed order (bit-reproducible); the slot is released right after the read
-      uint32_t xit = 0, lt = 0;
-      float* nrm = reinterpret_cast<float*>(smem + kOffPart);          // [2 tile parities][128 px]
-      const uint8_t* lane_base = smem + (lane >> 4) * 8192 + (lane & 1) * 8;
-      const int gran = (lane & 15) >> 1;                               // 16-byte granule of the row (before the swizzle)
-      for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters, ++lt) {
-        float ss0 = 0.f, ss1 = 0.f, ss2 = 0.f, ss3 = 0.f;
+      uint32_t xit = 0;
+      for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters) {
         for (int c = 0; c < n_dchunks; ++c, ++xit) {
           const int st = xit % kXStages;
           RC_WAIT(mbar_wait, &bars->xf[st], (xit / kXStages) & 1, 14);
-          if (lane == 0) arrive_leader(&bars->xfull[st]);
-          if (RC_PAIR_NORM_WARP) {
-            const uint8_t* base = lane_base + st * kStageBytes;
-            if (!(prm.ablate & 64)) {
-#pragma unroll 8
-              for (int rowd = 0; rowd < 64; ++rowd) {
-                const uint2 v = *reinterpret_cast<const uint2*>(base + rowd * 128 + ((gran ^ (rowd & 7)) << 4));
-                ss0 = sqacc_bf16x2_lo(ss0, v.x); ss1 = sqacc_bf16x2_hi(ss1, v.x);
-                ss2 = sqacc_bf16x2_lo(ss2, v.y); ss3 = sqacc_bf16x2_hi(ss3, v.y);
-              }
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&bars->xempty[st]);
-          }
-        }
-        if (RC_PAIR_NORM_WARP) {
-          // nrm[lt & 1] was last read by the softmax warps of tile lt - 2
-          if (lt >= 2) RC_WAIT(mbar_wait, &bars->n_empty[lt & 1], ((lt >> 1) & 1) ^ 1, 13);
-          float4 o;
-          o.x = 1.f / fmaxf(sqrtf(ss0), 1e-12f); o.y = 1.f / fmaxf(sqrtf(ss1), 1e-12f);
-          o.z = 1.f / fmaxf(sqrtf(ss2), 1e-12f); o.w = 1.f / fmaxf(sqrtf(ss3), 1e-12f);
-          reinterpret_cast<float4*>(nrm + (lt & 1) * 128)[lane] = o;
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bars->n_full[lt & 1]);
+          arrive_leader(&bars->xfull[st]);
         }
       }
     }
@@ -615,7 +428,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
     // otherwise wait for its S GEMM: the X chunks are read where they sit in the operand ring ([64 d][2 x 64 px],
     // 128-byte swizzle).  thread = (8-pixel group g, row phase r); sums of squares meet in shared memory.
     float* part_s = reinterpret_cast<float*>(smem + kOffPart);   // [8 warps][128 px] partial sums of squares
-    const int st_ = rtid - 128;                                  // 0..255
+    const int st_ = threadIdx.x - 128;                           // 0..255
     const int ng = st_ & 15, nr = st_ >> 4;
     uint32_t nit = 0;
     float inv_n_next = 0.f;
@@ -625,7 +438,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       for (int j = 0; j < 8; ++j) ss[j] = 0.f;
       for (int c = 0; c < n_dchunks; ++c, ++nit) {
         const int st = nit % kXStages;
-        ROLE_WAIT_SMX(warp == 4, &bars->xf[st], (nit / kXStages) & 1, 15, 8);
+        RC_WAIT(mbar_wait, &bars->xf[st], (nit / kXStages) & 1, 15);
         const uint8_t* base = smem + st * kStageBytes + (ng >> 3) * 8192 + nr * 128;
         const int ch = ng & 7;
 #pragma unroll
@@ -656,8 +469,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       for (int wv = 0; wv < 8; ++wv) q += part_s[wv * 128 + row];
       inv_n_next = 1.f / fmaxf(sqrtf(q), 1e-12f);
     };
-    if (!RC_PAIR_NORM_WARP && cluster_id < prm.n_pairs) norm_tile();
-    const float* nrm = reinterpret_cast<const float*>(smem + kOffPart);
+    if (cluster_id < prm.n_pairs) norm_tile();
     const float inv_tau = prm.log_tau_dev != nullptr ? expf(-__ldg(prm.log_tau_dev)) : prm.inv_tau;
     const int K_valid = prm.k_dev != nullptr ? max(1, min(__ldg(prm.k_dev), prm.K)) : prm.K;      // rows past it are zero pads
     const bool use_bound = inv_tau * (2.02f * kLog2e) < 100.f;
@@ -674,7 +486,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       const bool valid = tile_ok && px < prm.HW;
       // dText mode: the bulk store of the previous tile's G must have read the P buffer before anyone rewrites it
       // (every thread passes the named barrier below before its next P store)
-      if (kBwd && prm.store_g && rtid == 128) tma_store_wait_read0();
+      if (kBwd && prm.store_g && threadIdx.x == 128) tma_store_wait_read0();
       const int64_t m = (int64_t)b * prm.HW + px;
       // candidates in this tile's block (kb mode: the last block may be short; its zero pad rows are masked like any pad)
       const int Kt = (kKB && prm.kb > 0) ? min(256, prm.K - 256 * b) : K_valid;
@@ -683,21 +495,15 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       const float wi = (R == 1 && (yi >= 0 || (kKB && prm.keep_w))) ? nx_w : 0.f;
       load_pixel_scalars(pj + n_clusters);
       float* xch = xch_base + (lt & 1) * (4 * 2 * 128);      // double-buffered: one named barrier per tile suffices
-      if (RC_PAIR_NORM_WARP) {
-        RC_WAIT(mbar_wait, &bars->n_full[lt & 1], (lt >> 1) & 1, 15);
-        inv_n_next = nrm[(lt & 1) * 128 + row];
-        __syncwarp();
-        if (elect_one()) mbar_arrive(&bars->n_empty[lt & 1]);
-      }
       const float inv_n = px_ok ? inv_n_next : 0.f;
       const float zs = inv_n * inv_tau;
       const float zl = zs * kLog2e;
       // forward-only: the tensor pipe runs one pair ahead (two S buffers), so the next tile's row norms are taken
       // first -- its X chunks are already streaming and their ring slots are refilled only after these reads
-      if (!RC_PAIR_NORM_WARP && !kBwd && pj + n_clusters < prm.n_pairs) norm_tile();
+      if (!kBwd && pj + n_clusters < prm.n_pairs) norm_tile();
       const uint32_t sidx = kBwd ? 0u : (lt & 1u);
       const uint32_t trow = trow0 + sidx * 256;
-      ROLE_WAIT_SMX(warp == 4, &bars->s_full[sidx], (kBwd ? lt : (lt >> 1)) & 1u, 8, 8);
+      RC_WAIT(mbar_wait, &bars->s_full[sidx], (kBwd ? lt : (lt >> 1)) & 1u, 8);
       tc_fence_after();
       if (warp == 4) RC_EV(lt, 10);    // S(lt) complete (seen by the softmax warps)
       RC_T0(tsm);
@@ -759,32 +565,13 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
           }
         }
       };
-      if (RC_SMX_DOUBLE_BUFFER) {
-        // the TMEM load of step c+1 is in flight while step c is computed (two 16-column register buffers)
-        uint32_t ra[16], rb[16];
-        tmem_ld_32x16(trow, ra);
 #pragma unroll
-        for (int c = 0; c < 8; c += 2) {
-          if (c * 16 < Kh) {
-            tmem_ld_wait16(ra);
-            if ((c + 1) * 16 < Kh) tmem_ld_32x16(trow + (c + 1) * 16, rb);
-            smx_step(ra, c);
-          }
-          if ((c + 1) * 16 < Kh) {
-            tmem_ld_wait16(rb);
-            if ((c + 2) * 16 < Kh) tmem_ld_32x16(trow + (c + 2) * 16, ra);
-            smx_step(rb, c + 1);
-          }
-        }
-      } else {
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          if (c * 16 < Kh) {
-            uint32_t r[16];
-            tmem_ld_32x16(trow + c * 16, r);
-            tmem_ld_wait();
-            smx_step(r, c);
-          }
+      for (int c = 0; c < 8; ++c) {
+        if (c * 16 < Kh) {
+          uint32_t r[16];
+          tmem_ld_32x16(trow + c * 16, r);
+          tmem_ld_wait();
+          smx_step(r, c);
         }
       }
       tc_fence_before();
@@ -861,7 +648,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
           if (row == 0) mbar_arrive_expect_tx(&bars->sc_full[lt & 1], 64 * 4);   // the peer's 64 st.async land here
         }
         // the dX MMAs of the previous pair have finished reading P: store this pair's P
-        ROLE_WAIT_SMX(warp == 4, &bars->p_empty, (lt & 1) ^ 1, 9, 8);
+        RC_WAIT(mbar_wait, &bars->p_empty, (lt & 1) ^ 1, 9);
         if (warp == 4) RC_EV(lt, 12);  // P buffer free
         RC_T0(tst);
         const uint32_t rs2 = pack_bf16x2(rsv, rsv);
@@ -904,94 +691,18 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
         RC_TACC(2, tst);
         if (prm.store_g) {                        // dText: the finished G tile goes to global memory as it sits in smem
           named_bar_sync(6, 256);
-          if (rtid == 128 && tile_ok) {
+          if (threadIdx.x == 128 && tile_ok) {
             const int gpx0 = px - row;
             for (int j = 0; j < n_kchunks; ++j) tma_store_3d(&map_g, smem + kOffP + j * 16384, j * 64, gpx0, b);
             tma_store_commit();
           }
         }
         if (half == 0 && valid && prm.lse && !(kKB && prm.lse_in != nullptr)) prm.lse[m] = lse;      // after the hand-off: nothing waits behind this store
-        uint32_t sxq[2][16];
-        int s_n8 = 0;
-        int64_t s_off = 0;
-        const bool smx_unit = RC_PAIR_SMX_UNIT && !(kKB && prm.acc_dx);
-        if (smx_unit) {
-          // x of unit 1 (own channel row, pixels [64,128) of the tile this warp half covers): requested now, used after the norms
-          const int t1 = 2 * pj + half;
-          if (t1 < prm.n_tiles) {
-            const int b1 = div_tiles(prm, t1);
-            const int px1 = (t1 - b1 * prm.tiles_per_img) * kTilePx + 64;
-            const int d1 = (int)rank * 128 + row;
-            s_off = ((int64_t)((kKB && prm.kb > 0) ? 0 : b1) * prm.D + d1) * prm.HW + px1;
-            const int64_t left = prm.HW - px1;
-            s_n8 = left >= 64 ? 8 : (left > 0 ? (int)(left >> 3) : 0);
-          }
-          const int slb = lane & 1;
-#pragma unroll
-          for (int c = 0; c < 2; ++c) {
-            const int n8 = min(2, max(0, s_n8 - (c * 2 + slb) * 2));
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-              ldg_px16(prm.x + s_off + (int64_t)(j - slb) * prm.HW + c * 32 + slb * 16, prm.wide != 0, n8, &sxq[c][j * 8], 0);
-          }
-        }
-        if (RC_PAIR_SMX_UNIT != 2 && !RC_PAIR_NORM_WARP && pj + n_clusters < prm.n_pairs) norm_tile();
+        if (pj + n_clusters < prm.n_pairs) norm_tile();
         if (warp == 4) RC_EV(lt, 14);  // row norms of the next tile done
-        if (smx_unit) {
-          const int slb = lane & 1;
-          const uint32_t upp = 2u * (uint32_t)n_blk;
-          const uint32_t uc1 = lt * upp + 1u;                                   // the epilogue's unit counter at (this pair, unit 1)
-          RC_WAIT(mbar_wait, &bars->sc_full[lt & 1], (lt >> 1) & 1, 10);       // -cs of both tiles (the peer's arrive by st.async)
-          const uint32_t* sc = sc_s + (lt % kScaleBufs) * 128 + half * 64;
-          RC_WAIT(mbar_wait, &bars->acc_full[1], (uc1 >> 1) & 1, 11);
-          tc_fence_after();
-          const uint32_t tacc = tmem + ((uint32_t)((warp & 3) * 32) << 16) + 256 + half * 64 + 128;     // accumulator buffer 1
-#pragma unroll
-          for (int c = 0; c < 2; ++c) {
-            uint32_t acc[32];
-            tmem_ld_32x32(tacc + c * 32, acc);
-            tmem_ld_wait();
-            if (c == 1) { tc_fence_before(); arrive_leader_warp(&bars->acc_empty[1]); }
-            {       // (row 2p+j, piece b) -> own row, pixels [c*32, +32)
-#pragma unroll
-              for (int r = 0; r < 8; ++r) {
-                const uint32_t send = slb ? sxq[c][r] : sxq[c][8 + r];
-                const uint32_t recv = __shfl_xor_sync(0xffffffffu, send, 1);
-                if (slb) sxq[c][r] = recv; else sxq[c][8 + r] = recv;
-              }
-            }
-            const uint4* scp = reinterpret_cast<const uint4*>(sc + 32 + c * 16);          // pxh = 1
-            uint32_t o[16];
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              const uint4 sv = scp[g];
-              const uint32_t cs4[4] = {sv.x, sv.y, sv.z, sv.w};
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const int i = 4 * g + j;
-                const uint32_t a = pack_bf16x2(__uint_as_float(acc[2 * i]), __uint_as_float(acc[2 * i + 1]));
-                o[i] = bf2_fma(cs4[j], sxq[c][i], a);
-              }
-            }
-            {       // own row -> (row 2p+j, piece b): 64 contiguous bytes per lane pair and row, straight to global memory
-#pragma unroll
-              for (int r = 0; r < 8; ++r) {
-                const uint32_t send = slb ? o[r] : o[8 + r];
-                const uint32_t recv = __shfl_xor_sync(0xffffffffu, send, 1);
-                if (slb) o[r] = recv; else o[8 + r] = recv;
-              }
-            }
-            const int n8 = min(2, max(0, s_n8 - (c * 2 + slb) * 2));
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-              stg_px16(prm.dx + ((kKB && prm.kb > 0) ? (int64_t)div_tiles(prm, 2 * pj + half) * prm.D * prm.HW : 0) + s_off +
-                           (int64_t)(j - slb) * prm.HW + c * 32 + slb * 16, prm.wide != 0, n8, &o[j * 8]);
-          }
-        }
-        if (RC_PAIR_SMX_UNIT == 2 && !RC_PAIR_NORM_WARP && pj + n_clusters < prm.n_pairs) norm_tile();
       }
     }
-    if (kBwd && prm.store_g && rtid == 128) tma_store_wait_all0();
+    if (kBwd && prm.store_g && threadIdx.x == 128) tma_store_wait_all0();
     if (half == 0) {
       loss_acc = warp_sum(loss_acc); w_acc = warp_sum(w_acc); dlt_acc = warp_sum(dlt_acc);
       if (lane == 0) {
@@ -1027,10 +738,8 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
         f_n8 = left >= 64 ? 8 : (left > 0 ? (int)(left >> 3) : 0);
       }
     };
-    const bool smx_unit = RC_PAIR_SMX_UNIT && !(kKB && prm.acc_dx);      // unit 1 of every pair is drained by the softmax warps
     auto cursor_next = [&]() {
       ++f_unit;
-      if (smx_unit && f_unit == 1) ++f_unit;
       if (f_unit >= units_per_pair) { f_unit = 0; f_pj += n_clusters; }
       cursor_set();
     };
@@ -1039,7 +748,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
     // covers 16 rows x 64 contiguous bytes instead of 32 rows x 32 bytes (half the L1 tag work).  A 2x2 exchange
     // inside the pair (pair_swap) turns "row 2p+j, piece b" into "own row, piece j" and back.
     const int lb = lane & 1;
-    const uint64_t pol_x = RC_EPI_X_HINT ? l2_policy_evict_first() : 0;     // last use of these X lines in this kernel
+    const uint64_t pol_x = l2_policy_evict_first();     // last use of these X lines in this kernel
     uint32_t xq[2][16];       // chunk c of the current unit; before pair_swap: [j][8] = (row 2p+j, piece b)
     auto pair_swap = [&](uint32_t* e) {
 #pragma unroll
@@ -1056,22 +765,20 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       for (int j = 0; j < 2; ++j)
         ldg_px16(prm.x + f_off + (int64_t)(j - lb) * prm.HW + c * 32 + lb * 16, wide, n8, &xq[c][j * 8], pol_x);
     };
-    uint8_t* stg0 = smem + kOffStg + (warp - 12) * kStgBufs * kStgBytes;
-    uint32_t sc_ = 0;                                    // chunks staged so far (buffer = parity)
+    uint8_t* stg = smem + kOffStg + (warp - 12) * kStgBytes;
     const uint64_t pol_first = l2_policy_evict_first();  // dX is write-once: keep it from displacing X in L2
     cursor_set();
     fetch(0); fetch(1);
     uint32_t uc = 0, lt = 0;
     for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters, ++lt) {
-      ROLE_WAIT_EPI(warp == 12, &bars->sc_full[lt & 1], (lt >> 1) & 1, 10, 7);
+      RC_WAIT(mbar_wait, &bars->sc_full[lt & 1], (lt >> 1) & 1, 10);
       const uint32_t* sc = sc_s + (lt % kScaleBufs) * 128 + half * 64;
       for (int unit = 0; unit < units_per_pair; ++unit, ++uc) {
-        if (smx_unit && unit == 1) continue;
         const int ab = uc & 1;
         const int pxh = unit & 1;
         // where this unit's output goes (same cursor arithmetic as the prefetch, one unit behind)
         const int o_b = f_b, o_px = f_px, o_d = f_d;
-        ROLE_WAIT_EPI(warp == 12, &bars->acc_full[ab], (uc >> 1) & 1, 11, 7);
+        RC_WAIT(mbar_wait, &bars->acc_full[ab], (uc >> 1) & 1, 11);
         tc_fence_after();
         if (warp == 12) RC_EV(lt, 20 + unit * 2);      // accumulator of this unit complete
         RC_T0(tep);
@@ -1103,23 +810,10 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
             }
           }
           RC_TACC(7, t7);
-          // x of the NEXT unit's chunk c: requested as soon as this chunk's x registers are free (before the staging wait
-          // and the store, not after them) -- the first use of the prefetched x is the hottest stall of the launch
-          if (RC_EPI_FETCH_EARLY) {
-            RC_T0(t6);
-            if (c == 0) cursor_next();        // both chunks of the next unit are fetched relative to the advanced cursor
-            fetch(c);
-            RC_TACC(6, t6);
-          }
           {
             // own row of the warp's [32 d][32 px] staging tile (64-byte swizzle), then one TMA store per warp
             RC_T0(t5);
-            uint8_t* stg = stg0 + (kStgBufs == 2 ? (sc_ & 1u) * kStgBytes : 0u);
-            ++sc_;
-            if (lane == 0) {                                  // the store that last used THIS buffer has read it
-              if (kStgBufs == 2) tma_store_wait_read0_keep1();
-              else tma_store_wait_read0();
-            }
+            if (lane == 0) tma_store_wait_read0();           // the previous store has read the staging buffer
             __syncwarp();
             RC_TACC(5, t5);
             RC_T0(t8);
@@ -1141,12 +835,12 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
             }
             RC_TACC(12, t12);
           }
-          if (!RC_EPI_FETCH_EARLY) {
-            RC_T0(t6);
-            if (c == 0) cursor_next();
-            fetch(c);
-            RC_TACC(6, t6);
-          }
+          // x of the NEXT unit's chunk c, into the registers this chunk has just released (both chunks of the next unit
+          // are fetched relative to the advanced cursor)
+          RC_T0(t6);
+          if (c == 0) cursor_next();
+          fetch(c);
+          RC_TACC(6, t6);
         }
         RC_TACC(2, tep);
         if (warp == 12) RC_EV(lt, 21 + unit * 2);      // unit drained and stored
@@ -1174,7 +868,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
 
 bool infonce_pair_supported(int D) { return D == 256 || D == 512; }
 
-// launch helper used by rc_infonce_bf16 (infonce_umma.cu owns argument checking, the pre-pass and text maps)
+// launch helper used by rc_infonce_bf16 (infonce.cu owns argument checking and the pre-pass)
 int launch_infonce_pair(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
                         const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
                         const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, void* g_out,
@@ -1227,10 +921,8 @@ int launch_infonce_pair(const void* xsrc, void* dx, const void* t_bf16, const vo
   prm.x = reinterpret_cast<const __nv_bfloat16*>(xsrc);
   prm.dx = reinterpret_cast<__nv_bfloat16*>(dx);
   prm.ablate = 0;
-  prm.split_c = prm.split_b = -1;
-#ifdef RC_BRINGUP      // ablation / issue-order switches of the bring-up build; the shipped library has no environment knobs
+#ifdef RC_BRINGUP      // ablation switches of the bring-up build (tools/ablate_pair.py); the shipped library has no environment knobs
   { const char* ab = getenv("RANGECLIP_B200_ABLATE"); prm.ablate = ab ? atoi(ab) : 0; }
-  if (const char* sp = getenv("RANGECLIP_B200_SPLIT")) sscanf(sp, "%d,%d", &prm.split_c, &prm.split_b);
 #endif
   prm.wide = (HW % 16 == 0) && (reinterpret_cast<uintptr_t>(xsrc) % 32 == 0) && (reinterpret_cast<uintptr_t>(dx) % 32 == 0);
   prm.inv_norm = inv_norm; prm.y = y; prm.w = w; prm.inv_tau = inv_tau; prm.grad_scale = grad_scale;

@@ -4,7 +4,6 @@
 // forward and one read of X (+ one read-modify-write of dX) for the backward.  sign(0) = 0 as
 // torch.sgn (SURVEY Q8: the nearest-upsampled decoder makes half of all differences exactly 0).
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace rc {
 
@@ -451,22 +450,12 @@ tv_bwd_direct_kernel(const T* __restrict__ x, int64_t planes, int H, int W, cons
 // a drained load pipeline): measured at 256 x 256 planes, forward 0.77 -> 0.87 of HBM with 128-row tiles (66 KB, opt-in
 // shared memory, three resident blocks), backward 0.82 -> 0.85 and fused backward 0.85 -> 0.865 with 86-row tiles
 // (48 KB); 64 KB+ tiles lose again on the backward.  Rows are balanced over the tiles of a plane (a plane is never
-// split into two large tiles and a sliver).  RANGECLIP_B200_TV_ROWS / _TV_SMEM_KB override cap and budget (bring-up).
-static int tv_tile_budget_bytes(bool vec, int dflt) {
-  int bytes = dflt;
-#ifdef RC_BRINGUP
-  if (vec) if (const char* e = getenv("RANGECLIP_B200_TV_SMEM_KB")) { const int v = atoi(e); if (v >= 8 && v <= 224) bytes = v * 1024; }
-#endif
-  return bytes;
-}
+// split into two large tiles and a sliver).
 static int tv_tile_rows(int H, int W, int halo, int elt_bytes, bool vec, bool fwd) {
   const bool big = vec && elt_bytes == 2;
-  const int budget = tv_tile_budget_bytes(vec, (big && fwd) ? 66 * 1024 + 512 : kTvSmemFloats * 4);
+  const int budget = (big && fwd) ? 66 * 1024 + 512 : kTvSmemFloats * 4;
   int r = (budget / elt_bytes) / W - halo;
-  int cap = big ? (fwd ? 128 : 94) : 32;
-#ifdef RC_BRINGUP
-  if (const char* e = getenv("RANGECLIP_B200_TV_ROWS")) { const int v = atoi(e); if (v > 0) cap = v; }
-#endif
+  const int cap = big ? (fwd ? 128 : 94) : 32;
   if (r > cap) r = cap;
   if (r > H) r = H;
   if (r >= 1) {                        // balance: same number of tiles, equal heights

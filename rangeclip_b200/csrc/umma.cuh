@@ -34,10 +34,7 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
 // try_wait suspends the thread in hardware until the phase completes or the time hint expires; with the default
 // (short) limit a waiting warp comes back every ~100 cycles and its polling loop steals issue slots from the
 // warps that share its scheduler.
-#ifndef RC_SUSPEND_NS
-#define RC_SUSPEND_NS 200000u
-#endif
-constexpr uint32_t kSuspendHintNs = RC_SUSPEND_NS;
+constexpr uint32_t kSuspendHintNs = 200000u;
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -131,13 +128,6 @@ __device__ __forceinline__ void tma_load_3d_2sm_hint(void* dst, const CUtensorMa
       "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;" ::"r"(
           smem_u32(dst)),
       "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "r"(c2), "l"(pol)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm_hint(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint64_t pol) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-          smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "l"(pol)
       : "memory");
 }
 __device__ __forceinline__ void tma_store_3d_hint(const CUtensorMap* m, const void* src, int c0, int c1, int c2, uint64_t pol) {
@@ -242,13 +232,6 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 // wait that also "redefines" the destination registers of an earlier, still outstanding tcgen05.ld, so that the
 // compiler cannot schedule a use of them ahead of the wait (for loads issued early to overlap with other work)
-__device__ __forceinline__ void tmem_ld_wait16(uint32_t (&r)[16]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
-                 "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-               :
-               : "memory");
-}
 __device__ __forceinline__ void tmem_ld_wait32(uint32_t (&r)[32]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;"
                : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
@@ -436,7 +419,7 @@ __device__ __forceinline__ void mma_commit_2sm(uint64_t* bar) {
 
 }  // namespace umma
 
-// ---- host: tensor-map encoding through the driver entry point (no -lcuda link dependency) ------
+// ---- host (umma.cu): tensor-map encoding through the driver entry point (no -lcuda link dependency) ------
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);

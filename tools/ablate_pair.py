@@ -37,7 +37,7 @@ if len(sys.argv) > 1 and sys.argv[1] == "child":
         e0.record(); run(); e1.record(); torch.cuda.synchronize(); ts.append(e0.elapsed_time(e1))
     print(json.dumps({"lib": os.path.basename(os.environ["RANGECLIP_B200_LIB"]), "ablate": int(os.environ.get("RANGECLIP_B200_ABLATE", 0)), "ms_min": min(ts), "ms_med": sorted(ts)[3]}))
 elif len(sys.argv) > 1 and sys.argv[1] == "ab":
-    # same-box A/B of library variants (make -C rangeclip_b200/csrc variant NAME=.. DEFS=..): python tools/ablate_pair.py ab base norm ...
+    # same-box A/B of library variants (make -C rangeclip_b200/csrc variant NAME=.. DEFS=..): python tools/ablate_pair.py ab base x ...
     names = sys.argv[2:]
     for rep in range(2):
         for n in names:
