@@ -62,18 +62,37 @@ long long* debug_timing_buffer();   // bring-up instrumentation target (rc_debug
 int launch_infonce_1cta(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
                         const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
                         const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, cudaStream_t s);
-// CTA-pair (cta_group::2) version of the fused InfoNCE kernel (infonce_umma2.cu)
+// CTA-pair (cta_group::2) versions of the fused InfoNCE kernel, D = 256 / 512: SS (infonce_umma2.cu, both dX operands in
+// shared memory) and TS (infonce_ts.cu, the softmax tile as a tensor-memory operand); infonce_pair.cuh holds what they share
 bool infonce_pair_supported(int D);
-int launch_infonce_pair(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
-                        const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
-                        const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, void* g_out,
-                        int rep, int keep_w, const float* lse_in, int kb, int acc_dx, const int32_t* k_dev,
-                        const float* log_tau_dev, cudaStream_t s);
-// same problem with the softmax tile as a tensor-memory operand (infonce_ts.cu): backward launches without dText
-int launch_infonce_ts(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
-                      const int32_t* y, const float* w, float inv_tau, const float* grad_scale, const double* w_sum_in,
-                      float* lse, double* loss_sum, double* w_sum, double* dlogtau, int rep, int keep_w, const float* lse_in,
-                      int kb, int acc_dx, cudaStream_t s);
+struct InfoncePairArgs {
+  const void* xsrc;             // bf16 X [B][D][HW] (kb > 0: one image)
+  void* dx;                     // bf16 dX [B][D][HW], null: forward only
+  const void* t_bf16;           // T [Kall][D]
+  const void* tt_bf16;          // T^T [D][Kall] (backward)
+  int B, D;
+  int64_t HW;
+  int K;
+  const int32_t* y;
+  const float* w;
+  float inv_tau;
+  const float* grad_scale;
+  const double* w_sum_in;
+  float* lse;
+  double* loss_sum;
+  double* w_sum;
+  double* dlogtau;
+  int rep;                      // targets per row: 1, or 4 (the shared 2x2 form)
+  int keep_w, acc_dx, kb;       // K-blocked launches (see cta_pair::Tiling)
+  const float* lse_in;
+  // SS only
+  void* g_out;                  // dText: G = rs (P - sum onehot), bf16 [B][HW][Kp]
+  const int32_t* k_dev;         // rc_infonce_bf16_dyn: valid candidate rows and log tau in device memory
+  const float* log_tau_dev;
+};
+int launch_infonce_pair(const InfoncePairArgs& a, cudaStream_t s);
+// backward launches without dText, device-side K or device-side tau
+int launch_infonce_ts(const InfoncePairArgs& a, cudaStream_t s);
 // dText = G^T X on the tensor cores (infonce_dt_umma.cu); G is the bf16 [B][HW][Kp] tensor the pair kernel writes
 int launch_infonce_dt(const void* g, const void* xsrc, int B, int D, int64_t HW, int K, float* dt, cudaStream_t s);
 

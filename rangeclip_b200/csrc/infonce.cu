@@ -313,26 +313,23 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   if ((rcode = infonce_prepass_impl(x, x_dtype, B, D, HW, workspace, workspace_bytes, skip_prepass ? (cudaStream_t)-1 : s,
                                     &inv_norm, &xb))) return rcode;
   const void* xsrc = (x_dtype == RC_F32) ? (const void*)xb : x;
-
+  if (!use_pair)
+    return launch_infonce_1cta(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
+                               loss_sum, w_sum, dlogtau, s);
+  InfoncePairArgs a{xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, y, w, inv_tau, grad_scale, w_sum_in, lse, loss_sum, w_sum, dlogtau,
+                    rep, keep_w, acc_dx, /*kb*/ 0, lse_in, /*g_out*/ nullptr, k_dev, log_tau_dev};
   if (dt != nullptr) {
     // dText: the pair kernel also writes G = rs (P - sum onehot) (bf16 [B][HW][Kp]) into the workspace, then one
     // split-K GEMM over the pixels (infonce_dt_umma.cu) adds G^T X to dt.
     const int64_t base = rc_infonce_workspace_bytes(B, D, HW, K, x_dtype);
     uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
-    void* g = ws + ((base + 255) / 256) * 256;
-    if ((rcode = launch_infonce_pair(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
-                                     loss_sum, w_sum, dlogtau, g, rep, 0, nullptr, 0, 0, k_dev, log_tau_dev, s))) return rcode;
-    return launch_infonce_dt(g, xsrc, B, D, HW, K, dt, s);
+    a.g_out = ws + ((base + 255) / 256) * 256;
+    if ((rcode = launch_infonce_pair(a, s))) return rcode;
+    return launch_infonce_dt(a.g_out, xsrc, B, D, HW, K, dt, s);
   }
-  if (!use_pair)
-    return launch_infonce_1cta(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
-                               loss_sum, w_sum, dlogtau, s);
   // backward launches: the softmax tile as a tensor-memory operand of the dX GEMM (infonce_ts.cu) unless RC_INFONCE_SS_KERNEL
-  if (bwd && !(flags & RC_INFONCE_SS_KERNEL) && k_dev == nullptr && log_tau_dev == nullptr)
-    return launch_infonce_ts(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, y, w, inv_tau, grad_scale, w_sum_in, lse, loss_sum, w_sum,
-                             dlogtau, rep, keep_w, lse_in, 0, acc_dx, s);
-  return launch_infonce_pair(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
-                             loss_sum, w_sum, dlogtau, nullptr, rep, keep_w, lse_in, 0, acc_dx, k_dev, log_tau_dev, s);
+  if (bwd && !(flags & RC_INFONCE_SS_KERNEL) && k_dev == nullptr && log_tau_dev == nullptr) return launch_infonce_ts(a, s);
+  return launch_infonce_pair(a, s);
 }
 
 extern "C" int rc_infonce_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16,
@@ -387,9 +384,10 @@ extern "C" int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, i
   if ((rcode = infonce_prepass_impl(x, x_dtype, 1, D, HW, workspace, workspace_bytes, skip_prepass ? (cudaStream_t)-1 : s, &inv_norm, &xb))) return rcode;
   const void* xsrc = (x_dtype == RC_F32) ? (const void*)xb : x;
   const float* lse_in = (flags & RC_INFONCE_LSE_GIVEN) ? lse : nullptr;
-  if (bwd && !(flags & RC_INFONCE_SS_KERNEL))
-    return launch_infonce_ts(xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, y_rel, w_rep, inv_tau, grad_scale, w_sum_in,
-                             lse, loss_sum, w_sum, dlogtau, 1, 1, lse_in, n_blocks, 0, s);
-  return launch_infonce_pair(xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, inv_norm, y_rel, w_rep, inv_tau, grad_scale,
-                             w_sum_in, lse, loss_sum, w_sum, dlogtau, nullptr, 1, 1, lse_in, n_blocks, 0, nullptr, nullptr, s);
+  // the kb blocks of 256 candidate rows are the "images" of one launch; every target keeps its weight
+  const InfoncePairArgs a{xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, y_rel, w_rep, inv_tau, grad_scale,
+                          w_sum_in, lse, loss_sum, w_sum, dlogtau, /*rep*/ 1, /*keep_w*/ 1, /*acc_dx*/ 0, /*kb*/ n_blocks, lse_in,
+                          nullptr, nullptr, nullptr};
+  if (bwd && !(flags & RC_INFONCE_SS_KERNEL)) return launch_infonce_ts(a, s);
+  return launch_infonce_pair(a, s);
 }

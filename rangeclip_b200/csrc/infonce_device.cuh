@@ -39,11 +39,16 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {     // one cloc
 // %globaltimer of event `id` of tile-pair iteration `iter` in [40, 44)
 #define RC_EV(iter, id) do { if (prm.dbg != nullptr && blockIdx.x < 2 && lane == 0 && (iter) >= 40u && (iter) < 44u) \
     prm.dbg[256 + blockIdx.x * 192 + ((iter) - 40u) * 48 + (id)] = (long long)globaltimer_ns(); } while (0)
+// a device function with RC_WAIT inside takes the caller's counters: f(... RC_WT_PARAM) called as f(... RC_WT)
+#define RC_WT_PARAM , long long (&wt)[16]
+#define RC_WT , wt
 #else
 #define RC_T0(name)
 #define RC_TACC(idx, name)
 #define RC_WAIT(fn, bar, par, tag) fn(bar, par, tag)
 #define RC_EV(iter, id)
+#define RC_WT_PARAM
+#define RC_WT
 #endif
 
 }  // namespace rc

@@ -1,7 +1,10 @@
-// K1/K2 with the softmax tile as a TENSOR-MEMORY operand (TS-mode tcgen05.mma) and TWO tile pairs in flight per CTA pair.
+// K1/K2 with the softmax tile as a TENSOR-MEMORY operand (TS-mode tcgen05.mma) and TWO tile pairs in flight per CTA pair:
+// the fused pixel-text InfoNCE forward + backward (model.py:272-291 and its autograd) for backward launches without dText.
+// The tiling, the operand producers, the relay and the softmax arithmetic are shared with the SS kernel
+// (infonce_umma2.cu) through infonce_pair.cuh, so that both give bit-identical dX and lse.  This file holds the TS
+// pipeline (MMA issue order, tensor-memory slots), the P store into tensor memory and the dX epilogue.
 //
-// Same problem as infonce_umma2.cu (fused pixel-text InfoNCE forward + backward, model.py:272-291 and its autograd).
-// That kernel computes dX^T = T^T P^T with both operands in shared memory (SS mode) and keeps ONE S accumulator: the tensor
+// The SS kernel computes dX^T = T^T P^T with both operands in shared memory and keeps ONE S accumulator: the tensor
 // pipe, the softmax warps and the dX epilogue wait for one another in a chain S(i) -> exp(i) -> P(i) -> dX(i), and the SS
 // operand reads (96-128 B/clk) saturate the 128 B/clk shared-memory pipe.  Here
 //   S  = X^T T^T    M = 256 px (128 per CTA; A = own X chunk [64 d][128 px], MN-major, shared memory), N = Kp,
@@ -14,27 +17,23 @@
 // Tensor memory holds TWO slots (2 x 256 columns); tile pairs alternate between them.  MMA issue order
 //   S(0) | dX(0)[0,2) S(1) dX(0)[2,n) | dX(1)[0,2) S(2) dX(1)[2,n) | ...      ([a,b): 64-channel blocks of dX)
 // so the exp pass of pair j+1 runs while the tensor pipe works on dX(j) of the OTHER slot, and the dX epilogue drains the
-// first two blocks of dX(j) while S(j+1) is computed: no role waits for a hand-off it has just produced.  Pixels stay on the TMEM lanes for both GEMMs, so a CTA's softmax and dX epilogue work on
-// its own tile only (no row-scale exchange between the CTAs).  The dX epilogue thread owns a pixel: 32 channels per step
-// come out of TMEM, the x values of the same [32 ch][32 px] box arrive by TMA in a small per-warp ring (the box doubles as
-// the staging tile of the TMA store), dx = acc - cs x is formed in place and the box goes back with one TMA store.
-// The row norms 1/|x_p| (model.py:272 F.normalize) are computed by the relay warp from the X chunks in the operand ring.
-#include "common.cuh"
-#include "umma.cuh"
-#include "infonce_device.cuh"
-#include <float.h>
-#include <stdlib.h>
+// first two blocks of dX(j) while S(j+1) is computed: no role waits for a hand-off it has just produced.  Pixels stay on
+// the TMEM lanes for both GEMMs, so a CTA's softmax and dX epilogue work on its own tile only (no row-scale exchange
+// between the CTAs).  The dX epilogue thread owns a pixel: 32 channels per step come out of TMEM, the x values of the same
+// [32 ch][32 px] box arrive by TMA in a small per-warp ring (the box doubles as the staging tile of the TMA store),
+// dx = acc - cs x is formed in place and the box goes back with one TMA store.  The row norms 1/|x_p| are computed by the
+// softmax warps from the X chunks in the operand ring.
+#include "infonce_pair.cuh"
 
 namespace rc {
 using namespace umma;
 
 namespace ts {
+using namespace cta_pair;
 
-constexpr int kTilePx = 128;
-constexpr int kThreads = 640;          // warps: 0 text TMA, 1 MMA (leader CTA), 2 relay + row norms + TMEM alloc, 3 X TMA, 4-11 softmax, 12-19 dX epilogue
+constexpr int kThreads = 640;          // warps: 0 text TMA, 1 MMA (leader CTA), 2 relay + TMEM alloc, 3 X TMA, 4-11 softmax, 12-19 dX epilogue
 constexpr int kXStages = 6;            // X ring: own X chunks [64 d][128 px]; deep, so that most of the next tile is resident early
 constexpr int kTStages = 3;            // text ring: text half-chunks [Kp/2][64 d] for S, own T^T rows [32 ch][Kp] of a dX block
-constexpr int kStageBytes = 16 * 1024;
 constexpr int kEpiBufs = 4;            // per epilogue warp: ring of [32 ch][32 px] bf16 boxes (x in, dX out)
 constexpr int kEpiAhead = 2;           // x boxes requested this many steps ahead
 constexpr int kEpiBufBytes = 2048;
@@ -66,44 +65,8 @@ constexpr int kOffBars = kOffAcc + 3 * 128 * 4;                       // per-pix
 constexpr int kSmemBytes = kOffBars + (int)sizeof(Bars);
 static_assert(kSmemBytes <= 232448, "shared-memory budget of one SM (227 KB)");
 
-struct Params {
-  long long* dbg;           // timing build: per-role wait cycles and the event trace (tools/timing_ts.py)
-  int ablate;               // bring-up only (RANGECLIP_B200_ABLATE): 1 no epilogue x loads, 2 no dX stores, 256 no text reloads
-  int B, D, K, Kp;
-  int64_t HW;
-  int tiles_per_img, n_tiles, n_pairs;
-  uint32_t tpi_magic;       // floor(2^32 / tiles_per_img)
-  int keep_w;               // K-blocked launches, see infonce_umma2.cu
-  int acc_dx;               // dX += this launch's gradient (TMA reduce-add store)
-  const float* lse_in;
-  int kb;
-  const int32_t* y;
-  const float* w;
-  float inv_tau;
-  const float* grad_scale;
-  const double* w_sum_in;
-  float* lse;
-  double* loss_sum;
-  double* w_sum;
-  double* dlogtau;
-};
-
-__device__ __forceinline__ int div_tiles(const Params& prm, int tile) {
-  int q = (int)__umulhi((uint32_t)tile, prm.tpi_magic);
-  if (tile - q * prm.tiles_per_img >= prm.tiles_per_img) ++q;
-  return q;
-}
-
-// tile -> (image, first pixel); tiles past the end map to image index B (out of bounds for every tensor map)
-__device__ __forceinline__ void tile_coords(const Params& prm, int tile, int& b, int& px0) {
-  if (tile < prm.n_tiles) {
-    b = div_tiles(prm, tile);
-    px0 = (tile - b * prm.tiles_per_img) * kTilePx;
-  } else {
-    b = prm.B;
-    px0 = 0;
-  }
-}
+// bring-up ablation bits (Tiling::ablate): 1 no epilogue x loads, 2 no dX stores, 256 no text reloads
+struct Params : Tiling {};
 
 // R = targets per embedding row (1, or 4 for the shared 2x2 form); kKB: K-blocked launches (keep_w / lse_in / kb)
 template <int R, bool kKB>
@@ -123,7 +86,6 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
   const int n_dchunks = prm.D / 64;      // 64-channel chunks of the S GEMM
   const int n_blk = prm.D / 64;          // 64-channel blocks of the dX GEMM
   const int n_kchunks = prm.Kp / 64;
-  const int Nh = prm.Kp / 2;             // text rows staged by each CTA
   const int n_clusters = gridDim.x / 2;
   const int cluster_id = blockIdx.x / 2;
   const int my_pairs = cluster_id < prm.n_pairs ? (prm.n_pairs - cluster_id + n_clusters - 1) / n_clusters : 0;
@@ -156,17 +118,8 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
 #endif
   const uint32_t idesc_s = make_idesc_bf16(256, prm.Kp, /*A MN-major*/ 1, /*B K-major*/ 0);
   const uint32_t idesc_d = make_idesc_bf16(256, kAccCols, 0, 0);
-  auto arrive_leader = [&](uint64_t* bar) {
-    if (leader_cta) mbar_arrive(bar);
-    else mbar_arrive_remote(map_to_cta(bar, 0));
-  };
-  auto arrive_leader_warp = [&](uint64_t* bar) {
-    __syncwarp();
-    if (elect_one()) arrive_leader(bar);
-  };
   // l-th tile pair of this cluster
   auto pair_of = [&](int l) -> int { return cluster_id + l * n_clusters; };
-  auto koff_of = [&](int pj) -> int { return (kKB && prm.kb > 0) ? div_tiles(prm, 2 * pj) * 256 : 0; };
 
   if (warp < 4) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsCtl));
@@ -175,20 +128,11 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       // ring order == MMA issue order: S(0) | dX(0)[0,2) S(1) dX(0)[2,n) | dX(1)[0,2) S(2) dX(1)[2,n) | ...
       uint32_t it = 0;
       auto load_s = [&](int l) {
-        const int koff = koff_of(pair_of(l));
-        for (int c = 0; c < n_dchunks; ++c, ++it) {   // own half (Nh rows) of text chunk c
-          const int st = it % kTStages;
-          RC_WAIT(mbar_wait, &bars->tempty[st], ((it / kTStages) & 1) ^ 1, 1);
-          if ((prm.ablate & 256) && it >= (uint32_t)kTStages) {      // bring-up: no text traffic after the first ring pass (stale operands)
-            if (leader_cta) mbar_arrive(&bars->tfull[st]);
-            continue;
-          }
-          if (leader_cta) mbar_arrive_expect_tx(&bars->tfull[st], 2 * Nh * 128);
-          tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_t, &bars->tfull[st], c * 64, koff + (int)rank * Nh);
-        }
+        load_text_s<kTStages>(prm, &map_t, smem + kOffT, bars->tfull, bars->tempty, it, 0, n_dchunks,
+                              text_row0<kKB>(prm, pair_of(l)), rank RC_WT);
       };
       auto load_dx = [&](int l, int b0, int b1) {     // per 64-channel block: own 32 rows of T^T, all Kp columns (4 KB per 64 k)
-        const int koff = koff_of(pair_of(l));
+        const int koff = text_row0<kKB>(prm, pair_of(l));
         for (int blk = b0; blk < b1; ++blk, ++it) {
           const int st = it % kTStages;
           RC_WAIT(mbar_wait, &bars->tempty[st], ((it / kTStages) & 1) ^ 1, 2);
@@ -215,19 +159,9 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       // between the L2 sees about 2 x 74 clusters x 256 KB of other X and as much dX written.  These loads mark the lines
       // evict_last and the epilogue's (last) load marks them evict_first, so that kept lines are released once consumed.
       const uint64_t pol_keep = l2_policy_evict_last();
-      for (int l = 0; l < my_pairs; ++l) {
-        int b, px0;
-        tile_coords(prm, 2 * pair_of(l) + (int)rank, b, px0);
-        for (int c = 0; c < n_dchunks; ++c, ++xit) {
-          const int st = xit % kXStages;
-          RC_WAIT(mbar_wait, &bars->xempty[st], ((xit / kXStages) & 1) ^ 1, 3);
-          uint8_t* sb = smem + st * kStageBytes;
-          mbar_arrive_expect_tx(&bars->xf[st], 2 * 8192);          // CTA-local: the row-norm warp reads the chunk too
-          const int bx = (kKB && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;      // kb mode: the one image of X (1 = out of bounds)
-          tma_load_3d_hint(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx, pol_keep);
-          tma_load_3d_hint(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx, pol_keep);
-        }
-      }
+      for (int l = 0; l < my_pairs; ++l)
+        load_x_tile<kXStages, kKB, true>(prm, &map_x_s, smem, bars->xf, bars->xempty, xit, 2 * pair_of(l) + (int)rank, n_dchunks,
+                                         pol_keep, 3 RC_WT);
     } else if (warp == 1 && leader_cta) {
       // =============================== MMA issuer (leader CTA) ================================
       // whole warp converged (addresses / descriptors in uniform registers), one elected lane issues
@@ -310,12 +244,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     } else if (warp == 2 && lane == 0) {
       // ========== relay (both CTAs): "own X chunk has landed" (CTA-local xf) -> the leader's full barrier ==========
       uint32_t xit = 0;
-      for (int l = 0; l < my_pairs; ++l)
-        for (int c = 0; c < n_dchunks; ++c, ++xit) {
-          const int st = xit % kXStages;
-          mbar_wait(&bars->xf[st], (xit / kXStages) & 1, 10);
-          arrive_leader(&bars->xfull[st]);
-        }
+      for (int l = 0; l < my_pairs; ++l) relay_x_tile<kXStages, false>(n_dchunks, bars->xf, bars->xfull, xit, leader_cta, 10 RC_WT);
     }
   } else if (warp < 12) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsSoftmax));
@@ -330,78 +259,18 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     // pass (96 registers at compile time)
     float* acc_s = reinterpret_cast<float*>(smem + kOffAcc) + row;
     if (half == 0) acc_s[0] = acc_s[128] = acc_s[256] = 0.f;
-    float coefb;               // d loss / d (mean) = grad_scale / sum of weights
-    {
-      const double ws = prm.w_sum_in[0];
-      coefb = (prm.grad_scale ? prm.grad_scale[0] : 1.f) * (ws > 0.0 ? (float)(1.0 / ws) : 0.f);
-    }
-    float nx_ok = 0.f, nx_w = 0.f;
-    int nx_y = -1;
-    auto load_pixel_scalars = [&](int l) {
-      nx_ok = 0.f; nx_w = 0.f; nx_y = -1;
-      if (l >= my_pairs) return;
-      const int t = 2 * pair_of(l) + (int)rank;
-      if (t < prm.n_tiles) {
-        const int tb = div_tiles(prm, t);
-        const int tpx = (t - tb * prm.tiles_per_img) * kTilePx + row;
-        if (tpx < prm.HW) {
-          const int64_t tm = (int64_t)tb * prm.HW + tpx;
-          nx_ok = 1.f;
-          if (R == 1) {
-            nx_y = __ldg(prm.y + tm);
-            nx_w = __ldg(prm.w + tm);
-          } else {               // four targets, 8 bits each (K <= 256)
-            const int4 y4 = __ldg(reinterpret_cast<const int4*>(prm.y) + tm);
-            nx_y = (y4.x & 255) | ((y4.y & 255) << 8) | ((y4.z & 255) << 16) | ((y4.w & 255) << 24);
-          }
-        }
-      }
-    };
-    load_pixel_scalars(0);
-    // Row norms 1/|x_p| (model.py:272 F.normalize) of a tile from its X chunks where they sit in the operand ring
-    // ([64 d][2 x 64 px], 128-byte swizzle): thread = (8-pixel group, row phase); sums of squares meet in shared memory.
-    // The X ring holds most of a tile, so the chunks are normally resident when this runs (right before the tile's exp pass).
-    float* part_s = reinterpret_cast<float*>(smem + kOffPart);   // [8 warps][128 px] partial sums of squares
-    const int st_ = threadIdx.x - 128;                           // 0..255
-    const int ng = st_ & 15, nr = st_ >> 4;
+    float gscale, inv_wsum;
+    grad_scales(prm, gscale, inv_wsum);
+    const float coefb = gscale * inv_wsum;
+    float nx_ok, nx_w;         // pixel scalars of the next tile
+    int nx_y;
+    load_pixel_scalars<R>(prm, 0 < my_pairs, 2 * pair_of(0) + (int)rank, row, nx_ok, nx_w, nx_y);
+    // Row norms: the X ring holds most of a tile, so its chunks are normally resident when they are taken, right before
+    // the tile's exp pass.
+    float* part_s = reinterpret_cast<float*>(smem + kOffPart);
+    int ng, nr;
+    norm_coords(ng, nr);
     uint32_t nit = 0;
-    auto norm_tile = [&]() -> float {
-      float ss[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) ss[j] = 0.f;
-      for (int c = 0; c < n_dchunks; ++c, ++nit) {
-        const int st = nit % kXStages;
-        RC_WAIT(mbar_wait, &bars->xf[st], (nit / kXStages) & 1, 11);
-        const uint8_t* base = smem + st * kStageBytes + (ng >> 3) * 8192 + nr * 128;
-        const int ch = ng & 7;
-#pragma unroll
-        for (int rr = 0; rr < 4; ++rr) {
-          const int rowd = nr + rr * 16;
-          const uint4 v = *reinterpret_cast<const uint4*>(base + rr * 2048 + ((ch ^ (rowd & 7)) << 4));
-          const uint32_t u[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {       // FHFMA.BF16 on the word's halves: no unpack instructions
-            ss[2 * j] = sqacc_bf16x2_lo(ss[2 * j], u[j]);
-            ss[2 * j + 1] = sqacc_bf16x2_hi(ss[2 * j + 1], u[j]);
-          }
-        }
-        __syncwarp();
-        if (elect_one()) mbar_arrive(&bars->xempty[st]);
-      }
-      // fixed-order reduction (bit-reproducible): lane pairs, then the eight warps' partials through shared memory
-#pragma unroll
-      for (int j = 0; j < 8; ++j) ss[j] += __shfl_xor_sync(0xffffffffu, ss[j], 16);
-      if (lane < 16) {
-        float4* dst = reinterpret_cast<float4*>(part_s + (warp - 4) * 128 + ng * 8);
-        dst[0] = make_float4(ss[0], ss[1], ss[2], ss[3]);
-        dst[1] = make_float4(ss[4], ss[5], ss[6], ss[7]);
-      }
-      named_bar_sync(5, 256);
-      float q = 0.f;
-#pragma unroll
-      for (int wv = 0; wv < 8; ++wv) q += part_s[wv * 128 + row];
-      return 1.f / fmaxf(sqrtf(q), 1e-12f);
-    };
     const bool use_bound = prm.inv_tau * (2.02f * kLog2e) < 100.f;
     const float ml_bound = prm.inv_tau * (1.01f * kLog2e);
     for (int l = 0; l < my_pairs; ++l) {
@@ -413,14 +282,16 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       const bool valid = tile_ok && px < prm.HW;
       const int64_t m = (int64_t)b * prm.HW + px;
       const int Kt = (kKB && prm.kb > 0) ? min(256, prm.K - 256 * b) : prm.K;
-      const bool px_ok = nx_ok != 0.f;
+      const float ok = nx_ok;
+      const bool px_ok = ok != 0.f;
       const int yi = nx_y;
       const float wi = (R == 1 && (yi >= 0 || (kKB && prm.keep_w))) ? nx_w : 0.f;
-      load_pixel_scalars(l + 1);
+      load_pixel_scalars<R>(prm, l + 1 < my_pairs, 2 * pair_of(l + 1) + (int)rank, row, nx_ok, nx_w, nx_y);
       float* xch = xch_base + (l & 1) * (4 * 2 * 128);
       const uint32_t trow = lane_base + sl * kSlotCols + cb;
       RC_T0(tnorm);
-      const float inv_n_tile = norm_tile();
+      const float inv_n_tile = norm_tile<kXStages>(smem, bars->xf, bars->xempty, nit, n_dchunks, part_s, warp, lane, row, ng, nr, false,
+                                                   11 RC_WT);
       RC_TACC(1, tnorm);
       if (warp == 4) RC_EV(l, 12);      // row norms of the tile done
       const float inv_n = px_ok ? inv_n_tile : 0.f;
@@ -430,95 +301,17 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       tc_fence_after();
       if (warp == 4) RC_EV(l, 13);      // S(l) complete (seen by the softmax warps)
       RC_T0(texp);
-      float ml = ml_bound;
-      if (!use_bound) {
-        float mx = -FLT_MAX;
-        for (int c = 0; c * 32 < Kh; ++c) {
-          const int nvalid = Kt - (cb + c * 32);
-          if (nvalid <= 0) break;
-          uint32_t r[32];
-          tmem_ld_32x32(trow + c * 32, r);
-          tmem_ld_wait();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) if (i < nvalid) mx = fmaxf(mx, __uint_as_float(r[i]));
-        }
-        xch[(0 * 2 + half) * 128 + row] = mx;
-        named_bar_sync(3, 256);
-        mx = fmaxf(mx, xch[(0 * 2 + (half ^ 1)) * 128 + row]);
-        ml = mx * zl;
-      }
+      const float ml = use_bound ? ml_bound : row_max(trow, Kt, cb, Kh, xch, half, row, zl);
       uint32_t pk[64];
-      float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f, q0 = 0.f, q1 = 0.f, q2 = 0.f, q3 = 0.f;
       float sy[R];
-#pragma unroll
-      for (int j = 0; j < R; ++j) sy[j] = 0.f;
-#pragma unroll
-      for (int c = 0; c < 8; ++c) {
-        if (c * 16 < Kh) {
-          uint32_t r[16];
-          tmem_ld_32x16(trow + c * 16, r);
-          tmem_ld_wait();
-          const int k0 = cb + c * 16;
-          const int nvalid = Kt - k0;
-#pragma unroll
-          for (int j = 0; j < R; ++j) {                          // target logit(s): once per row, not per column
-            const int yrel = (R == 1 ? yi : (int)(((uint32_t)yi >> (8 * j)) & 255u)) - k0;
-            if ((unsigned)yrel < 16u) sy[j] = select16(r, yrel);
-          }
-          if (nvalid >= 16) {
-#pragma unroll
-            for (int i = 0; i < 16; i += 4) {
-              const float a0 = __uint_as_float(r[i]), a1 = __uint_as_float(r[i + 1]);
-              const float a2 = __uint_as_float(r[i + 2]), a3 = __uint_as_float(r[i + 3]);
-              const float e0 = fast_exp2(fmaf(a0, zl, -ml)), e1 = fast_exp2(fmaf(a1, zl, -ml));
-              const float e2 = fast_exp2(fmaf(a2, zl, -ml)), e3 = fast_exp2(fmaf(a3, zl, -ml));
-              s0 += e0; s1 += e1; s2 += e2; s3 += e3;
-              q0 = fmaf(e0, a0, q0); q1 = fmaf(e1, a1, q1); q2 = fmaf(e2, a2, q2); q3 = fmaf(e3, a3, q3);
-              pk[c * 8 + (i >> 1)] = pack_bf16x2(e0, e1);
-              pk[c * 8 + (i >> 1) + 1] = pack_bf16x2(e2, e3);
-            }
-          } else {          // the step that straddles K, or padding columns only
-#pragma unroll
-            for (int i = 0; i < 16; i += 2) {
-              const float a0 = __uint_as_float(r[i]), a1 = __uint_as_float(r[i + 1]);
-              const float e0 = (i < nvalid) ? fast_exp2(fmaf(a0, zl, -ml)) : 0.f;
-              const float e1 = (i + 1 < nvalid) ? fast_exp2(fmaf(a1, zl, -ml)) : 0.f;
-              s0 += e0; s1 += e1;
-              q0 = fmaf(e0, a0, q0); q1 = fmaf(e1, a1, q1);
-              pk[c * 8 + (i >> 1)] = pack_bf16x2(e0, e1);
-            }
-          }
-        }
-      }
-      float sum = (s0 + s1) + (s2 + s3);
-      float sez = (q0 + q1) + (q2 + q3);
+      float sum, sez;
+      exp_pass<R>(trow, cb, Kh, Kt, yi, zl, ml, pk, sy, sum, sez);
       int yj[R];
       float wj[R];
-      if (R == 1) {
-        yj[0] = yi; wj[0] = wi;
-      } else {
-        int4 y4 = make_int4(-1, -1, -1, -1);
-        float4 w4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (px_ok) {
-          y4 = __ldg(reinterpret_cast<const int4*>(prm.y) + m);
-          w4 = __ldg(reinterpret_cast<const float4*>(prm.w) + m);
-        }
-        const int ya[4] = {y4.x, y4.y, y4.z, y4.w};
-        const float wa[4] = {w4.x, w4.y, w4.z, w4.w};
-#pragma unroll
-        for (int j = 0; j < R; ++j) { yj[j] = ya[j]; wj[j] = ya[j] >= 0 ? wa[j] : 0.f; }
-      }
-      float wtot = 0.f, tz = 0.f;
       bool mine[R];
-#pragma unroll
-      for (int j = 0; j < R; ++j) {
-        mine[j] = yj[j] >= cb && yj[j] < cb + Kh;
-        wtot += wj[j];
-        tz += mine[j] ? wj[j] * sy[j] : 0.f;
-      }
-      xch[(1 * 2 + half) * 128 + row] = sum;
-      xch[(2 * 2 + half) * 128 + row] = sez;
-      xch[(3 * 2 + half) * 128 + row] = tz;
+      float wtot, tz;
+      gather_targets<R>(prm, yi, wi, ok, m, cb, Kh, sy, yj, wj, mine, wtot, tz);
+      post_sums(xch, half, row, sum, sez, tz);
       // every softmax warp has read its S columns (tcgen05.wait::ld above): after this barrier the slot's columns may be
       // overwritten with P
       RC_TACC(2, texp);
@@ -529,22 +322,13 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       RC_TACC(13, txch);
       tc_fence_after();
       RC_T0(tpst);
-      sum += xch[(1 * 2 + (half ^ 1)) * 128 + row];
-      sez += xch[(2 * 2 + (half ^ 1)) * 128 + row];
-      tz += xch[(3 * 2 + (half ^ 1)) * 128 + row];
-      if (kKB && prm.lse_in != nullptr && valid) sum = fast_exp2(fmaf(__ldg(prm.lse_in + (prm.kb > 0 ? (int64_t)px : m)), kLog2e, -ml));   // 1 / sum = exp(m - lse)
-      float lse = 0.f;
-      if (half == 0) {
-        lse = (ml + __log2f(sum)) * kLn2;
-        acc_s[0] += wtot * lse - tz * zs;
-        acc_s[128] += wtot;
-      }
+      add_peer_sums(xch, half, row, sum, sez, tz);
+      const float lse = row_lse<kKB>(prm, valid, px, m, half, ml, wtot, tz, zs, sum, acc_s[0], acc_s[128]);
       const float coef = coefb * wtot;
       const float inv_sum = 1.f / sum;
-      // P is stored pre-scaled: G[p][k] = rs_p (e_pk - sum_p [k = y_p]) = d loss / d(xhat_p . that_k) / |x_p|
-      const float rsv = inv_n * prm.inv_tau * coef * inv_sum;
+      const float rsv = p_scale(inv_n, prm.inv_tau, coef, inv_sum);
       if (half == 0) {
-        const float cj = coef * sez * zs * inv_sum - coefb * tz * zs;
+        const float cj = proj_coef(coef, coefb, sez, tz, zs, inv_sum);
         sc_s[(l & (kScaleBufs - 1)) * 128 + row] = -(inv_n * inv_n * cj);      // dx = acc + (-cs) x
         acc_s[256] -= cj;
         __syncwarp();
@@ -553,7 +337,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       {
         const uint32_t prow = lane_base + sl * kSlotCols + (cb >> 1);
         const uint32_t rs2 = pack_bf16x2(rsv, rsv);
-        // G[row][y_j] = rs (e_y - sum * (weight of target y_j) / (weight of the row)), formed in fp32 before rounding
+        // the target entries of G, rounded to bf16, patched into the packed P words below
         uint32_t g16[R];
         int grel[R];
 #pragma unroll
@@ -561,16 +345,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
           grel[j] = -1;
           g16[j] = 0;
           if (mine[j]) {
-            const float ey = fast_exp2(fmaf(sy[j], zl, -ml));
-            float gv;
-            if (R == 1) {
-              gv = (ey - sum) * rsv;
-            } else {
-              float wk = 0.f;
-#pragma unroll
-              for (int i = 0; i < R; ++i) wk += (yj[i] == yj[j]) ? wj[i] : 0.f;
-              gv = (ey - sum * (wtot > 0.f ? wk / wtot : 0.f)) * rsv;
-            }
+            const float gv = target_g<R>(j, sy, yj, wj, wtot, sum, zl, ml, rsv);
             grel[j] = yj[j] - cb;
             g16[j] = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(gv));
           }
@@ -596,20 +371,13 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
         }
         tmem_st_wait();
         tc_fence_before();
-        arrive_leader_warp(&bars->p_full[sl]);
+        arrive_leader_warp(leader_cta, &bars->p_full[sl]);
       }
       RC_TACC(3, tpst);
       if (warp == 4) RC_EV(l, 15);      // P(l) stored
       if (half == 0 && valid && prm.lse && !(kKB && prm.lse_in != nullptr)) prm.lse[m] = lse;
     }
-    if (half == 0) {
-      const float loss_acc = warp_sum(acc_s[0]), w_acc = warp_sum(acc_s[128]), dlt_acc = warp_sum(acc_s[256]);
-      if (lane == 0) {
-        if (prm.loss_sum) atomicAdd(prm.loss_sum, (double)loss_acc);
-        if (prm.w_sum) atomicAdd(prm.w_sum, (double)w_acc);
-        if (prm.dlogtau) atomicAdd(prm.dlogtau, (double)dlt_acc);
-      }
-    }
+    if (half == 0) add_sums<true>(prm, lane, acc_s[0], acc_s[128], acc_s[256]);
   } else {
     // ================ dX epilogue warps: own tile, thread = pixel, one 64-channel block = one step of 32 channels ================
     // warp (q, h): TMEM lane quarter q = pixels [32 q, +32) of the tile, accumulator columns [32 h, +32) of every block
@@ -695,7 +463,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
           }
         }
         tc_fence_before();
-        arrive_leader_warp(&bars->acc_empty[sl][ab]);
+        arrive_leader_warp(leader_cta, &bars->acc_empty[sl][ab]);
         RC_TACC(3, tld);
         const int bi = s % kEpiBufs;
         RC_WAIT(mbar_wait, &ebar[bi], (s / kEpiBufs) & 1, 4);
@@ -757,58 +525,24 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
 }  // namespace ts
 
 // launch helper used by rc_infonce_bf16 for backward launches without dText (infonce.cu owns argument checking)
-int launch_infonce_ts(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
-                      const int32_t* y, const float* w, float inv_tau, const float* grad_scale, const double* w_sum_in,
-                      float* lse, double* loss_sum, double* w_sum, double* dlogtau, int rep, int keep_w, const float* lse_in,
-                      int kb, int acc_dx, cudaStream_t s) {
+int launch_infonce_ts(const InfoncePairArgs& a, cudaStream_t s) {
   using namespace ts;
-  const int Kp = kb > 0 ? 256 : (K + 63) / 64 * 64;
-  const int Kall = kb > 0 ? kb * 256 : Kp;          // rows of the text matrices
   CUtensorMap m_xs, m_t, m_tt, m_xe, m_dx;
   int rcode;
-  {
-    const uint64_t dims[3] = {(uint64_t)HW, (uint64_t)D, (uint64_t)B};
-    const uint64_t xdims[3] = {(uint64_t)HW, (uint64_t)D, (uint64_t)(kb > 0 ? 1 : B)};
-    const uint64_t str[3] = {2, (uint64_t)HW * 2, (uint64_t)D * HW * 2};
-    const uint32_t box_s[3] = {64, 64, 1};
-    if ((rcode = make_tmap_bf16(&m_xs, xsrc, 3, xdims, str, box_s, "ts map_x_s"))) return rcode;
-    const uint32_t box_o[3] = {32, 32, 1};
-    if ((rcode = make_tmap_bf16(&m_xe, xsrc, 3, xdims, str, box_o, "ts map_xe"))) return rcode;
-    if ((rcode = make_tmap_bf16(&m_dx, dx, 3, dims, str, box_o, "ts map_dx"))) return rcode;
-    const uint64_t tdims[2] = {(uint64_t)D, (uint64_t)Kall}, tstr[2] = {2, (uint64_t)D * 2};
-    const uint32_t tbox[2] = {64, (uint32_t)(Kp / 2)};
-    if ((rcode = make_tmap_bf16(&m_t, t_bf16, 2, tdims, tstr, tbox, "ts map_t"))) return rcode;
-    const uint64_t ttdims[2] = {(uint64_t)Kall, (uint64_t)D}, ttstr[2] = {2, (uint64_t)Kall * 2};
-    const uint32_t ttbox[2] = {64, 32};
-    if ((rcode = make_tmap_bf16(&m_tt, tt_bf16, 2, ttdims, ttstr, ttbox, "ts map_tt"))) return rcode;
-  }
+  if ((rcode = make_operand_maps(a, 32, {"ts map_x_s", "ts map_t", "ts map_tt"}, &m_xs, &m_t, &m_tt))) return rcode;
+  if ((rcode = make_xmap(&m_xe, a.xsrc, a, a.kb > 0 ? 1 : a.B, 32, 32, "ts map_xe"))) return rcode;
+  if ((rcode = make_xmap(&m_dx, a.dx, a, a.B, 32, 32, "ts map_dx"))) return rcode;
   Params prm;
-  prm.dbg = debug_timing_buffer();
-  prm.ablate = 0;
-#ifdef RC_BRINGUP      // ablation switches of the bring-up build (tools/timing_ts.py ablate); the shipped library has no environment knobs
-  { const char* ab = getenv("RANGECLIP_B200_ABLATE"); prm.ablate = ab ? atoi(ab) : 0; }
-#endif
-  prm.B = B; prm.D = D; prm.K = K; prm.Kp = Kp; prm.HW = HW;
-  prm.tiles_per_img = (int)((HW + kTilePx - 1) / kTilePx);
-  if ((int64_t)B * prm.tiles_per_img > 0x3fffffff) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: too many tiles");
-  prm.n_tiles = B * prm.tiles_per_img;
-  prm.tpi_magic = prm.tiles_per_img == 1 ? 0xffffffffu : (uint32_t)(0x100000000ull / (uint64_t)prm.tiles_per_img);
-  prm.n_pairs = (prm.n_tiles + 1) / 2;
-  prm.y = y; prm.w = w; prm.inv_tau = inv_tau; prm.grad_scale = grad_scale;
-  prm.w_sum_in = w_sum_in; prm.lse = lse; prm.loss_sum = loss_sum; prm.w_sum = w_sum; prm.dlogtau = dlogtau;
-  prm.keep_w = keep_w; prm.lse_in = lse_in; prm.kb = kb; prm.acc_dx = acc_dx;
-  if (kb > 0 && (prm.tiles_per_img & 1)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: HW must be a multiple of 256");
-  int n_clusters = num_sms() / 2;
-  if (n_clusters > prm.n_pairs) n_clusters = prm.n_pairs;
-  const int grid = 2 * n_clusters;
+  int grid = 0;
+  if ((rcode = fill_tiling(prm, a, &grid))) return rcode;
   auto launch = [&](auto kernel) -> int {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) return fail(RC_ERR_CUDA, "rc_infonce_bf16(ts): smem opt-in: %s", cudaGetErrorString(e));
     kernel<<<grid, kThreads, kSmemBytes, s>>>(m_xs, m_t, m_tt, m_xe, m_dx, prm);
     return check_launch("rc_infonce_bf16(ts)");
   };
-  if (rep == 4) return launch(infonce_ts_kernel<4, false>);
-  if (keep_w || lse_in != nullptr || kb > 0 || acc_dx) return launch(infonce_ts_kernel<1, true>);
+  if (a.rep == 4) return launch(infonce_ts_kernel<4, false>);
+  if (launch_kblocked(a)) return launch(infonce_ts_kernel<1, true>);
   return launch(infonce_ts_kernel<1, false>);
 }
 

@@ -24,22 +24,23 @@
 // consumer-release barriers live in the leader and receive remote arrivals from the peer.  The per-pixel
 // row scales of a tile are exchanged through distributed shared memory (the dX epilogue of a CTA covers
 // pixels of both tiles).
-#include "common.cuh"
-#include "umma.cuh"
-#include "infonce_device.cuh"
-#include <float.h>
-#include <stdlib.h>
+//
+// This kernel runs forward-only launches, the dText path (it writes G for infonce_dt_umma.cu), rc_infonce_bf16_dyn and
+// RC_INFONCE_SS_KERNEL; backward launches otherwise run the TS kernel (infonce_ts.cu).  The tiling, the operand
+// producers, the relay and the softmax arithmetic are shared with it through infonce_pair.cuh, so that both give
+// bit-identical dX and lse; this file holds the SS pipeline, the P store into shared memory (and the G store), the
+// row-scale exchange between the CTAs and the dX epilogue.
+#include "infonce_pair.cuh"
 
 namespace rc {
 using namespace umma;
 
 namespace pair {
+using namespace cta_pair;
 
-constexpr int kTilePx = 128;
 constexpr int kThreads = 640;          // warps: 0 text TMA, 1 MMA (leader CTA only), 2 relay + TMEM alloc, 3 X TMA, 4-11 softmax, 12-19 dX epilogue
 constexpr int kXStages = 4;            // X ring: own X chunks [64 d][128 px] (first touch: HBM latency; also read by the row norms)
 constexpr int kTStages = 4;            // text ring: text half-chunks [Kp/2][64 d] for S, own T^T rows [128 d][64 k] for dX (L2 hits)
-constexpr int kStageBytes = 16 * 1024;
 static_assert(kTStages >= 4, "a dX block keeps Kp/64 <= 4 slots of the text ring at once");
 constexpr int kPBytes = 64 * 1024;
 constexpr int kTmemCols = 512;
@@ -67,50 +68,17 @@ constexpr int kOffBars = kOffPart + 8 * 128 * 4;            // row-norm partial 
 constexpr int kSmemBytes = kOffBars + (int)sizeof(Bars);
 static_assert(kSmemBytes <= 232448, "shared-memory budget of one SM (227 KB)");
 
-struct Params {
-  long long* dbg;
-  int B, D, K, Kp;
-  int64_t HW;
-  int tiles_per_img, n_tiles, n_pairs;
-  uint32_t tpi_magic;       // floor(2^32 / tiles_per_img): tile / tiles_per_img as a multiply-high + one correction
-  int ablate;               // bring-up only (RANGECLIP_B200_ABLATE): 1 no epilogue x loads, 2 no dX stores, 64 no row-norm reads, 128 no dX staging, 256 no text reloads
+// bring-up ablation bits (Tiling::ablate): 1 no epilogue x loads, 2 no dX stores, 64 no row-norm reads, 128 no dX
+// staging, 256 no text reloads
+struct Params : Tiling {
   int store_g;              // 1: also write G = rs (P - sum onehot) (bf16 [B][HW][Kp]) for the dText GEMM
   int wide;                 // 1: rows of X / dX are 32-byte aligned (256-bit global accesses allowed)
   const __nv_bfloat16* x;
-  __nv_bfloat16* dx;
-  const float* inv_norm;
-  // K-blocked use (more than 256 candidates, e.g. the area-image loss at thousands of objects): the candidates are split
-  // into launches of <= 256 rows.  keep_w: a target outside this launch's rows keeps its weight (only the one-hot term is
-  // dropped).  lse_in: the row's logsumexp over ALL candidates, from a first round of forward launches; the softmax of
-  // this block is then exp(z - lse_in) instead of exp(z - m) / (block sum).
-  int keep_w;
-  int acc_dx;               // K-blocked backward launches after the first: dX += this block's gradient (TMA reduce-add store)
-  const float* lse_in;
-  // kb > 0: ALL candidate blocks in one launch.  The "images" of the tile index are the kb blocks of 256 candidate rows:
-  // X (one image) is read with image coordinate 0, everything else (y, w, lse, dX, text rows) is indexed by the block.
-  // K is then the total number of candidates; lse_in is indexed by the pixel alone.
-  int kb;
-  const int32_t* y;
-  const float* w;
-  float inv_tau;
   // sync-free callers (device-side contrast-set builder, SURVEY 8f-2): the number of valid candidate rows and the log
   // temperature are read from device memory at kernel start (nullable: K / inv_tau above are used)
   const int32_t* k_dev;
   const float* log_tau_dev;
-  const float* grad_scale;
-  const double* w_sum_in;
-  float* lse;
-  double* loss_sum;
-  double* w_sum;
-  double* dlogtau;
 };
-
-// tile / tiles_per_img without the ~20-instruction runtime division (exact for tile < 2^32: the estimate is low by at most 1)
-__device__ __forceinline__ int div_tiles(const Params& prm, int tile) {
-  int q = (int)__umulhi((uint32_t)tile, prm.tpi_magic);
-  if (tile - q * prm.tiles_per_img >= prm.tiles_per_img) ++q;
-  return q;
-}
 
 // 16 pixels (32 bytes) of one channel row, straight from global memory.  `n8` = number of valid
 // 8-pixel groups (0, 1 or 2); the 256-bit form needs 32-byte alignment (`wide`).
@@ -132,21 +100,7 @@ __device__ __forceinline__ void ldg_px16(const __nv_bfloat16* p, bool wide, int 
     }
   }
 }
-// tile -> (image, first pixel); tiles past the end map to image index B, which is out of bounds for every
-// tensor map (TMA loads return zeros)
-__device__ __forceinline__ void tile_coords(const Params& prm, int tile, int& b, int& px0) {
-  if (tile < prm.n_tiles) {
-    b = div_tiles(prm, tile);
-    px0 = (tile - b * prm.tiles_per_img) * kTilePx;
-  } else {
-    b = prm.B;
-    px0 = 0;
-  }
-}
-
-// R = targets per embedding row: 1 = one pixel per row (y, w are [B*HW]); 4 = every row stands for the four pixels of a
-// 2x2 block that share one embedding (decoder.py:113 nearest x2): y, w are [B*HW][4], the loss of the row is
-// sum_j w_j (lse - z[y_j]) and dX is the gradient with respect to the shared embedding (the sum over the block).
+// R = targets per embedding row (1, or 4 for the shared 2x2 form, see infonce_pair.cuh)
 // kKB: K-blocked launches (Params::keep_w / lse_in); a template flag so that the headline instantiation carries none of it
 template <bool kBwd, int R, bool kKB>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
@@ -170,7 +124,6 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
   // this pair, so that the dX epilogue drains accumulators while the tensor pipe works on S
   const int c_half = n_dchunks / 2;
   const int b_half = (n_blk + 1) / 2;
-  const int Nh = prm.Kp / 2;             // text rows staged by each CTA
   const int n_clusters = gridDim.x / 2;
   const int cluster_id = blockIdx.x / 2;
 
@@ -207,16 +160,6 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
 #endif
   const uint32_t idesc_s = make_idesc_bf16(256, prm.Kp, /*A MN-major*/ 1, /*B K-major*/ 0);
   const uint32_t idesc_d = make_idesc_bf16(256, 128, 0, 0);
-  // consumer-release barriers live in the leader CTA
-  auto arrive_leader = [&](uint64_t* bar) {
-    if (leader_cta) mbar_arrive(bar);
-    else mbar_arrive_remote(map_to_cta(bar, 0));
-  };
-  // one arrival for the whole warp: every lane has fenced its own accesses, __syncwarp orders them before lane 0's arrive
-  auto arrive_leader_warp = [&](uint64_t* bar) {
-    __syncwarp();
-    if (elect_one()) arrive_leader(bar);
-  };
 
   if (warp < 4) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsCtl));
@@ -226,19 +169,9 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       // text ring, in MMA issue order: S(first), then per tile pair
       //   [S(next) first half] [dX(this) first blocks] [S(next) second half] [dX(this) remaining blocks]
       uint32_t it = 0;
-      // first candidate row of the pair's block (kb mode: both tiles of a pair lie in one block, tiles_per_img is even)
-      auto koff_of = [&](int pj) -> int { return (kKB && prm.kb > 0) ? div_tiles(prm, 2 * pj) * 256 : 0; };
+      auto koff_of = [&](int pj) -> int { return text_row0<kKB>(prm, pj); };
       auto load_s = [&](int c_begin, int c_end, int koff) {
-        for (int c = c_begin; c < c_end; ++c, ++it) {   // own half (Nh rows) of text chunk c
-          const int st = it % kTStages;
-          RC_WAIT(mbar_wait, &bars->tempty[st], ((it / kTStages) & 1) ^ 1, 1);
-          if ((prm.ablate & 256) && it >= (uint32_t)kTStages) {      // bring-up: no text traffic after the first ring pass (stale operands)
-            if (leader_cta) mbar_arrive(&bars->tfull[st]);
-            continue;
-          }
-          if (leader_cta) mbar_arrive_expect_tx(&bars->tfull[st], 2 * Nh * 128);
-          tma_load_2d_2sm(smem + kOffT + st * kStageBytes, &map_t, &bars->tfull[st], c * 64, koff + (int)rank * Nh);
-        }
+        load_text_s<kTStages>(prm, &map_t, smem + kOffT, bars->tfull, bars->tempty, it, c_begin, c_end, koff, rank RC_WT);
       };
       auto load_dx = [&](int b_begin, int b_end, int koff) {
         for (int blk = b_begin; blk < b_end; ++blk)
@@ -267,19 +200,8 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       // own X chunks of every tile, as far ahead as the X ring allows (the next tile's first chunks are in flight
       // while the dX GEMM of the previous pair runs)
       uint32_t xit = 0;
-      for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters) {
-        int b, px0;
-        tile_coords(prm, 2 * pj + (int)rank, b, px0);
-        for (int c = 0; c < n_dchunks; ++c, ++xit) {
-          const int st = xit % kXStages;
-          RC_WAIT(mbar_wait, &bars->xempty[st], ((xit / kXStages) & 1) ^ 1, 1);
-          uint8_t* sb = smem + st * kStageBytes;
-          mbar_arrive_expect_tx(&bars->xf[st], 2 * 8192);          // CTA-local: the softmax warps read the chunk too
-          const int bx = (kKB && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;      // kb mode: the one image of X (1 = out of bounds)
-          tma_load_3d(sb, &map_x_s, &bars->xf[st], px0, c * 64, bx);
-          tma_load_3d(sb + 8192, &map_x_s, &bars->xf[st], px0 + 64, c * 64, bx);
-        }
-      }
+      for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters)
+        load_x_tile<kXStages, kKB, false>(prm, &map_x_s, smem, bars->xf, bars->xempty, xit, 2 * pj + (int)rank, n_dchunks, 0, 1 RC_WT);
     } else if (warp == 1 && leader_cta) {
       // =============================== MMA issuer (leader CTA) ================================
       // The whole warp runs the loop converged, so stage indices, addresses and descriptors live in uniform
@@ -376,13 +298,8 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
     else if (warp == 2 && lane == 0) {
       // ========== relay (both CTAs): "own X chunk has landed" (CTA-local xf) -> the leader's full barrier ==========
       uint32_t xit = 0;
-      for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters) {
-        for (int c = 0; c < n_dchunks; ++c, ++xit) {
-          const int st = xit % kXStages;
-          RC_WAIT(mbar_wait, &bars->xf[st], (xit / kXStages) & 1, 14);
-          arrive_leader(&bars->xfull[st]);
-        }
-      }
+      for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters)
+        relay_x_tile<kXStages, true>(n_dchunks, bars->xf, bars->xfull, xit, leader_cta, 14 RC_WT);
     }
   } else if (warp < 12) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsSoftmax));
@@ -396,80 +313,22 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
     const int sw = row & 7;
     float* xch_base = reinterpret_cast<float*>(smem + kOffXch);
     float loss_acc = 0.f, w_acc = 0.f, dlt_acc = 0.f;
-    float inv_wsum = 0.f, gscale = 1.f;
-    if (kBwd) {
-      const double ws = prm.w_sum_in[0];
-      inv_wsum = ws > 0.0 ? (float)(1.0 / ws) : 0.f;
-      if (prm.grad_scale) gscale = prm.grad_scale[0];
-    }
-    float nx_inv_n = 0.f, nx_w = 0.f;
-    int nx_y = -1;
-    auto load_pixel_scalars = [&](int pj) {
-      nx_inv_n = 0.f; nx_w = 0.f; nx_y = -1;
-      const int t = 2 * pj + (int)rank;
-      if (pj < prm.n_pairs && t < prm.n_tiles) {
-        const int tb = div_tiles(prm, t);
-        const int tpx = (t - tb * prm.tiles_per_img) * kTilePx + row;
-        if (tpx < prm.HW) {
-          const int64_t tm = (int64_t)tb * prm.HW + tpx;
-          nx_inv_n = 1.f;        // valid pixel (the value itself comes from the norm warps)
-          if (R == 1) {
-            nx_y = __ldg(prm.y + tm);
-            nx_w = __ldg(prm.w + tm);
-          } else {               // four targets, 8 bits each (K <= 256); ignored targets are sorted out when w is read
-            const int4 y4 = __ldg(reinterpret_cast<const int4*>(prm.y) + tm);
-            nx_y = (y4.x & 255) | ((y4.y & 255) << 8) | ((y4.z & 255) << 16) | ((y4.w & 255) << 24);
-          }
-        }
-      }
-    };
-    load_pixel_scalars(cluster_id);
-    // Row norms 1/|x_p| (model.py:272 F.normalize) of the NEXT tile, computed by these warps while they would
-    // otherwise wait for its S GEMM: the X chunks are read where they sit in the operand ring ([64 d][2 x 64 px],
-    // 128-byte swizzle).  thread = (8-pixel group g, row phase r); sums of squares meet in shared memory.
-    float* part_s = reinterpret_cast<float*>(smem + kOffPart);   // [8 warps][128 px] partial sums of squares
-    const int st_ = threadIdx.x - 128;                           // 0..255
-    const int ng = st_ & 15, nr = st_ >> 4;
+    float gscale = 1.f, inv_wsum = 0.f;
+    if (kBwd) grad_scales(prm, gscale, inv_wsum);
+    float nx_ok, nx_w;         // pixel scalars of the next tile
+    int nx_y;
+    load_pixel_scalars<R>(prm, cluster_id < prm.n_pairs, 2 * cluster_id + (int)rank, row, nx_ok, nx_w, nx_y);
+    // Row norms of the NEXT tile, computed by these warps while they would otherwise wait for its S GEMM
+    float* part_s = reinterpret_cast<float*>(smem + kOffPart);
+    int ng, nr;
+    norm_coords(ng, nr);
     uint32_t nit = 0;
     float inv_n_next = 0.f;
-    auto norm_tile = [&]() {
-      float ss[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) ss[j] = 0.f;
-      for (int c = 0; c < n_dchunks; ++c, ++nit) {
-        const int st = nit % kXStages;
-        RC_WAIT(mbar_wait, &bars->xf[st], (nit / kXStages) & 1, 15);
-        const uint8_t* base = smem + st * kStageBytes + (ng >> 3) * 8192 + nr * 128;
-        const int ch = ng & 7;
-#pragma unroll
-        for (int rr = 0; rr < ((prm.ablate & 64) ? 0 : 4); ++rr) {
-          const int rowd = nr + rr * 16;
-          const uint4 v = *reinterpret_cast<const uint4*>(base + rr * 2048 + ((ch ^ (rowd & 7)) << 4));
-          const uint32_t u[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {       // FHFMA.BF16 on the word's halves: no unpack instructions
-            ss[2 * j] = sqacc_bf16x2_lo(ss[2 * j], u[j]);
-            ss[2 * j + 1] = sqacc_bf16x2_hi(ss[2 * j + 1], u[j]);
-          }
-        }
-        __syncwarp();
-        if (elect_one()) mbar_arrive(&bars->xempty[st]);     // (elect.sync: no lane id to re-materialise in this hot loop)
-      }
-      // fixed-order reduction (bit-reproducible): lane pairs, then the eight warps' partials through shared memory
-#pragma unroll
-      for (int j = 0; j < 8; ++j) ss[j] += __shfl_xor_sync(0xffffffffu, ss[j], 16);     // lanes l and l^16: same pixels, other rows
-      if (lane < 16) {
-        float4* dst = reinterpret_cast<float4*>(part_s + (warp - 4) * 128 + ng * 8);
-        dst[0] = make_float4(ss[0], ss[1], ss[2], ss[3]);
-        dst[1] = make_float4(ss[4], ss[5], ss[6], ss[7]);
-      }
-      named_bar_sync(5, 256);
-      float q = 0.f;
-#pragma unroll
-      for (int wv = 0; wv < 8; ++wv) q += part_s[wv * 128 + row];
-      inv_n_next = 1.f / fmaxf(sqrtf(q), 1e-12f);
+    auto norm_next = [&]() {
+      inv_n_next = norm_tile<kXStages>(smem, bars->xf, bars->xempty, nit, n_dchunks, part_s, warp, lane, row, ng, nr,
+                                       (prm.ablate & 64) != 0, 15 RC_WT);
     };
-    if (cluster_id < prm.n_pairs) norm_tile();
+    if (cluster_id < prm.n_pairs) norm_next();
     const float inv_tau = prm.log_tau_dev != nullptr ? expf(-__ldg(prm.log_tau_dev)) : prm.inv_tau;
     const int K_valid = prm.k_dev != nullptr ? max(1, min(__ldg(prm.k_dev), prm.K)) : prm.K;      // rows past it are zero pads
     const bool use_bound = inv_tau * (2.02f * kLog2e) < 100.f;
@@ -490,149 +349,55 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       const int64_t m = (int64_t)b * prm.HW + px;
       // candidates in this tile's block (kb mode: the last block may be short; its zero pad rows are masked like any pad)
       const int Kt = (kKB && prm.kb > 0) ? min(256, prm.K - 256 * b) : K_valid;
-      const bool px_ok = nx_inv_n != 0.f;
+      const float ok = nx_ok;
+      const bool px_ok = ok != 0.f;
       const int yi = nx_y;
       const float wi = (R == 1 && (yi >= 0 || (kKB && prm.keep_w))) ? nx_w : 0.f;
-      load_pixel_scalars(pj + n_clusters);
+      load_pixel_scalars<R>(prm, pj + n_clusters < prm.n_pairs, 2 * (pj + n_clusters) + (int)rank, row, nx_ok, nx_w, nx_y);
       float* xch = xch_base + (lt & 1) * (4 * 2 * 128);      // double-buffered: one named barrier per tile suffices
       const float inv_n = px_ok ? inv_n_next : 0.f;
       const float zs = inv_n * inv_tau;
       const float zl = zs * kLog2e;
       // forward-only: the tensor pipe runs one pair ahead (two S buffers), so the next tile's row norms are taken
       // first -- its X chunks are already streaming and their ring slots are refilled only after these reads
-      if (!kBwd && pj + n_clusters < prm.n_pairs) norm_tile();
+      if (!kBwd && pj + n_clusters < prm.n_pairs) norm_next();
       const uint32_t sidx = kBwd ? 0u : (lt & 1u);
       const uint32_t trow = trow0 + sidx * 256;
       RC_WAIT(mbar_wait, &bars->s_full[sidx], (kBwd ? lt : (lt >> 1)) & 1u, 8);
       tc_fence_after();
       if (warp == 4) RC_EV(lt, 10);    // S(lt) complete (seen by the softmax warps)
       RC_T0(tsm);
-      float ml = ml_bound;
-      if (!use_bound) {
-        float mx = -FLT_MAX;
-        for (int c = 0; c * 32 < Kh; ++c) {
-          const int nvalid = Kt - (cb + c * 32);
-          if (nvalid <= 0) break;
-          uint32_t r[32];
-          tmem_ld_32x32(trow + c * 32, r);
-          tmem_ld_wait();
-#pragma unroll
-          for (int i = 0; i < 32; ++i) if (i < nvalid) mx = fmaxf(mx, __uint_as_float(r[i]));
-        }
-        xch[(0 * 2 + half) * 128 + row] = mx;
-        named_bar_sync(3, 256);
-        mx = fmaxf(mx, xch[(0 * 2 + (half ^ 1)) * 128 + row]);
-        ml = mx * zl;
-      }
-      // e = exp(z - m) for this half's columns; P stays in registers as packed bf16 until the P buffer is free.
-      // (Measured, not adopted: the scale / sum / e*s arithmetic as packed fp32x2 -- FFMA2 / FADD2, 6 instead of 9
-      // issued instructions per two columns -- is 2.7 % slower, 2.57 against 2.50 ms.)
+      const float ml = use_bound ? ml_bound : row_max(trow, Kt, cb, Kh, xch, half, row, zl);
+      // e = exp(z - m) for this half's columns; P stays in registers as packed bf16 until the P buffer is free
       uint32_t pk[64];
-      float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f, q0 = 0.f, q1 = 0.f, q2 = 0.f, q3 = 0.f;
       float sy[R];
-#pragma unroll
-      for (int j = 0; j < R; ++j) sy[j] = 0.f;
-      // 16 text columns per step
-      auto smx_step = [&](const uint32_t (&r)[16], int c) {
-        const int k0 = cb + c * 16;
-        const int nvalid = Kt - k0;
-#pragma unroll
-        for (int j = 0; j < R; ++j) {                          // target logit(s): once per row, not per column
-          const int yrel = (R == 1 ? yi : (int)(((uint32_t)yi >> (8 * j)) & 255u)) - k0;
-          if ((unsigned)yrel < 16u) sy[j] = select16(r, yrel);
-        }
-        if (nvalid >= 16) {
-#pragma unroll
-          for (int i = 0; i < 16; i += 4) {
-            const float a0 = __uint_as_float(r[i]), a1 = __uint_as_float(r[i + 1]);
-            const float a2 = __uint_as_float(r[i + 2]), a3 = __uint_as_float(r[i + 3]);
-            const float e0 = fast_exp2(fmaf(a0, zl, -ml)), e1 = fast_exp2(fmaf(a1, zl, -ml));
-            const float e2 = fast_exp2(fmaf(a2, zl, -ml)), e3 = fast_exp2(fmaf(a3, zl, -ml));
-            s0 += e0; s1 += e1; s2 += e2; s3 += e3;
-            q0 = fmaf(e0, a0, q0); q1 = fmaf(e1, a1, q1); q2 = fmaf(e2, a2, q2); q3 = fmaf(e3, a3, q3);
-            pk[c * 8 + (i >> 1)] = pack_bf16x2(e0, e1);
-            pk[c * 8 + (i >> 1) + 1] = pack_bf16x2(e2, e3);
-          }
-        } else {          // the step that straddles K, or padding columns only
-#pragma unroll
-          for (int i = 0; i < 16; i += 2) {
-            const float a0 = __uint_as_float(r[i]), a1 = __uint_as_float(r[i + 1]);
-            const float e0 = (i < nvalid) ? fast_exp2(fmaf(a0, zl, -ml)) : 0.f;
-            const float e1 = (i + 1 < nvalid) ? fast_exp2(fmaf(a1, zl, -ml)) : 0.f;
-            s0 += e0; s1 += e1;
-            q0 = fmaf(e0, a0, q0); q1 = fmaf(e1, a1, q1);
-            pk[c * 8 + (i >> 1)] = pack_bf16x2(e0, e1);
-          }
-        }
-      };
-#pragma unroll
-      for (int c = 0; c < 8; ++c) {
-        if (c * 16 < Kh) {
-          uint32_t r[16];
-          tmem_ld_32x16(trow + c * 16, r);
-          tmem_ld_wait();
-          smx_step(r, c);
-        }
-      }
+      float sum, sez;
+      exp_pass<R>(trow, cb, Kh, Kt, yi, zl, ml, pk, sy, sum, sez);
       tc_fence_before();
       if (warp == 4) RC_EV(lt, 11);    // exp pass done
       if (warp == 11) RC_EV(lt, 15);   // exp pass done (last softmax warp)
-      arrive_leader_warp(&bars->s_empty[sidx]);      // S columns are free: the tensor pipe may start the next S in them
-      float sum = (s0 + s1) + (s2 + s3);
-      float sez = (q0 + q1) + (q2 + q3);
-      // targets of this row: y_j, w_j (w_j = 0: ignored); tz = sum_j w_j s[y_j] over the targets in this half's columns
+      arrive_leader_warp(leader_cta, &bars->s_empty[sidx]);      // S columns are free: the tensor pipe may start the next S in them
       int yj[R];
       float wj[R];
-      if (R == 1) {
-        yj[0] = yi; wj[0] = wi;
-      } else {
-        int4 y4 = make_int4(-1, -1, -1, -1);
-        float4 w4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (px_ok) {
-          y4 = __ldg(reinterpret_cast<const int4*>(prm.y) + m);
-          w4 = __ldg(reinterpret_cast<const float4*>(prm.w) + m);
-        }
-        const int ya[4] = {y4.x, y4.y, y4.z, y4.w};
-        const float wa[4] = {w4.x, w4.y, w4.z, w4.w};
-#pragma unroll
-        for (int j = 0; j < R; ++j) { yj[j] = ya[j]; wj[j] = ya[j] >= 0 ? wa[j] : 0.f; }
-      }
-      float wtot = 0.f, tz = 0.f;
       bool mine[R];
-#pragma unroll
-      for (int j = 0; j < R; ++j) {
-        mine[j] = yj[j] >= cb && yj[j] < cb + Kh;
-        wtot += wj[j];
-        tz += mine[j] ? wj[j] * sy[j] : 0.f;
-      }
-      xch[(1 * 2 + half) * 128 + row] = sum;
-      xch[(2 * 2 + half) * 128 + row] = sez;
-      xch[(3 * 2 + half) * 128 + row] = tz;
+      float wtot, tz;
+      gather_targets<R>(prm, yi, wi, ok, m, cb, Kh, sy, yj, wj, mine, wtot, tz);
+      post_sums(xch, half, row, sum, sez, tz);
       named_bar_sync(2, 256);
-      sum += xch[(1 * 2 + (half ^ 1)) * 128 + row];
-      sez += xch[(2 * 2 + (half ^ 1)) * 128 + row];
-      tz += xch[(3 * 2 + (half ^ 1)) * 128 + row];
-      if (kKB && prm.lse_in != nullptr && valid) sum = fast_exp2(fmaf(__ldg(prm.lse_in + (prm.kb > 0 ? (int64_t)px : m)), kLog2e, -ml));   // 1 / sum = exp(m - lse)
-      float lse = 0.f;
-      if (half == 0) {
-        lse = (ml + __log2f(sum)) * kLn2;
-        loss_acc += wtot * lse - tz * zs;
-        w_acc += wtot;
-      }
+      add_peer_sums(xch, half, row, sum, sez, tz);
+      const float lse = row_lse<kKB>(prm, valid, px, m, half, ml, wtot, tz, zs, sum, loss_acc, w_acc);
       RC_TACC(1, tsm);
       if (!kBwd) {
         if (half == 0 && valid && prm.lse) prm.lse[m] = lse;
         continue;
       }
       {
-        const float coefb = gscale * inv_wsum;
+        const float coefb = gscale * inv_wsum;      // formed per tile: kept live across the loop it costs time
         const float coef = coefb * wtot;
         const float inv_sum = 1.f / sum;
-        // P is stored pre-scaled: G[p][k] = rs_p (e_pk - sum_p [k = y_p]) = d loss / d(xhat_p . that_k) / |x_p|, so the
-        // dX accumulators need no row scale and the same tile is the A operand of the dText GEMM (dT = G^T X).
-        const float rsv = inv_n * inv_tau * coef * inv_sum;
+        const float rsv = p_scale(inv_n, inv_tau, coef, inv_sum);
         if (half == 0) {
-          const float cj = coef * sez * zs * inv_sum - coefb * tz * zs;
+          const float cj = proj_coef(coef, coefb, sez, tz, zs, inv_sum);
           const float csv = inv_n * inv_n * cj;
           // the dX epilogue works on packed bf16 pixel pairs: dx = acc + (-cs) * x
           const float cs_n = __shfl_down_sync(0xffffffffu, csv, 1);
@@ -665,27 +430,18 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
                              bf2_mul(pk[c * 16 + g * 4 + 2], rs2), bf2_mul(pk[c * 16 + g * 4 + 3], rs2));
           }
         }
-        // G[row][y_j] = rs (e_y - sum * (weight of target y_j) / (weight of the row))  (softmax - onehot), formed before rounding
+        // the target entries of G, over the rounded P entries
 #pragma unroll
         for (int j = 0; j < R; ++j) {
           if (mine[j]) {
-            const float ey = fast_exp2(fmaf(sy[j], zl, -ml));
-            float gv;
-            if (R == 1) {
-              gv = (ey - sum) * rsv;
-            } else {
-              float wk = 0.f;                 // targets of the block that name the same text row
-#pragma unroll
-              for (int i = 0; i < R; ++i) wk += (yj[i] == yj[j]) ? wj[i] : 0.f;
-              gv = (ey - sum * (wtot > 0.f ? wk / wtot : 0.f)) * rsv;      // rs = rsv carries the block's total weight
-            }
+            const float gv = target_g<R>(j, sy, yj, wj, wtot, sum, zl, ml, rsv);
             const int kk = yj[j] & 63;
             uint8_t* sub = prow + (yj[j] >> 6) * 16384;
             *reinterpret_cast<__nv_bfloat16*>(sub + (((kk >> 3) ^ sw) << 4) + (kk & 7) * 2) = __float2bfloat16_rn(gv);
           }
         }
         fence_proxy_async_smem();                 // P is read by the tensor cores (async proxy)
-        arrive_leader_warp(&bars->p_full);
+        arrive_leader_warp(leader_cta, &bars->p_full);
         if (warp == 4) RC_EV(lt, 13);  // P(lt) stored
         if (warp == 11) RC_EV(lt, 16); // P(lt) stored (last softmax warp)
         RC_TACC(2, tst);
@@ -698,19 +454,12 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
           }
         }
         if (half == 0 && valid && prm.lse && !(kKB && prm.lse_in != nullptr)) prm.lse[m] = lse;      // after the hand-off: nothing waits behind this store
-        if (pj + n_clusters < prm.n_pairs) norm_tile();
+        if (pj + n_clusters < prm.n_pairs) norm_next();
         if (warp == 4) RC_EV(lt, 14);  // row norms of the next tile done
       }
     }
     if (kBwd && prm.store_g && threadIdx.x == 128) tma_store_wait_all0();
-    if (half == 0) {
-      loss_acc = warp_sum(loss_acc); w_acc = warp_sum(w_acc); dlt_acc = warp_sum(dlt_acc);
-      if (lane == 0) {
-        if (prm.loss_sum) atomicAdd(prm.loss_sum, (double)loss_acc);
-        if (prm.w_sum) atomicAdd(prm.w_sum, (double)w_acc);
-        if (kBwd && prm.dlogtau) atomicAdd(prm.dlogtau, (double)dlt_acc);
-      }
-    }
+    if (half == 0) add_sums<kBwd>(prm, lane, loss_acc, w_acc, dlt_acc);
   } else if (kBwd) {
     // ================ dX epilogue warps: own channel rows, 64 contiguous pixels per accumulator ================
     // Warps 12-15 (half 0) take accumulator columns [0,64) = pixels of CTA 0's tile, warps 16-19 (half 1) columns
@@ -790,7 +539,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
           tmem_ld_wait();
           RC_TACC(3, t3);
           RC_T0(t13);
-          if (c == 1) { tc_fence_before(); arrive_leader_warp(&bars->acc_empty[ab]); }
+          if (c == 1) { tc_fence_before(); arrive_leader_warp(leader_cta, &bars->acc_empty[ab]); }
           RC_TACC(13, t13);
           RC_T0(t4);
           pair_swap(&xq[c][0]);             // -> own row, pixels [c*32, +32) in order
@@ -869,78 +618,39 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
 bool infonce_pair_supported(int D) { return D == 256 || D == 512; }
 
 // launch helper used by rc_infonce_bf16 (infonce.cu owns argument checking and the pre-pass)
-int launch_infonce_pair(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
-                        const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
-                        const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, void* g_out,
-                        int rep, int keep_w, const float* lse_in, int kb, int acc_dx, const int32_t* k_dev,
-                        const float* log_tau_dev, cudaStream_t s) {
+int launch_infonce_pair(const InfoncePairArgs& a, cudaStream_t s) {
   using namespace pair;
-  const bool bwd = dx != nullptr;
-  // kb > 0: all kb blocks of 256 candidate rows in one launch -- B counts the blocks (virtual images), X has ONE image,
-  // the text maps span all blocks (row offset = block * 256), dX has one [D][HW] slab per block
-  const int Kp = kb > 0 ? 256 : (K + 63) / 64 * 64;
-  const int Kall = kb > 0 ? kb * 256 : Kp;          // rows of the text matrices
+  const bool bwd = a.dx != nullptr;
   CUtensorMap m_xs, m_t, m_tt, m_dx, m_g;
   int rcode;
-  {
-    const uint64_t dims[3] = {(uint64_t)HW, (uint64_t)D, (uint64_t)B};
-    const uint64_t xdims[3] = {(uint64_t)HW, (uint64_t)D, (uint64_t)(kb > 0 ? 1 : B)};
-    const uint64_t str[3] = {2, (uint64_t)HW * 2, (uint64_t)D * HW * 2};
-    const uint32_t box_s[3] = {64, 64, 1};
-    if ((rcode = make_tmap_bf16(&m_xs, xsrc, 3, xdims, str, box_s, "pair map_x_s"))) return rcode;
-    const uint32_t box_o[3] = {32, 32, 1};
-    if ((rcode = make_tmap_bf16(&m_dx, bwd ? dx : xsrc, 3, bwd ? dims : xdims, str, box_o, "pair map_dx"))) return rcode;
-    const uint64_t tdims[2] = {(uint64_t)D, (uint64_t)Kall}, tstr[2] = {2, (uint64_t)D * 2};
-    const uint32_t tbox[2] = {64, (uint32_t)(Kp / 2)};
-    if ((rcode = make_tmap_bf16(&m_t, t_bf16, 2, tdims, tstr, tbox, "pair map_t"))) return rcode;
-    const uint64_t ttdims[2] = {(uint64_t)Kall, (uint64_t)D}, ttstr[2] = {2, (uint64_t)Kall * 2};
-    const uint32_t ttbox[2] = {64, 128};
-    if ((rcode = make_tmap_bf16(&m_tt, bwd ? tt_bf16 : t_bf16, 2, bwd ? ttdims : tdims, bwd ? ttstr : tstr,
-                                bwd ? ttbox : tbox, "pair map_tt"))) return rcode;
-  }
-  {
+  if ((rcode = make_operand_maps(a, 128, {"pair map_x_s", "pair map_t", "pair map_tt"}, &m_xs, &m_t, &m_tt))) return rcode;
+  // dX [B][D][HW] (forward only: X again, unread)
+  if ((rcode = make_xmap(&m_dx, bwd ? a.dx : a.xsrc, a, bwd || a.kb == 0 ? a.B : 1, 32, 32, "pair map_dx"))) return rcode;
+  if (a.g_out != nullptr) {
     // G [B][HW][Kp] bf16: a tile is stored exactly as it sits in shared memory (four K-major 128B-swizzled sub-tiles)
-    const uint64_t gdims[3] = {(uint64_t)Kp, (uint64_t)HW, (uint64_t)B};
-    const uint64_t gstr[3] = {2, (uint64_t)Kp * 2, (uint64_t)HW * Kp * 2};
+    const int Kp = launch_kp(a);
+    const uint64_t gdims[3] = {(uint64_t)Kp, (uint64_t)a.HW, (uint64_t)a.B};
+    const uint64_t gstr[3] = {2, (uint64_t)Kp * 2, (uint64_t)a.HW * Kp * 2};
     const uint32_t gbox[3] = {64, 128, 1};
-    if (g_out != nullptr) {
-      if ((rcode = make_tmap_bf16(&m_g, g_out, 3, gdims, gstr, gbox, "pair map_g"))) return rcode;
-    } else {
-      m_g = m_dx;
-    }
+    if ((rcode = make_tmap_bf16(&m_g, a.g_out, 3, gdims, gstr, gbox, "pair map_g"))) return rcode;
+  } else {
+    m_g = m_dx;
   }
   Params prm;
-  prm.store_g = g_out != nullptr;
-  prm.dbg = debug_timing_buffer();
-  prm.B = B; prm.D = D; prm.K = K; prm.Kp = Kp; prm.HW = HW;
-  prm.tiles_per_img = (int)((HW + kTilePx - 1) / kTilePx);
-  if ((int64_t)B * prm.tiles_per_img > 0x3fffffff) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: too many tiles");
-  prm.n_tiles = B * prm.tiles_per_img;
-  prm.tpi_magic = prm.tiles_per_img == 1 ? 0xffffffffu : (uint32_t)(0x100000000ull / (uint64_t)prm.tiles_per_img);
-  prm.n_pairs = (prm.n_tiles + 1) / 2;
-  prm.x = reinterpret_cast<const __nv_bfloat16*>(xsrc);
-  prm.dx = reinterpret_cast<__nv_bfloat16*>(dx);
-  prm.ablate = 0;
-#ifdef RC_BRINGUP      // ablation switches of the bring-up build (tools/ablate_pair.py); the shipped library has no environment knobs
-  { const char* ab = getenv("RANGECLIP_B200_ABLATE"); prm.ablate = ab ? atoi(ab) : 0; }
-#endif
-  prm.wide = (HW % 16 == 0) && (reinterpret_cast<uintptr_t>(xsrc) % 32 == 0) && (reinterpret_cast<uintptr_t>(dx) % 32 == 0);
-  prm.inv_norm = inv_norm; prm.y = y; prm.w = w; prm.inv_tau = inv_tau; prm.grad_scale = grad_scale;
-  prm.w_sum_in = w_sum_in; prm.lse = lse; prm.loss_sum = loss_sum; prm.w_sum = w_sum; prm.dlogtau = dlogtau;
-  prm.keep_w = keep_w; prm.lse_in = lse_in; prm.kb = kb; prm.acc_dx = acc_dx;
-  prm.k_dev = k_dev; prm.log_tau_dev = log_tau_dev;
-  if (kb > 0 && (prm.tiles_per_img & 1)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: HW must be a multiple of 256");
-  int n_clusters = num_sms() / 2;
-  if (n_clusters > prm.n_pairs) n_clusters = prm.n_pairs;
-  const int grid = 2 * n_clusters;
+  int grid = 0;
+  if ((rcode = fill_tiling(prm, a, &grid))) return rcode;
+  prm.store_g = a.g_out != nullptr;
+  prm.wide = (a.HW % 16 == 0) && (reinterpret_cast<uintptr_t>(a.xsrc) % 32 == 0) && (reinterpret_cast<uintptr_t>(a.dx) % 32 == 0);
+  prm.x = reinterpret_cast<const __nv_bfloat16*>(a.xsrc);
+  prm.k_dev = a.k_dev; prm.log_tau_dev = a.log_tau_dev;
   auto launch = [&](auto kernel) -> int {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) return fail(RC_ERR_CUDA, "rc_infonce_bf16(pair): smem opt-in: %s", cudaGetErrorString(e));
     kernel<<<grid, kThreads, kSmemBytes, s>>>(m_xs, m_t, m_tt, m_dx, m_g, prm);
     return check_launch("rc_infonce_bf16(pair)");
   };
-  if (rep == 4) return bwd ? launch(infonce_umma_pair_kernel<true, 4, false>) : launch(infonce_umma_pair_kernel<false, 4, false>);
-  if (keep_w || lse_in != nullptr || kb > 0 || acc_dx) return bwd ? launch(infonce_umma_pair_kernel<true, 1, true>) : launch(infonce_umma_pair_kernel<false, 1, true>);
+  if (a.rep == 4) return bwd ? launch(infonce_umma_pair_kernel<true, 4, false>) : launch(infonce_umma_pair_kernel<false, 4, false>);
+  if (launch_kblocked(a)) return bwd ? launch(infonce_umma_pair_kernel<true, 1, true>) : launch(infonce_umma_pair_kernel<false, 1, true>);
   return bwd ? launch(infonce_umma_pair_kernel<true, 1, false>) : launch(infonce_umma_pair_kernel<false, 1, false>);
 }
 
