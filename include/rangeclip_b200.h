@@ -301,6 +301,14 @@ int rc_eval_topk_dyn_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t
                           int64_t* out /*nullable*/, const int64_t* gt, const uint8_t* E, const int64_t* cmap, int C,
                           int64_t* hist /*nullable [5][C]*/, int64_t* counters /*[3]*/,
                           void* workspace, int64_t workspace_bytes, void* stream);
+/* rc_eval_topk_bf16 / _hist_bf16 / _dyn_bf16 on the decoder's half-resolution rows x [B][D][h*w] (the output_conv result,
+ * SURVEY 8f-1): the top-k of row (i, j) is the top-k of the four full-resolution pixels (2i+a, 2j+b) of the nearest-x2
+ * upsampled tensor; out [B][k][2h][2w] and gt [B][2h][2w] are FULL resolution.  k_dev nullable (NULL: K valid rows);
+ * out and hist optional, at least one given; hist / counters are added to.  h*w % 8 == 0. */
+int rc_eval_topk_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int h, int w, const void* t_bf16, int K,
+                           const int32_t* k_dev, const int64_t* index_map, int k, int64_t* out, const int64_t* gt,
+                           const uint8_t* E, const int64_t* cmap, int C, int64_t* hist, int64_t* counters,
+                           void* workspace, int64_t workspace_bytes, void* stream);
 int rc_eval_hist(const int64_t* gt, const int64_t* topk, int B, int64_t HW, int k,
                  const uint8_t* E, const int64_t* cmap, int C,
                  int64_t* hist /*[5][C]*/, int64_t* counters /*[3]*/, void* stream);

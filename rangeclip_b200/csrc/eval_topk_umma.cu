@@ -11,6 +11,7 @@
 #include "umma.cuh"
 #include "eval_metrics.cuh"
 #include <float.h>
+#include <type_traits>
 
 namespace rc {
 using namespace umma;
@@ -61,6 +62,7 @@ struct Params {
   int C;
   unsigned long long* hist;              // [5][C]
   unsigned long long* counters;          // [3]
+  int w;                                 // R = 4: width of the half-resolution rows (HW = h * w); out / gt are [2h][2w]
 };
 
 // KT > 0: compile-time k (the insertion network has exactly k stages); KT == 0: run-time k <= kMaxK
@@ -162,7 +164,10 @@ __device__ __forceinline__ uint32_t push_gt(uint32_t m, float v, float kth) {
 // barriers of both CTAs, the scan warps of both CTAs release the S buffer at the leader.
 // P = scan threads per pixel (2 or 4): each keeps its own running top-k over 256 / P columns of every block; more lists mean
 // more insertions in total but twice the warps to hide the dependent chains behind.
-template <int KT, bool kPair, int P>
+// R = targets per row: 1, or 4 when the rows are the decoder's half-resolution output (SURVEY 8f-1) and every row stands for
+// the 2x2 block (2i + a, 2j + b) of the nearest-x2 upsampled map -- the scan is the same, the epilogue writes the ids to the
+// block's four pixels and scores each of them against its own full-resolution ground truth.
+template <int KT, bool kPair, int P, int R = 1>
 __global__ void __launch_bounds__(128 + 128 * P, 1)
 eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][HW], box (64 px, 64 d, 1)
                       const __grid_constant__ CUtensorMap map_t,    // T [Kp][D], box (64 d, 256 rows; pair: 128 rows), OOB rows = 0
@@ -469,30 +474,59 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
         int64_t ids[kMaxK];
 #pragma unroll
         for (int j = 0; j < kMaxK; ++j) ids[j] = (inb && j < prm.k && bi[j] >= 0) ? __ldg(prm.index_map + bi[j]) : -1;
-        if (inb && prm.out != nullptr) {
+        auto id_of = [&](int j) {
+          int64_t v = ids[0];
 #pragma unroll
-          for (int j = 0; j < kMaxK; ++j)
-            if (j < prm.k) prm.out[((int64_t)b * prm.k + j) * prm.HW + px] = ids[j];
-        }
-        if (prm.hist != nullptr) {
-          // Fused metrics: the pixel's top-k ids never leave the registers on their way into the five class histograms
-          // (warp-aggregated atomics: one per distinct class per warp); same per-pixel function as rc_eval_hist.
+          for (int q = 1; q < kMaxK; ++q) v = (j == q) ? ids[q] : v;
+          return v;
+        };
+        // Fused metrics: the pixel's top-k ids never leave the registers on their way into the five class histograms
+        // (warp-aggregated atomics: one per distinct class per warp); same per-pixel function as rc_eval_hist.
+        auto count = [&](int64_t g) {
           PixelMetric m;
           m.ok = false; m.ge = 0; m.p1 = 0; m.orc = 0; m.top1_same = false; m.orc_same = false; m.any_eq1 = false; m.any_eqk = false;
-          if (inb) {
-            m = pixel_metric(__ldg(prm.gt + (int64_t)b * prm.HW + px), prm.k, [&](int j) {
-              int64_t v = ids[0];
-#pragma unroll
-              for (int q = 1; q < kMaxK; ++q) v = (j == q) ? ids[q] : v;
-              return v;
-            }, prm.E, prm.cmap, prm.C);
-          }
+          if (inb) m = pixel_metric(g, prm.k, id_of, prm.E, prm.cmap, prm.C);
           if (m.ok) { m_c1 += m.any_eq1 ? 1u : 0u; m_ck += m.any_eqk ? 1u : 0u; m_tot += 1u; }
           warp_agg_add(prm.hist + 0 * (int64_t)prm.C, m.ge, m.ok);
           warp_agg_add(prm.hist + 1 * (int64_t)prm.C, m.p1, m.ok);
           warp_agg_add(prm.hist + 2 * (int64_t)prm.C, m.ge, m.ok && m.top1_same);
           warp_agg_add(prm.hist + 3 * (int64_t)prm.C, m.orc, m.ok);
           warp_agg_add(prm.hist + 4 * (int64_t)prm.C, m.ge, m.ok && m.orc_same);
+        };
+        if (R == 1) {
+          if (inb && prm.out != nullptr) {
+#pragma unroll
+            for (int j = 0; j < kMaxK; ++j)
+              if (j < prm.k) prm.out[((int64_t)b * prm.k + j) * prm.HW + px] = ids[j];
+          }
+          if (prm.hist != nullptr) count(inb ? __ldg(prm.gt + (int64_t)b * prm.HW + px) : 0);
+        } else {
+          // row (i, j) = full-resolution pixels (2i + a, 2j + c) of a [2h][2w] map: per image row a the two pixels are adjacent
+          // from an even index, so each id is one 16-byte store per image row and their gt words one 16-byte load
+          const int i = px / prm.w, jx = px - i * prm.w;
+          const int64_t W2 = 2 * (int64_t)prm.w, HW4 = 4 * prm.HW;
+          const int64_t p00 = 2 * (int64_t)i * W2 + 2 * jx;
+          if (inb && prm.out != nullptr) {
+#pragma unroll
+            for (int j = 0; j < kMaxK; ++j)
+              if (j < prm.k) {
+                longlong2* o = reinterpret_cast<longlong2*>(prm.out + ((int64_t)b * prm.k + j) * HW4 + p00);
+                const longlong2 v = make_longlong2(ids[j], ids[j]);
+                o[0] = v;
+                o[W2 / 2] = v;
+              }
+          }
+          if (prm.hist != nullptr) {
+            longlong2 g0 = make_longlong2(0, 0), g1 = g0;
+            if (inb) {
+              const longlong2* gp = reinterpret_cast<const longlong2*>(prm.gt + (int64_t)b * HW4 + p00);
+              g0 = __ldg(gp);
+              g1 = __ldg(gp + W2 / 2);
+            }
+            // the four pixels share the id list and are counted one by one, exactly as the upsampled launch counts them
+#pragma unroll 1
+            for (int q = 0; q < 4; ++q) count(q == 0 ? g0.x : q == 1 ? g0.y : q == 2 ? g1.x : g1.y);
+          }
         }
       }
     }
@@ -525,13 +559,19 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
 static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16, int K,
                                const int64_t* index_map, int k, int64_t* out, const int64_t* gt, const uint8_t* E,
                                const int64_t* cmap, int C, int64_t* hist, int64_t* counters, void* workspace,
-                               int64_t workspace_bytes, void* stream, const char* who, const int32_t* k_dev = nullptr) {
+                               int64_t workspace_bytes, void* stream, const char* who, const int32_t* k_dev = nullptr,
+                               int rep_w = 0) {
+  // rep_w = 0: one target per row (x is [B][D][HW], out / gt [B][HW]); rep_w = w > 0: x holds the half-resolution rows
+  // [B][D][h*w] (HW = h*w) and out / gt are the full-resolution [B][2h][2w] maps (four targets per row)
   using namespace rc;
   RC_REQUIRE(x && t_bf16 && index_map && (out || hist), "%s: null pointer", who);
   RC_REQUIRE(B >= 0 && HW >= 0 && K >= 1 && k >= 1 && k <= topk::kMaxK && k <= K, "%s: bad shape (k=%d K=%d)", who, k, K);
   if (hist != nullptr) RC_REQUIRE(gt && E && cmap && counters && C >= 1, "%s: the fused metrics need gt, E, cmap, counters and C >= 1", who);
   if (D < 64 || D > 512 || D % 64 != 0) return fail(RC_ERR_UNSUPPORTED, "%s: D=%d must be a multiple of 64 and <= 512", who, D);
   if (HW % 8 != 0) return fail(RC_ERR_UNSUPPORTED, "%s: HW=%lld must be a multiple of 8", who, (long long)HW);
+  if (rep_w > 0)             // 16-byte stores of the ids / loads of the gt words (pixel pairs from an even index)
+    RC_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0 && (reinterpret_cast<uintptr_t>(gt) & 15) == 0,
+               "%s: out and gt must be 16-byte aligned", who);
   RC_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(t_bf16) & 15) == 0,
              "%s: x and t must be 16-byte aligned", who);
   if (B == 0 || HW == 0) return RC_OK;
@@ -568,6 +608,7 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   prm.index_map = index_map; prm.out = out; prm.k_dev = k_dev;
   prm.gt = gt; prm.E = E; prm.cmap = cmap; prm.C = C;
   prm.hist = reinterpret_cast<unsigned long long*>(hist); prm.counters = reinterpret_cast<unsigned long long*>(counters);
+  prm.w = rep_w;
   // CTA pairs (two tiles per cluster, text chunks shared between the two SMs) whenever there is more than one tile
   const bool pair = prm.n_tiles >= 2 && (prm.n_blocks >= 2 || k == 1);       // one text block per tile: nothing to share, the coupling costs 5 %
   CUtensorMap m_tp = m_t;
@@ -605,14 +646,18 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   // Two scan threads per pixel.  Measured, not adopted (P = 4, 640 threads, setmaxnreg 40 / 104): four lists per pixel mean 23 %
   // more insertions and the scan is close to its instruction-throughput bound (ALU + FMA pipe at one warp instruction per two
   // cycles each): K = 1024 top-5 1041 against 1147 Mpix/s, K = 256 2258 against 2764.
-  if (pair) {
-    if (k == 1) return launch(topk::eval_topk_umma_kernel<1, true, 2>, true, 384);
-    if (k == 5) return launch(topk::eval_topk_umma_kernel<5, true, 2>, true, 384);
-    return launch(topk::eval_topk_umma_kernel<0, true, 2>, true, 384);
-  }
-  if (k == 1) return launch(topk::eval_topk_umma_kernel<1, false, 2>, false, 384);
-  if (k == 5) return launch(topk::eval_topk_umma_kernel<5, false, 2>, false, 384);
-  return launch(topk::eval_topk_umma_kernel<0, false, 2>, false, 384);
+  auto dispatch = [&](auto r) -> int {
+    constexpr int R = decltype(r)::value;
+    if (pair) {
+      if (k == 1) return launch(topk::eval_topk_umma_kernel<1, true, 2, R>, true, 384);
+      if (k == 5) return launch(topk::eval_topk_umma_kernel<5, true, 2, R>, true, 384);
+      return launch(topk::eval_topk_umma_kernel<0, true, 2, R>, true, 384);
+    }
+    if (k == 1) return launch(topk::eval_topk_umma_kernel<1, false, 2, R>, false, 384);
+    if (k == 5) return launch(topk::eval_topk_umma_kernel<5, false, 2, R>, false, 384);
+    return launch(topk::eval_topk_umma_kernel<0, false, 2, R>, false, 384);
+  };
+  return rep_w > 0 ? dispatch(std::integral_constant<int, 4>()) : dispatch(std::integral_constant<int, 1>());
 }
 
 extern "C" int rc_eval_topk_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16, int K,
@@ -641,4 +686,16 @@ extern "C" int rc_eval_topk_dyn_bf16(const void* x, rc_dtype x_dtype, int B, int
   RC_REQUIRE(k_dev != nullptr, "rc_eval_topk_dyn_bf16: k_dev is required");
   return eval_topk_bf16_impl(x, x_dtype, B, D, HW, t_bf16, K, index_map, k, out, gt, E, cmap, C, hist, counters, workspace,
                              workspace_bytes, stream, "rc_eval_topk_dyn_bf16", k_dev);
+}
+
+/* The same on the decoder's half-resolution rows x [B][D][h*w] (the output_conv result): row (i, j) stands for the 2x2 block
+ * (2i + a, 2j + b) of the nearest-x2 upsampled map, whose four pixels have the same top-k; out and gt are full resolution. */
+extern "C" int rc_eval_topk_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int h, int w, const void* t_bf16, int K,
+                                      const int32_t* k_dev, const int64_t* index_map, int k, int64_t* out, const int64_t* gt,
+                                      const uint8_t* E, const int64_t* cmap, int C, int64_t* hist, int64_t* counters,
+                                      void* workspace, int64_t workspace_bytes, void* stream) {
+  RC_REQUIRE(x && t_bf16 && index_map && (out || hist), "rc_eval_topk_bf16_rep4: null pointer");
+  RC_REQUIRE(h >= 1 && w >= 1, "rc_eval_topk_bf16_rep4: bad shape (h=%d w=%d)", h, w);
+  return eval_topk_bf16_impl(x, x_dtype, B, D, (int64_t)h * w, t_bf16, K, index_map, k, out, gt, E, cmap, C, hist, counters,
+                             workspace, workspace_bytes, stream, "rc_eval_topk_bf16_rep4", k_dev, w);
 }

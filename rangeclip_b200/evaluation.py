@@ -53,13 +53,40 @@ def build_reduced_candidates_device(segmentation: torch.Tensor, candidate_text_e
     return reduced, tb, kinfo
 
 
+def _check_shared2x2(pixel_embeddings, segmentation):
+    """``shared2x2=True`` takes the decoder's ``output_conv`` result [B,D,h,w] and the full-resolution segmentation [B,2h,2w]."""
+    if pixel_embeddings.dim() != 4 or segmentation is None or not pixel_embeddings.is_cuda or not segmentation.is_cuda:
+        raise RuntimeError("shared2x2: needs CUDA tensors, embeddings [B, D, h, w] and a segmentation")
+    B, _, h, w = pixel_embeddings.shape
+    if tuple(segmentation.shape) != (B, 2 * h, 2 * w):
+        raise RuntimeError(f"shared2x2: the segmentation must be [B, 2h, 2w] = [{B}, {2 * h}, {2 * w}], "
+                           f"got {list(segmentation.shape)}")
+
+
 def predict_from_embeddings(pixel_embeddings, candidate_text_embeddings, segmentation, num_negatives=300, top_k=5,
-                            precision="auto", candidate_builder="reference"):
+                            precision="auto", candidate_builder="reference", shared2x2=False):
     """model.py:144-173 given the decoder output: returns (topk ids [B,k,H,W] int64 in the ORIGINAL
     index space, L2-normalised embeddings).  The [B,Kr,HW] logits are never materialised.
     ``candidate_builder="device"``: the reduced candidate set is built on the GPU and its size stays there
-    (``build_reduced_candidates_device``): no host synchronisation; a pixel gets -1 where fewer than ``top_k`` candidates exist."""
+    (``build_reduced_candidates_device``): no host synchronisation; a pixel gets -1 where fewer than ``top_k`` candidates exist.
+    ``shared2x2=True``: ``pixel_embeddings`` is the decoder's ``output_conv`` result [B,D,H/2,W/2], before the tail
+    (nearest x2 -> normalize, decoder.py:113-115) that makes every 2x2 block one embedding; the top-k is ranked once per
+    block (rc_eval_topk_bf16_rep4, tensor cores only) and the ids come out at full resolution [B,k,H,W].  The second
+    result is then the L2-normalised half-resolution rows."""
     total = candidate_text_embeddings.shape[0]
+    if shared2x2:
+        if precision == "fp32":
+            raise ValueError("shared2x2=True runs on the tensor cores only (precision 'auto' or 'bf16')")
+        _check_shared2x2(pixel_embeddings, segmentation)
+        if candidate_builder == "device" and device_candidates_supported(pixel_embeddings, total):
+            reduced, tb, kinfo = build_reduced_candidates_device(segmentation, candidate_text_embeddings, num_negatives)
+            topk = ops.eval_topk_rep4(pixel_embeddings, tb, reduced, min(top_k, total), k_dev=kinfo)
+        else:
+            reduced = build_reduced_candidates(segmentation, total, num_negatives)
+            index_tensor = torch.tensor(reduced, device=pixel_embeddings.device)
+            t_norm, _, _ = ops.text_prepare(candidate_text_embeddings, index_tensor, want_f32=True)
+            topk = ops.eval_topk_rep4(pixel_embeddings, ops.text_to_bf16(t_norm)[0], index_tensor, min(top_k, len(reduced)))
+        return topk, F.normalize(pixel_embeddings, dim=1)
     if candidate_builder == "device" and segmentation is not None and device_candidates_supported(pixel_embeddings, total) \
             and precision != "fp32":
         reduced, tb, kinfo = build_reduced_candidates_device(segmentation, candidate_text_embeddings, num_negatives)
@@ -73,22 +100,26 @@ def predict_from_embeddings(pixel_embeddings, candidate_text_embeddings, segment
 
 
 def predict_and_accumulate(pixel_embeddings, candidate_text_embeddings, segmentation, accumulator, num_negatives=300, top_k=5,
-                           batch_index=None, want_ids=True, candidate_builder="reference"):
+                           batch_index=None, want_ids=True, candidate_builder="reference", shared2x2=False):
     """``predict_from_embeddings`` + ``MetricAccumulator.update`` as one fused kernel per batch: same reduced candidate
     set (same ``random.sample`` draw, Q6), same ids, same histograms -- the ids never make the round trip through HBM
     between the two steps.  Returns (topk ids or None, L2-normalised embeddings).  ``candidate_builder="device"``: see
-    ``predict_from_embeddings`` -- the whole validation batch then runs without a host synchronisation."""
+    ``predict_from_embeddings`` -- the whole validation batch then runs without a host synchronisation.
+    ``shared2x2=True``: ``pixel_embeddings`` is the ``output_conv`` result [B,D,H/2,W/2] (see ``predict_from_embeddings``);
+    every full-resolution pixel of ``segmentation`` [B,H,W] is counted, as on the upsampled tensor."""
     total = candidate_text_embeddings.shape[0]
+    if shared2x2:
+        _check_shared2x2(pixel_embeddings, segmentation)
     if candidate_builder == "device" and device_candidates_supported(pixel_embeddings, total):
         reduced, tb, kinfo = build_reduced_candidates_device(segmentation, candidate_text_embeddings, num_negatives)
         ids = accumulator.update_from_device_candidates(pixel_embeddings, tb, kinfo, reduced, segmentation, min(top_k, total),
-                                                        batch_index=batch_index, want_ids=want_ids)
+                                                        batch_index=batch_index, want_ids=want_ids, shared2x2=shared2x2)
         return ids, F.normalize(pixel_embeddings, dim=1)
     reduced = build_reduced_candidates(segmentation, total, num_negatives)
     index_tensor = torch.tensor(reduced, device=pixel_embeddings.device)
     t_norm, _, _ = ops.text_prepare(candidate_text_embeddings, index_tensor, want_f32=True)
     ids = accumulator.update_from_embeddings(pixel_embeddings, t_norm, index_tensor, segmentation, min(top_k, len(reduced)),
-                                             batch_index=batch_index, want_ids=want_ids)
+                                             batch_index=batch_index, want_ids=want_ids, shared2x2=shared2x2)
     return ids, F.normalize(pixel_embeddings, dim=1)
 
 
@@ -129,22 +160,34 @@ class MetricAccumulator:
 
     def update_from_embeddings(self, pixel_embeddings: torch.Tensor, t_norm: torch.Tensor, index_tensor: torch.Tensor,
                                segmentation: torch.Tensor, top_k: int = 5, batch_index: Optional[int] = None,
-                               t_bf16=None, want_ids: bool = True):
+                               t_bf16=None, want_ids: bool = True, shared2x2: bool = False):
         """One validation batch straight from the pixel embeddings: ONE kernel does the top-k over the text rows and the
-        metric histograms (rc_eval_topk_hist_bf16); the ids are returned only if ``want_ids``."""
+        metric histograms (rc_eval_topk_hist_bf16); the ids are returned only if ``want_ids``.  ``shared2x2=True``: the
+        embeddings are the ``output_conv`` result [B,D,H/2,W/2] of the full-resolution ``segmentation`` (rc_eval_topk_bf16_rep4)."""
         self._hist.zero_()
-        ids = ops.eval_topk_hist(pixel_embeddings, t_norm, index_tensor, top_k, segmentation, self.E, self.cmap, self._hist,
-                                 self.counters, t_bf16=t_bf16, want_ids=want_ids)
+        if shared2x2:
+            _check_shared2x2(pixel_embeddings, segmentation)
+            tb = t_bf16 if t_bf16 is not None else ops.text_to_bf16(t_norm)[0]
+            ids = ops.eval_topk_rep4(pixel_embeddings, tb, index_tensor, top_k, segmentation, self.E, self.cmap, self._hist,
+                                     self.counters, want_ids=want_ids)
+        else:
+            ids = ops.eval_topk_hist(pixel_embeddings, t_norm, index_tensor, top_k, segmentation, self.E, self.cmap, self._hist,
+                                     self.counters, t_bf16=t_bf16, want_ids=want_ids)
         ops.eval_fold(self._hist, self.n_batches if batch_index is None else batch_index, self.acc, self.first_seen)
         self.n_batches += 1
         return ids
 
     def update_from_device_candidates(self, pixel_embeddings, t_bf16, kinfo, index_tensor, segmentation, top_k: int = 5,
-                                      batch_index: Optional[int] = None, want_ids: bool = True):
+                                      batch_index: Optional[int] = None, want_ids: bool = True, shared2x2: bool = False):
         """``update_from_embeddings`` for a candidate set whose size lives on the device (``build_reduced_candidates_device``)."""
         self._hist.zero_()
-        ids = ops.eval_topk_dyn(pixel_embeddings, t_bf16, kinfo, index_tensor, top_k, segmentation, self.E, self.cmap, self._hist,
-                                self.counters, want_ids=want_ids)
+        if shared2x2:
+            _check_shared2x2(pixel_embeddings, segmentation)
+            ids = ops.eval_topk_rep4(pixel_embeddings, t_bf16, index_tensor, top_k, segmentation, self.E, self.cmap, self._hist,
+                                     self.counters, k_dev=kinfo, want_ids=want_ids)
+        else:
+            ids = ops.eval_topk_dyn(pixel_embeddings, t_bf16, kinfo, index_tensor, top_k, segmentation, self.E, self.cmap,
+                                    self._hist, self.counters, want_ids=want_ids)
         ops.eval_fold(self._hist, self.n_batches if batch_index is None else batch_index, self.acc, self.first_seen)
         self.n_batches += 1
         return ids

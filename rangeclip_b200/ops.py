@@ -674,6 +674,48 @@ def eval_topk_dyn(x: torch.Tensor, t_bf16: torch.Tensor, k_dev: torch.Tensor, in
     return out
 
 
+def eval_topk_rep4(x: torch.Tensor, t_bf16: torch.Tensor, index_map: torch.Tensor, k: int, gt=None, E_u8=None, cmap=None,
+                   hist=None, counters=None, k_dev=None, want_ids: bool = True):
+    """``eval_topk_dyn`` on the decoder's half-resolution rows (the ``output_conv`` result, SURVEY 8f-1): ``x`` [B,D,h,w] bf16 or
+    fp32 stands for its nearest-x2 upsampled, normalised map, whose 2x2 blocks share one embedding and hence one top-k.  The
+    ranking runs once per row; the ids [B,k,2h,2w] (returned when ``want_ids``) and, with ``hist`` / ``counters``, the metrics
+    of the four pixels against the full-resolution ``gt`` [B,2h,2w] are those of the upsampled launch (rc_eval_topk_bf16_rep4).
+    ``t_bf16`` [Kp,D] holds the normalised rows of ``index_map`` [K]; ``k_dev`` (int32, first entry, optional) how many are valid."""
+    _need_cuda(x, t_bf16, k_dev, index_map, gt, E_u8, cmap, hist, counters)
+    if x.dim() != 4:
+        raise RuntimeError("eval_topk_rep4: x must be [B, D, h, w]")
+    B, D, h, w = x.shape
+    x = x.contiguous()
+    if not topk_bf16_supported(D, h * w):
+        raise RuntimeError(f"eval_topk_rep4: the tensor-core kernel does not cover D={D}, h*w={h * w}")
+    K = int(index_map.numel())
+    k = min(int(k), K)
+    out = torch.empty((B, k, 2 * h, 2 * w), device=x.device, dtype=torch.int64) if (want_ids or hist is None) else None
+    index_map = index_map.to(torch.int64).contiguous()
+    if (gt is not None or hist is not None) and (gt is None or tuple(gt.shape) != (B, 2 * h, 2 * w)):
+        raise RuntimeError(f"eval_topk_rep4: gt must be the full-resolution [B, 2h, 2w] = [{B}, {2 * h}, {2 * w}] segmentation")
+    C = 0
+    if hist is not None:
+        C = cmap.numel()
+        if hist.dtype != torch.int64 or tuple(hist.shape) != (5, C) or counters.dtype != torch.int64 or counters.numel() != 3:
+            raise RuntimeError("eval_topk_rep4: hist must be int64 [5, C], counters int64 [3]")
+        gt = gt.to(torch.int64).contiguous()
+        if gt.data_ptr() % 16:               # the kernel loads the gt words of two adjacent pixels at once
+            gt = gt.clone()
+        E_u8, cmap = E_u8.contiguous(), cmap.to(torch.int64).contiguous()
+    L = _lib.lib()
+    xdt = _dt(x)
+    ws, ws_bytes = None, 0
+    if xdt == RC_F32:
+        ws_bytes = int(L.rc_infonce_workspace_bytes(B, D, h * w, K, xdt))
+        ws = torch.empty(ws_bytes, device=x.device, dtype=torch.uint8)
+    kd = k_dev.to(torch.int32) if k_dev is not None else None
+    check(L.rc_eval_topk_bf16_rep4(_p(x), xdt, B, D, h, w, _p(t_bf16), K, _p(kd), _p(index_map), k, _p(out), _p(gt), _p(E_u8),
+                                   _p(cmap), C, _p(hist), _p(counters), _p(ws), ws_bytes, _stream(x)),
+          "rc_eval_topk_bf16_rep4")
+    return out
+
+
 def eval_hist(gt: torch.Tensor, topk: torch.Tensor, E_u8: torch.Tensor, cmap: torch.Tensor,
               hist: Optional[torch.Tensor] = None, counters: Optional[torch.Tensor] = None):
     """One batch of validate.py:88-139 as five class histograms + three counters (int64, added to)."""
@@ -1200,6 +1242,22 @@ def _(x, t_norm, index_map, k, gt, E_u8, cmap, hist, counters, t_bf16, want_ids)
     if not want_ids:
         return torch.empty(0, device=x.device, dtype=torch.int64)
     return torch.empty((x.shape[0], k) + tuple(x.shape[2:]), device=x.device, dtype=torch.int64)
+
+
+@_op("rangeclip::eval_topk_rep4", mutates_args=("hist", "counters"), device_types="cuda")
+def _op_eval_topk_rep4(x: torch.Tensor, t_bf16: torch.Tensor, index_map: torch.Tensor, k: int, gt: Optional[torch.Tensor],
+                       E_u8: Optional[torch.Tensor], cmap: Optional[torch.Tensor], hist: Optional[torch.Tensor],
+                       counters: Optional[torch.Tensor], k_dev: Optional[torch.Tensor], want_ids: bool) -> torch.Tensor:
+    ids = eval_topk_rep4(x, t_bf16, index_map, k, gt, E_u8, cmap, hist, counters, k_dev=k_dev, want_ids=want_ids)
+    return ids if ids is not None else torch.empty(0, device=x.device, dtype=torch.int64)
+
+
+@_op_eval_topk_rep4.register_fake
+def _(x, t_bf16, index_map, k, gt, E_u8, cmap, hist, counters, k_dev, want_ids):
+    if not want_ids and hist is not None:
+        return torch.empty(0, device=x.device, dtype=torch.int64)
+    k = min(k, index_map.numel())
+    return torch.empty((x.shape[0], k, 2 * x.shape[2], 2 * x.shape[3]), device=x.device, dtype=torch.int64)
 
 
 @_op("rangeclip::eval_fold", mutates_args=("acc", "first_seen"), device_types="cuda")
