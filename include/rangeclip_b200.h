@@ -94,7 +94,11 @@ int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t ld_b,
  *   RC_INFONCE_KEEP_WEIGHT  a row whose target is outside this launch keeps its weight (its one-hot term is dropped);
  *                           round 1 = forward launches with this flag: lse per block, loss_sum = sum w lse_blk - sum_{y in blk} w z_y
  *   RC_INFONCE_LSE_GIVEN    `lse` is an INPUT: the row's logsumexp over all candidates (logsumexp of the per-block values);
- *                           round 2 = backward launches with both flags: dx and dlogtau of each block add up to the full gradient */
+ *                           round 2 = backward launches with both flags: dx and dlogtau of each block add up to the full gradient
+ * rc_infonce_bf16_rep4 takes the same flags (D = 256 / 512, no dt): y4 holds each target relative to the launch's first
+ * row, w4 is 0 for every ignored target, lse is [B*hw] (one value per shared row: per block out, or in), and round 1's
+ * loss_sum = sum_q wtot_q lse_blk - sum_{y_qj in blk} w_qj z_qy with wtot_q = sum_j w_qj.  rc_infonce_bf16_dyn and
+ * rc_infonce_bf16_kblocks take one target per row only. */
 #define RC_INFONCE_KEEP_WEIGHT 2
 #define RC_INFONCE_LSE_GIVEN 4
 /* Backward launches (dx given, no dt) of D = 256 / 512 with K and log tau given by the host (rc_infonce_bf16, _rep4 and the

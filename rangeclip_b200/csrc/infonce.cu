@@ -291,9 +291,9 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   const int acc_dx = (flags & RC_INFONCE_ACCUMULATE_DX) ? 1 : 0;
   const float* lse_in = (flags & RC_INFONCE_LSE_GIVEN) ? lse : nullptr;
   if (acc_dx) RC_REQUIRE(bwd, "rc_infonce_bf16: RC_INFONCE_ACCUMULATE_DX needs dx");
-  if (keep_w || lse_in || acc_dx) {
-    if (!use_pair || rep != 1 || dt != nullptr)
-      return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: the K-blocked flags need D = 256 or 512, one target per row and no dText");
+  if (keep_w || lse_in || acc_dx) {      // rep = 1 or 4 (rc_infonce_bf16_dyn rejects these flags before it gets here)
+    if (!use_pair || dt != nullptr)
+      return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: the K-blocked flags need D = 256 or 512 and no dText");
     RC_REQUIRE(!(flags & RC_INFONCE_LSE_GIVEN) || lse != nullptr, "rc_infonce_bf16: RC_INFONCE_LSE_GIVEN needs lse");
   }
   if (rep != 1) {

@@ -162,6 +162,9 @@ __device__ __forceinline__ void relay_x_tile(int n_dchunks, uint64_t* xf, uint64
 
 // Target(s) and weight of the thread's pixel of tile t, read one tile ahead (`live`: t belongs to this cluster).
 // ok = 1 for a valid pixel; R = 4: the four targets, 8 bits each (K <= 256); ignored targets are sorted out when w is read.
+// In K-blocked launches a relative target outside [0, 256) (ignored, or in another block) aliases to some column of this
+// block here.  That is harmless only because the logit it picks up (exp_pass: sy[j]) is used solely under mine[j], which
+// gather_targets computes from the full 32-bit target.
 template <int R>
 __device__ __forceinline__ void load_pixel_scalars(const Tiling& prm, bool live, int t, int row, float& ok, float& w, int& y) {
   ok = 0.f; w = 0.f; y = -1;
@@ -252,7 +255,8 @@ __device__ __forceinline__ float row_max(uint32_t trow, int Kt, int cb, int Kh, 
 
 // The exp pass over this half's Kh columns of S (TMEM at trow, 16 columns per step): e = exp(z - m), kept in registers as
 // packed bf16 (pk), with sum = sum e and sez = sum e z (up to the scale zs) of the valid columns (k < Kt), and sy[j] = the
-// raw logit of target j if it lies in this half.  yi: the target (R = 1) or the four packed targets (R = 4).
+// raw logit of target j if it lies in this half.  yi: the target (R = 1) or the four packed targets (R = 4).  R = 4: sy[j]
+// may hold an aliased column's logit (load_pixel_scalars); every reader must guard it with mine[j].
 // (Measured, not adopted: the scale / sum / e*s arithmetic as packed fp32x2 -- FFMA2 / FADD2, 6 instead of 9 issued
 // instructions per two columns -- is 2.7 % slower, 2.57 against 2.50 ms.)
 template <int R>
@@ -305,8 +309,10 @@ __device__ __forceinline__ void exp_pass(uint32_t trow, int cb, int Kh, int Kt, 
 
 // Targets of the row: y_j, w_j (w_j = 0: ignored), mine[j] = target j lies in this half's columns [cb, cb + Kh),
 // wtot = sum_j w_j and tz = sum_j w_j sy[j] over the targets in this half.  R = 1 takes yi / wi from the pixel scalars;
-// R = 4 reads the four targets and weights of pixel m if its pixel-scalar flag `ok` is set.
-template <int R>
+// R = 4 reads the four targets and weights of pixel m if its pixel-scalar flag `ok` is set.  K-blocked launches with
+// keep_w (kKB): a target outside this launch's rows (y < 0 included) keeps its weight, so that wtot is the row's weight
+// over all blocks; ignored targets then carry w = 0 (rangeclip_b200.h, RC_INFONCE_KEEP_WEIGHT).
+template <int R, bool kKB>
 __device__ __forceinline__ void gather_targets(const Tiling& prm, int yi, float wi, float ok, int64_t m, int cb, int Kh,
                                                const float (&sy)[R], int (&yj)[R], float (&wj)[R], bool (&mine)[R],
                                                float& wtot, float& tz) {
@@ -322,7 +328,7 @@ __device__ __forceinline__ void gather_targets(const Tiling& prm, int yi, float 
     const int ya[4] = {y4.x, y4.y, y4.z, y4.w};
     const float wa[4] = {w4.x, w4.y, w4.z, w4.w};
 #pragma unroll
-    for (int j = 0; j < R; ++j) { yj[j] = ya[j]; wj[j] = ya[j] >= 0 ? wa[j] : 0.f; }
+    for (int j = 0; j < R; ++j) { yj[j] = ya[j]; wj[j] = (ya[j] >= 0 || (kKB && prm.keep_w)) ? wa[j] : 0.f; }
   }
   wtot = 0.f; tz = 0.f;
 #pragma unroll
@@ -347,7 +353,8 @@ __device__ __forceinline__ void add_peer_sums(const float* xch, int half, int ro
 }
 
 // The row's logsumexp (half 0; 0 in half 1), and its loss and weight added to loss / wsum.  K-blocked rounds with
-// lse_in: sum becomes exp(lse_in - m), so that 1 / sum = exp(m - lse) normalises this block's softmax.
+// lse_in: sum becomes exp(lse_in - m), so that 1 / sum = exp(m - lse) normalises this block's softmax.  lse_in is indexed
+// by the embedding row m (R = 4: one lse per shared row) or, in kb mode, by the pixel.
 template <bool kKB>
 __device__ __forceinline__ float row_lse(const Tiling& prm, bool valid, int px, int64_t m, int half, float ml, float wtot,
                                          float tz, float zs, float& sum, float& loss, float& wsum) {

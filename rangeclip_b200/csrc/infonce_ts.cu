@@ -83,6 +83,9 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
   const bool leader_cta = rank == 0;
+  // kb mode (every candidate block in one launch, rc_infonce_bf16_kblocks) exists for R = 1 only; without this the
+  // R = 4 K-blocked instantiation spills
+  constexpr bool kKbAll = kKB && R == 1;
   const int n_dchunks = prm.D / 64;      // 64-channel chunks of the S GEMM
   const int n_blk = prm.D / 64;          // 64-channel blocks of the dX GEMM
   const int n_kchunks = prm.Kp / 64;
@@ -129,10 +132,10 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       uint32_t it = 0;
       auto load_s = [&](int l) {
         load_text_s<kTStages>(prm, &map_t, smem + kOffT, bars->tfull, bars->tempty, it, 0, n_dchunks,
-                              text_row0<kKB>(prm, pair_of(l)), rank RC_WT);
+                              text_row0<kKbAll>(prm, pair_of(l)), rank RC_WT);
       };
       auto load_dx = [&](int l, int b0, int b1) {     // per 64-channel block: own 32 rows of T^T, all Kp columns (4 KB per 64 k)
-        const int koff = text_row0<kKB>(prm, pair_of(l));
+        const int koff = text_row0<kKbAll>(prm, pair_of(l));
         for (int blk = b0; blk < b1; ++blk, ++it) {
           const int st = it % kTStages;
           RC_WAIT(mbar_wait, &bars->tempty[st], ((it / kTStages) & 1) ^ 1, 2);
@@ -160,7 +163,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       // evict_last and the epilogue's (last) load marks them evict_first, so that kept lines are released once consumed.
       const uint64_t pol_keep = l2_policy_evict_last();
       for (int l = 0; l < my_pairs; ++l)
-        load_x_tile<kXStages, kKB, true>(prm, &map_x_s, smem, bars->xf, bars->xempty, xit, 2 * pair_of(l) + (int)rank, n_dchunks,
+        load_x_tile<kXStages, kKbAll, true>(prm, &map_x_s, smem, bars->xf, bars->xempty, xit, 2 * pair_of(l) + (int)rank, n_dchunks,
                                          pol_keep, 3 RC_WT);
     } else if (warp == 1 && leader_cta) {
       // =============================== MMA issuer (leader CTA) ================================
@@ -281,7 +284,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       const int px = tile_ok ? (tile - b * prm.tiles_per_img) * kTilePx + row : 0;
       const bool valid = tile_ok && px < prm.HW;
       const int64_t m = (int64_t)b * prm.HW + px;
-      const int Kt = (kKB && prm.kb > 0) ? min(256, prm.K - 256 * b) : prm.K;
+      const int Kt = (kKbAll && prm.kb > 0) ? min(256, prm.K - 256 * b) : prm.K;
       const float ok = nx_ok;
       const bool px_ok = ok != 0.f;
       const int yi = nx_y;
@@ -310,7 +313,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       float wj[R];
       bool mine[R];
       float wtot, tz;
-      gather_targets<R>(prm, yi, wi, ok, m, cb, Kh, sy, yj, wj, mine, wtot, tz);
+      gather_targets<R, kKB>(prm, yi, wi, ok, m, cb, Kh, sy, yj, wj, mine, wtot, tz);
       post_sums(xch, half, row, sum, sez, tz);
       // every softmax warp has read its S columns (tcgen05.wait::ld above): after this barrier the slot's columns may be
       // overwritten with P
@@ -394,7 +397,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       tile_coords(prm, 2 * pair_of(cu.l) + (int)rank, b, px0);
       cu.px = px0 + q * 32;
       cu.bo = b;
-      cu.bx = (kKB && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;
+      cu.bx = (kKbAll && prm.kb > 0) ? (b < prm.B ? 0 : 1) : b;
     };
     auto cursor_next = [&](Cursor& cu) {
       if (++cu.u == n_blk) { cu.u = 0; ++cu.l; cursor_pair(cu); }
@@ -541,7 +544,7 @@ int launch_infonce_ts(const InfoncePairArgs& a, cudaStream_t s) {
     kernel<<<grid, kThreads, kSmemBytes, s>>>(m_xs, m_t, m_tt, m_xe, m_dx, prm);
     return check_launch("rc_infonce_bf16(ts)");
   };
-  if (a.rep == 4) return launch(infonce_ts_kernel<4, false>);
+  if (a.rep == 4) return launch_kblocked(a) ? launch(infonce_ts_kernel<4, true>) : launch(infonce_ts_kernel<4, false>);
   if (launch_kblocked(a)) return launch(infonce_ts_kernel<1, true>);
   return launch(infonce_ts_kernel<1, false>);
 }

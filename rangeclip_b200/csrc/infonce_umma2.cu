@@ -117,6 +117,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
   const int warp = (int)(threadIdx.x >> 5);
   const uint32_t rank = cluster_ctarank();
   const bool leader_cta = rank == 0;
+  constexpr bool kKbAll = kKB && R == 1;      // kb mode (rc_infonce_bf16_kblocks) exists for R = 1 only
   const int n_dchunks = prm.D / 64;      // 64-channel chunks of the S GEMM
   const int n_blk = prm.D / 256;         // 256-channel blocks of the dX GEMM
   const int n_kchunks = prm.Kp / 64;
@@ -169,7 +170,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       // text ring, in MMA issue order: S(first), then per tile pair
       //   [S(next) first half] [dX(this) first blocks] [S(next) second half] [dX(this) remaining blocks]
       uint32_t it = 0;
-      auto koff_of = [&](int pj) -> int { return text_row0<kKB>(prm, pj); };
+      auto koff_of = [&](int pj) -> int { return text_row0<kKbAll>(prm, pj); };
       auto load_s = [&](int c_begin, int c_end, int koff) {
         load_text_s<kTStages>(prm, &map_t, smem + kOffT, bars->tfull, bars->tempty, it, c_begin, c_end, koff, rank RC_WT);
       };
@@ -201,7 +202,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       // while the dX GEMM of the previous pair runs)
       uint32_t xit = 0;
       for (int pj = cluster_id; pj < prm.n_pairs; pj += n_clusters)
-        load_x_tile<kXStages, kKB, false>(prm, &map_x_s, smem, bars->xf, bars->xempty, xit, 2 * pj + (int)rank, n_dchunks, 0, 1 RC_WT);
+        load_x_tile<kXStages, kKbAll, false>(prm, &map_x_s, smem, bars->xf, bars->xempty, xit, 2 * pj + (int)rank, n_dchunks, 0, 1 RC_WT);
     } else if (warp == 1 && leader_cta) {
       // =============================== MMA issuer (leader CTA) ================================
       // The whole warp runs the loop converged, so stage indices, addresses and descriptors live in uniform
@@ -348,7 +349,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       if (kBwd && prm.store_g && threadIdx.x == 128) tma_store_wait_read0();
       const int64_t m = (int64_t)b * prm.HW + px;
       // candidates in this tile's block (kb mode: the last block may be short; its zero pad rows are masked like any pad)
-      const int Kt = (kKB && prm.kb > 0) ? min(256, prm.K - 256 * b) : K_valid;
+      const int Kt = (kKbAll && prm.kb > 0) ? min(256, prm.K - 256 * b) : K_valid;
       const float ok = nx_ok;
       const bool px_ok = ok != 0.f;
       const int yi = nx_y;
@@ -381,7 +382,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       float wj[R];
       bool mine[R];
       float wtot, tz;
-      gather_targets<R>(prm, yi, wi, ok, m, cb, Kh, sy, yj, wj, mine, wtot, tz);
+      gather_targets<R, kKB>(prm, yi, wi, ok, m, cb, Kh, sy, yj, wj, mine, wtot, tz);
       post_sums(xch, half, row, sum, sez, tz);
       named_bar_sync(2, 256);
       add_peer_sums(xch, half, row, sum, sez, tz);
@@ -482,7 +483,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
         const int px0 = (t - b * prm.tiles_per_img) * kTilePx + (f_unit & 1) * 64;
         const int d = (f_unit >> 1) * 256 + (int)rank * 128 + row;
         f_b = b; f_px = px0; f_d = d - lane;
-        f_off = ((int64_t)((kKB && prm.kb > 0) ? 0 : b) * prm.D + d) * prm.HW + px0;      // kb mode: X has one image
+        f_off = ((int64_t)((kKbAll && prm.kb > 0) ? 0 : b) * prm.D + d) * prm.HW + px0;      // kb mode: X has one image
         const int64_t left = prm.HW - px0;
         f_n8 = left >= 64 ? 8 : (left > 0 ? (int)(left >> 3) : 0);
       }
@@ -649,7 +650,10 @@ int launch_infonce_pair(const InfoncePairArgs& a, cudaStream_t s) {
     kernel<<<grid, kThreads, kSmemBytes, s>>>(m_xs, m_t, m_tt, m_dx, m_g, prm);
     return check_launch("rc_infonce_bf16(pair)");
   };
-  if (a.rep == 4) return bwd ? launch(infonce_umma_pair_kernel<true, 4, false>) : launch(infonce_umma_pair_kernel<false, 4, false>);
+  if (a.rep == 4) {
+    if (launch_kblocked(a)) return bwd ? launch(infonce_umma_pair_kernel<true, 4, true>) : launch(infonce_umma_pair_kernel<false, 4, true>);
+    return bwd ? launch(infonce_umma_pair_kernel<true, 4, false>) : launch(infonce_umma_pair_kernel<false, 4, false>);
+  }
   if (launch_kblocked(a)) return bwd ? launch(infonce_umma_pair_kernel<true, 1, true>) : launch(infonce_umma_pair_kernel<false, 1, true>);
   return bwd ? launch(infonce_umma_pair_kernel<true, 1, false>) : launch(infonce_umma_pair_kernel<false, 1, false>);
 }

@@ -195,13 +195,17 @@ def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embed
         return loss, aux
     if shared2x2:
         K = int(contrast.shape[0])
-        if precision != "fp32" and D in (256, 512) and ops.bf16_path_supported(D, (H // 2) * (W // 2), K):
+        rows = (H // 2) * (W // 2)
+        # more than 256 contrast rows (their number is data dependent, model.py:268): the four-target kernel over blocks of
+        # 256 candidate rows (ops.infonce_kblocked_raw), for frozen text
+        kblocked = K > 256 and ops.kblocked_supported(D, rows) and not candidate_text_embeddings.requires_grad
+        if precision != "fp32" and D in (256, 512) and (ops.bf16_path_supported(D, rows, K) or kblocked):
             y, w = group_2x2(y.view(B, H, W)), group_2x2(w.view(B, H, W))
             loss = ops.infonce(pixel_embeddings, t_norm, log_temperature_text, y, w, precision, rep=4, t_bf16=t_bf16)
         else:
-            # outside what the four-target kernel covers (more than 256 contrast rows -- their number is data dependent,
-            # model.py:268 --, D not 256 / 512, fp32 parity mode): the loss of the upsampled tensor itself, as the decoder
-            # would emit it (decoder.py:113); autograd sums the four pixel gradients of a block below the interpolation
+            # outside what the four-target kernel covers (D not 256 / 512, fp32 parity mode, more than 256 contrast rows
+            # with trainable text): the loss of the upsampled tensor itself, as the decoder would emit it (decoder.py:113);
+            # autograd sums the four pixel gradients of a block below the interpolation
             up = torch.nn.functional.interpolate(pixel_embeddings, scale_factor=2, mode="nearest")
             loss = ops.infonce(up, t_norm, log_temperature_text, y, w, precision, t_bf16=t_bf16)
     else:

@@ -204,15 +204,20 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
         raise RuntimeError("infonce: rep must be 1 or 4")
     if y.numel() != M * rep or w.numel() != M * rep:
         raise RuntimeError("infonce: y / w must have `rep` entries per embedding row")
+    kblocked = precision == "auto" and rep == 1 and K > 256 and not need_dt and kblocked_supported(D, HW)
     if rep == 4:
-        if precision == "fp32" or need_dt and not need_dx or D not in (256, 512) or not bf16_path_supported(D, HW, K):
-            raise RuntimeError(f"infonce(rep=4): needs the tensor-core path (D in (256, 512), K <= 256, HW % 8 == 0); "
-                               f"got D={D}, HW={HW}, K={K}, precision={precision!r}")
+        # more than 256 candidates: the four-target kernel over blocks of 256 candidate rows (host-given K and tau only)
+        kblocked = (precision != "fp32" and K > 256 and not need_dt and k_dev is None and log_tau_dev is None
+                    and kblocked_supported(D, HW))
+        if not kblocked and (precision == "fp32" or need_dt and not need_dx or D not in (256, 512)
+                             or not bf16_path_supported(D, HW, K)):
+            raise RuntimeError(f"infonce(rep=4): needs the tensor-core path (D in (256, 512), HW % 8 == 0, K <= 256 or "
+                               f"no dText); got D={D}, HW={HW}, K={K}, precision={precision!r}")
         precision = "bf16"
-    if precision == "auto" and rep == 1 and K > 256 and not need_dt and kblocked_supported(D, HW):
+    if kblocked:
         # more candidates than one launch takes: tensor cores over blocks of 256 candidate rows instead of the CUDA-core
         # kernel (which needs ~100x longer at full size)
-        r = infonce_kblocked_raw(x, t_norm, y, w, inv_tau, need_dx)
+        r = infonce_kblocked_raw(x, t_norm, y, w, inv_tau, need_dx, rep=rep)
         dx = r["dx"]
         if dx is not None and grad_scale is not None:
             dx = dx * grad_scale.detach().reshape(1).to(device=dev, dtype=dx.dtype)
@@ -305,20 +310,29 @@ def kblocked_supported(D: int, HW: int) -> bool:
 
 
 def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch.Tensor, inv_tau: float,
-                         need_dx: bool, block: int = 256, keep_bf16: bool = False):
+                         need_dx: bool, block: int = 256, keep_bf16: bool = False, rep: int = 1):
     """InfoNCE against MORE than 256 candidates on the tensor cores (model.py:304-321 at thousands of objects): the
     candidate rows are split into launches of <= 256.  Round 1: forward launches give the per-block logsumexp; their
     logsumexp is the row's lse over all candidates.  Round 2: fwd+bwd launches with that lse given produce per-block dx /
-    dlogtau that add up to the full gradient.  Returns dict(loss, lse, dx, dlogtau, w_sum); bf16 operands, fp32 sums."""
+    dlogtau that add up to the full gradient.  Returns dict(loss, lse, dx, dlogtau, w_sum); bf16 operands, fp32 sums.
+    rep = 4: every row of x is the embedding shared by a 2x2 block of pixels, y / w are [rows, 4] (rc_infonce_bf16_rep4,
+    one launch per block and round); lse is per row and a row's weight is the sum of its four."""
     _need_cuda(x, t_norm, y, w)
     x, B, D, HW = _emb3(x)
     if not kblocked_supported(D, HW):
         raise RuntimeError(f"infonce_kblocked: needs D in (256, 512) and HW % 8 == 0; got D={D}, HW={HW}")
+    if rep not in (1, 4):
+        raise RuntimeError("infonce_kblocked: rep must be 1 or 4")
     K = t_norm.shape[0]
     M = B * HW
     dev = x.device
-    y = y.reshape(-1).to(torch.int32)
-    w = (w.reshape(-1).to(torch.float32) * (y >= 0)).contiguous()        # ignored rows: weight 0 (targets may leave the block)
+    y = y.reshape(-1, 4) if rep == 4 else y.reshape(-1)
+    if y.numel() != M * rep or w.numel() != M * rep:
+        raise RuntimeError("infonce_kblocked: y / w must have `rep` entries per embedding row")
+    y = y.to(torch.int32)
+    # ignored targets: weight 0 (targets may leave the block)
+    w = (w.reshape(y.shape).to(torch.float32) * (y >= 0)).contiguous()
+    w_row = w.double().sum(dim=1) if rep == 4 else w.double()           # the weight each row's lse carries
     L = _lib.lib()
     st = _stream(x)
     xdt = _dt(x)
@@ -330,7 +344,7 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
         check(L.rc_infonce_prepass(_p(x), xdt, B, D, HW, _p(ws), ws_bytes, st), "rc_infonce_prepass")
     starts = list(range(0, K, block))
     nb = len(starts)
-    if B == 1 and HW % 256 == 0 and block == 256:
+    if rep == 1 and B == 1 and HW % 256 == 0 and block == 256:
         # one image of rows (the area-image loss): every candidate block in ONE launch per round -- the kernel's image
         # index runs over the blocks (rc_infonce_bf16_kblocks)
         tb_all = torch.zeros(nb * 256, D, device=dev, dtype=torch.bfloat16)
@@ -369,19 +383,20 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
         texts = [(tb_full[i * block:(i + 1) * block], ttb_full[i]) for i in range(n_full)]
     texts += [text_to_bf16(t_norm[s0:s0 + block]) for s0 in starts[n_full:]]
     ys = [(y - s0).contiguous() for s0 in starts]
+    entry = L.rc_infonce_bf16 if rep == 1 else L.rc_infonce_bf16_rep4
     lse_blk = torch.empty(nb, M, device=dev, dtype=torch.float32)
     acc = torch.zeros(nb, 4, device=dev, dtype=torch.float64)             # per block: loss_sum, w_sum, dlogtau, w_sum_in
     wsum = w.double().sum()
     acc[:, 3] = wsum
     for i, s0 in enumerate(starts):
         Kb = min(block, K - s0)
-        check(L.rc_infonce_bf16(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
-                                lse_blk[i].data_ptr(), acc[i, 0:].data_ptr(), acc[i, 1:].data_ptr(), None, None, None, None, None,
-                                _p(ws), ws_bytes, 1 | RC_INFONCE_KEEP_WEIGHT, st), "rc_infonce_bf16(K block, forward)")
+        check(entry(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
+                    lse_blk[i].data_ptr(), acc[i, 0:].data_ptr(), acc[i, 1:].data_ptr(), None, None, None, None, None,
+                    _p(ws), ws_bytes, 1 | RC_INFONCE_KEEP_WEIGHT, st), "rc_infonce_bf16(K block, forward)")
     lse = torch.logsumexp(lse_blk, dim=0)
     # sum_p w z[p, y_p] from the blocks that own the targets: loss_sum_b = sum_p w lse_b - sum_{y in b} w z_y
-    wz = ((lse_blk.double() * w.double()).sum(dim=1) - acc[:, 0]).sum()
-    loss = torch.where(wsum > 0, ((lse.double() * w.double()).sum() - wz) / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
+    wz = ((lse_blk.double() * w_row).sum(dim=1) - acc[:, 0]).sum()
+    loss = torch.where(wsum > 0, ((lse.double() * w_row).sum() - wz) / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
     dx = dlogtau = None
     if need_dx:
         dxb = torch.empty(B, D, HW, device=dev, dtype=torch.bfloat16)     # the tensor-core kernel always writes bf16
@@ -395,9 +410,9 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
         for i, s0 in enumerate(starts):
             Kb = min(block, K - s0)
             fl = 1 | RC_INFONCE_KEEP_WEIGHT | RC_INFONCE_LSE_GIVEN | (RC_INFONCE_ACCUMULATE_DX if (in_kernel and i > 0) else 0)
-            check(L.rc_infonce_bf16(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
-                                    _p(lse), acc2[i, 0:].data_ptr(), acc2[i, 1:].data_ptr(), acc2[i, 3:].data_ptr(), None, _p(dxb),
-                                    None, acc2[i, 2:].data_ptr(), _p(ws), ws_bytes, fl, st), "rc_infonce_bf16(K block, backward)")
+            check(entry(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
+                        _p(lse), acc2[i, 0:].data_ptr(), acc2[i, 1:].data_ptr(), acc2[i, 3:].data_ptr(), None, _p(dxb),
+                        None, acc2[i, 2:].data_ptr(), _p(ws), ws_bytes, fl, st), "rc_infonce_bf16(K block, backward)")
             if not in_kernel:
                 dx = dxb.float() if dx is None else dx.add_(dxb)
         dlogtau = acc2[:, 2].sum()
@@ -760,7 +775,7 @@ def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: i
     D = x.shape[1]
     HW = x[0, 0].numel() if x.shape[0] and D else 0
     if rep == 4:
-        return "bf16"
+        return "kblocked" if (precision != "fp32" and K > 256 and not need_dt and kblocked_supported(D, HW)) else "bf16"
     if precision == "auto" and K > 256 and not need_dt and kblocked_supported(D, HW):
         return "kblocked"
     if precision == "auto":
