@@ -253,6 +253,20 @@ __device__ __forceinline__ float row_max(uint32_t trow, int Kt, int cb, int Kh, 
   return mx * zl;
 }
 
+// The row's exp offset ml (log2 units): the fixed bound, or the row maximum (row_max; every softmax thread takes the same
+// branch, it holds a named barrier).  K-blocked rounds with lse_in: the row's logsumexp over ALL candidates, so that
+// e = exp(z - lse) is the softmax itself and row_lse sets sum = 1.  (With this block's own maximum as the offset, sum =
+// exp(lse - m) overflows ex2.approx to +inf once lse exceeds the block's largest logit by 128 ln 2 = 88.7 nats -- at tau =
+// 0.01 a cosine gap of 0.89 -- and the row's target entry of G becomes (e_y - inf) * 0 = NaN.)  Rows past the end of
+// the image (zl = 0, weight 0) take offset 0: e = 1, a finite sum.
+template <bool kKB>
+__device__ __forceinline__ float row_offset(const Tiling& prm, bool valid, int px, int64_t m, bool use_bound, float ml_bound,
+                                            uint32_t trow, int Kt, int cb, int Kh, float* xch, int half, int row, float zl) {
+  if (kKB && prm.lse_in != nullptr)
+    return valid ? __ldg(prm.lse_in + (prm.kb > 0 ? (int64_t)px : m)) * kLog2e : 0.f;
+  return use_bound ? ml_bound : row_max(trow, Kt, cb, Kh, xch, half, row, zl);
+}
+
 // The exp pass over this half's Kh columns of S (TMEM at trow, 16 columns per step): e = exp(z - m), kept in registers as
 // packed bf16 (pk), with sum = sum e and sez = sum e z (up to the scale zs) of the valid columns (k < Kt), and sy[j] = the
 // raw logit of target j if it lies in this half.  yi: the target (R = 1) or the four packed targets (R = 4).  R = 4: sy[j]
@@ -353,12 +367,12 @@ __device__ __forceinline__ void add_peer_sums(const float* xch, int half, int ro
 }
 
 // The row's logsumexp (half 0; 0 in half 1), and its loss and weight added to loss / wsum.  K-blocked rounds with
-// lse_in: sum becomes exp(lse_in - m), so that 1 / sum = exp(m - lse) normalises this block's softmax.  lse_in is indexed
-// by the embedding row m (R = 4: one lse per shared row) or, in kb mode, by the pixel.
+// lse_in: the exp offset was lse_in itself (row_offset), so e is already the softmax over all candidates and sum = 1.
+// lse_in is indexed by the embedding row m (R = 4: one lse per shared row) or, in kb mode, by the pixel.
 template <bool kKB>
-__device__ __forceinline__ float row_lse(const Tiling& prm, bool valid, int px, int64_t m, int half, float ml, float wtot,
-                                         float tz, float zs, float& sum, float& loss, float& wsum) {
-  if (kKB && prm.lse_in != nullptr && valid) sum = fast_exp2(fmaf(__ldg(prm.lse_in + (prm.kb > 0 ? (int64_t)px : m)), kLog2e, -ml));
+__device__ __forceinline__ float row_lse(const Tiling& prm, bool valid, float ml, int half, float wtot, float tz, float zs,
+                                         float& sum, float& loss, float& wsum) {
+  if (kKB && prm.lse_in != nullptr && valid) sum = 1.f;
   float lse = 0.f;
   if (half == 0) {
     lse = (ml + __log2f(sum)) * kLn2;

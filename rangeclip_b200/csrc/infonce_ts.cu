@@ -304,7 +304,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       tc_fence_after();
       if (warp == 4) RC_EV(l, 13);      // S(l) complete (seen by the softmax warps)
       RC_T0(texp);
-      const float ml = use_bound ? ml_bound : row_max(trow, Kt, cb, Kh, xch, half, row, zl);
+      const float ml = row_offset<kKB>(prm, valid, px, m, use_bound, ml_bound, trow, Kt, cb, Kh, xch, half, row, zl);
       uint32_t pk[64];
       float sy[R];
       float sum, sez;
@@ -326,7 +326,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       tc_fence_after();
       RC_T0(tpst);
       add_peer_sums(xch, half, row, sum, sez, tz);
-      const float lse = row_lse<kKB>(prm, valid, px, m, half, ml, wtot, tz, zs, sum, acc_s[0], acc_s[128]);
+      const float lse = row_lse<kKB>(prm, valid, ml, half, wtot, tz, zs, sum, acc_s[0], acc_s[128]);
       const float coef = coefb * wtot;
       const float inv_sum = 1.f / sum;
       const float rsv = p_scale(inv_n, prm.inv_tau, coef, inv_sum);

@@ -368,7 +368,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       tc_fence_after();
       if (warp == 4) RC_EV(lt, 10);    // S(lt) complete (seen by the softmax warps)
       RC_T0(tsm);
-      const float ml = use_bound ? ml_bound : row_max(trow, Kt, cb, Kh, xch, half, row, zl);
+      const float ml = row_offset<kKB>(prm, valid, px, m, use_bound, ml_bound, trow, Kt, cb, Kh, xch, half, row, zl);
       // e = exp(z - m) for this half's columns; P stays in registers as packed bf16 until the P buffer is free
       uint32_t pk[64];
       float sy[R];
@@ -386,7 +386,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
       post_sums(xch, half, row, sum, sez, tz);
       named_bar_sync(2, 256);
       add_peer_sums(xch, half, row, sum, sez, tz);
-      const float lse = row_lse<kKB>(prm, valid, px, m, half, ml, wtot, tz, zs, sum, loss_acc, w_acc);
+      const float lse = row_lse<kKB>(prm, valid, ml, half, wtot, tz, zs, sum, loss_acc, w_acc);
       RC_TACC(1, tsm);
       if (!kBwd) {
         if (half == 0 && valid && prm.lse) prm.lse[m] = lse;
