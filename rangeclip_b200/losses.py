@@ -87,10 +87,11 @@ def similarity_csr(label_similarity_sets, C: int, use_medium: bool, use_hard: bo
     return off_d, items_d
 
 
-def device_builder_supported(D: int, hw_rows: int, C: int, text_requires_grad: bool, precision: str) -> bool:
-    """Shapes the sync-free path covers: CTA-pair kernel (D = 256 / 512, rows % 8 == 0), label histogram in shared memory
-    (C <= 12000), frozen text embeddings, not the fp32 parity mode."""
-    return D in (256, 512) and hw_rows > 0 and hw_rows % 8 == 0 and 2 <= C <= 12000 and not text_requires_grad and precision != "fp32"
+def device_builder_supported(x: torch.Tensor, rep: int, C: int, k_cap: int, text_requires_grad: bool, precision: str) -> bool:
+    """Calls the sync-free path covers: label histogram in shared memory (2 <= C <= 12000), not the fp32 parity mode, and a
+    tensor-core launch that reads K and tau from device memory (``ops._infonce_plan``: the CTA-pair kernel, frozen text)."""
+    return (2 <= C <= 12000 and precision != "fp32"
+            and ops._infonce_plan(x, k_cap, text_requires_grad, "bf16", rep, dev_params=True) is not None)
 
 
 def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embeddings, label_similarity_sets,
@@ -129,15 +130,15 @@ def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embed
     aux = dict(rand_indices=rand_indices, contrast_indices=None)
     if contrast_builder not in ("reference", "device"):
         raise RuntimeError(f"contrast_builder must be 'reference' or 'device', got {contrast_builder!r}")
-    rows_hw = (H // 2) * (W // 2) if shared2x2 else hw
-    if contrast_builder == "device" and device_builder_supported(D, rows_hw, C, candidate_text_embeddings.requires_grad, precision):
+    k_cap = max(2, min(int(max_contrast), 256, C))
+    if contrast_builder == "device" and device_builder_supported(pixel_embeddings, 4 if shared2x2 else 1, C, k_cap,
+                                                                 candidate_text_embeddings.requires_grad, precision):
         # ---- sync-free path (SURVEY 8f-2): label histogram -> contrast set, label map, text operands and the loss launch
         # without one device->host read; the set size and the temperature reach the kernel through device memory
         n_medium = int(k_distractors * pct_medium)
         n_hard = int(k_distractors * pct_hard)
         n_rand = k_distractors - n_medium - n_hard
         sim_off, sim_items = similarity_csr(label_similarity_sets, C, n_medium > 0, n_hard > 0, device)
-        k_cap = max(2, min(int(max_contrast), 256, C))
         seed_dev = None
         if torch.cuda.is_current_stream_capturing():
             # CUDA-graph capture: a host-side seed would be frozen into the graph.  The CUDA generator is graph-safe (its
@@ -194,12 +195,10 @@ def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embed
         aux["smoothness"] = smooth
         return loss, aux
     if shared2x2:
-        K = int(contrast.shape[0])
-        rows = (H // 2) * (W // 2)
-        # more than 256 contrast rows (their number is data dependent, model.py:268): the four-target kernel over blocks of
-        # 256 candidate rows (ops.infonce_kblocked_raw), for frozen text
-        kblocked = K > 256 and ops.kblocked_supported(D, rows) and not candidate_text_embeddings.requires_grad
-        if precision != "fp32" and D in (256, 512) and (ops.bf16_path_supported(D, rows, K) or kblocked):
+        # the four-target kernel: one launch, or blocks of 256 candidate rows for frozen text above 256 contrast rows (their
+        # number is data dependent, model.py:268).  The plan is asked with the text's requires_grad, not the grad mode's
+        # view of it, so a no_grad call with trainable text takes the same route as the training step
+        if ops._infonce_plan(pixel_embeddings, int(contrast.shape[0]), candidate_text_embeddings.requires_grad, precision, 4) is not None:
             y, w = group_2x2(y.view(B, H, W)), group_2x2(w.view(B, H, W))
             loss = ops.infonce(pixel_embeddings, t_norm, log_temperature_text, y, w, precision, rep=4, t_bf16=t_bf16)
         else:
@@ -225,23 +224,19 @@ def image_contrastive_loss(area_embeddings, image_embeddings, log_temperature_im
     transposed to the kernels' [D][n] layout first (n*D elements; plumbing).
 
     ``precision``: "fp32" = CUDA-core kernel (1e-5 path; what the reference's n <= batch size needs -- the call is
-    launch-bound there); "bf16" = tensor cores with the candidates in blocks of 256 (``ops.infonce_kblocked``; the
-    fp32 kernel takes 9 ms at n = 4096); "auto" = bf16 from n = 512 when the shape allows it (D in (256, 512), n % 8 == 0,
-    frozen image embeddings)."""
+    launch-bound there); "bf16" = tensor cores with the candidates in blocks of 256 (``ops.infonce`` with
+    ``precision="kblocked"``; the fp32 kernel takes 9 ms at n = 4096); "auto" = bf16 from n = 512 when the shape allows it
+    (D in (256, 512), n % 8 == 0, frozen image embeddings)."""
     n, D = area_embeddings.shape
-    blocked_ok = ops.kblocked_supported(D, n) and not image_embeddings.requires_grad
+    x = area_embeddings.float().t().contiguous().view(1, D, n, 1)
+    blocked_ok = ops._infonce_plan(x, n, image_embeddings.requires_grad, "kblocked", 1) is not None
     if precision == "auto":
         precision = "bf16" if (blocked_ok and n >= 512) else "fp32"
     if precision == "bf16":
         if not blocked_ok:
             raise RuntimeError(f"image_contrastive_loss: the tensor-core path needs D in (256, 512), n % 8 == 0 and frozen "
                                f"image embeddings; got n={n}, D={D}")
-        x = area_embeddings.float().t().contiguous().view(1, D, n, 1)
-        t_norm, _, _ = torch.ops.rangeclip.text_prepare(image_embeddings, None)
-        y = torch.arange(n, device=x.device, dtype=torch.int32)
-        w = torch.ones(n, device=x.device, dtype=torch.float32)
-        return ops.infonce_kblocked(x, t_norm, log_temperature_image, y, w)
-    x = area_embeddings.float().t().contiguous().view(1, D, n, 1)
+        precision = "kblocked"
     if image_embeddings.requires_grad:
         t_norm = torch.nn.functional.normalize(image_embeddings.float(), dim=1)
     else:

@@ -7,6 +7,10 @@ Three tiers, top to bottom of this file:
     them as single opaque nodes (north_star: "exposed as PyTorch custom ops");
   * the public functions the drop-ins call (``infonce``, ``pixel_losses``, ``smoothness``, ``masked_pool``, ...), thin
     shims over the registered operators.
+Which InfoNCE kernel family a call takes (CUDA-core, one tensor-core launch, or tensor cores over blocks of 256 candidate
+rows) is decided in one place, ``_infonce_plan``: ``infonce_raw`` dispatches on it, the fake-tensor rules of
+``rangeclip::infonce`` / ``rangeclip::pixel_losses`` derive their outputs from it, and the loss drop-ins ask it whether a
+kernel takes a call.
 PyTorch is used for device memory, streams and autograd plumbing only; every computation is a kernel in
 ``librangeclip_b200.so``.  All functions require CUDA tensors on an sm_100 device and raise ``RuntimeError``
 otherwise -- there is no CPU or eager-PyTorch fallback.
@@ -52,11 +56,6 @@ def _emb3(x: torch.Tensor) -> Tuple[torch.Tensor, int, int, int]:
     x = x.contiguous()
     B, D = x.shape[0], x.shape[1]
     return x, B, D, x[0, 0].numel() if B and D else 0
-
-
-def bf16_path_supported(D: int, HW: int, K: int) -> bool:
-    """Shapes the tcgen05 InfoNCE kernel covers (everything else runs on the fp32 kernel)."""
-    return 1 <= K <= 256 and D in (128, 256, 384, 512) and HW % 8 == 0 and HW > 0
 
 
 # ----------------------------------------------------------------------------------------------
@@ -176,45 +175,88 @@ def contrast_build(counts: torch.Tensor, sim_off: Optional[torch.Tensor], sim_it
 # InfoNCE
 # ----------------------------------------------------------------------------------------------
 
+def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: int, need_dx: bool = True,
+                  dev_params: bool = False) -> Optional[str]:
+    """The route of one InfoNCE call; the only place that chooses it.  ``infonce_raw`` runs it, the fake-tensor rules of
+    rangeclip::infonce / pixel_losses derive dX's dtype from it and the loss drop-ins ask it whether a kernel takes a call.
+      'fp32'      the CUDA-core kernel (rc_infonce_f32): any shape, one target per row, host K and tau;
+      'bf16'      one tensor-core launch (rc_infonce_bf16 / _rep4 / _dyn): K <= 256, D in (128, 256, 384, 512), HW % 8 == 0;
+                  four targets, dText (with dX) and the device-parameter form only on the CTA-pair kernel (D in (256, 512));
+      'kblocked'  tensor cores over blocks of 256 candidate rows (``infonce_kblocked_raw``): D in (256, 512), HW % 8 == 0, no
+                  dText, host K and tau; what "auto" (and, for four targets, "bf16") takes above 256 candidates;
+      None        no kernel covers the call.
+    x: a tensor or meta tensor [B, D, H, W] / [B, D, HW]; K: rows of t_norm; precision: 'auto', 'fp32', 'bf16' or 'kblocked';
+    need_dx: dX is wanted (the autograd operators always want it with dText); dev_params: K and log(tau) are read from device
+    memory (k_dev / log_tau_dev)."""
+    if rep not in (1, 4) or precision not in ("auto", "fp32", "bf16", "kblocked"):
+        return None
+    D = x.shape[1]
+    HW = x[0, 0].numel() if x.shape[0] and D else 0
+    kblocked = kblocked_supported(D, HW) and not need_dt and not dev_params
+    if precision == "kblocked":
+        return "kblocked" if kblocked else None
+    if precision == "fp32":
+        return "fp32" if rep == 1 and not dev_params else None
+    if kblocked and K > 256 and (precision == "auto" or rep == 4):
+        return "kblocked"
+    one_launch = 1 <= K <= 256 and D in (128, 256, 384, 512) and HW % 8 == 0 and HW > 0
+    if rep == 4 or need_dt or dev_params:         # forms only the CTA-pair kernel has
+        one_launch = one_launch and D in (256, 512)
+    if need_dt:                                   # tensor-core dText: pair kernel + split-K GEMM, from the dX pass
+        one_launch = one_launch and need_dx and not dev_params
+    if one_launch:
+        return "bf16"
+    return "fp32" if precision == "auto" and rep == 1 and not dev_params else None
+
+
+def _infonce_route(x: torch.Tensor, K: int, need_dx: bool, need_dt: bool, precision: str, rep: int, dev_params: bool) -> str:
+    """``_infonce_plan``, or the error of a call no kernel covers (raised alike by the op and by its fake-tensor rules)."""
+    route = _infonce_plan(x, K, need_dt, precision, rep, need_dx, dev_params)
+    if route is None:
+        D = x.shape[1]
+        HW = x[0, 0].numel() if x.shape[0] and D else 0
+        raise RuntimeError(f"infonce: no kernel covers D={D}, HW={HW}, K={K}, precision={precision!r}, rep={rep} "
+                           f"(need_dx={need_dx}, need_dt={need_dt}, device parameters={dev_params}); see _infonce_plan")
+    return route
+
+
+def _fused_tv(x: torch.Tensor, route: Optional[str]) -> bool:
+    """Whether the launch's pre-pass over x also gives the smoothness sums of x -- and, with dX, the difference signs for
+    tv_backward_codes (rc_infonce_prepass_tv): an fp32 NCHW x with W % 8 == 0 on the tensor-core route."""
+    return route == "bf16" and x.dim() == 4 and x.dtype == torch.float32 and x.shape[3] % 8 == 0 and x.numel() > 0
+
+
 def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch.Tensor, inv_tau: float,
                 need_dx: bool, need_dt: bool, precision: str = "auto",
                 grad_scale: Optional[torch.Tensor] = None, t_bf16=None, rep: int = 1, keep_bf16: bool = False,
                 flags: int = 0, k_dev: Optional[torch.Tensor] = None, log_tau_dev: Optional[torch.Tensor] = None,
                 fuse_tv: bool = False):
     """One fused pass: returns dict(loss_sum, w_sum (double[1] tensors), lse, dx, dt, dlogtau).
-    loss = loss_sum / w_sum; dx/dt/dlogtau are gradients of that mean loss times grad_scale.
+    loss = loss_sum / w_sum; dx/dt/dlogtau are gradients of that mean loss times grad_scale.  The kernel family is
+    ``_infonce_plan``'s route; a call no kernel covers raises ``RuntimeError``.
     rep = 4: every row of x is the embedding shared by a 2x2 block of pixels (decoder.py:113, Q8);
-    y / w are [rows, 4] and dx is the gradient w.r.t. the shared row (tensor-core path only).
-    keep_bf16: leave the tensor-core path's dx in bf16 whatever x's dtype (the autograd wrappers widen and scale it
+    y / w are [rows, 4] and dx is the gradient w.r.t. the shared row (tensor-core paths only).
+    keep_bf16: leave the tensor-core launch's dx in bf16 whatever x's dtype (the autograd wrappers widen and scale it
     in one pass at backward time); flags: extra RC_INFONCE_* bits for rc_infonce_bf16 (e.g. RC_INFONCE_SS_KERNEL).
     k_dev / log_tau_dev (device int32[>=1] / float[1]): the sync-free form (rc_infonce_bf16_dyn) -- the number of valid rows of
     t_norm and log(tau) are read by the kernel from device memory; ``inv_tau`` is ignored; CTA-pair kernel shapes only.
-    fuse_tv: the caller also wants tv_sums(x); where the launch has a pre-pass over x anyway (fp32 NCHW x on the tensor-core
-    path, W % 8 == 0) the sums come out of that pass (rc_infonce_prepass_tv) as ``tv_sums`` -- and with need_dx the difference
-    signs for tv_backward_codes as ``tv_codes`` --, else both keys are None."""
+    fuse_tv: the caller also wants tv_sums(x); where the launch has a pre-pass over x anyway (``_fused_tv``) the sums come
+    out of that pass (rc_infonce_prepass_tv) as ``tv_sums`` -- and with need_dx the difference signs for tv_backward_codes
+    as ``tv_codes`` --, else both keys are None."""
     _need_cuda(x, t_norm, y, w)
-    tv_hw = tuple(x.shape[2:]) if (fuse_tv and x.dim() == 4 and x.dtype == torch.float32 and x.shape[3] % 8 == 0) else None
+    x_in = x
     x, B, D, HW = _emb3(x)
     K = t_norm.shape[0]
+    dev_params = log_tau_dev is not None
+    route = _infonce_route(x, K, need_dx, need_dt, precision, rep, dev_params)
+    tv_hw = tuple(x_in.shape[2:]) if (fuse_tv and _fused_tv(x_in, route)) else None
     dev = x.device
     M = B * HW
     y = y.reshape(-1).to(torch.int32).contiguous()
     w = w.reshape(-1).to(torch.float32).contiguous()
-    if rep not in (1, 4):
-        raise RuntimeError("infonce: rep must be 1 or 4")
     if y.numel() != M * rep or w.numel() != M * rep:
         raise RuntimeError("infonce: y / w must have `rep` entries per embedding row")
-    kblocked = precision == "auto" and rep == 1 and K > 256 and not need_dt and kblocked_supported(D, HW)
-    if rep == 4:
-        # more than 256 candidates: the four-target kernel over blocks of 256 candidate rows (host-given K and tau only)
-        kblocked = (precision != "fp32" and K > 256 and not need_dt and k_dev is None and log_tau_dev is None
-                    and kblocked_supported(D, HW))
-        if not kblocked and (precision == "fp32" or need_dt and not need_dx or D not in (256, 512)
-                             or not bf16_path_supported(D, HW, K)):
-            raise RuntimeError(f"infonce(rep=4): needs the tensor-core path (D in (256, 512), HW % 8 == 0, K <= 256 or "
-                               f"no dText); got D={D}, HW={HW}, K={K}, precision={precision!r}")
-        precision = "bf16"
-    if kblocked:
+    if route == "kblocked":
         # more candidates than one launch takes: tensor cores over blocks of 256 candidate rows instead of the CUDA-core
         # kernel (which needs ~100x longer at full size)
         r = infonce_kblocked_raw(x, t_norm, y, w, inv_tau, need_dx, rep=rep)
@@ -224,11 +266,8 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
         dlt = r["dlogtau"] if r["dlogtau"] is not None else torch.zeros((), device=dev, dtype=torch.float64)
         if grad_scale is not None:
             dlt = dlt * grad_scale.detach().reshape(()).to(device=dev, dtype=torch.float64)
-        return dict(loss_sum=r["loss"] * r["w_sum"], w_sum=r["w_sum"], dlogtau=dlt, lse=r["lse"], dx=dx, dt=None,
-                    precision="bf16-kblocked", tv_sums=None)
-    dt_on_tc = need_dt and need_dx and D in (256, 512)       # tensor-core dText: pair kernel + split-K GEMM
-    if precision == "auto":
-        precision = "bf16" if (bf16_path_supported(D, HW, K) and (not need_dt or dt_on_tc)) else "fp32"
+        return dict(loss_sum=r["loss_sum"], w_sum=r["w_sum"], dlogtau=dlt, lse=r["lse"], dx=dx, dt=None,
+                    precision="bf16-kblocked", tv_sums=None, tv_codes=None)
     acc = torch.zeros(4, device=dev, dtype=torch.float64)        # loss_sum, w_sum, dlogtau, w_sum_in
     lse = torch.empty(M, device=dev, dtype=torch.float32)
     need_grad = need_dx or need_dt
@@ -240,7 +279,8 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
     if grad_scale is not None:
         gs = grad_scale.detach().reshape(1).to(device=dev, dtype=torch.float32)
     dt = torch.zeros(K, D, device=dev, dtype=torch.float32) if need_dt else None
-    if precision == "fp32":
+    tv = tv_codes = None
+    if route == "fp32":
         xf = x if x.dtype == torch.float32 else x.float()
         tf = t_norm.detach().float().contiguous()
         dx = torch.empty_like(xf) if need_dx else None
@@ -250,11 +290,7 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
                                _p(dx), _p(dt), acc[2:].data_ptr() if need_grad else None, st), "rc_infonce_f32")
         if dx is not None and dx.dtype != x.dtype:
             dx = dx.to(x.dtype)
-    elif precision == "bf16":
-        if not bf16_path_supported(D, HW, K):
-            raise RuntimeError(f"infonce: bf16 tensor-core path does not cover D={D}, HW={HW}, K={K}")
-        if need_dt and not dt_on_tc:
-            raise RuntimeError("infonce: dText on the bf16 path needs dx and D in (256, 512); use precision='fp32'")
+    else:
         if t_bf16 is None:
             t_bf16 = text_to_bf16(t_norm)
         tb, ttb = t_bf16
@@ -262,8 +298,7 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
         ws_bytes = int((L.rc_infonce_workspace_bytes_dt if need_dt else L.rc_infonce_workspace_bytes)(B, D, HW, K, xdt))
         ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
         dxb = torch.empty(B, D, HW, device=dev, dtype=torch.bfloat16) if need_dx else None
-        tv = tv_codes = None
-        if tv_hw is not None and M > 0:
+        if tv_hw is not None:
             # fp32 x: the bf16 copy, the row norms, the smoothness sums and (for the backward) the signs of the differences,
             # 4 bits per element, from one read of x
             tv = torch.zeros(2, device=dev, dtype=torch.float64)
@@ -272,33 +307,21 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
             check(L.rc_infonce_prepass_tv(_p(x), B, D, int(tv_hw[0]), int(tv_hw[1]), _p(ws), ws_bytes, _p(tv), _p(tv_codes), st),
                   "rc_infonce_prepass_tv")
             flags = int(flags) | RC_INFONCE_PREPASS_DONE
-        if log_tau_dev is not None:
-            if need_dt or D not in (256, 512):
-                raise RuntimeError("infonce: the device-parameter form needs D in (256, 512) and no dText")
+        sums = (_p(lse), acc[0:].data_ptr(), acc[1:].data_ptr(), acc[3:].data_ptr() if need_grad else None, _p(gs), _p(dxb))
+        if dev_params:
             kd = k_dev.to(torch.int32) if k_dev is not None else None
             lt = log_tau_dev.detach().reshape(1).to(device=dev, dtype=torch.float32)
-            check(L.rc_infonce_bf16_dyn(_p(x), xdt, B, D, HW, _p(tb), _p(ttb), K, _p(kd), _p(y), _p(w), _p(lt), rep, _p(lse),
-                                        acc[0:].data_ptr(), acc[1:].data_ptr(), acc[3:].data_ptr() if need_grad else None,
-                                        _p(gs), _p(dxb), acc[2:].data_ptr() if need_dx else None, _p(ws), ws_bytes, int(flags),
-                                        st), "rc_infonce_bf16_dyn")
-            dx = None
-            if dxb is not None:
-                dx = dxb.view(x.shape) if (x.dtype == torch.bfloat16 or keep_bf16) else scale_to(dxb.view(x.shape), x.dtype)
-            return dict(loss_sum=acc[0], w_sum=acc[1], dlogtau=acc[2], lse=lse, dx=dx, dt=None, precision=precision, tv_sums=tv,
-                        tv_codes=tv_codes)
-        entry = L.rc_infonce_bf16 if rep == 1 else L.rc_infonce_bf16_rep4
-        check(entry(_p(x), xdt, B, D, HW, _p(tb), _p(ttb), K, _p(y), _p(w), float(inv_tau), _p(lse),
-                    acc[0:].data_ptr(), acc[1:].data_ptr(),
-                    acc[3:].data_ptr() if need_grad else None, _p(gs), _p(dxb), _p(dt),
-                    acc[2:].data_ptr() if need_dx else None, _p(ws), ws_bytes, int(flags), st),
-              "rc_infonce_bf16" if rep == 1 else "rc_infonce_bf16_rep4")
+            entry, args = "rc_infonce_bf16_dyn", (_p(kd), _p(y), _p(w), _p(lt), rep) + sums
+        else:
+            entry = "rc_infonce_bf16" if rep == 1 else "rc_infonce_bf16_rep4"
+            args = (_p(y), _p(w), float(inv_tau)) + sums + (_p(dt),)
+        check(getattr(L, entry)(_p(x), xdt, B, D, HW, _p(tb), _p(ttb), K, *args, acc[2:].data_ptr() if need_dx else None,
+                                _p(ws), ws_bytes, int(flags), st), entry)
         dx = None
         if dxb is not None:
             dx = dxb.view(x.shape) if (x.dtype == torch.bfloat16 or keep_bf16) else scale_to(dxb.view(x.shape), x.dtype)
-    else:
-        raise RuntimeError(f"infonce: unknown precision {precision!r}")
-    return dict(loss_sum=acc[0], w_sum=acc[1], dlogtau=acc[2], lse=lse, dx=dx, dt=dt, precision=precision,
-                tv_sums=tv if precision == "bf16" else None, tv_codes=tv_codes if precision == "bf16" else None)
+    return dict(loss_sum=acc[0], w_sum=acc[1], dlogtau=acc[2], lse=lse, dx=dx, dt=dt, precision=route, tv_sums=tv,
+                tv_codes=tv_codes)
 
 
 RC_INFONCE_PREPASS_DONE, RC_INFONCE_KEEP_WEIGHT, RC_INFONCE_LSE_GIVEN, RC_INFONCE_TS_KERNEL, RC_INFONCE_ACCUMULATE_DX = 1, 2, 4, 8, 16
@@ -314,7 +337,8 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
     """InfoNCE against MORE than 256 candidates on the tensor cores (model.py:304-321 at thousands of objects): the
     candidate rows are split into launches of <= 256.  Round 1: forward launches give the per-block logsumexp; their
     logsumexp is the row's lse over all candidates.  Round 2: fwd+bwd launches with that lse given produce per-block dx /
-    dlogtau that add up to the full gradient.  Returns dict(loss, lse, dx, dlogtau, w_sum); bf16 operands, fp32 sums.
+    dlogtau that add up to the full gradient.  Returns dict(loss, loss_sum, lse, dx, dlogtau, w_sum), loss = loss_sum / w_sum;
+    bf16 operands, fp32 sums.
     rep = 4: every row of x is the embedding shared by a 2x2 block of pixels, y / w are [rows, 4] (rc_infonce_bf16_rep4,
     one launch per block and round); lse is per row and a row's weight is the sum of its four."""
     _need_cuda(x, t_norm, y, w)
@@ -361,7 +385,8 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
                                         ws_bytes, 1, st), "rc_infonce_bf16_kblocks(forward)")
         lse = torch.logsumexp(lse_blk, dim=0)
         wz = (lse_blk.double() * w.double()[None, :]).sum() - acc[0]
-        loss = torch.where(wsum > 0, ((lse.double() * w.double()).sum() - wz) / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
+        loss_sum = (lse.double() * w.double()).sum() - wz
+        loss = torch.where(wsum > 0, loss_sum / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
         dx = dlogtau = None
         if need_dx:
             dxb = torch.empty(nb, D, HW, device=dev, dtype=torch.bfloat16)
@@ -373,7 +398,7 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
                   "rc_infonce_bf16_kblocks(backward)")
             dx = dxb.float().sum(dim=0).view(x.shape).to(x.dtype)
             dlogtau = acc2[2].clone()
-        return dict(loss=loss, lse=lse, dx=dx, dlogtau=dlogtau, w_sum=wsum)
+        return dict(loss=loss, loss_sum=loss_sum, lse=lse, dx=dx, dlogtau=dlogtau, w_sum=wsum)
     # bf16 operand copies of the candidate blocks: all full blocks with two tensor ops, a shorter last block on its own
     n_full = K // block if block % 64 == 0 else 0
     texts = []
@@ -396,7 +421,8 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
     lse = torch.logsumexp(lse_blk, dim=0)
     # sum_p w z[p, y_p] from the blocks that own the targets: loss_sum_b = sum_p w lse_b - sum_{y in b} w z_y
     wz = ((lse_blk.double() * w_row).sum(dim=1) - acc[:, 0]).sum()
-    loss = torch.where(wsum > 0, ((lse.double() * w_row).sum() - wz) / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
+    loss_sum = (lse.double() * w_row).sum() - wz
+    loss = torch.where(wsum > 0, loss_sum / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
     dx = dlogtau = None
     if need_dx:
         dxb = torch.empty(B, D, HW, device=dev, dtype=torch.bfloat16)     # the tensor-core kernel always writes bf16
@@ -420,7 +446,7 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
             dx = dxb.view(x.shape) if (x.dtype == torch.bfloat16 or keep_bf16) else scale_to(dxb.view(x.shape), x.dtype)
         else:
             dx = dx.view(x.shape).to(x.dtype)
-    return dict(loss=loss, lse=lse, dx=dx, dlogtau=dlogtau, w_sum=wsum)
+    return dict(loss=loss, loss_sum=loss_sum, lse=lse, dx=dx, dlogtau=dlogtau, w_sum=wsum)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -770,20 +796,6 @@ def _empty(like: torch.Tensor) -> torch.Tensor:
     return like.new_empty(0)
 
 
-def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: int) -> str:
-    """Which kernel family ``infonce_raw`` takes for this call: 'kblocked', 'bf16' or 'fp32' (shape logic only)."""
-    D = x.shape[1]
-    HW = x[0, 0].numel() if x.shape[0] and D else 0
-    if rep == 4:
-        return "kblocked" if (precision != "fp32" and K > 256 and not need_dt and kblocked_supported(D, HW)) else "bf16"
-    if precision == "auto" and K > 256 and not need_dt and kblocked_supported(D, HW):
-        return "kblocked"
-    if precision == "auto":
-        dt_on_tc = need_dt and D in (256, 512)
-        return "bf16" if (bf16_path_supported(D, HW, K) and (not need_dt or dt_on_tc)) else "fp32"
-    return precision
-
-
 def _mean_loss(r) -> torch.Tensor:
     wsum = r["w_sum"]
     return torch.where(wsum > 0, r["loss_sum"] / wsum.clamp_min(1e-300), torch.zeros_like(wsum)).float().reshape(())
@@ -803,12 +815,10 @@ def _op_infonce(x: torch.Tensor, t_norm: torch.Tensor, log_tau: torch.Tensor, y:
 def _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev, fuse_tv):
     """Body of rangeclip::infonce (and of the InfoNCE half of rangeclip::pixel_losses): (loss, dx, dt, dlogtau, tv_sums | None, tv_codes | None)."""
     tb = (t_bf16, tt_bf16) if (t_bf16 is not None and tt_bf16 is not None) else None
-    if k_dev is not None:
-        r = infonce_raw(x, t_norm, y, w, 0.0, need_grad, False, "bf16", t_bf16=tb, rep=rep, keep_bf16=True, k_dev=k_dev,
-                        log_tau_dev=log_tau, fuse_tv=fuse_tv)
-    else:
-        inv_tau = float(torch.exp(-log_tau.detach().float()))          # one scalar sync, as .item() in the reference
-        r = infonce_raw(x, t_norm, y, w, inv_tau, need_grad, need_dt, precision, t_bf16=tb, rep=rep, keep_bf16=True, fuse_tv=fuse_tv)
+    dyn = k_dev is not None
+    inv_tau = 0.0 if dyn else float(torch.exp(-log_tau.detach().float()))      # one scalar sync, as .item() in the reference
+    r = infonce_raw(x, t_norm, y, w, inv_tau, need_grad, need_dt, precision, t_bf16=tb, rep=rep, keep_bf16=True, k_dev=k_dev,
+                    log_tau_dev=log_tau if dyn else None, fuse_tv=fuse_tv)
     dx, dt = r["dx"], r["dt"]
     return (_mean_loss(r), dx if dx is not None else _empty(x), dt if dt is not None else _empty(t_norm),
             r["dlogtau"].float().reshape(()), r.get("tv_sums"), r.get("tv_codes"))
@@ -816,8 +826,8 @@ def _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, re
 
 @_op_infonce.register_fake
 def _(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev=None):
-    plan = "bf16" if k_dev is not None else _infonce_plan(x, t_norm.shape[0], need_dt, precision, rep)
-    dx_dtype = torch.bfloat16 if plan == "bf16" else x.dtype
+    route = _infonce_route(x, t_norm.shape[0], need_grad, need_dt, precision, rep, k_dev is not None)
+    dx_dtype = torch.bfloat16 if route == "bf16" else x.dtype
     f32 = dict(device=x.device, dtype=torch.float32)
     return (torch.empty((), **f32), torch.empty(x.shape, device=x.device, dtype=dx_dtype) if need_grad else _empty(x),
             torch.empty(t_norm.shape, **f32) if need_dt else _empty(t_norm), torch.empty((), **f32))
@@ -887,10 +897,10 @@ def _op_pixel_losses(x: torch.Tensor, t_norm: torch.Tensor, log_tau: torch.Tenso
 
 @_op_pixel_losses.register_fake
 def _(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, t_bf16, tt_bf16, k_dev=None):
-    plan = "bf16" if k_dev is not None else _infonce_plan(x, t_norm.shape[0], need_dt, precision, 1)
-    dx_dtype = torch.bfloat16 if plan == "bf16" else x.dtype
+    route = _infonce_route(x, t_norm.shape[0], need_grad, need_dt, precision, 1, k_dev is not None)
+    dx_dtype = torch.bfloat16 if route == "bf16" else x.dtype
     f32 = dict(device=x.device, dtype=torch.float32)
-    fused = (plan == "bf16" and need_grad and x.dim() == 4 and x.dtype == torch.float32 and x.shape[3] % 8 == 0 and x.numel() > 0)
+    fused = need_grad and _fused_tv(x, route)
     return (torch.empty((), **f32), torch.empty((), **f32),
             torch.empty(x.shape, device=x.device, dtype=dx_dtype) if need_grad else _empty(x),
             torch.empty(t_norm.shape, **f32) if need_dt else _empty(t_norm), torch.empty((), **f32),
@@ -927,39 +937,6 @@ def _pixel_losses_backward(ctx, g_text, g_smooth, *_unused):
 
 
 _op_pixel_losses.register_autograd(_pixel_losses_backward, setup_context=_pixel_losses_setup)
-
-
-@_op("rangeclip::infonce_kblocked", mutates_args=(), device_types="cuda")
-def _op_infonce_kblocked(x: torch.Tensor, t_norm: torch.Tensor, log_tau: torch.Tensor, y: torch.Tensor, w: torch.Tensor,
-                         need_grad: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """(loss, dx, dlogtau) against MORE than 256 candidates (``infonce_kblocked_raw``); the candidate rows are constants."""
-    inv_tau = float(torch.exp(-log_tau.detach().float()))
-    r = infonce_kblocked_raw(x, t_norm, y, w, inv_tau, need_grad)
-    z = torch.zeros((), device=x.device, dtype=torch.float32)
-    return (r["loss"].float().reshape(()), r["dx"] if r["dx"] is not None else _empty(x),
-            r["dlogtau"].float().reshape(()) if r["dlogtau"] is not None else z)
-
-
-@_op_infonce_kblocked.register_fake
-def _(x, t_norm, log_tau, y, w, need_grad):
-    f32 = dict(device=x.device, dtype=torch.float32)
-    return torch.empty((), **f32), torch.empty_like(x) if need_grad else _empty(x), torch.empty((), **f32)
-
-
-def _kblocked_setup(ctx, inputs, output):
-    ctx.save_for_backward(output[1], output[2])
-    ctx.set_materialize_grads(False)         # see _infonce_setup
-
-
-def _kblocked_backward(ctx, g, *_unused):
-    dx, dlt = ctx.saved_tensors
-    need = ctx.needs_input_grad
-    if g is None:
-        return (None,) * 6
-    return (dx * g.to(dx.dtype) if need[0] else None, None, (dlt * g).reshape(()) if need[2] else None, None, None, None)
-
-
-_op_infonce_kblocked.register_autograd(_kblocked_backward, setup_context=_kblocked_setup)
 
 
 @_op("rangeclip::scale_to", mutates_args=(), device_types="cuda")
@@ -1290,8 +1267,9 @@ def _tb(t_bf16):
 
 def infonce(x, t_norm, log_tau, y, w, precision="auto", rep=1, t_bf16=None, k_dev=None):
     """Autograd-aware fused InfoNCE (torch.ops.rangeclip.infonce); x [B,D,H,W], t_norm [K,D] normalised, y/w per pixel
-    (rep = 4: x holds the embeddings shared by 2x2 pixel blocks, y/w are [B*H*W, 4]).  ``t_bf16`` = (bf16 [Kp,D], bf16
-    [D,Kp]) copies of t_norm from ``text_prepare`` (optional: built on the fly otherwise)."""
+    (rep = 4: x holds the embeddings shared by 2x2 pixel blocks, y/w are [B*H*W, 4]).  ``precision``: 'auto', 'fp32', 'bf16'
+    or 'kblocked', the kernel family as ``_infonce_plan`` routes it.  ``t_bf16`` = (bf16 [Kp,D], bf16 [D,Kp]) copies of
+    t_norm from ``text_prepare`` (optional: built on the fly otherwise)."""
     _need_cuda(x, t_norm, y, w)
     tb, ttb = _tb(t_bf16)
     need_grad = bool(torch.is_grad_enabled() and (x.requires_grad or log_tau.requires_grad))
@@ -1307,12 +1285,6 @@ def pixel_losses(x, t_norm, log_tau, y, w, precision="auto", t_bf16=None, k_dev=
     need_dt = bool(torch.is_grad_enabled() and t_norm.requires_grad)
     out = torch.ops.rangeclip.pixel_losses(x, t_norm, log_tau, y, w, need_grad or need_dt, need_dt, precision, tb, ttb, k_dev)
     return out[0], out[1]
-
-
-def infonce_kblocked(x, t_norm, log_tau, y, w):
-    _need_cuda(x, t_norm, y, w)
-    need = bool(torch.is_grad_enabled() and (x.requires_grad or log_tau.requires_grad))
-    return torch.ops.rangeclip.infonce_kblocked(x, t_norm, log_tau, y, w, need)[0]
 
 
 def smoothness(x: torch.Tensor, denominators=None) -> torch.Tensor:

@@ -263,12 +263,14 @@ def _small_infonce_args(D=256, HW=64, K=40, requires_grad=True):
 
 def test_custom_ops_are_registered_and_pass_opcheck():
     import rangeclip_b200  # noqa: F401  (registers torch.ops.rangeclip.*)
-    for name in ("infonce", "pixel_losses", "infonce_kblocked", "smoothness", "tv_bwd", "scale_to", "scale_", "masked_pool", "masked_pool_bwd",
+    for name in ("infonce", "pixel_losses", "smoothness", "tv_bwd", "scale_to", "scale_", "masked_pool", "masked_pool_bwd",
                  "sample_weights", "text_prepare", "eval_topk", "eval_hist", "eval_topk_hist", "eval_fold"):
         assert hasattr(torch.ops.rangeclip, name), name
     x, t, log_tau, y, w = _small_infonce_args()
     tests = ("test_schema", "test_faketensor", "test_autograd_registration")
     torch.library.opcheck(torch.ops.rangeclip.infonce.default, (x, t, log_tau, y, w, True, False, "auto", 1, None, None), test_utils=tests)
+    torch.library.opcheck(torch.ops.rangeclip.infonce.default, (x, t, log_tau, y, w, True, False, "kblocked", 1, None, None),
+                          test_utils=tests)
     torch.library.opcheck(torch.ops.rangeclip.smoothness.default, (x, 10.0, 12.0), test_utils=tests)
     torch.library.opcheck(torch.ops.rangeclip.scale_to.default, (x.detach(), torch.tensor(0.5, device=dev()), 0), test_utils=tests)
     seg = torch.randint(0, 5, (2, 8, 8), device=dev())

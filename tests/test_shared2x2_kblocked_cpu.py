@@ -1,5 +1,5 @@
 """CPU-side checks of the K-blocked four-target loss (more than 256 contrast rows on the shared 2x2 embeddings): which kernel
-family rangeclip::infonce plans for (its fake-tensor dX dtype depends on it), and the entry points that keep rejecting the
+family rangeclip::infonce plans for (its fake-tensor dX dtype depends on it; None = no kernel takes the call), and the entry points that keep rejecting the
 K-blocked flags for four targets per row."""
 import pytest
 import torch
@@ -18,22 +18,23 @@ def test_rep4_above_256_candidates_plans_the_kblocked_rounds(D, K, precision):
     assert ops._infonce_plan(_x(D, dtype=torch.float32), K, False, precision, 4) == "kblocked"
 
 
-@pytest.mark.parametrize("D,K,need_dt,precision,h,w", [
-    (128, 300, False, "auto", 16, 16),     # no CTA-pair kernel for D = 128
-    (512, 300, False, "fp32", 16, 16),     # fp32 parity mode
-    (512, 300, True, "auto", 16, 16),      # dText
-    (512, 256, False, "auto", 16, 16),     # one launch covers every candidate
-    (512, 300, False, "auto", 3, 3),       # rows % 8 != 0
+@pytest.mark.parametrize("D,K,need_dt,precision,h,w,route", [
+    (128, 300, False, "auto", 16, 16, None),     # no CTA-pair kernel for D = 128
+    (512, 300, False, "fp32", 16, 16, None),     # fp32 parity mode
+    (512, 300, True, "auto", 16, 16, None),      # dText
+    (512, 256, False, "auto", 16, 16, "bf16"),   # one launch covers every candidate
+    (512, 300, False, "auto", 3, 3, None),       # rows % 8 != 0
 ])
-def test_rep4_plan_is_unchanged_outside_the_kblocked_shapes(D, K, need_dt, precision, h, w):
+def test_rep4_plan_outside_the_kblocked_shapes(D, K, need_dt, precision, h, w, route):
+    """Outside the K-blocked shapes a four-target call takes one tensor-core launch, or no kernel takes it (None)."""
     from rangeclip_b200 import ops
-    assert ops._infonce_plan(_x(D, h, w), K, need_dt, precision, 4) == "bf16"
+    assert ops._infonce_plan(_x(D, h, w), K, need_dt, precision, 4) == route
 
 
-def test_rep1_plan_is_unchanged():
+def test_rep1_plan():
     from rangeclip_b200 import ops
     assert ops._infonce_plan(_x(512), 300, False, "auto", 1) == "kblocked"
-    assert ops._infonce_plan(_x(512), 300, False, "bf16", 1) == "bf16"
+    assert ops._infonce_plan(_x(512), 300, False, "bf16", 1) is None          # one launch takes at most 256 candidates
     assert ops._infonce_plan(_x(128), 300, False, "auto", 1) == "fp32"
 
 
