@@ -97,12 +97,12 @@ int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t ld_b,
  *                           round 2 = backward launches with both flags: dx and dlogtau of each block add up to the full gradient
  * rc_infonce_bf16_rep4 takes the same flags (D = 256 / 512, no dt): y4 holds each target relative to the launch's first
  * row, w4 is 0 for every ignored target, lse is [B*hw] (one value per shared row: per block out, or in), and round 1's
- * loss_sum = sum_q wtot_q lse_blk - sum_{y_qj in blk} w_qj z_qy with wtot_q = sum_j w_qj.  rc_infonce_bf16_dyn and
- * rc_infonce_bf16_kblocks take one target per row only. */
+ * loss_sum = sum_q wtot_q lse_blk - sum_{y_qj in blk} w_qj z_qy with wtot_q = sum_j w_qj.  rc_infonce_bf16_dyn rejects
+ * these flags (its K-blocked form is rc_infonce_bf16_dyn_kblock); rc_infonce_bf16_kblocks takes one target per row only. */
 #define RC_INFONCE_KEEP_WEIGHT 2
 #define RC_INFONCE_LSE_GIVEN 4
 /* Backward launches (dx given, no dt) of D = 256 / 512 with K and log tau given by the host (rc_infonce_bf16, _rep4 and the
- * K-blocked rounds) run the kernel whose softmax tile is a tensor-memory operand of the dX GEMM (TS-mode tcgen05.mma,
+ * K-blocked rounds), and those of rc_infonce_bf16_dyn_kblock, run the kernel whose softmax tile is a tensor-memory operand of the dX GEMM (TS-mode tcgen05.mma,
  * csrc/infonce_ts.cu).  Forward-only launches, launches with dt and rc_infonce_bf16_dyn run the kernel with both operands in
  * shared memory (SS, csrc/infonce_umma2.cu).  Both give the same results bit for bit; DESIGN.md records their speed.
  *   RC_INFONCE_SS_KERNEL  run the SS kernel for a backward launch too (A/B measurements)
@@ -162,6 +162,28 @@ int rc_infonce_bf16_dyn(const void* x, rc_dtype x_dtype, int B, int D, int64_t H
                         const double* w_sum_in, const float* grad_scale,
                         void* dx, double* dlogtau,
                         void* workspace, int64_t workspace_bytes, int flags, void* stream);
+/* rc_infonce_bf16_dyn for one block of the K-blocked rounds (more than 256 rows in the contrast set of the sync-free loss,
+ * e.g. rc_contrast_build with k_cap up to 1024): the launch is shaped for rows [k0, k0 + K) of the set, K <= 256, and
+ * reads the set's valid row count from k_dev and log(tau) from log_tau_dev (both required) when it starts.
+ *   valid rows of the launch = min(K, *k_dev - k0); for k0 = 0 at least 1, as rc_infonce_bf16_dyn
+ *   t_bf16 / tt_bf16 the block's rows as [Kp][D] / [D][Kp] (rows past the valid ones are zero pad rows)
+ *   y, w     every launch runs the RC_INFONCE_KEEP_WEIGHT form: y is relative to k0 and may fall outside [0, K); w is 0 for
+ *            every ignored target.  rep = 1 or 4 (y, w [B*HW] or [B*HW][4])
+ *   lse      [B*HW], one value per embedding row: OUT per block in round 1, IN with RC_INFONCE_LSE_GIVEN in round 2
+ *   flags    RC_INFONCE_KEEP_WEIGHT, RC_INFONCE_LSE_GIVEN, RC_INFONCE_ACCUMULATE_DX, RC_INFONCE_SS_KERNEL,
+ *            RC_INFONCE_PREPASS_DONE.  Backward launches run the TS kernel unless RC_INFONCE_SS_KERNEL (bit-identical).
+ * EMPTY LAUNCH: when no row of the block is valid (k0 > 0 and *k_dev <= k0) the kernel returns at once.  It writes no lse
+ * and no dx and adds nothing to loss_sum, w_sum or dlogtau, so an RC_INFONCE_ACCUMULATE_DX launch leaves dx as it was.
+ * The block at k0 = 0 is never empty; it should be the launch that stores dx.  A caller shapes its launches for the
+ * capacity of the set (ceil(capacity / 256) blocks) and combines the per-block results on the device, treating an empty
+ * block's lse as -inf.  D = 256 or 512, no dText; everything else as rc_infonce_bf16_dyn. */
+int rc_infonce_bf16_dyn_kblock(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW,
+                               const void* t_bf16, const void* tt_bf16, int K, const int32_t* k_dev, int k0,
+                               const int32_t* y, const float* w, const float* log_tau_dev, int rep,
+                               float* lse, double* loss_sum, double* w_sum,
+                               const double* w_sum_in, const float* grad_scale,
+                               void* dx, double* dlogtau,
+                               void* workspace, int64_t workspace_bytes, int flags, void* stream);
 /* The pre-pass alone: 1/|x_p| of the bf16-rounded rows (+ bf16 copy of an f32 x) into workspace. */
 int rc_infonce_prepass(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW,
                        void* workspace, int64_t workspace_bytes, void* stream);

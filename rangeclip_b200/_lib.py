@@ -33,6 +33,8 @@ PROTOTYPES = {
                              _vp, _vp, _vp, _vp, _i64, _i32, _vp],
     "rc_infonce_bf16_dyn": [_vp, _i32, _i32, _i32, _i64, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp,
                             _vp, _vp, _vp, _i64, _i32, _vp],
+    "rc_infonce_bf16_dyn_kblock": [_vp, _i32, _i32, _i32, _i64, _vp, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp,
+                                   _vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp],
     "rc_contrast_build": [_vp, _i32, _vp, _vp, _i32, _i32, _i32, C.c_uint64, _vp, _i32, _vp, _vp, _vp, _vp],
     "rc_infonce_bf16_kblocks": [_vp, _i32, _i32, _i64, _vp, _vp, _i32, _i32, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                 _vp, _i64, _i32, _vp],

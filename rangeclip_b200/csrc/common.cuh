@@ -87,11 +87,14 @@ struct InfoncePairArgs {
   const float* lse_in;
   // SS only
   void* g_out;                  // dText: G = rs (P - sum onehot), bf16 [B][HW][Kp]
-  const int32_t* k_dev;         // rc_infonce_bf16_dyn: valid candidate rows and log tau in device memory
+  // rc_infonce_bf16_dyn (SS) and rc_infonce_bf16_dyn_kblock (SS forward, TS backward): valid candidate rows and log tau in
+  // device memory; k0 = the first contrast row of a K-blocked launch's block
+  const int32_t* k_dev;
   const float* log_tau_dev;
+  int k0;
 };
 int launch_infonce_pair(const InfoncePairArgs& a, cudaStream_t s);
-// backward launches without dText, device-side K or device-side tau
+// backward launches without dText, with host-side K and tau, or K-blocked with device-side K and tau
 int launch_infonce_ts(const InfoncePairArgs& a, cudaStream_t s);
 // dText = G^T X on the tensor cores (infonce_dt_umma.cu); G is the bf16 [B][HW][Kp] tensor the pair kernel writes
 int launch_infonce_dt(const void* g, const void* xsrc, int B, int D, int64_t HW, int K, float* dt, cudaStream_t s);

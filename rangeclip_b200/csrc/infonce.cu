@@ -3,7 +3,7 @@
 // arguments, runs the pre-pass and launches one of the kernels:
 //   dText   infonce_umma2.cu (writes G) + infonce_dt_umma.cu (dT = G^T X)
 //   1-CTA   infonce_umma.cu   D = 128 / 384
-//   TS      infonce_ts.cu     backward launches without dText, D = 256 / 512
+//   TS      infonce_ts.cu     backward launches without dText, D = 256 / 512 (rc_infonce_bf16_dyn's excepted)
 //   SS      infonce_umma2.cu  forward-only launches, rc_infonce_bf16_dyn and RC_INFONCE_SS_KERNEL, D = 256 / 512
 #include "common.cuh"
 #include <stdlib.h>
@@ -262,7 +262,8 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
                              const void* tt_bf16, int K, const int32_t* y, const float* w, float inv_tau, float* lse,
                              double* loss_sum, double* w_sum, const double* w_sum_in, const float* grad_scale, void* dx,
                              float* dt, double* dlogtau, void* workspace, int64_t workspace_bytes, int flags, int rep,
-                             void* stream, const int32_t* k_dev = nullptr, const float* log_tau_dev = nullptr) {
+                             void* stream, const int32_t* k_dev = nullptr, const float* log_tau_dev = nullptr,
+                             bool dev_blocks = false, int k0 = 0) {
   using namespace rc;
   RC_REQUIRE(x && t_bf16 && y && w && workspace, "rc_infonce_bf16: null pointer");
   RC_REQUIRE(B >= 0 && HW >= 0, "rc_infonce_bf16: bad shape");
@@ -287,7 +288,8 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   const char* impl = nullptr;
 #endif
   const bool use_pair = (rep != 1 || !(impl != nullptr && impl[0] == '1')) && infonce_pair_supported(D);
-  const int keep_w = (flags & RC_INFONCE_KEEP_WEIGHT) ? 1 : 0;
+  // rc_infonce_bf16_dyn_kblock: y is relative to k0 and w = 0 marks an ignored target, the RC_INFONCE_KEEP_WEIGHT form
+  const int keep_w = (dev_blocks || (flags & RC_INFONCE_KEEP_WEIGHT)) ? 1 : 0;
   const int acc_dx = (flags & RC_INFONCE_ACCUMULATE_DX) ? 1 : 0;
   const float* lse_in = (flags & RC_INFONCE_LSE_GIVEN) ? lse : nullptr;
   if (acc_dx) RC_REQUIRE(bwd, "rc_infonce_bf16: RC_INFONCE_ACCUMULATE_DX needs dx");
@@ -317,7 +319,7 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
     return launch_infonce_1cta(xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, inv_norm, y, w, inv_tau, grad_scale, w_sum_in, lse,
                                loss_sum, w_sum, dlogtau, s);
   InfoncePairArgs a{xsrc, dx, t_bf16, tt_bf16, B, D, HW, K, y, w, inv_tau, grad_scale, w_sum_in, lse, loss_sum, w_sum, dlogtau,
-                    rep, keep_w, acc_dx, /*kb*/ 0, lse_in, /*g_out*/ nullptr, k_dev, log_tau_dev};
+                    rep, keep_w, acc_dx, /*kb*/ 0, lse_in, /*g_out*/ nullptr, k_dev, log_tau_dev, k0};
   if (dt != nullptr) {
     // dText: the pair kernel also writes G = rs (P - sum onehot) (bf16 [B][HW][Kp]) into the workspace, then one
     // split-K GEMM over the pixels (infonce_dt_umma.cu) adds G^T X to dt.
@@ -327,8 +329,10 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
     if ((rcode = launch_infonce_pair(a, s))) return rcode;
     return launch_infonce_dt(a.g_out, xsrc, B, D, HW, K, dt, s);
   }
-  // backward launches: the softmax tile as a tensor-memory operand of the dX GEMM (infonce_ts.cu) unless RC_INFONCE_SS_KERNEL
-  if (bwd && !(flags & RC_INFONCE_SS_KERNEL) && k_dev == nullptr && log_tau_dev == nullptr) return launch_infonce_ts(a, s);
+  // backward launches: the softmax tile as a tensor-memory operand of the dX GEMM (infonce_ts.cu) unless RC_INFONCE_SS_KERNEL;
+  // the one-launch device-parameter form (rc_infonce_bf16_dyn) runs the SS kernel
+  if (bwd && !(flags & RC_INFONCE_SS_KERNEL) && (dev_blocks || (k_dev == nullptr && log_tau_dev == nullptr)))
+    return launch_infonce_ts(a, s);
   return launch_infonce_pair(a, s);
 }
 
@@ -362,6 +366,23 @@ extern "C" int rc_infonce_bf16_dyn(const void* x, rc_dtype x_dtype, int B, int D
                            nullptr, dlogtau, workspace, workspace_bytes, flags, rep, stream, k_dev, log_tau_dev);
 }
 
+// rc_infonce_bf16_dyn for one block of the K-blocked rounds: rows [k0, k0 + K) of a contrast set whose valid row count is
+// *k_dev; a launch whose block holds no valid row returns at once in the kernel (rangeclip_b200.h)
+extern "C" int rc_infonce_bf16_dyn_kblock(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16,
+                                          const void* tt_bf16, int K, const int32_t* k_dev, int k0, const int32_t* y,
+                                          const float* w, const float* log_tau_dev, int rep, float* lse, double* loss_sum,
+                                          double* w_sum, const double* w_sum_in, const float* grad_scale, void* dx,
+                                          double* dlogtau, void* workspace, int64_t workspace_bytes, int flags, void* stream) {
+  using namespace rc;
+  RC_REQUIRE(k_dev != nullptr && log_tau_dev != nullptr, "rc_infonce_bf16_dyn_kblock: k_dev and log_tau_dev are required");
+  RC_REQUIRE(rep == 1 || rep == 4, "rc_infonce_bf16_dyn_kblock: rep must be 1 or 4");
+  RC_REQUIRE(k0 >= 0, "rc_infonce_bf16_dyn_kblock: k0=%d must be >= 0", k0);
+  if (K < 1 || K > 256) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn_kblock: K=%d outside [1,256] (one block)", K);
+  if (!infonce_pair_supported(D)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn_kblock: D=%d must be 256 or 512", D);
+  return infonce_bf16_impl(x, x_dtype, B, D, HW, t_bf16, tt_bf16, K, y, w, 0.f, lse, loss_sum, w_sum, w_sum_in, grad_scale, dx,
+                           nullptr, dlogtau, workspace, workspace_bytes, flags, rep, stream, k_dev, log_tau_dev, true, k0);
+}
+
 extern "C" int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, int64_t HW, const void* t_bf16_all,
                                        const void* tt_bf16_all, int K, int n_blocks, const int32_t* y_rel, const float* w_rep,
                                        float inv_tau, float* lse, double* loss_sum, double* w_sum, const double* w_sum_in,
@@ -387,7 +408,7 @@ extern "C" int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, i
   // the kb blocks of 256 candidate rows are the "images" of one launch; every target keeps its weight
   const InfoncePairArgs a{xsrc, dx_blocks, t_bf16_all, tt_bf16_all, n_blocks, D, HW, K, y_rel, w_rep, inv_tau, grad_scale,
                           w_sum_in, lse, loss_sum, w_sum, dlogtau, /*rep*/ 1, /*keep_w*/ 1, /*acc_dx*/ 0, /*kb*/ n_blocks, lse_in,
-                          nullptr, nullptr, nullptr};
+                          nullptr, nullptr, nullptr, 0};
   if (bwd && !(flags & RC_INFONCE_SS_KERNEL)) return launch_infonce_ts(a, s);
   return launch_infonce_pair(a, s);
 }

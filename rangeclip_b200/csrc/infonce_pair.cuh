@@ -81,6 +81,14 @@ __device__ __forceinline__ int text_row0(const Tiling& prm, int pj) {
   return (kKB && prm.kb > 0) ? div_tiles(prm, 2 * pj) * 256 : 0;
 }
 
+// K-blocked launches with the row count in device memory (rc_infonce_bf16_dyn_kblock): the valid rows of the launch's
+// block, rows [k0, k0 + K) of the contrast set, of which *k_dev are valid in all.  0 or fewer: an empty launch.  The first
+// block keeps at least one row, as the one-launch form does (rows past *k_dev are zero pad rows).
+__device__ __forceinline__ int block_rows(const int32_t* k_dev, int k0, int K) {
+  const int v = min(K, __ldg(k_dev) - k0);
+  return k0 == 0 ? max(1, v) : v;
+}
+
 // consumer-release barriers live in the leader CTA
 __device__ __forceinline__ void arrive_leader(bool leader_cta, uint64_t* bar) {
   if (leader_cta) mbar_arrive(bar);

@@ -66,7 +66,13 @@ constexpr int kSmemBytes = kOffBars + (int)sizeof(Bars);
 static_assert(kSmemBytes <= 232448, "shared-memory budget of one SM (227 KB)");
 
 // bring-up ablation bits (Tiling::ablate): 1 no epilogue x loads, 2 no dX stores, 256 no text reloads
-struct Params : Tiling {};
+// K-blocked launches of rc_infonce_bf16_dyn_kblock (read by the kKB instantiations only): the contrast set's valid rows and
+// log(tau) in device memory (nullable: K and inv_tau are used), k0 = the first row of this launch's block (block_rows)
+struct Params : Tiling {
+  const int32_t* k_dev;
+  const float* log_tau_dev;
+  int k0;
+};
 
 // R = targets per embedding row (1, or 4 for the shared 2x2 form); kKB: K-blocked launches (keep_w / lse_in / kb)
 template <int R, bool kKB>
@@ -92,6 +98,9 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
   const int n_clusters = gridDim.x / 2;
   const int cluster_id = blockIdx.x / 2;
   const int my_pairs = cluster_id < prm.n_pairs ? (prm.n_pairs - cluster_id + n_clusters - 1) / n_clusters : 0;
+  // an empty K block: the whole cluster leaves before any barrier or tensor memory exists (infonce_umma2.cu); dX, lse and the
+  // sums stay untouched, so an RC_INFONCE_ACCUMULATE_DX launch adds nothing
+  if (kKB && prm.k_dev != nullptr && block_rows(prm.k_dev, prm.k0, prm.K) <= 0) return;
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&map_x_s); tma_prefetch_desc(&map_t); tma_prefetch_desc(&map_tt);
@@ -274,8 +283,12 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
     int ng, nr;
     norm_coords(ng, nr);
     uint32_t nit = 0;
-    const bool use_bound = prm.inv_tau * (2.02f * kLog2e) < 100.f;
-    const float ml_bound = prm.inv_tau * (1.01f * kLog2e);
+    // log(tau) in device memory (kKB only): inv_tau formed as the SS kernel forms it, so that both stay bit-identical.  The
+    // other instantiations read prm.inv_tau at every use, as they always have (a local copy changes their code).
+    const float inv_tau_dev = (kKB && prm.log_tau_dev != nullptr) ? expf(-__ldg(prm.log_tau_dev)) : 0.f;
+    auto inv_tau = [&]() { return (kKB && prm.log_tau_dev != nullptr) ? inv_tau_dev : prm.inv_tau; };
+    const bool use_bound = inv_tau() * (2.02f * kLog2e) < 100.f;
+    const float ml_bound = inv_tau() * (1.01f * kLog2e);
     for (int l = 0; l < my_pairs; ++l) {
       const int sl = l & 1;
       const int tile = 2 * pair_of(l) + (int)rank;
@@ -284,7 +297,10 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       const int px = tile_ok ? (tile - b * prm.tiles_per_img) * kTilePx + row : 0;
       const bool valid = tile_ok && px < prm.HW;
       const int64_t m = (int64_t)b * prm.HW + px;
-      const int Kt = (kKbAll && prm.kb > 0) ? min(256, prm.K - 256 * b) : prm.K;
+      // valid candidate rows (rows past them are zero pads): kb mode's last block may be short; a block of
+      // rc_infonce_bf16_dyn_kblock has block_rows of them
+      const int Kt = (kKbAll && prm.kb > 0) ? min(256, prm.K - 256 * b)
+                     : ((kKB && prm.k_dev != nullptr) ? block_rows(prm.k_dev, prm.k0, prm.K) : prm.K);
       const float ok = nx_ok;
       const bool px_ok = ok != 0.f;
       const int yi = nx_y;
@@ -298,7 +314,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       RC_TACC(1, tnorm);
       if (warp == 4) RC_EV(l, 12);      // row norms of the tile done
       const float inv_n = px_ok ? inv_n_tile : 0.f;
-      const float zs = inv_n * prm.inv_tau;
+      const float zs = inv_n * inv_tau();
       const float zl = zs * kLog2e;
       RC_WAIT(mbar_wait, &bars->s_full[sl], (l >> 1) & 1, 12);
       tc_fence_after();
@@ -329,7 +345,7 @@ infonce_ts_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B][D][HW]
       const float lse = row_lse<kKB>(prm, valid, ml, half, wtot, tz, zs, sum, acc_s[0], acc_s[128]);
       const float coef = coefb * wtot;
       const float inv_sum = 1.f / sum;
-      const float rsv = p_scale(inv_n, prm.inv_tau, coef, inv_sum);
+      const float rsv = p_scale(inv_n, inv_tau(), coef, inv_sum);
       if (half == 0) {
         const float cj = proj_coef(coef, coefb, sez, tz, zs, inv_sum);
         sc_s[(l & (kScaleBufs - 1)) * 128 + row] = -(inv_n * inv_n * cj);      // dx = acc + (-cs) x
@@ -538,6 +554,7 @@ int launch_infonce_ts(const InfoncePairArgs& a, cudaStream_t s) {
   Params prm;
   int grid = 0;
   if ((rcode = fill_tiling(prm, a, &grid))) return rcode;
+  prm.k_dev = a.k_dev; prm.log_tau_dev = a.log_tau_dev; prm.k0 = a.k0;
   auto launch = [&](auto kernel) -> int {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) return fail(RC_ERR_CUDA, "rc_infonce_bf16(ts): smem opt-in: %s", cudaGetErrorString(e));

@@ -26,7 +26,8 @@
 // pixels of both tiles).
 //
 // This kernel runs forward-only launches, the dText path (it writes G for infonce_dt_umma.cu), rc_infonce_bf16_dyn and
-// RC_INFONCE_SS_KERNEL; backward launches otherwise run the TS kernel (infonce_ts.cu).  The tiling, the operand
+// RC_INFONCE_SS_KERNEL; backward launches otherwise run the TS kernel (infonce_ts.cu), those of rc_infonce_bf16_dyn_kblock
+// included.  The tiling, the operand
 // producers, the relay and the softmax arithmetic are shared with it through infonce_pair.cuh, so that both give
 // bit-identical dX and lse; this file holds the SS pipeline, the P store into shared memory (and the G store), the
 // row-scale exchange between the CTAs and the dX epilogue.
@@ -78,6 +79,7 @@ struct Params : Tiling {
   // temperature are read from device memory at kernel start (nullable: K / inv_tau above are used)
   const int32_t* k_dev;
   const float* log_tau_dev;
+  int k0;                   // K-blocked launches with k_dev: first contrast row of this launch's block (block_rows)
 };
 
 // 16 pixels (32 bytes) of one channel row, straight from global memory.  `n8` = number of valid
@@ -127,6 +129,9 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
   const int b_half = (n_blk + 1) / 2;
   const int n_clusters = gridDim.x / 2;
   const int cluster_id = blockIdx.x / 2;
+  // an empty K block (rc_infonce_bf16_dyn_kblock): every CTA reads the same count, so the whole cluster leaves before any
+  // barrier or tensor memory exists, and nothing is written
+  if (kKB && prm.k_dev != nullptr && block_rows(prm.k_dev, prm.k0, prm.K) <= 0) return;
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&map_x_s); tma_prefetch_desc(&map_t);
@@ -331,7 +336,9 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
     };
     if (cluster_id < prm.n_pairs) norm_next();
     const float inv_tau = prm.log_tau_dev != nullptr ? expf(-__ldg(prm.log_tau_dev)) : prm.inv_tau;
-    const int K_valid = prm.k_dev != nullptr ? max(1, min(__ldg(prm.k_dev), prm.K)) : prm.K;      // rows past it are zero pads
+    // rows past K_valid are zero pads; K-blocked launches with k_dev: the rows of their block (block_rows)
+    const int K_valid = (kKB && prm.k_dev != nullptr) ? block_rows(prm.k_dev, prm.k0, prm.K)
+                        : (prm.k_dev != nullptr ? max(1, min(__ldg(prm.k_dev), prm.K)) : prm.K);
     const bool use_bound = inv_tau * (2.02f * kLog2e) < 100.f;
     const float ml_bound = inv_tau * (1.01f * kLog2e);
     // peer copies of the row-scale arrays (same offsets in the other CTA's shared memory)
@@ -643,7 +650,7 @@ int launch_infonce_pair(const InfoncePairArgs& a, cudaStream_t s) {
   prm.store_g = a.g_out != nullptr;
   prm.wide = (a.HW % 16 == 0) && (reinterpret_cast<uintptr_t>(a.xsrc) % 32 == 0) && (reinterpret_cast<uintptr_t>(a.dx) % 32 == 0);
   prm.x = reinterpret_cast<const __nv_bfloat16*>(a.xsrc);
-  prm.k_dev = a.k_dev; prm.log_tau_dev = a.log_tau_dev;
+  prm.k_dev = a.k_dev; prm.log_tau_dev = a.log_tau_dev; prm.k0 = a.k0;
   auto launch = [&](auto kernel) -> int {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) return fail(RC_ERR_CUDA, "rc_infonce_bf16(pair): smem opt-in: %s", cudaGetErrorString(e));

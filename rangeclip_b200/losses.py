@@ -88,10 +88,11 @@ def similarity_csr(label_similarity_sets, C: int, use_medium: bool, use_hard: bo
 
 
 def device_builder_supported(x: torch.Tensor, rep: int, C: int, k_cap: int, text_requires_grad: bool, precision: str) -> bool:
-    """Calls the sync-free path covers: label histogram in shared memory (2 <= C <= 12000), not the fp32 parity mode, and a
-    tensor-core launch that reads K and tau from device memory (``ops._infonce_plan``: the CTA-pair kernel, frozen text)."""
+    """Calls the sync-free path covers: label histogram in shared memory (2 <= C <= 12000), not the fp32 parity mode, and
+    tensor-core launches that read K and tau from device memory (``ops._infonce_plan`` with ``dev_blocks``: the CTA-pair
+    kernel, frozen text, one launch up to 256 contrast rows and the K-blocked rounds up to 1024)."""
     return (2 <= C <= 12000 and precision != "fp32"
-            and ops._infonce_plan(x, k_cap, text_requires_grad, "bf16", rep, dev_params=True) is not None)
+            and ops._infonce_plan(x, k_cap, text_requires_grad, "bf16", rep, dev_params=True, dev_blocks=True) is not None)
 
 
 def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embeddings, label_similarity_sets,
@@ -130,7 +131,7 @@ def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embed
     aux = dict(rand_indices=rand_indices, contrast_indices=None)
     if contrast_builder not in ("reference", "device"):
         raise RuntimeError(f"contrast_builder must be 'reference' or 'device', got {contrast_builder!r}")
-    k_cap = max(2, min(int(max_contrast), 256, C))
+    k_cap = max(2, min(int(max_contrast), 1024, C))
     if contrast_builder == "device" and device_builder_supported(pixel_embeddings, 4 if shared2x2 else 1, C, k_cap,
                                                                  candidate_text_embeddings.requires_grad, precision):
         # ---- sync-free path (SURVEY 8f-2): label histogram -> contrast set, label map, text operands and the loss launch
@@ -156,13 +157,13 @@ def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embed
         t_norm, tb, ttb = torch.ops.rangeclip.text_prepare(candidate_text_embeddings, contrast)
         if with_smoothness:
             loss, smooth = ops.pixel_losses(pixel_embeddings, t_norm, log_temperature_text, y, w, "bf16", t_bf16=(tb, ttb),
-                                            k_dev=kinfo)
+                                            k_dev=kinfo, dev_blocks=True)
             aux["smoothness"] = smooth
             return loss, aux
         if shared2x2:
             y, w = group_2x2(y.view(B, H, W)), group_2x2(w.view(B, H, W))
         loss = ops.infonce(pixel_embeddings, t_norm, log_temperature_text, y, w, "bf16", rep=4 if shared2x2 else 1,
-                           t_bf16=(tb, ttb), k_dev=kinfo)
+                           t_bf16=(tb, ttb), k_dev=kinfo, dev_blocks=True)
         return (loss, aux) if return_aux else loss
     # the sampled foreground labels (model.py:222-233: gather, drop label 0, torch.unique) from a label histogram of the
     # sampled pixels: one small kernel instead of a 3M-element gather + boolean index + sort
@@ -256,7 +257,9 @@ def compute_loss(self, pixel_embeddings, target_indices, candidate_text_embeddin
     counter-based stream seeded from the CPU torch generator -- NOT the reference's NumPy / randperm streams, so the drawn
     distractors differ from the reference's for the same seeds), its size and the temperatures stay in device memory, and
     ``loss_info`` is a ``LazyLossInfo`` whose floats are fetched on first access: the call never synchronises with the
-    host.  At most ``max_contrast`` (<= 256) rows; distractors are trimmed to fit."""
+    host.  At most ``max_contrast`` (<= 1024) rows; distractors are trimmed to fit.  Up to 256 rows the loss is one
+    tensor-core launch; above, K-blocked rounds shaped for ``max_contrast`` rows, each launch reading from device memory how
+    many of its rows the drawn set fills."""
     return _compute_loss(self, pixel_embeddings, target_indices, candidate_text_embeddings, label_similarity_sets,
                          area_embeddings, image_embeddings, W_text, W_image, W_smooth, percent_image_sampling,
                          k_distractors, pct_medium, pct_hard, pct_rand, precision, shared2x2=False,

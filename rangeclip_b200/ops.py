@@ -176,22 +176,29 @@ def contrast_build(counts: torch.Tensor, sim_off: Optional[torch.Tensor], sim_it
 # ----------------------------------------------------------------------------------------------
 
 def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: int, need_dx: bool = True,
-                  dev_params: bool = False) -> Optional[str]:
+                  dev_params: bool = False, dev_blocks: bool = False) -> Optional[str]:
     """The route of one InfoNCE call; the only place that chooses it.  ``infonce_raw`` runs it, the fake-tensor rules of
     rangeclip::infonce / pixel_losses derive dX's dtype from it and the loss drop-ins ask it whether a kernel takes a call.
       'fp32'      the CUDA-core kernel (rc_infonce_f32): any shape, one target per row, host K and tau;
       'bf16'      one tensor-core launch (rc_infonce_bf16 / _rep4 / _dyn): K <= 256, D in (128, 256, 384, 512), HW % 8 == 0;
                   four targets, dText (with dX) and the device-parameter form only on the CTA-pair kernel (D in (256, 512));
       'kblocked'  tensor cores over blocks of 256 candidate rows (``infonce_kblocked_raw``): D in (256, 512), HW % 8 == 0, no
-                  dText, host K and tau; what "auto" (and, for four targets, "bf16") takes above 256 candidates;
+                  dText, host K and tau; what "auto" (and, for four targets, "bf16") takes above 256 candidates; with
+                  ``dev_blocks`` also for K and tau in device memory, up to 1024 rows (rc_infonce_bf16_dyn_kblock);
       None        no kernel covers the call.
     x: a tensor or meta tensor [B, D, H, W] / [B, D, HW]; K: rows of t_norm; precision: 'auto', 'fp32', 'bf16' or 'kblocked';
     need_dx: dX is wanted (the autograd operators always want it with dText); dev_params: K and log(tau) are read from device
-    memory (k_dev / log_tau_dev)."""
+    memory (k_dev / log_tau_dev).  dev_blocks (opt-in, implies dev_params): K is the CAPACITY of the contrast set (its valid
+    row count stays in device memory); above 256 the K-blocked rounds read it from there -- 'kblocked' up to 1024 rows,
+    'bf16' (the one-launch form) up to 256."""
     if rep not in (1, 4) or precision not in ("auto", "fp32", "bf16", "kblocked"):
         return None
     D = x.shape[1]
     HW = x[0, 0].numel() if x.shape[0] and D else 0
+    if dev_blocks:
+        if precision == "fp32" or need_dt or not kblocked_supported(D, HW) or not 1 <= K <= _DEV_BLOCKS_MAX_ROWS:
+            return None
+        return "kblocked" if (K > 256 or precision == "kblocked") else "bf16"
     kblocked = kblocked_supported(D, HW) and not need_dt and not dev_params
     if precision == "kblocked":
         return "kblocked" if kblocked else None
@@ -209,14 +216,16 @@ def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: i
     return "fp32" if precision == "auto" and rep == 1 and not dev_params else None
 
 
-def _infonce_route(x: torch.Tensor, K: int, need_dx: bool, need_dt: bool, precision: str, rep: int, dev_params: bool) -> str:
+def _infonce_route(x: torch.Tensor, K: int, need_dx: bool, need_dt: bool, precision: str, rep: int, dev_params: bool,
+                   dev_blocks: bool = False) -> str:
     """``_infonce_plan``, or the error of a call no kernel covers (raised alike by the op and by its fake-tensor rules)."""
-    route = _infonce_plan(x, K, need_dt, precision, rep, need_dx, dev_params)
+    route = _infonce_plan(x, K, need_dt, precision, rep, need_dx, dev_params, dev_blocks)
     if route is None:
         D = x.shape[1]
         HW = x[0, 0].numel() if x.shape[0] and D else 0
         raise RuntimeError(f"infonce: no kernel covers D={D}, HW={HW}, K={K}, precision={precision!r}, rep={rep} "
-                           f"(need_dx={need_dx}, need_dt={need_dt}, device parameters={dev_params}); see _infonce_plan")
+                           f"(need_dx={need_dx}, need_dt={need_dt}, device parameters={dev_params}, device blocks={dev_blocks}); "
+                           "see _infonce_plan")
     return route
 
 
@@ -230,7 +239,7 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
                 need_dx: bool, need_dt: bool, precision: str = "auto",
                 grad_scale: Optional[torch.Tensor] = None, t_bf16=None, rep: int = 1, keep_bf16: bool = False,
                 flags: int = 0, k_dev: Optional[torch.Tensor] = None, log_tau_dev: Optional[torch.Tensor] = None,
-                fuse_tv: bool = False):
+                fuse_tv: bool = False, dev_blocks: bool = False):
     """One fused pass: returns dict(loss_sum, w_sum (double[1] tensors), lse, dx, dt, dlogtau).
     loss = loss_sum / w_sum; dx/dt/dlogtau are gradients of that mean loss times grad_scale.  The kernel family is
     ``_infonce_plan``'s route; a call no kernel covers raises ``RuntimeError``.
@@ -240,6 +249,8 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
     in one pass at backward time); flags: extra RC_INFONCE_* bits for rc_infonce_bf16 (e.g. RC_INFONCE_SS_KERNEL).
     k_dev / log_tau_dev (device int32[>=1] / float[1]): the sync-free form (rc_infonce_bf16_dyn) -- the number of valid rows of
     t_norm and log(tau) are read by the kernel from device memory; ``inv_tau`` is ignored; CTA-pair kernel shapes only.
+    dev_blocks (with k_dev / log_tau_dev): t_norm may hold up to 1024 rows; above 256 the K-blocked rounds run on them
+    (``infonce_kblocked_raw``), each launch reading its valid rows from k_dev.
     fuse_tv: the caller also wants tv_sums(x); where the launch has a pre-pass over x anyway (``_fused_tv``) the sums come
     out of that pass (rc_infonce_prepass_tv) as ``tv_sums`` -- and with need_dx the difference signs for tv_backward_codes
     as ``tv_codes`` --, else both keys are None."""
@@ -248,7 +259,9 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
     x, B, D, HW = _emb3(x)
     K = t_norm.shape[0]
     dev_params = log_tau_dev is not None
-    route = _infonce_route(x, K, need_dx, need_dt, precision, rep, dev_params)
+    if dev_blocks and (k_dev is None or not dev_params):
+        raise RuntimeError("infonce: dev_blocks needs k_dev and log_tau_dev")
+    route = _infonce_route(x, K, need_dx, need_dt, precision, rep, dev_params, dev_blocks)
     tv_hw = tuple(x_in.shape[2:]) if (fuse_tv and _fused_tv(x_in, route)) else None
     dev = x.device
     M = B * HW
@@ -259,7 +272,7 @@ def infonce_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch
     if route == "kblocked":
         # more candidates than one launch takes: tensor cores over blocks of 256 candidate rows instead of the CUDA-core
         # kernel (which needs ~100x longer at full size)
-        r = infonce_kblocked_raw(x, t_norm, y, w, inv_tau, need_dx, rep=rep)
+        r = infonce_kblocked_raw(x, t_norm, y, w, inv_tau, need_dx, rep=rep, k_dev=k_dev, log_tau_dev=log_tau_dev)
         dx = r["dx"]
         if dx is not None and grad_scale is not None:
             dx = dx * grad_scale.detach().reshape(1).to(device=dev, dtype=dx.dtype)
@@ -328,20 +341,29 @@ RC_INFONCE_PREPASS_DONE, RC_INFONCE_KEEP_WEIGHT, RC_INFONCE_LSE_GIVEN, RC_INFONC
 RC_INFONCE_SS_KERNEL = 32
 
 
+_DEV_BLOCKS_MAX_ROWS = 1024      # contrast-set capacity of the device-parameter K-blocked rounds: four blocks, dX summed in-kernel
+
+
 def kblocked_supported(D: int, HW: int) -> bool:
     return D in (256, 512) and HW % 8 == 0 and HW > 0
 
 
 def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch.Tensor, inv_tau: float,
-                         need_dx: bool, block: int = 256, keep_bf16: bool = False, rep: int = 1):
+                         need_dx: bool, block: int = 256, keep_bf16: bool = False, rep: int = 1,
+                         k_dev: Optional[torch.Tensor] = None, log_tau_dev: Optional[torch.Tensor] = None):
     """InfoNCE against MORE than 256 candidates on the tensor cores (model.py:304-321 at thousands of objects): the
     candidate rows are split into launches of <= 256.  Round 1: forward launches give the per-block logsumexp; their
     logsumexp is the row's lse over all candidates.  Round 2: fwd+bwd launches with that lse given produce per-block dx /
     dlogtau that add up to the full gradient.  Returns dict(loss, loss_sum, lse, dx, dlogtau, w_sum), loss = loss_sum / w_sum;
     bf16 operands, fp32 sums.
     rep = 4: every row of x is the embedding shared by a 2x2 block of pixels, y / w are [rows, 4] (rc_infonce_bf16_rep4,
-    one launch per block and round); lse is per row and a row's weight is the sum of its four."""
-    _need_cuda(x, t_norm, y, w)
+    one launch per block and round); lse is per row and a row's weight is the sum of its four.
+    k_dev / log_tau_dev (device int32, first entry / float[1]; both or neither): the sync-free form.  t_norm's rows are the
+    CAPACITY of the contrast set (<= 1024, the rows past k_dev[0] are zero pads) and shape the launches; each launch
+    (rc_infonce_bf16_dyn_kblock) reads how many of its block's rows are valid and log(tau) from device memory, and a block
+    past the valid rows is an empty launch.  The blocks are combined on the device with that block mask: nothing is read
+    back, ``inv_tau`` is ignored."""
+    _need_cuda(x, t_norm, y, w, k_dev, log_tau_dev)
     x, B, D, HW = _emb3(x)
     if not kblocked_supported(D, HW):
         raise RuntimeError(f"infonce_kblocked: needs D in (256, 512) and HW % 8 == 0; got D={D}, HW={HW}")
@@ -350,6 +372,15 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
     K = t_norm.shape[0]
     M = B * HW
     dev = x.device
+    dyn = k_dev is not None or log_tau_dev is not None
+    if dyn:
+        if k_dev is None or log_tau_dev is None:
+            raise RuntimeError("infonce_kblocked: k_dev and log_tau_dev go together")
+        if block != 256 or K > _DEV_BLOCKS_MAX_ROWS:
+            raise RuntimeError(f"infonce_kblocked: the device-parameter form takes blocks of 256 and at most "
+                               f"{_DEV_BLOCKS_MAX_ROWS} rows; got K={K}")
+        kd = k_dev.reshape(-1)[:1].to(torch.int32)
+        lt = log_tau_dev.detach().reshape(1).to(device=dev, dtype=torch.float32)
     y = y.reshape(-1, 4) if rep == 4 else y.reshape(-1)
     if y.numel() != M * rep or w.numel() != M * rep:
         raise RuntimeError("infonce_kblocked: y / w must have `rep` entries per embedding row")
@@ -368,7 +399,7 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
         check(L.rc_infonce_prepass(_p(x), xdt, B, D, HW, _p(ws), ws_bytes, st), "rc_infonce_prepass")
     starts = list(range(0, K, block))
     nb = len(starts)
-    if rep == 1 and B == 1 and HW % 256 == 0 and block == 256:
+    if rep == 1 and B == 1 and HW % 256 == 0 and block == 256 and not dyn:
         # one image of rows (the area-image loss): every candidate block in ONE launch per round -- the kernel's image
         # index runs over the blocks (rc_infonce_bf16_kblocks)
         tb_all = torch.zeros(nb * 256, D, device=dev, dtype=torch.bfloat16)
@@ -409,18 +440,34 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
     texts += [text_to_bf16(t_norm[s0:s0 + block]) for s0 in starts[n_full:]]
     ys = [(y - s0).contiguous() for s0 in starts]
     entry = L.rc_infonce_bf16 if rep == 1 else L.rc_infonce_bf16_rep4
+
+    def launch(i, s0, lse_ptr, a, w_sum_in, dx_ptr, dlt_ptr, fl, what):
+        Kb = min(block, K - s0)
+        if dyn:       # the valid rows and log(tau) come from device memory; an empty block's launch returns at once
+            check(L.rc_infonce_bf16_dyn_kblock(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(kd), s0, _p(ys[i]),
+                                               _p(w), _p(lt), rep, lse_ptr, a[0:].data_ptr(), a[1:].data_ptr(), w_sum_in, None,
+                                               dx_ptr, dlt_ptr, _p(ws), ws_bytes, fl, st), f"rc_infonce_bf16_dyn_kblock({what})")
+        else:
+            check(entry(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
+                        lse_ptr, a[0:].data_ptr(), a[1:].data_ptr(), w_sum_in, None, dx_ptr, None, dlt_ptr,
+                        _p(ws), ws_bytes, fl, st), f"rc_infonce_bf16({what})")
+
     lse_blk = torch.empty(nb, M, device=dev, dtype=torch.float32)
     acc = torch.zeros(nb, 4, device=dev, dtype=torch.float64)             # per block: loss_sum, w_sum, dlogtau, w_sum_in
     wsum = w.double().sum()
     acc[:, 3] = wsum
     for i, s0 in enumerate(starts):
-        Kb = min(block, K - s0)
-        check(entry(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
-                    lse_blk[i].data_ptr(), acc[i, 0:].data_ptr(), acc[i, 1:].data_ptr(), None, None, None, None, None,
-                    _p(ws), ws_bytes, 1 | RC_INFONCE_KEEP_WEIGHT, st), "rc_infonce_bf16(K block, forward)")
-    lse = torch.logsumexp(lse_blk, dim=0)
+        launch(i, s0, lse_blk[i].data_ptr(), acc[i], None, None, None, 1 | RC_INFONCE_KEEP_WEIGHT, "K block, forward")
     # sum_p w z[p, y_p] from the blocks that own the targets: loss_sum_b = sum_p w lse_b - sum_{y in b} w z_y
-    wz = ((lse_blk.double() * w_row).sum(dim=1) - acc[:, 0]).sum()
+    wz_blk = (lse_blk.double() * w_row).sum(dim=1) - acc[:, 0]
+    if dyn:
+        # blocks past the valid rows were empty launches: their lse (never written) counts as -inf, their terms as 0
+        first_rows = torch.arange(0, K, block, device=dev, dtype=torch.int32)
+        live = (kd > first_rows) | (first_rows == 0)          # (the first block is never empty)
+        lse_blk = torch.where(live[:, None], lse_blk, torch.full((), float("-inf"), device=dev))
+        wz_blk = torch.where(live, wz_blk, torch.zeros((), device=dev, dtype=torch.float64))
+    lse = torch.logsumexp(lse_blk, dim=0)
+    wz = wz_blk.sum()
     loss_sum = (lse.double() * w_row).sum() - wz
     loss = torch.where(wsum > 0, loss_sum / wsum.clamp_min(1e-300), torch.zeros_like(wsum))
     dx = dlogtau = None
@@ -430,15 +477,13 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
         acc2[:, 3] = wsum
         # up to four blocks: every launch after the first ADDS its gradient to the same bf16 tensor inside the kernel
         # (RC_INFONCE_ACCUMULATE_DX, TMA reduce-add stores: one extra rounding per block, launch order = summation order);
-        # more blocks are summed in fp32 here, block by block
+        # more blocks are summed in fp32 here, block by block.  The device-parameter form (at most four blocks) always
+        # accumulates in the kernel: an empty launch leaves dX as it is, where the fp32 sum would add a stale buffer.
         in_kernel = nb <= 4
         dx = None
         for i, s0 in enumerate(starts):
-            Kb = min(block, K - s0)
             fl = 1 | RC_INFONCE_KEEP_WEIGHT | RC_INFONCE_LSE_GIVEN | (RC_INFONCE_ACCUMULATE_DX if (in_kernel and i > 0) else 0)
-            check(entry(_p(x), xdt, B, D, HW, _p(texts[i][0]), _p(texts[i][1]), Kb, _p(ys[i]), _p(w), float(inv_tau),
-                        _p(lse), acc2[i, 0:].data_ptr(), acc2[i, 1:].data_ptr(), acc2[i, 3:].data_ptr(), None, _p(dxb),
-                        None, acc2[i, 2:].data_ptr(), _p(ws), ws_bytes, fl, st), "rc_infonce_bf16(K block, backward)")
+            launch(i, s0, _p(lse), acc2[i], acc2[i, 3:].data_ptr(), _p(dxb), acc2[i, 2:].data_ptr(), fl, "K block, backward")
             if not in_kernel:
                 dx = dxb.float() if dx is None else dx.add_(dxb)
         dlogtau = acc2[:, 2].sum()
@@ -804,29 +849,33 @@ def _mean_loss(r) -> torch.Tensor:
 @_op("rangeclip::infonce", mutates_args=(), device_types="cuda")
 def _op_infonce(x: torch.Tensor, t_norm: torch.Tensor, log_tau: torch.Tensor, y: torch.Tensor, w: torch.Tensor,
                 need_grad: bool, need_dt: bool, precision: str, rep: int, t_bf16: Optional[torch.Tensor],
-                tt_bf16: Optional[torch.Tensor], k_dev: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+                tt_bf16: Optional[torch.Tensor], k_dev: Optional[torch.Tensor] = None,
+                dev_blocks: bool = False) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
     """(loss, dx, dt, dlogtau): weighted InfoNCE(x, t_norm, y, w) / tau with the gradients of the MEAN loss produced by
     the same fused launch (single pass over x).  dx stays in the kernel's dtype (bf16 on the tensor-core path).
     ``k_dev`` (int32 device tensor, first entry = valid rows of t_norm): the sync-free form -- the kernel reads the row
-    count and log(tau) from device memory, nothing is read back here."""
-    return _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev, False)[:4]
+    count and log(tau) from device memory, nothing is read back here.  ``dev_blocks`` (with k_dev, opt-in): t_norm's rows are
+    the contrast set's capacity, up to 1024; above 256 the K-blocked rounds run on them (``_infonce_plan``)."""
+    return _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev, False,
+                            dev_blocks)[:4]
 
 
-def _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev, fuse_tv):
+def _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev, fuse_tv,
+                     dev_blocks=False):
     """Body of rangeclip::infonce (and of the InfoNCE half of rangeclip::pixel_losses): (loss, dx, dt, dlogtau, tv_sums | None, tv_codes | None)."""
     tb = (t_bf16, tt_bf16) if (t_bf16 is not None and tt_bf16 is not None) else None
     dyn = k_dev is not None
     inv_tau = 0.0 if dyn else float(torch.exp(-log_tau.detach().float()))      # one scalar sync, as .item() in the reference
     r = infonce_raw(x, t_norm, y, w, inv_tau, need_grad, need_dt, precision, t_bf16=tb, rep=rep, keep_bf16=True, k_dev=k_dev,
-                    log_tau_dev=log_tau if dyn else None, fuse_tv=fuse_tv)
+                    log_tau_dev=log_tau if dyn else None, fuse_tv=fuse_tv, dev_blocks=dev_blocks)
     dx, dt = r["dx"], r["dt"]
     return (_mean_loss(r), dx if dx is not None else _empty(x), dt if dt is not None else _empty(t_norm),
             r["dlogtau"].float().reshape(()), r.get("tv_sums"), r.get("tv_codes"))
 
 
 @_op_infonce.register_fake
-def _(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev=None):
-    route = _infonce_route(x, t_norm.shape[0], need_grad, need_dt, precision, rep, k_dev is not None)
+def _(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, rep, t_bf16, tt_bf16, k_dev=None, dev_blocks=False):
+    route = _infonce_route(x, t_norm.shape[0], need_grad, need_dt, precision, rep, k_dev is not None, dev_blocks)
     dx_dtype = torch.bfloat16 if route == "bf16" else x.dtype
     f32 = dict(device=x.device, dtype=torch.float32)
     return (torch.empty((), **f32), torch.empty(x.shape, device=x.device, dtype=dx_dtype) if need_grad else _empty(x),
@@ -857,7 +906,7 @@ def _infonce_backward(ctx, g, *_unused):
     need = ctx.needs_input_grad
     gx = None
     if g is None:
-        return (None,) * 12
+        return (None,) * 13
     if need[0]:
         if dx.dtype == ctx.x_dtype and not _graph_is_retained():
             # the common training case (loss.backward()): nobody can run this node again, so the saved gradient is scaled
@@ -870,7 +919,7 @@ def _infonce_backward(ctx, g, *_unused):
             gx = torch.ops.rangeclip.scale_to(dx, g, _DT_CODE[ctx.x_dtype])
     gt = dt * g if need[1] else None
     gl = (dlt * g).reshape(()) if need[2] else None
-    return (gx, gt, gl) + (None,) * 9
+    return (gx, gt, gl) + (None,) * 10
 
 
 _op_infonce.register_autograd(_infonce_backward, setup_context=_infonce_setup)
@@ -879,12 +928,13 @@ _op_infonce.register_autograd(_infonce_backward, setup_context=_infonce_setup)
 @_op("rangeclip::pixel_losses", mutates_args=(), device_types="cuda")
 def _op_pixel_losses(x: torch.Tensor, t_norm: torch.Tensor, log_tau: torch.Tensor, y: torch.Tensor, w: torch.Tensor,
                      need_grad: bool, need_dt: bool, precision: str, t_bf16: Optional[torch.Tensor],
-                     tt_bf16: Optional[torch.Tensor], k_dev: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+                     tt_bf16: Optional[torch.Tensor], k_dev: Optional[torch.Tensor] = None,
+                     dev_blocks: bool = False) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
     """(text InfoNCE, smoothness, dx_text, dt, dlogtau, tv_codes) of the SAME pixel embeddings: one autograd node for both
     terms, so that the backward is a single pass (model.py:272-291, 332-334 and their autograd).  tv_codes: the difference
     signs the backward needs, when the fp32 pre-pass produced them with the sums (else empty)."""
     loss, dx, dt, dlt, sums, codes = _infonce_forward(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, 1, t_bf16, tt_bf16,
-                                                      k_dev, True)
+                                                      k_dev, True, dev_blocks)
     if sums is None:
         sums = tv_sums(x)
     if codes is None:
@@ -896,8 +946,8 @@ def _op_pixel_losses(x: torch.Tensor, t_norm: torch.Tensor, log_tau: torch.Tenso
 
 
 @_op_pixel_losses.register_fake
-def _(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, t_bf16, tt_bf16, k_dev=None):
-    route = _infonce_route(x, t_norm.shape[0], need_grad, need_dt, precision, 1, k_dev is not None)
+def _(x, t_norm, log_tau, y, w, need_grad, need_dt, precision, t_bf16, tt_bf16, k_dev=None, dev_blocks=False):
+    route = _infonce_route(x, t_norm.shape[0], need_grad, need_dt, precision, 1, k_dev is not None, dev_blocks)
     dx_dtype = torch.bfloat16 if route == "bf16" else x.dtype
     f32 = dict(device=x.device, dtype=torch.float32)
     fused = need_grad and _fused_tv(x, route)
@@ -917,7 +967,7 @@ def _pixel_losses_backward(ctx, g_text, g_smooth, *_unused):
     need = ctx.needs_input_grad
     gx = None
     if g_text is None and g_smooth is None:
-        return (None,) * 11
+        return (None,) * 12
     if g_text is None:
         g_text = torch.zeros((), device=x.device, dtype=torch.float32)
     if g_smooth is None:
@@ -933,7 +983,7 @@ def _pixel_losses_backward(ctx, g_text, g_smooth, *_unused):
             gx = torch.ops.rangeclip.tv_bwd(x, scale, dx, g_text.float())
     gt = dt * g_text if need[1] else None
     gl = (dlt * g_text).reshape(()) if need[2] else None
-    return (gx, gt, gl) + (None,) * 8
+    return (gx, gt, gl) + (None,) * 9
 
 
 _op_pixel_losses.register_autograd(_pixel_losses_backward, setup_context=_pixel_losses_setup)
@@ -1265,25 +1315,30 @@ def _tb(t_bf16):
     return (None, None) if t_bf16 is None else (t_bf16[0], t_bf16[1])
 
 
-def infonce(x, t_norm, log_tau, y, w, precision="auto", rep=1, t_bf16=None, k_dev=None):
+def infonce(x, t_norm, log_tau, y, w, precision="auto", rep=1, t_bf16=None, k_dev=None, dev_blocks=False):
     """Autograd-aware fused InfoNCE (torch.ops.rangeclip.infonce); x [B,D,H,W], t_norm [K,D] normalised, y/w per pixel
     (rep = 4: x holds the embeddings shared by 2x2 pixel blocks, y/w are [B*H*W, 4]).  ``precision``: 'auto', 'fp32', 'bf16'
     or 'kblocked', the kernel family as ``_infonce_plan`` routes it.  ``t_bf16`` = (bf16 [Kp,D], bf16 [D,Kp]) copies of
-    t_norm from ``text_prepare`` (optional: built on the fly otherwise)."""
+    t_norm from ``text_prepare`` (optional: built on the fly otherwise).  ``k_dev``: the valid rows of t_norm in device memory
+    (log(tau) is then read from ``log_tau`` on the device as well); ``dev_blocks``: t_norm may then hold up to 1024 rows
+    (the K-blocked rounds above 256)."""
     _need_cuda(x, t_norm, y, w)
     tb, ttb = _tb(t_bf16)
     need_grad = bool(torch.is_grad_enabled() and (x.requires_grad or log_tau.requires_grad))
     need_dt = bool(torch.is_grad_enabled() and t_norm.requires_grad)
-    return torch.ops.rangeclip.infonce(x, t_norm, log_tau, y, w, need_grad or need_dt, need_dt, precision, rep, tb, ttb, k_dev)[0]
+    return torch.ops.rangeclip.infonce(x, t_norm, log_tau, y, w, need_grad or need_dt, need_dt, precision, rep, tb, ttb, k_dev,
+                                       dev_blocks)[0]
 
 
-def pixel_losses(x, t_norm, log_tau, y, w, precision="auto", t_bf16=None, k_dev=None):
-    """(text InfoNCE, smoothness) with a fused single-pass backward (torch.ops.rangeclip.pixel_losses)."""
+def pixel_losses(x, t_norm, log_tau, y, w, precision="auto", t_bf16=None, k_dev=None, dev_blocks=False):
+    """(text InfoNCE, smoothness) with a fused single-pass backward (torch.ops.rangeclip.pixel_losses); k_dev, dev_blocks as
+    for ``infonce``."""
     _need_cuda(x, t_norm, y, w)
     tb, ttb = _tb(t_bf16)
     need_grad = bool(torch.is_grad_enabled() and (x.requires_grad or log_tau.requires_grad))
     need_dt = bool(torch.is_grad_enabled() and t_norm.requires_grad)
-    out = torch.ops.rangeclip.pixel_losses(x, t_norm, log_tau, y, w, need_grad or need_dt, need_dt, precision, tb, ttb, k_dev)
+    out = torch.ops.rangeclip.pixel_losses(x, t_norm, log_tau, y, w, need_grad or need_dt, need_dt, precision, tb, ttb, k_dev,
+                                           dev_blocks)
     return out[0], out[1]
 
 
