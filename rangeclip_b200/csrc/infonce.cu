@@ -77,7 +77,7 @@ rownorm_kernel(const T* __restrict__ x, int B, int D, int64_t HW, __nv_bfloat16*
 // lanes = consecutive 8-pixel groups of the same rows), rounds to bf16 for the copy and the norms, and keeps the TV terms on
 // the unrounded fp32 values as rc_tv_fwd does.  kCodes: the signs of those differences are kept as well -- 4 bits per element,
 // one 32-bit word per 8-pixel group: pixel j at bits 4j..4j+3, low pair sgn(x[h][w] - x[h][w+1]), high pair
-// sgn(x[h][w] - x[h+1][w]), each a 2-bit two's-complement -1 / 0 / +1 (0 past the last column / row) -- which is all the
+// sgn(x[h][w] - x[h+1][w]), each stored as sgn + 1 in two bits (0 / 1 / 2; 1 past the last column / row) -- which is all the
 // smoothness BACKWARD needs (rc_tv_bwd_codes: 0.5 bytes per element read instead of x again).
 constexpr int kPrepassTvRows = 4;      // R: rows per strip
 constexpr int kPrepassTvThreads = 128;
