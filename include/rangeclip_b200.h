@@ -62,7 +62,7 @@ int64_t rc_infonce_workspace_bytes(int B, int D, int64_t HW, int K, rc_dtype x_d
 /* Same, including the bf16 [B][HW][Kp] tensor G the tensor-core dText path needs (rc_infonce_bf16 with dt). */
 int64_t rc_infonce_workspace_bytes_dt(int B, int D, int64_t HW, int K, rc_dtype x_dtype);
 
-/* fp32 CUDA-core path (any K >= 1, D % 8 == 0, D <= 512).  Parity path: 1e-5 relative.
+/* fp32 CUDA-core path (any K >= 1, D % 4 == 0, D <= 1024; wider: RC_ERR_UNSUPPORTED).  Parity path: 1e-5 relative.
  *   dx (nullable) [B][D][HW] f32 = grad_scale * d(loss)/dx, dt (nullable) [K][D] f32 ADDED to.
  *   w_sum_in: device double[1] holding sum_p w_p (needed when dx/dt/dlogtau are requested);
  *   grad_scale: device float[1] upstream gradient (nullable = 1).                             */
@@ -72,7 +72,7 @@ int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t ld_b,
                    const double* w_sum_in, const float* grad_scale,
                    float* dx, float* dt, double* dlogtau, void* stream);
 
-/* bf16 tcgen05/TMEM path (K <= 256, D % 64 == 0, D <= 512, HW % 8 == 0).
+/* bf16 tcgen05/TMEM path (K <= 256, D in {128, 256, 384, 512, 768, 1024}, HW % 8 == 0; other D: RC_ERR_UNSUPPORTED).
  *   x        [B][D][HW] f32 or bf16 (x_dtype); f32 input is rounded to bf16 by the pre-pass
  *   t_bf16   [Kp][D] bf16 normalised rows, Kp = K rounded up to 64, pad rows zero
  *   tt_bf16  [D][Kp] bf16 = transpose of t_bf16 (operand of the dX GEMM)
@@ -84,24 +84,24 @@ int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t ld_b,
  *   workspace from rc_infonce_workspace_bytes; holds bf16 copy of x (f32 input) and 1/|x|.
  *   flags    RC_INFONCE_PREPASS_DONE: the workspace already holds the pre-pass results for this
  *            x (written by rc_infonce_prepass or an earlier call); skip the pre-pass kernel.
- * D = 256 / 512 run the CTA-pair kernel, which computes 1/|x_p| itself from the operand tiles in
+ * D = 256 / 512 / 768 / 1024 run the CTA-pair kernel, which computes 1/|x_p| itself from the operand tiles in
  * shared memory: a bf16 x then needs no pre-pass at all.  D = 128 / 384 run the single-CTA kernel
  * (pre-pass + fused kernel).                                                                      */
 #define RC_INFONCE_PREPASS_DONE 1
 /* More than 256 candidates (e.g. the area-image loss at thousands of objects): split the candidate rows into launches of
- * <= 256 (D = 256 / 512, no dt).  y is then the target index RELATIVE to the launch's first row and may fall outside
+ * <= 256 (D = 256 / 512 / 768 / 1024, no dt).  y is then the target index RELATIVE to the launch's first row and may fall outside
  * [0, K); ignored rows are encoded by w = 0 only.
  *   RC_INFONCE_KEEP_WEIGHT  a row whose target is outside this launch keeps its weight (its one-hot term is dropped);
  *                           round 1 = forward launches with this flag: lse per block, loss_sum = sum w lse_blk - sum_{y in blk} w z_y
  *   RC_INFONCE_LSE_GIVEN    `lse` is an INPUT: the row's logsumexp over all candidates (logsumexp of the per-block values);
  *                           round 2 = backward launches with both flags: dx and dlogtau of each block add up to the full gradient
- * rc_infonce_bf16_rep4 takes the same flags (D = 256 / 512, no dt): y4 holds each target relative to the launch's first
+ * rc_infonce_bf16_rep4 takes the same flags (D = 256 / 512 / 768 / 1024, no dt): y4 holds each target relative to the launch's first
  * row, w4 is 0 for every ignored target, lse is [B*hw] (one value per shared row: per block out, or in), and round 1's
  * loss_sum = sum_q wtot_q lse_blk - sum_{y_qj in blk} w_qj z_qy with wtot_q = sum_j w_qj.  rc_infonce_bf16_dyn rejects
  * these flags (its K-blocked form is rc_infonce_bf16_dyn_kblock); rc_infonce_bf16_kblocks takes one target per row only. */
 #define RC_INFONCE_KEEP_WEIGHT 2
 #define RC_INFONCE_LSE_GIVEN 4
-/* Backward launches (dx given, no dt) of D = 256 / 512 with K and log tau given by the host (rc_infonce_bf16, _rep4 and the
+/* Backward launches (dx given, no dt) of D = 256 / 512 / 768 / 1024 with K and log tau given by the host (rc_infonce_bf16, _rep4 and the
  * K-blocked rounds), and those of rc_infonce_bf16_dyn_kblock, run the kernel whose softmax tile is a tensor-memory operand of the dX GEMM (TS-mode tcgen05.mma,
  * csrc/infonce_ts.cu).  Forward-only launches, launches with dt and rc_infonce_bf16_dyn run the kernel with both operands in
  * shared memory (SS, csrc/infonce_umma2.cu).  Both give the same results bit for bit; DESIGN.md records their speed.
@@ -127,8 +127,8 @@ int rc_infonce_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW,
  *   dx     = gradient with respect to the shared row = the sum of the four pixel gradients -- what autograd
  *            returns below F.interpolate(mode='nearest')
  *   lse    [B*hw]; w_sum_in = sum of all 4 B hw weights (rc_weight_sum over the flat arrays).
- * One quarter of the tensor-core work and HBM traffic of rc_infonce_bf16 on the upsampled tensor.  D = 256 or 512
- * (CTA-pair kernel); everything else as rc_infonce_bf16. */
+ * One quarter of the tensor-core work and HBM traffic of rc_infonce_bf16 on the upsampled tensor.  D = 256, 512, 768 or
+ * 1024 (CTA-pair kernel); everything else as rc_infonce_bf16. */
 int rc_infonce_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW,
                          const void* t_bf16, const void* tt_bf16, int K,
                          const int32_t* y4, const float* w4, float inv_tau,
@@ -137,7 +137,7 @@ int rc_infonce_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int64_t 
                          void* dx, float* dt, double* dlogtau,
                          void* workspace, int64_t workspace_bytes, int flags, void* stream);
 /* All candidate blocks of the K-blocked scheme in ONE launch (K > 256 candidates against ONE image of rows, HW % 256 == 0,
- * D = 256 / 512): the kernel's image index runs over the n_blocks = ceil(K / 256) blocks of candidate rows.
+ * D = 256 / 512 / 768 / 1024): the kernel's image index runs over the n_blocks = ceil(K / 256) blocks of candidate rows.
  *   t_bf16_all [n_blocks*256][D], tt_bf16_all [D][n_blocks*256] (zero pad rows / columns past K)
  *   y_rel, w_rep [n_blocks][HW]: target index relative to the block's first row (any value outside [0,256) when the
  *       target lives in another block), the row weight repeated per block (0 = ignored row)
@@ -154,7 +154,7 @@ int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, int64_t HW,
  *   K        rows of t_bf16 / tt_bf16 the launch is shaped for (<= 256; rows past *k_dev are zero pad rows)
  *   k_dev    device int32[1], valid rows in [1, K] (nullable = K); e.g. k_out[0] of rc_contrast_build
  *   log_tau_dev device float[1] = log(tau) (model.py:99-103 `log_temperature_text`); replaces inv_tau = exp(-log tau)
- * D = 256 or 512 (CTA-pair kernel), no dText, no K-blocked flags; everything else as rc_infonce_bf16. */
+ * D = 256, 512, 768 or 1024 (CTA-pair kernel), no dText, no K-blocked flags; everything else as rc_infonce_bf16. */
 int rc_infonce_bf16_dyn(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW,
                         const void* t_bf16, const void* tt_bf16, int K, const int32_t* k_dev,
                         const int32_t* y, const float* w, const float* log_tau_dev, int rep,
@@ -176,7 +176,7 @@ int rc_infonce_bf16_dyn(const void* x, rc_dtype x_dtype, int B, int D, int64_t H
  * and no dx and adds nothing to loss_sum, w_sum or dlogtau, so an RC_INFONCE_ACCUMULATE_DX launch leaves dx as it was.
  * The block at k0 = 0 is never empty; it should be the launch that stores dx.  A caller shapes its launches for the
  * capacity of the set (ceil(capacity / 256) blocks) and combines the per-block results on the device, treating an empty
- * block's lse as -inf.  D = 256 or 512, no dText; everything else as rc_infonce_bf16_dyn. */
+ * block's lse as -inf.  D = 256, 512, 768 or 1024, no dText; everything else as rc_infonce_bf16_dyn. */
 int rc_infonce_bf16_dyn_kblock(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW,
                                const void* t_bf16, const void* tt_bf16, int K, const int32_t* k_dev, int k0,
                                const int32_t* y, const float* w, const float* log_tau_dev, int rep,
@@ -298,6 +298,9 @@ int rc_tv_bwd_from(const void* x, rc_dtype x_dtype, int64_t planes, int H, int W
  * Evaluation  (replaces model.py:164-173 and validate.py:88-139)
  * rc_eval_topk_f32 / rc_eval_topk_bf16: top-k (k <= 8) text ids per pixel by cosine logit,
  *   ties broken towards the smaller reduced index; out[b][j][p] = index_map[arg] (int64).
+ *   rc_eval_topk_f32: D % 4 == 0, D <= 1024.  rc_eval_topk_bf16 and the other tensor-core forms below: D % 64 == 0,
+ *   D <= 1024, HW % 8 == 0; above 512 channels the pixel tile is streamed through shared memory once per 256 text rows.
+ *   Wider rows: RC_ERR_UNSUPPORTED.
  * rc_eval_hist: per-batch histograms over equivalence classes
  *   hist[0][L]=#(ge==L) hist[1][L]=#(p1==L) hist[2][L]=#(ge==L & p1==L)
  *   hist[3][L]=#(oracle==L) hist[4][L]=#(ge==L & oracle==L); counters {correct_top1,

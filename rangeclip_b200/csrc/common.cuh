@@ -62,7 +62,7 @@ long long* debug_timing_buffer();   // bring-up instrumentation target (rc_debug
 int launch_infonce_1cta(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
                         const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
                         const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, cudaStream_t s);
-// CTA-pair (cta_group::2) versions of the fused InfoNCE kernel, D = 256 / 512: SS (infonce_umma2.cu, both dX operands in
+// CTA-pair (cta_group::2) versions of the fused InfoNCE kernel, D = 256 / 512 / 768 / 1024: SS (infonce_umma2.cu, both dX operands in
 // shared memory) and TS (infonce_ts.cu, the softmax tile as a tensor-memory operand); infonce_pair.cuh holds what they share
 bool infonce_pair_supported(int D);
 struct InfoncePairArgs {

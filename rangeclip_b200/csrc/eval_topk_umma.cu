@@ -7,6 +7,9 @@
 // j+1) and every thread keeps the running top-k of its pixel in registers.
 // The ranking by cosine similarity equals the ranking by raw dot product (the per-pixel norm is a
 // positive constant), so no normalisation pass over X is needed; ties go to the smaller text index.
+// Above 512 channels (CLIP ViT-L/14: 768, ViT-H/14: 1024) the tile no longer fits next to the text ring: the streamed-X form
+// (kStreamX) turns the same 128 KB into a ring of eight 64-channel chunks that is refilled for every text block, so X is
+// re-read from the L2 once per block of 256 text rows.
 #include "common.cuh"
 #include "umma.cuh"
 #include "eval_metrics.cuh"
@@ -21,7 +24,7 @@ namespace topk {
 
 constexpr int kThreads = 384;            // warps: 0 TMA, 1 MMA, 2 TMEM alloc, 3 spare, 4-11 top-k scan (two threads per pixel)
 constexpr int kTilePx = 128;
-constexpr int kXBytes = 128 * 1024;      // X tile [D <= 512][128 px] bf16: D/64 chunks of 16 KB
+constexpr int kXBytes = 128 * 1024;      // X tile [D <= 512][128 px] bf16: D/64 chunks of 16 KB (streamed X: 8 ring slots)
 constexpr int kStages = 3;
 constexpr int kStageBytes = 32 * 1024;   // text block chunk [256 k][64 d]
 // CTA-pair form (cta_group::2, two tiles per pair): each CTA stages HALF of a text chunk ([128 k][64 d], 16 KB) and the tensor
@@ -33,11 +36,12 @@ constexpr int kMaxStages = 6;
 constexpr int kNB = 256;                 // text rows per block (MMA N)
 constexpr int kTmemCols = 512;
 constexpr int kMaxK = 8;
-constexpr int kMaxChunks = 8;            // D <= 512
+constexpr int kMaxChunks = 8;            // D <= 512 resident; the streamed-X ring has as many slots
+constexpr int kMaxStreamD = 1024;
 
 struct __align__(8) Bars {
   uint64_t full[kMaxStages], empty[kMaxStages];
-  uint64_t x_full[kMaxChunks], x_empty[kMaxChunks];   // per 64-channel chunk of the resident X tile
+  uint64_t x_full[kMaxChunks], x_empty[kMaxChunks];   // per 64-channel chunk of the resident X tile / per slot of the X ring
   uint64_t s_full[2], s_empty[2];
   uint32_t tmem_base, pad;
 };
@@ -167,11 +171,10 @@ __device__ __forceinline__ uint32_t push_gt(uint32_t m, float v, float kth) {
 // R = targets per row: 1, or 4 when the rows are the decoder's half-resolution output (SURVEY 8f-1) and every row stands for
 // the 2x2 block (2i + a, 2j + b) of the nearest-x2 upsampled map -- the scan is the same, the epilogue writes the ids to the
 // block's four pixels and scores each of them against its own full-resolution ground truth.
-template <int KT, bool kPair, int P, int R = 1>
-__global__ void __launch_bounds__(128 + 128 * P, 1)
-eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][HW], box (64 px, 64 d, 1)
-                      const __grid_constant__ CUtensorMap map_t,    // T [Kp][D], box (64 d, 256 rows; pair: 128 rows), OOB rows = 0
-                      const Params prm) {
+// kStreamX: X chunk c goes through the ring slot of the chunk's running count (not slot c) for EVERY text block; the producer
+// loads it and the MMA issuer waits for it and releases it per (block, chunk), in the order both walk the text ring.
+template <int KT, bool kPair, int P, int R, bool kStreamX>
+__device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const CUtensorMap& map_t, const Params& prm) {
   extern __shared__ __align__(1024) uint8_t smem[];
   Bars* bars = reinterpret_cast<Bars*>(smem + kOffBars);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -214,7 +217,7 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
     // =============================== TMA producer ===============================
     // X chunk c of the next tile is refilled as soon as the last text block of this tile has consumed it, so the
     // tile transition overlaps with the tail of the tensor work.
-    uint32_t it = 0, lt = 0;
+    uint32_t it = 0, lt = 0, xit = 0;
     for (int u = unit0; u < n_units; u += unit_step, ++lt) {
       const int tile = tile_of(u);
       const bool tile_ok = tile < prm.n_tiles;
@@ -222,17 +225,20 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
       const int px0 = tile_ok ? (tile - b * prm.tiles_per_img) * kTilePx : 0;
       for (int nb = 0; nb < n_blocks; ++nb)
         for (int c = 0; c < n_dchunks; ++c, ++it) {
-          if (nb == 0) {
-            mbar_wait(&bars->x_empty[c], (lt & 1) ^ 1, 1);
+          // X chunk c into slot xs: resident, slot c once per tile; streamed, the next ring slot for every block
+          const int xs = kStreamX ? (int)(xit % kMaxChunks) : c;
+          if (kStreamX || nb == 0) {
+            mbar_wait(&bars->x_empty[xs], ((kStreamX ? xit / kMaxChunks : lt) & 1) ^ 1, 1);
             if (kPair) {          // both CTAs' bytes are credited to the leader's barrier
-              if (leader_cta) mbar_arrive_expect_tx(&bars->x_full[c], 2 * 16384);
-              tma_load_3d_2sm(smem + c * 16384, &map_x, &bars->x_full[c], px0, c * 64, b);
-              tma_load_3d_2sm(smem + c * 16384 + 8192, &map_x, &bars->x_full[c], px0 + 64, c * 64, b);
+              if (leader_cta) mbar_arrive_expect_tx(&bars->x_full[xs], 2 * 16384);
+              tma_load_3d_2sm(smem + xs * 16384, &map_x, &bars->x_full[xs], px0, c * 64, b);
+              tma_load_3d_2sm(smem + xs * 16384 + 8192, &map_x, &bars->x_full[xs], px0 + 64, c * 64, b);
             } else {
-              mbar_arrive_expect_tx(&bars->x_full[c], 16384);
-              tma_load_3d(smem + c * 16384, &map_x, &bars->x_full[c], px0, c * 64, b);
-              tma_load_3d(smem + c * 16384 + 8192, &map_x, &bars->x_full[c], px0 + 64, c * 64, b);
+              mbar_arrive_expect_tx(&bars->x_full[xs], 16384);
+              tma_load_3d(smem + xs * 16384, &map_x, &bars->x_full[xs], px0, c * 64, b);
+              tma_load_3d(smem + xs * 16384 + 8192, &map_x, &bars->x_full[xs], px0 + 64, c * 64, b);
             }
+            if (kStreamX) ++xit;
           }
           const int st = it % kRingStages;
           mbar_wait(&bars->empty[st], ((it / kRingStages) & 1) ^ 1, 2);
@@ -248,7 +254,7 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
   } else if (warp == 1 && leader_cta) {
     // =============================== MMA issuer (leader CTA in the pair form) ================================
     // whole warp converged (addresses / descriptors in uniform registers), one elected lane issues
-    uint32_t it = 0, lt = 0, nbc = 0;
+    uint32_t it = 0, lt = 0, nbc = 0, xit = 0;
     const uint32_t smem_base = smem_u32(smem);
     const uint64_t dsc_x = desc_mnmajor_sw128(0, 8192) + (smem_base >> 4);
     const uint64_t dsc_t = desc_kmajor_sw128(0) + ((smem_base + kOffRing) >> 4);
@@ -260,10 +266,12 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
         const bool last = nb + 1 == n_blocks;
         for (int c = 0; c < n_dchunks; ++c, ++it) {
           const int st = it % kRingStages;
-          if (nb == 0) mbar_wait(&bars->x_full[c], lt & 1, 3);
+          const int xs = kStreamX ? (int)(xit % kMaxChunks) : c;
+          if (kStreamX) mbar_wait(&bars->x_full[xs], (xit / kMaxChunks) & 1, 3);
+          else if (nb == 0) mbar_wait(&bars->x_full[c], lt & 1, 3);
           mbar_wait(&bars->full[st], (it / kRingStages) & 1, 5);
           tc_fence_after();
-          const uint64_t xa = dsc_x + ((c * 16384) >> 4);
+          const uint64_t xa = dsc_x + ((xs * 16384) >> 4);
           const uint64_t tb = dsc_t + ((st * kRingBytes) >> 4);
           if (elect_one()) {
             if (kPair) {
@@ -271,16 +279,17 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
               for (int ks = 0; ks < 4; ++ks)
                 mma_bf16_ss_2sm(tmem + sbuf * kNB, xa + ((ks * 2048) >> 4), tb + ((ks * 32) >> 4), idesc, (c | ks) != 0);
               mma_commit_2sm(&bars->empty[st]);
-              if (last) mma_commit_2sm(&bars->x_empty[c]);
+              if (kStreamX || last) mma_commit_2sm(&bars->x_empty[xs]);
             } else {
 #pragma unroll
               for (int ks = 0; ks < 4; ++ks)
                 mma_bf16_ss(tmem + sbuf * kNB, xa + ((ks * 2048) >> 4), tb + ((ks * 32) >> 4), idesc, (c | ks) != 0);
               mma_commit(&bars->empty[st]);
-              if (last) mma_commit(&bars->x_empty[c]);       // this X chunk has been read for the last time
+              if (kStreamX || last) mma_commit(&bars->x_empty[xs]);       // this X chunk has been read for the last time (by this block)
             }
           }
           __syncwarp();
+          if (kStreamX) ++xit;
         }
         if (elect_one()) {
           if (kPair) mma_commit_2sm(&bars->s_full[sbuf]);
@@ -553,6 +562,22 @@ eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][
   }
 }
 
+// D <= 512: X tile resident for all text blocks
+template <int KT, bool kPair, int P, int R = 1>
+__global__ void __launch_bounds__(128 + 128 * P, 1)
+eval_topk_umma_kernel(const __grid_constant__ CUtensorMap map_x,    // X [B][D][HW], box (64 px, 64 d, 1)
+                      const __grid_constant__ CUtensorMap map_t,    // T [Kp][D], box (64 d, 256 rows; pair: 128 rows), OOB rows = 0
+                      const Params prm) {
+  eval_topk_body<KT, kPair, P, R, false>(map_x, map_t, prm);
+}
+
+// 512 < D <= 1024: X streamed through the 8-slot chunk ring, once per text block
+template <int KT, bool kPair, int P, int R = 1>
+__global__ void __launch_bounds__(128 + 128 * P, 1)
+eval_topk_umma_xs_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_t, const Params prm) {
+  eval_topk_body<KT, kPair, P, R, true>(map_x, map_t, prm);
+}
+
 }  // namespace topk
 }  // namespace rc
 
@@ -567,7 +592,8 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   RC_REQUIRE(x && t_bf16 && index_map && (out || hist), "%s: null pointer", who);
   RC_REQUIRE(B >= 0 && HW >= 0 && K >= 1 && k >= 1 && k <= topk::kMaxK && k <= K, "%s: bad shape (k=%d K=%d)", who, k, K);
   if (hist != nullptr) RC_REQUIRE(gt && E && cmap && counters && C >= 1, "%s: the fused metrics need gt, E, cmap, counters and C >= 1", who);
-  if (D < 64 || D > 512 || D % 64 != 0) return fail(RC_ERR_UNSUPPORTED, "%s: D=%d must be a multiple of 64 and <= 512", who, D);
+  if (D < 64 || D > topk::kMaxStreamD || D % 64 != 0)
+    return fail(RC_ERR_UNSUPPORTED, "%s: D=%d must be a multiple of 64 and <= %d", who, D, topk::kMaxStreamD);
   if (HW % 8 != 0) return fail(RC_ERR_UNSUPPORTED, "%s: HW=%lld must be a multiple of 8", who, (long long)HW);
   if (rep_w > 0)             // 16-byte stores of the ids / loads of the gt words (pixel pairs from an even index)
     RC_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0 && (reinterpret_cast<uintptr_t>(gt) & 15) == 0,
@@ -646,8 +672,19 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   // Two scan threads per pixel.  Measured, not adopted (P = 4, 640 threads, setmaxnreg 40 / 104): four lists per pixel mean 23 %
   // more insertions and the scan is close to its instruction-throughput bound (ALU + FMA pipe at one warp instruction per two
   // cycles each): K = 1024 top-5 1041 against 1147 Mpix/s, K = 256 2258 against 2764.
+  const bool stream_x = D > topk::kMaxChunks * 64;       // the tile does not fit the 128 KB X region
   auto dispatch = [&](auto r) -> int {
     constexpr int R = decltype(r)::value;
+    if (stream_x) {
+      if (pair) {
+        if (k == 1) return launch(topk::eval_topk_umma_xs_kernel<1, true, 2, R>, true, 384);
+        if (k == 5) return launch(topk::eval_topk_umma_xs_kernel<5, true, 2, R>, true, 384);
+        return launch(topk::eval_topk_umma_xs_kernel<0, true, 2, R>, true, 384);
+      }
+      if (k == 1) return launch(topk::eval_topk_umma_xs_kernel<1, false, 2, R>, false, 384);
+      if (k == 5) return launch(topk::eval_topk_umma_xs_kernel<5, false, 2, R>, false, 384);
+      return launch(topk::eval_topk_umma_xs_kernel<0, false, 2, R>, false, 384);
+    }
     if (pair) {
       if (k == 1) return launch(topk::eval_topk_umma_kernel<1, true, 2, R>, true, 384);
       if (k == 5) return launch(topk::eval_topk_umma_kernel<5, true, 2, R>, true, 384);

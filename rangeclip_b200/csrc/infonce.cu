@@ -3,8 +3,9 @@
 // arguments, runs the pre-pass and launches one of the kernels:
 //   dText   infonce_umma2.cu (writes G) + infonce_dt_umma.cu (dT = G^T X)
 //   1-CTA   infonce_umma.cu   D = 128 / 384
-//   TS      infonce_ts.cu     backward launches without dText, D = 256 / 512 (rc_infonce_bf16_dyn's excepted)
-//   SS      infonce_umma2.cu  forward-only launches, rc_infonce_bf16_dyn and RC_INFONCE_SS_KERNEL, D = 256 / 512
+//   TS      infonce_ts.cu     backward launches without dText, D = 256 / 512 / 768 / 1024 (rc_infonce_bf16_dyn's excepted)
+//   SS      infonce_umma2.cu  forward-only launches, dText (D = 256 / 512), rc_infonce_bf16_dyn and RC_INFONCE_SS_KERNEL,
+//                             D = 256 / 512 / 768 / 1024
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -268,7 +269,8 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   RC_REQUIRE(x && t_bf16 && y && w && workspace, "rc_infonce_bf16: null pointer");
   RC_REQUIRE(B >= 0 && HW >= 0, "rc_infonce_bf16: bad shape");
   if (K < 1 || K > 256) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: K=%d outside [1,256] (use rc_infonce_f32)", K);
-  if (D < 128 || D > 512 || D % 128 != 0) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: D=%d must be 128, 256, 384 or 512", D);
+  if (!(D == 128 || D == 384 || infonce_pair_supported(D)))
+    return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: D=%d must be 128, 256, 384, 512, 768 or 1024", D);
   RC_REQUIRE((reinterpret_cast<uintptr_t>(t_bf16) & 15) == 0, "rc_infonce_bf16: t must be 16-byte aligned");
   const bool bwd = dx != nullptr;
   if (bwd) RC_REQUIRE(tt_bf16 && w_sum_in && (reinterpret_cast<uintptr_t>(dx) & 15) == 0, "rc_infonce_bf16: backward needs tt_bf16, w_sum_in and aligned dx");
@@ -277,7 +279,7 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   int rcode = check_sm100("rc_infonce_bf16");
   if (rcode) return rcode;
   if ((k_dev != nullptr || log_tau_dev != nullptr) && !infonce_pair_supported(D))
-    return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn: device-side K / log tau need D = 256 or 512 (CTA-pair kernel)");
+    return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn: device-side K / log tau need D = 256, 512, 768 or 1024 (CTA-pair kernel)");
   // CTA-pair kernels (cta_group::2) when the channel count allows it; the bring-up build's RANGECLIP_B200_INFONCE=1cta
   // forces the single-CTA kernel (kept for D = 128 / 384 and as the A/B baseline).  The pair kernels compute 1/|x_p|
   // themselves from the operand tiles in shared memory, so a bf16 input needs no pre-pass at all (an fp32 input still
@@ -287,7 +289,7 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
 #else
   const char* impl = nullptr;
 #endif
-  const bool use_pair = (rep != 1 || !(impl != nullptr && impl[0] == '1')) && infonce_pair_supported(D);
+  const bool use_pair = (rep != 1 || D > 512 || !(impl != nullptr && impl[0] == '1')) && infonce_pair_supported(D);
   // rc_infonce_bf16_dyn_kblock: y is relative to k0 and w = 0 marks an ignored target, the RC_INFONCE_KEEP_WEIGHT form
   const int keep_w = (dev_blocks || (flags & RC_INFONCE_KEEP_WEIGHT)) ? 1 : 0;
   const int acc_dx = (flags & RC_INFONCE_ACCUMULATE_DX) ? 1 : 0;
@@ -295,16 +297,17 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   if (acc_dx) RC_REQUIRE(bwd, "rc_infonce_bf16: RC_INFONCE_ACCUMULATE_DX needs dx");
   if (keep_w || lse_in || acc_dx) {      // rep = 1 or 4 (rc_infonce_bf16_dyn rejects these flags before it gets here)
     if (!use_pair || dt != nullptr)
-      return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: the K-blocked flags need D = 256 or 512 and no dText");
+      return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: the K-blocked flags need D = 256, 512, 768 or 1024 and no dText");
     RC_REQUIRE(!(flags & RC_INFONCE_LSE_GIVEN) || lse != nullptr, "rc_infonce_bf16: RC_INFONCE_LSE_GIVEN needs lse");
   }
   if (rep != 1) {
-    if (!use_pair) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_rep4: D=%d must be 256 or 512", D);
+    if (!use_pair) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_rep4: D=%d must be 256 or 512 (or 768 / 1024)", D);
     RC_REQUIRE((reinterpret_cast<uintptr_t>(y) & 15) == 0 && (reinterpret_cast<uintptr_t>(w) & 15) == 0,
                "rc_infonce_bf16_rep4: y and w must be 16-byte aligned");
   }
   if (dt != nullptr) {
-    if (!use_pair || !bwd)
+    // the dText GEMM keeps all channels of a text row in the 512 tensor-memory columns of one CTA pair
+    if (!use_pair || !bwd || D > 512)
       return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16: dText needs dx and D = 256 or 512 (use rc_infonce_f32 otherwise)");
     RC_REQUIRE(workspace_bytes >= rc_infonce_workspace_bytes_dt(B, D, HW, K, x_dtype), "rc_infonce_bf16: workspace too small for dText");
   }
@@ -378,7 +381,7 @@ extern "C" int rc_infonce_bf16_dyn_kblock(const void* x, rc_dtype x_dtype, int B
   RC_REQUIRE(rep == 1 || rep == 4, "rc_infonce_bf16_dyn_kblock: rep must be 1 or 4");
   RC_REQUIRE(k0 >= 0, "rc_infonce_bf16_dyn_kblock: k0=%d must be >= 0", k0);
   if (K < 1 || K > 256) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn_kblock: K=%d outside [1,256] (one block)", K);
-  if (!infonce_pair_supported(D)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn_kblock: D=%d must be 256 or 512", D);
+  if (!infonce_pair_supported(D)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn_kblock: D=%d must be 256 or 512 (or 768 / 1024)", D);
   return infonce_bf16_impl(x, x_dtype, B, D, HW, t_bf16, tt_bf16, K, y, w, 0.f, lse, loss_sum, w_sum, w_sum_in, grad_scale, dx,
                            nullptr, dlogtau, workspace, workspace_bytes, flags, rep, stream, k_dev, log_tau_dev, true, k0);
 }
@@ -391,7 +394,7 @@ extern "C" int rc_infonce_bf16_kblocks(const void* x, rc_dtype x_dtype, int D, i
   using namespace rc;
   RC_REQUIRE(x && t_bf16_all && y_rel && w_rep && workspace && lse, "rc_infonce_bf16_kblocks: null pointer");
   RC_REQUIRE(HW >= 0 && K >= 1 && n_blocks >= 1 && n_blocks == (K + 255) / 256, "rc_infonce_bf16_kblocks: n_blocks must be ceil(K / 256)");
-  if (!infonce_pair_supported(D)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: D=%d must be 256 or 512", D);
+  if (!infonce_pair_supported(D)) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: D=%d must be 256 or 512 (or 768 / 1024)", D);
   if (HW % 256 != 0) return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_kblocks: HW=%lld must be a multiple of 256", (long long)HW);
   RC_REQUIRE((reinterpret_cast<uintptr_t>(t_bf16_all) & 15) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0, "rc_infonce_bf16_kblocks: alignment");
   const bool bwd = dx_blocks != nullptr;

@@ -9,6 +9,9 @@
 // Mapping: a block owns 32 consecutive pixel rows (lane = pixel, so global loads of the NCHW
 // tensor are coalesced along HW); its 8 warps each own one eighth of the D channels in registers.
 // Logits for 8 text rows at a time are reduced across the warps through shared memory.
+// 512 < D <= 1024 (CLIP ViT-L/14, ViT-H/14): the wide form, 16 warps of 64 channels each, keeps the normalised pixel rows
+// in shared memory instead ([D][32] fp32, lane = pixel: conflict-free) and only the dX accumulator in registers, so that
+// 512 threads fit in 128 registers each.  Same arithmetic and accumulation order per warp slice.
 #include "common.cuh"
 #include <float.h>
 
@@ -248,6 +251,267 @@ eval_topk_f32_kernel(const float* __restrict__ x, int B, int D, int64_t HW, int6
   }
 }
 
+// ---- wide form: 512 < D <= 1024 --------------------------------------------------------------
+
+constexpr int kWideWarps = 16;
+constexpr int kWideThreads = kWideWarps * 32;
+constexpr int kWideDPT = 64;                 // channels per warp slice
+constexpr int kWideMaxD = kWideWarps * kWideDPT;
+struct WideSmem {
+  float xs[kWideMaxD][32];                   // normalised pixel rows of the tile: [channel][lane = pixel]
+  float red[kWideWarps][32];
+  float part[2][kWideWarps][kSimtKB][32];
+};
+constexpr int kWideSmemBytes = (int)sizeof(WideSmem);
+
+// simt_load_tile with the slice in shared memory (each thread writes and reads only its own entries: no barrier between)
+__device__ __forceinline__ void wide_load_tile(WideSmem& sm, const float* __restrict__ x, int D, int64_t HW, int64_t ld_b,
+                                               int64_t M, int64_t m, int slice, float& inv_norm, bool& valid, int64_t& off) {
+  const int lane = threadIdx.x & 31;
+  valid = m < M;
+  const int64_t b = valid ? m / HW : 0;
+  const int64_t p = valid ? m - b * HW : 0;
+  off = b * ld_b + (int64_t)slice * kWideDPT * HW + p;
+  float ss = 0.f;
+#pragma unroll 8
+  for (int j = 0; j < kWideDPT; ++j) {
+    const int d = slice * kWideDPT + j;
+    const float v = (valid && d < D) ? __ldg(x + off + (int64_t)j * HW) : 0.f;
+    sm.xs[slice * kWideDPT + j][lane] = v;
+    ss = fmaf(v, v, ss);
+  }
+  sm.red[slice][lane] = ss;
+  __syncthreads();
+  float tot = 0.f;
+#pragma unroll
+  for (int s = 0; s < kWideWarps; ++s) tot += sm.red[s][lane];
+  __syncthreads();
+  const float nrm = fmaxf(sqrtf(tot), 1e-12f);   // F.normalize eps (model.py:273)
+  inv_norm = 1.f / nrm;
+#pragma unroll 8
+  for (int j = 0; j < kWideDPT; ++j) sm.xs[slice * kWideDPT + j][lane] = sm.xs[slice * kWideDPT + j][lane] / nrm;
+}
+
+// simt_logits with x̂ read from shared memory, in two steps: the slice partials into part[buf] (ends with a barrier), then
+// the logit of row k0 + kk summed over the slices in warp order (wide_logit)
+__device__ __forceinline__ void wide_partials(WideSmem& sm, const float* __restrict__ text, int D, int K, int k0, int slice,
+                                              int buf) {
+  const int lane = threadIdx.x & 31;
+  float acc[kSimtKB];
+#pragma unroll
+  for (int kk = 0; kk < kSimtKB; ++kk) acc[kk] = 0.f;
+  const int dbase = slice * kWideDPT;
+  const float* xs = &sm.xs[dbase][lane];
+  if (dbase + kWideDPT <= D) {
+#pragma unroll 1
+    for (int j = 0; j < kWideDPT; j += 4) {      // 8 text rows x 4 channels per step: 128 registers hold the dX slice too
+      const float x0 = xs[j * 32], x1 = xs[(j + 1) * 32], x2 = xs[(j + 2) * 32], x3 = xs[(j + 3) * 32];
+#pragma unroll
+      for (int kk = 0; kk < kSimtKB; ++kk) {
+        if (k0 + kk < K) {   // warp-uniform
+          const float4 tv = __ldg(reinterpret_cast<const float4*>(text + (int64_t)(k0 + kk) * D + dbase + j));
+          acc[kk] = fmaf(x0, tv.x, acc[kk]);
+          acc[kk] = fmaf(x1, tv.y, acc[kk]);
+          acc[kk] = fmaf(x2, tv.z, acc[kk]);
+          acc[kk] = fmaf(x3, tv.w, acc[kk]);
+        }
+      }
+    }
+  } else if (dbase < D) {
+#pragma unroll 1
+    for (int j = 0; j < kWideDPT && dbase + j < D; ++j) {
+      const float xv = xs[j * 32];
+#pragma unroll
+      for (int kk = 0; kk < kSimtKB; ++kk)
+        if (k0 + kk < K) acc[kk] = fmaf(xv, __ldg(text + (int64_t)(k0 + kk) * D + dbase + j), acc[kk]);
+    }
+  }
+#pragma unroll
+  for (int kk = 0; kk < kSimtKB; ++kk) sm.part[buf][slice][kk][lane] = acc[kk];
+  __syncthreads();
+}
+__device__ __forceinline__ float wide_logit(const WideSmem& sm, int buf, int kk, float scale) {
+  const int lane = threadIdx.x & 31;
+  float s = 0.f;
+#pragma unroll
+  for (int w = 0; w < kWideWarps; ++w) s += sm.part[buf][w][kk][lane];
+  return s * scale;
+}
+__device__ __forceinline__ void wide_logits(WideSmem& sm, const float* __restrict__ text, int D, int K, int k0, int slice,
+                                            int buf, float scale, float (&z)[kSimtKB]) {
+  wide_partials(sm, text, D, K, k0, slice, buf);
+#pragma unroll
+  for (int kk = 0; kk < kSimtKB; ++kk) z[kk] = wide_logit(sm, buf, kk, scale);
+}
+
+// infonce_f32_kernel at 512 < D <= 1024
+__global__ void __launch_bounds__(kWideThreads, 1)
+infonce_f32_wide_kernel(const float* __restrict__ x, int B, int D, int64_t HW, int64_t ld_b,
+                        const float* __restrict__ text, int K, const int32_t* __restrict__ y,
+                        const float* __restrict__ w, float inv_tau, float* __restrict__ lse_out,
+                        double* __restrict__ loss_sum, double* __restrict__ w_sum,
+                        const double* __restrict__ w_sum_in, const float* __restrict__ grad_scale_p,
+                        float* __restrict__ dx, float* __restrict__ dt, double* __restrict__ dlogtau) {
+  extern __shared__ __align__(16) uint8_t smem_raw[];
+  WideSmem& sm = *reinterpret_cast<WideSmem*>(smem_raw);
+  const int lane = threadIdx.x & 31, slice = threadIdx.x >> 5;
+  const int64_t M = (int64_t)B * HW;
+  const int64_t n_tiles = (M + 31) / 32;
+  const bool need_bwd = (dx != nullptr) || (dt != nullptr) || (dlogtau != nullptr);
+  double acc_loss = 0.0, acc_w = 0.0, acc_dlt = 0.0;
+  const float* xs = &sm.xs[slice * kWideDPT][lane];
+  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int64_t m = tile * 32 + lane;
+    float inv_norm;
+    bool valid;
+    int64_t off;
+    wide_load_tile(sm, x, D, HW, ld_b, M, m, slice, inv_norm, valid, off);
+    const int yi = valid ? y[m] : -1;
+    const float wi = (valid && yi >= 0) ? w[m] : 0.f;
+    // ---- forward: online logsumexp over the K text rows
+    float mx = -FLT_MAX, l = 0.f, zy = 0.f;
+    int buf = 0;
+    for (int k0 = 0; k0 < K; k0 += kSimtKB, buf ^= 1) {
+      float z[kSimtKB];
+      wide_logits(sm, text, D, K, k0, slice, buf, inv_tau, z);
+      float bm = mx;
+#pragma unroll
+      for (int kk = 0; kk < kSimtKB; ++kk) if (k0 + kk < K) bm = fmaxf(bm, z[kk]);
+      l *= expf(mx - bm);
+#pragma unroll
+      for (int kk = 0; kk < kSimtKB; ++kk)
+        if (k0 + kk < K) {
+          l += expf(z[kk] - bm);
+          if (k0 + kk == yi) zy = z[kk];
+        }
+      mx = bm;
+    }
+    const float lse = mx + logf(l);
+    if (slice == 0 && valid) {
+      if (lse_out) lse_out[m] = lse;
+      acc_loss += (double)(wi * (lse - zy));
+      acc_w += (double)wi;
+    }
+    if (!need_bwd) { __syncthreads(); continue; }     // the next tile rewrites the rows and the exchange buffers
+    // ---- backward: recompute logits, dz = coef * (softmax - onehot)
+    const double ws = w_sum_in[0];
+    const float grad_scale = grad_scale_p ? grad_scale_p[0] : 1.f;
+    const float coef = (ws > 0.0) ? grad_scale * wi / (float)ws : 0.f;
+    float dxh[kWideDPT];
+#pragma unroll
+    for (int j = 0; j < kWideDPT; ++j) dxh[j] = 0.f;
+    float c = 0.f;
+    const int dbase = slice * kWideDPT;
+    __syncthreads();
+    buf = 0;
+    for (int k0 = 0; k0 < K; k0 += kSimtKB, buf ^= 1) {
+      wide_partials(sm, text, D, K, k0, slice, buf);
+#pragma unroll 1
+      for (int kk = 0; kk < kSimtKB; ++kk) {
+        const int k = k0 + kk;
+        if (k < K) {
+          const float zk = wide_logit(sm, buf, kk, inv_tau);
+          const float pk = expf(zk - lse);
+          const float dz = coef * (pk - (k == yi ? 1.f : 0.f));
+          c = fmaf(dz, zk, c);
+          const float* row = text + (int64_t)k * D + dbase;
+          if (dx != nullptr) {
+            if (dbase + kWideDPT <= D) {
+#pragma unroll
+              for (int j = 0; j < kWideDPT; j += 4) {
+                const float4 tv = __ldg(reinterpret_cast<const float4*>(row + j));
+                dxh[j] = fmaf(dz, tv.x, dxh[j]);
+                dxh[j + 1] = fmaf(dz, tv.y, dxh[j + 1]);
+                dxh[j + 2] = fmaf(dz, tv.z, dxh[j + 2]);
+                dxh[j + 3] = fmaf(dz, tv.w, dxh[j + 3]);
+              }
+            } else {
+#pragma unroll
+              for (int j = 0; j < kWideDPT; ++j)
+                if (dbase + j < D) dxh[j] = fmaf(dz, __ldg(row + j), dxh[j]);
+            }
+          }
+          if (dt != nullptr) {
+            const float dzs = dz * inv_tau;
+#pragma unroll 4
+            for (int j = 0; j < kWideDPT; ++j) {
+              const float s = warp_sum(dzs * xs[j * 32]);
+              if (lane == 0 && dbase + j < D && s != 0.f) atomicAdd(&dt[(int64_t)k * D + dbase + j], s);
+            }
+          }
+        }
+      }
+    }
+    if (dx != nullptr && valid) {
+      // dx = (dxh/tau - xh * <xh, dxh/tau>) / |x|, with <xh, dxh/tau> = sum_k dz_k z_k = c  (Q2)
+#pragma unroll
+      for (int j = 0; j < kWideDPT; ++j)
+        if (dbase + j < D) dx[off + (int64_t)j * HW] = inv_norm * (inv_tau * dxh[j] - xs[j * 32] * c);
+    }
+    if (slice == 0 && valid) acc_dlt -= (double)c;   // d z / d log(tau) = -z
+    __syncthreads();
+  }
+  if (slice == 0) {
+    acc_loss = warp_sum(acc_loss);
+    acc_w = warp_sum(acc_w);
+    acc_dlt = warp_sum(acc_dlt);
+    if (lane == 0) {
+      if (loss_sum) atomicAdd(loss_sum, acc_loss);
+      if (w_sum) atomicAdd(w_sum, acc_w);
+      if (dlogtau && need_bwd) atomicAdd(dlogtau, acc_dlt);
+    }
+  }
+}
+
+// eval_topk_f32_kernel at 512 < D <= 1024
+__global__ void __launch_bounds__(kWideThreads, 1)
+eval_topk_f32_wide_kernel(const float* __restrict__ x, int B, int D, int64_t HW, int64_t ld_b,
+                          const float* __restrict__ text, int K, const int64_t* __restrict__ index_map, int k,
+                          int64_t* __restrict__ out) {
+  extern __shared__ __align__(16) uint8_t smem_raw[];
+  WideSmem& sm = *reinterpret_cast<WideSmem*>(smem_raw);
+  const int lane = threadIdx.x & 31, slice = threadIdx.x >> 5;
+  const int64_t M = (int64_t)B * HW;
+  const int64_t n_tiles = (M + 31) / 32;
+  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int64_t m = tile * 32 + lane;
+    float inv_norm;
+    bool valid;
+    int64_t off;
+    wide_load_tile(sm, x, D, HW, ld_b, M, m, slice, inv_norm, valid, off);
+    float bv[8];
+    int bi[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { bv[j] = -FLT_MAX; bi[j] = -1; }
+    int buf = 0;
+    for (int k0 = 0; k0 < K; k0 += kSimtKB, buf ^= 1) {
+      float z[kSimtKB];
+      wide_logits(sm, text, D, K, k0, slice, buf, 1.f, z);
+#pragma unroll
+      for (int kk = 0; kk < kSimtKB; ++kk) {
+        if (k0 + kk < K) {
+          float v = z[kk];
+          int id = k0 + kk;
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            if (j < k && v > bv[j]) {   // strict: earlier (smaller) index wins ties
+              const float tv = bv[j]; const int ti = bi[j];
+              bv[j] = v; bi[j] = id; v = tv; id = ti;
+            }
+          }
+        }
+      }
+    }
+    if (slice == 0 && valid) {
+      const int64_t b = m / HW, p = m - b * HW;
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        if (j < k) out[(b * k + j) * HW + p] = bi[j] >= 0 ? index_map[bi[j]] : -1;
+    }
+    __syncthreads();                 // the next tile rewrites the rows
+  }
+}
+
 // ---- small helpers ---------------------------------------------------------------------------
 
 // one warp per text row: F.normalize (model.py:272 / :161), write f32 / bf16 / transposed bf16
@@ -390,6 +654,14 @@ __global__ void __launch_bounds__(256) scale_to_kernel(const TI* __restrict__ x,
   for (int64_t i = nv * 8 + tid; i < n; i += nt) ElemIO<TO>::st(out + i, ElemIO<TI>::ld(x + i) * f);
 }
 
+// grid: one block per SM, the wide form's shared memory opted in once per kernel
+template <typename Kern>
+static int wide_prepare(Kern kernel, const char* who) {
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWideSmemBytes);
+  if (e != cudaSuccess) return fail(RC_ERR_CUDA, "%s: smem opt-in: %s", who, cudaGetErrorString(e));
+  return RC_OK;
+}
+
 template <template <int> class Launcher, typename... Args>
 static int dispatch_dpt(int D, Args... args) {
   if (D <= 64) return Launcher<8>::run(args...);
@@ -423,7 +695,8 @@ extern "C" int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t 
                               double* dlogtau, void* stream) {
   RC_REQUIRE(x && t && y && w, "rc_infonce_f32: null pointer");
   RC_REQUIRE(B >= 0 && HW >= 0 && K >= 1, "rc_infonce_f32: bad shape");
-  RC_REQUIRE(D >= 4 && D <= 512 && D % 4 == 0, "rc_infonce_f32: D=%d must be a multiple of 4 and <= 512", D);
+  RC_REQUIRE(D >= 4 && D % 4 == 0, "rc_infonce_f32: D=%d must be a multiple of 4", D);
+  if (D > rc::kWideMaxD) return rc::fail(RC_ERR_UNSUPPORTED, "rc_infonce_f32: D=%d is wider than %d", D, rc::kWideMaxD);
   RC_REQUIRE((reinterpret_cast<uintptr_t>(t) & 15) == 0, "rc_infonce_f32: text rows must be 16-byte aligned");
   if ((dx || dt || dlogtau) && !w_sum_in) return rc::fail(RC_ERR_INVALID, "rc_infonce_f32: gradients need w_sum_in");
   const int64_t M = (int64_t)B * HW;
@@ -431,6 +704,13 @@ extern "C" int rc_infonce_f32(const float* x, int B, int D, int64_t HW, int64_t 
   const int64_t tiles = (M + 31) / 32;
   const int64_t cap = (int64_t)rc::num_sms();
   const int grid = (int)(tiles < cap ? tiles : cap);
+  if (D > 512) {
+    int rcode = rc::wide_prepare(rc::infonce_f32_wide_kernel, "rc_infonce_f32");
+    if (rcode) return rcode;
+    rc::infonce_f32_wide_kernel<<<grid, rc::kWideThreads, rc::kWideSmemBytes, (cudaStream_t)stream>>>(
+        x, B, D, HW, ld_b, t, K, y, w, inv_tau, lse, loss_sum, w_sum, w_sum_in, grad_scale, dx, dt, dlogtau);
+    return rc::check_launch("rc_infonce_f32");
+  }
   rc::dispatch_dpt<rc::InfoNceLauncher>(D, grid, (cudaStream_t)stream, x, B, D, HW, ld_b, t, K, y, w, inv_tau, lse,
                                         loss_sum, w_sum, w_sum_in, grad_scale, dx, dt, dlogtau);
   return rc::check_launch("rc_infonce_f32");
@@ -440,12 +720,20 @@ extern "C" int rc_eval_topk_f32(const float* x, int B, int D, int64_t HW, int64_
                                 const int64_t* index_map, int k, int64_t* out, void* stream) {
   RC_REQUIRE(x && t && index_map && out, "rc_eval_topk_f32: null pointer");
   RC_REQUIRE(B >= 0 && HW >= 0 && K >= 1 && k >= 1 && k <= 8 && k <= K, "rc_eval_topk_f32: bad shape (k=%d K=%d)", k, K);
-  RC_REQUIRE(D >= 4 && D <= 512 && D % 4 == 0, "rc_eval_topk_f32: D=%d must be a multiple of 4 and <= 512", D);
+  RC_REQUIRE(D >= 4 && D % 4 == 0, "rc_eval_topk_f32: D=%d must be a multiple of 4", D);
+  if (D > rc::kWideMaxD) return rc::fail(RC_ERR_UNSUPPORTED, "rc_eval_topk_f32: D=%d is wider than %d", D, rc::kWideMaxD);
   const int64_t M = (int64_t)B * HW;
   if (M == 0) return RC_OK;
   const int64_t tiles = (M + 31) / 32;
   const int64_t cap = (int64_t)rc::num_sms();
   const int grid = (int)(tiles < cap ? tiles : cap);
+  if (D > 512) {
+    int rcode = rc::wide_prepare(rc::eval_topk_f32_wide_kernel, "rc_eval_topk_f32");
+    if (rcode) return rcode;
+    rc::eval_topk_f32_wide_kernel<<<grid, rc::kWideThreads, rc::kWideSmemBytes, (cudaStream_t)stream>>>(
+        x, B, D, HW, ld_b, t, K, index_map, k, out);
+    return rc::check_launch("rc_eval_topk_f32");
+  }
   rc::dispatch_dpt<rc::TopkLauncher>(D, grid, (cudaStream_t)stream, x, B, D, HW, ld_b, t, K, index_map, k, out);
   return rc::check_launch("rc_eval_topk_f32");
 }

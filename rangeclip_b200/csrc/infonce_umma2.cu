@@ -252,7 +252,7 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
             const int ab = uc & 1;
             RC_WAIT(mbar_wait, &bars->acc_empty[ab], ((uc >> 1) & 1) ^ 1, 6);
             tc_fence_after();
-            RC_EV(lt, 3 + blk * 2 + pxh);     // dX unit issue starts (accumulator free)
+            if (blk < 2) RC_EV(lt, 3 + blk * 2 + pxh);     // dX unit issue starts (accumulator free; event ids 3-6)
             const uint32_t dcol = tmem + 256 + ab * 128;
             for (int kc = 0; kc < n_kchunks; ++kc) {
               const int st = (it + kc) % kTStages;
@@ -623,7 +623,10 @@ infonce_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x_s,   // X [B]
 
 }  // namespace pair
 
-bool infonce_pair_supported(int D) { return D == 256 || D == 512; }
+// D / 64 chunks of the S GEMM and D / 256 blocks of the dX GEMM (SS; TS: D / 64), whatever their number: the pipelines are
+// tuned at D <= 512 and run unchanged at 768 and 1024 (CLIP ViT-L/14, ViT-H/14).  The X ring is shorter than a tile from
+// D = 512 on, so the row norms and the S GEMM release its slots in turn (same chunk order, no other wait between them).
+bool infonce_pair_supported(int D) { return D % 256 == 0 && D >= 256 && D <= 1024; }
 
 // launch helper used by rc_infonce_bf16 (infonce.cu owns argument checking and the pre-pass)
 int launch_infonce_pair(const InfoncePairArgs& a, cudaStream_t s) {

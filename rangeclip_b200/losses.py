@@ -203,7 +203,7 @@ def text_contrastive_loss(pixel_embeddings, target_indices, candidate_text_embed
             y, w = group_2x2(y.view(B, H, W)), group_2x2(w.view(B, H, W))
             loss = ops.infonce(pixel_embeddings, t_norm, log_temperature_text, y, w, precision, rep=4, t_bf16=t_bf16)
         else:
-            # outside what the four-target kernel covers (D not 256 / 512, fp32 parity mode, more than 256 contrast rows
+            # outside what the four-target kernel covers (D not 256 / 512 / 768 / 1024, fp32 parity mode, more than 256 contrast rows
             # with trainable text): the loss of the upsampled tensor itself, as the decoder would emit it (decoder.py:113);
             # autograd sums the four pixel gradients of a block below the interpolation
             up = torch.nn.functional.interpolate(pixel_embeddings, scale_factor=2, mode="nearest")
@@ -227,7 +227,7 @@ def image_contrastive_loss(area_embeddings, image_embeddings, log_temperature_im
     ``precision``: "fp32" = CUDA-core kernel (1e-5 path; what the reference's n <= batch size needs -- the call is
     launch-bound there); "bf16" = tensor cores with the candidates in blocks of 256 (``ops.infonce`` with
     ``precision="kblocked"``; the fp32 kernel takes 9 ms at n = 4096); "auto" = bf16 from n = 512 when the shape allows it
-    (D in (256, 512), n % 8 == 0, frozen image embeddings)."""
+    (D in (256, 512, 768, 1024), n % 8 == 0, frozen image embeddings)."""
     n, D = area_embeddings.shape
     x = area_embeddings.float().t().contiguous().view(1, D, n, 1)
     blocked_ok = ops._infonce_plan(x, n, image_embeddings.requires_grad, "kblocked", 1) is not None
@@ -235,7 +235,7 @@ def image_contrastive_loss(area_embeddings, image_embeddings, log_temperature_im
         precision = "bf16" if (blocked_ok and n >= 512) else "fp32"
     if precision == "bf16":
         if not blocked_ok:
-            raise RuntimeError(f"image_contrastive_loss: the tensor-core path needs D in (256, 512), n % 8 == 0 and frozen "
+            raise RuntimeError(f"image_contrastive_loss: the tensor-core path needs D in (256, 512, 768, 1024), n % 8 == 0 and frozen "
                                f"image embeddings; got n={n}, D={D}")
         precision = "kblocked"
     if image_embeddings.requires_grad:

@@ -179,10 +179,11 @@ def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: i
                   dev_params: bool = False, dev_blocks: bool = False) -> Optional[str]:
     """The route of one InfoNCE call; the only place that chooses it.  ``infonce_raw`` runs it, the fake-tensor rules of
     rangeclip::infonce / pixel_losses derive dX's dtype from it and the loss drop-ins ask it whether a kernel takes a call.
-      'fp32'      the CUDA-core kernel (rc_infonce_f32): any shape, one target per row, host K and tau;
-      'bf16'      one tensor-core launch (rc_infonce_bf16 / _rep4 / _dyn): K <= 256, D in (128, 256, 384, 512), HW % 8 == 0;
-                  four targets, dText (with dX) and the device-parameter form only on the CTA-pair kernel (D in (256, 512));
-      'kblocked'  tensor cores over blocks of 256 candidate rows (``infonce_kblocked_raw``): D in (256, 512), HW % 8 == 0, no
+      'fp32'      the CUDA-core kernel (rc_infonce_f32): D <= 1024, one target per row, host K and tau;
+      'bf16'      one tensor-core launch (rc_infonce_bf16 / _rep4 / _dyn): K <= 256, D in (128, 256, 384, 512, 768, 1024),
+                  HW % 8 == 0; four targets and the device-parameter form only on the CTA-pair kernel (D in _PAIR_D), dText
+                  (with dX) only at D in (256, 512);
+      'kblocked'  tensor cores over blocks of 256 candidate rows (``infonce_kblocked_raw``): D in _PAIR_D, HW % 8 == 0, no
                   dText, host K and tau; what "auto" (and, for four targets, "bf16") takes above 256 candidates; with
                   ``dev_blocks`` also for K and tau in device memory, up to 1024 rows (rc_infonce_bf16_dyn_kblock);
       None        no kernel covers the call.
@@ -202,18 +203,19 @@ def _infonce_plan(x: torch.Tensor, K: int, need_dt: bool, precision: str, rep: i
     kblocked = kblocked_supported(D, HW) and not need_dt and not dev_params
     if precision == "kblocked":
         return "kblocked" if kblocked else None
+    fp32 = rep == 1 and not dev_params and D <= _F32_MAX_D
     if precision == "fp32":
-        return "fp32" if rep == 1 and not dev_params else None
+        return "fp32" if fp32 else None
     if kblocked and K > 256 and (precision == "auto" or rep == 4):
         return "kblocked"
-    one_launch = 1 <= K <= 256 and D in (128, 256, 384, 512) and HW % 8 == 0 and HW > 0
+    one_launch = 1 <= K <= 256 and D in (128, 384) + _PAIR_D and HW % 8 == 0 and HW > 0
     if rep == 4 or need_dt or dev_params:         # forms only the CTA-pair kernel has
-        one_launch = one_launch and D in (256, 512)
-    if need_dt:                                   # tensor-core dText: pair kernel + split-K GEMM, from the dX pass
-        one_launch = one_launch and need_dx and not dev_params
+        one_launch = one_launch and D in _PAIR_D
+    if need_dt:                                   # tensor-core dText: pair kernel + split-K GEMM (all channels in 512 TMEM columns)
+        one_launch = one_launch and need_dx and not dev_params and D in _DTEXT_D
     if one_launch:
         return "bf16"
-    return "fp32" if precision == "auto" and rep == 1 and not dev_params else None
+    return "fp32" if precision == "auto" and fp32 else None
 
 
 def _infonce_route(x: torch.Tensor, K: int, need_dx: bool, need_dt: bool, precision: str, rep: int, dev_params: bool,
@@ -342,10 +344,13 @@ RC_INFONCE_SS_KERNEL = 32
 
 
 _DEV_BLOCKS_MAX_ROWS = 1024      # contrast-set capacity of the device-parameter K-blocked rounds: four blocks, dX summed in-kernel
+_PAIR_D = (256, 512, 768, 1024)  # widths of the CTA-pair kernels (CLIP ViT-B/32: 512, ViT-L/14: 768, ViT-H/14: 1024)
+_DTEXT_D = (256, 512)            # widths of the tensor-core dText GEMM
+_F32_MAX_D = 1024                # widest row of the CUDA-core kernels
 
 
 def kblocked_supported(D: int, HW: int) -> bool:
-    return D in (256, 512) and HW % 8 == 0 and HW > 0
+    return D in _PAIR_D and HW % 8 == 0 and HW > 0
 
 
 def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor, w: torch.Tensor, inv_tau: float,
@@ -366,7 +371,7 @@ def infonce_kblocked_raw(x: torch.Tensor, t_norm: torch.Tensor, y: torch.Tensor,
     _need_cuda(x, t_norm, y, w, k_dev, log_tau_dev)
     x, B, D, HW = _emb3(x)
     if not kblocked_supported(D, HW):
-        raise RuntimeError(f"infonce_kblocked: needs D in (256, 512) and HW % 8 == 0; got D={D}, HW={HW}")
+        raise RuntimeError(f"infonce_kblocked: needs D in {_PAIR_D} and HW % 8 == 0; got D={D}, HW={HW}")
     if rep not in (1, 4):
         raise RuntimeError("infonce_kblocked: rep must be 1 or 4")
     K = t_norm.shape[0]
@@ -656,7 +661,7 @@ def pool_backward(g: torch.Tensor, cnt: torch.Tensor, seg, lut: torch.Tensor, lu
 # ----------------------------------------------------------------------------------------------
 
 def topk_bf16_supported(D: int, HW: int) -> bool:
-    return D % 64 == 0 and 64 <= D <= 512 and HW % 8 == 0 and HW > 0
+    return D % 64 == 0 and 64 <= D <= 1024 and HW % 8 == 0 and HW > 0
 
 
 def eval_topk(x: torch.Tensor, t_norm: torch.Tensor, index_map: torch.Tensor, k: int, precision="auto", t_bf16=None):
@@ -699,7 +704,7 @@ def eval_topk_hist(x: torch.Tensor, t_norm: torch.Tensor, index_map: torch.Tenso
     """Fused evaluation batch (model.py:164-173 + validate.py:88-139): top-k on the tensor cores with the five class
     histograms and three counters built from the ids while they are still in registers (added to ``hist`` /
     ``counters``, int64).  Returns the ids [B,k,H,W] when ``want_ids`` (the drop-in ``predict`` needs them), else None.
-    Tensor-core path only (D % 64 == 0, D <= 512, HW % 8 == 0)."""
+    Tensor-core path only (D % 64 == 0, D <= 1024, HW % 8 == 0)."""
     _need_cuda(x, t_norm, index_map, gt, E_u8, cmap, hist, counters)
     x, B, D, HW = _emb3(x)
     if not topk_bf16_supported(D, HW):
