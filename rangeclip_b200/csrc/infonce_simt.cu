@@ -204,7 +204,8 @@ infonce_f32_kernel(const float* __restrict__ x, int B, int D, int64_t HW, int64_
   }
 }
 
-// fp32 top-k over cosine logits (model.py:144,161-173); ties -> smaller reduced index.
+// fp32 top-k over cosine logits (model.py:144,161-173); ties -> smaller reduced index (the index tie-break in the insertion
+// keeps that order when a better value shifts the list down past equal entries).
 template <int DPT>
 __global__ void __launch_bounds__(kSimtThreads, 1)
 eval_topk_f32_kernel(const float* __restrict__ x, int B, int D, int64_t HW, int64_t ld_b,
@@ -234,7 +235,8 @@ eval_topk_f32_kernel(const float* __restrict__ x, int B, int D, int64_t HW, int6
           int id = k0 + kk;
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
-            if (j < k && v > bv[j]) {   // strict: earlier (smaller) index wins ties
+            // explicit index tie-break: a displaced entry moving down must pass equal values with larger indices
+            if (j < k && (v > bv[j] || (v == bv[j] && (unsigned)id < (unsigned)bi[j]))) {
               const float tv = bv[j]; const int ti = bi[j];
               bv[j] = v; bi[j] = id; v = tv; id = ti;
             }
@@ -494,7 +496,8 @@ eval_topk_f32_wide_kernel(const float* __restrict__ x, int B, int D, int64_t HW,
           int id = k0 + kk;
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
-            if (j < k && v > bv[j]) {   // strict: earlier (smaller) index wins ties
+            // explicit index tie-break: a displaced entry moving down must pass equal values with larger indices
+            if (j < k && (v > bv[j] || (v == bv[j] && (unsigned)id < (unsigned)bi[j]))) {
               const float tv = bv[j]; const int ti = bi[j];
               bv[j] = v; bi[j] = id; v = tv; id = ti;
             }
