@@ -351,7 +351,7 @@ int rc_eval_fold(const int64_t* batch_hist /*[5][C]*/, int C, int32_t batch_inde
  *   variant 0: A K-major [128][Kd], B K-major [N][Kd]
  *   variant 1: A MN-major [Kd][128] (the NCHW pixel operand), B K-major [N][Kd]
  *
- * Bring-up entry points and environment switches (RANGECLIP_B200_ABLATE / _INFONCE / _DT) exist ONLY in
+ * Bring-up entry points and environment switches (RANGECLIP_B200_ABLATE / _DT) exist ONLY in
  * librangeclip_b200_bringup.so, built with -DRC_BRINGUP (`make -C rangeclip_b200/csrc bringup`); the shipped
  * librangeclip_b200.so exports none of them and reads no environment variable.
  * ------------------------------------------------------------------------------------------- */

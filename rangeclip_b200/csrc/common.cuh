@@ -58,7 +58,7 @@ int launch_rownorm_f32(const float* x, int B, int D, int64_t HW, __nv_bfloat16* 
 
 long long* debug_timing_buffer();   // bring-up instrumentation target (rc_debug_set_timing_buffer)
 // The fused InfoNCE kernels; infonce.cu validates the arguments, runs the pre-pass and picks one of them.
-// single-CTA version (infonce_umma.cu): D = 128 / 384, and the A/B baseline of the bring-up build
+// single-CTA version (infonce_umma.cu): D = 128 / 384
 int launch_infonce_1cta(const void* xsrc, void* dx, const void* t_bf16, const void* tt_bf16, int B, int D, int64_t HW, int K,
                         const float* inv_norm, const int32_t* y, const float* w, float inv_tau, const float* grad_scale,
                         const double* w_sum_in, float* lse, double* loss_sum, double* w_sum, double* dlogtau, cudaStream_t s);

@@ -7,7 +7,6 @@
 //   SS      infonce_umma2.cu  forward-only launches, dText (D = 256 / 512), rc_infonce_bf16_dyn and RC_INFONCE_SS_KERNEL,
 //                             D = 256 / 512 / 768 / 1024
 #include "common.cuh"
-#include <stdlib.h>
 
 extern "C" int64_t rc_infonce_workspace_bytes(int B, int D, int64_t HW, int K, rc_dtype x_dtype) {
   (void)K;
@@ -278,18 +277,12 @@ static int infonce_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, int6
   if (B == 0 || HW == 0) return RC_OK;
   int rcode = check_sm100("rc_infonce_bf16");
   if (rcode) return rcode;
-  if ((k_dev != nullptr || log_tau_dev != nullptr) && !infonce_pair_supported(D))
+  // CTA-pair kernels (cta_group::2) when the channel count allows it, the single-CTA kernel at D = 128 / 384.  The pair
+  // kernels compute 1/|x_p| themselves from the operand tiles in shared memory, so a bf16 input needs no pre-pass at all
+  // (an fp32 input still needs its bf16 copy).
+  const bool use_pair = infonce_pair_supported(D);
+  if ((k_dev != nullptr || log_tau_dev != nullptr) && !use_pair)
     return fail(RC_ERR_UNSUPPORTED, "rc_infonce_bf16_dyn: device-side K / log tau need D = 256, 512, 768 or 1024 (CTA-pair kernel)");
-  // CTA-pair kernels (cta_group::2) when the channel count allows it; the bring-up build's RANGECLIP_B200_INFONCE=1cta
-  // forces the single-CTA kernel (kept for D = 128 / 384 and as the A/B baseline).  The pair kernels compute 1/|x_p|
-  // themselves from the operand tiles in shared memory, so a bf16 input needs no pre-pass at all (an fp32 input still
-  // needs its bf16 copy).
-#ifdef RC_BRINGUP
-  const char* impl = getenv("RANGECLIP_B200_INFONCE");     // never compiled into the shipped library
-#else
-  const char* impl = nullptr;
-#endif
-  const bool use_pair = (rep != 1 || D > 512 || !(impl != nullptr && impl[0] == '1')) && infonce_pair_supported(D);
   // rc_infonce_bf16_dyn_kblock: y is relative to k0 and w = 0 marks an ignored target, the RC_INFONCE_KEEP_WEIGHT form
   const int keep_w = (dev_blocks || (flags & RC_INFONCE_KEEP_WEIGHT)) ? 1 : 0;
   const int acc_dx = (flags & RC_INFONCE_ACCUMULATE_DX) ? 1 : 0;

@@ -1,6 +1,5 @@
 // K1/K2, single-CTA version: the fused pixel-text InfoNCE forward + backward on the 5th-gen tensor cores (sm_100a).
-// rc_infonce_bf16 runs it for D = 128 / 384 (the CTA-pair kernels in infonce_umma2.cu / infonce_ts.cu need D % 256 == 0);
-// the bring-up build also takes it as the A/B baseline (RANGECLIP_B200_INFONCE=1cta).
+// rc_infonce_bf16 runs it for D = 128 / 384 (the CTA-pair kernels in infonce_umma2.cu / infonce_ts.cu need D % 256 == 0).
 //
 // Replaces model.py:272-291 (normalize, [N,512]@[512,K], /tau, cross_entropy) and its autograd
 // (CE backward, two matmuls, normalize backward, index_put/scatter_add).  Needs the pre-pass (rownorm_kernel,

@@ -41,8 +41,8 @@ for bwd in (True, False):
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / reps
     flops = (4 if bwd else 2) * K * D * B * HW
-    print(json.dumps({"kernel": "infonce_bf16" + ("_fwd_bwd" if bwd else "_fwd"), "impl": os.environ.get("RANGECLIP_B200_INFONCE", "pair"),
-                      "B": B, "H": H, "W": W, "ms": round(ms, 4), "TFLOPs": round(flops / ms / 1e9, 1), "Mpix_s": round(B * HW / ms / 1e3, 1)}), flush=True)
+    print(json.dumps({"kernel": "infonce_bf16" + ("_fwd_bwd" if bwd else "_fwd"), "B": B, "H": H, "W": W, "ms": round(ms, 4),
+                      "TFLOPs": round(flops / ms / 1e9, 1), "Mpix_s": round(B * HW / ms / 1e3, 1)}), flush=True)
 
 # fwd + dX + dText (tensor-core dText: the pair kernel also writes G, then the split-K GEMM)
 ws2_bytes = int(L.rc_infonce_workspace_bytes_dt(B, D, HW, K, _lib.RC_BF16))
