@@ -338,6 +338,17 @@ int rc_eval_topk_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int h,
                            const int32_t* k_dev, const int64_t* index_map, int k, int64_t* out, const int64_t* gt,
                            const uint8_t* E, const int64_t* cmap, int C, int64_t* hist, int64_t* counters,
                            void* workspace, int64_t workspace_bytes, void* stream);
+/* Open-vocabulary scores (no ground truth): the ids of rc_eval_topk_bf16 / _rep4, bit for bit, and for every ranked row its
+ * cosine <x_p / max(|x_p|, 1e-12), t_j> (fp32) and its softmax probability over all K rows at the temperature
+ * tau = exp(*log_tau) (fp32; log_tau is a DEVICE float, so the call needs no host synchronisation).  ids, cosine and prob are
+ * laid out as `out` above: [B][k][HW], or [B][k][2h][2w] on the half-resolution rows (ids 16-byte, cosine / prob 8-byte
+ * aligned).  Same shape limits as rc_eval_topk_bf16; an fp32 x needs the workspace of rc_eval_topk_bf16. */
+int rc_eval_topk_scores_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16, int K,
+                             const int64_t* index_map, int k, const float* log_tau, int64_t* ids, float* cosine, float* prob,
+                             void* workspace, int64_t workspace_bytes, void* stream);
+int rc_eval_topk_scores_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int h, int w, const void* t_bf16, int K,
+                                  const int64_t* index_map, int k, const float* log_tau, int64_t* ids, float* cosine,
+                                  float* prob, void* workspace, int64_t workspace_bytes, void* stream);
 int rc_eval_hist(const int64_t* gt, const int64_t* topk, int B, int64_t HW, int k,
                  const uint8_t* E, const int64_t* cmap, int C,
                  int64_t* hist /*[5][C]*/, int64_t* counters /*[3]*/, void* stream);

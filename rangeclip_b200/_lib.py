@@ -65,6 +65,9 @@ PROTOTYPES = {
                               _vp, _i64, _vp],
     "rc_eval_topk_bf16_rep4": [_vp, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _vp,
                                _vp, _i64, _vp],
+    "rc_eval_topk_scores_bf16": [_vp, _i32, _i32, _i32, _i64, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
+    "rc_eval_topk_scores_bf16_rep4": [_vp, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _i64,
+                                      _vp],
     "rc_eval_hist": [_vp, _vp, _i32, _i64, _i32, _vp, _vp, _i32, _vp, _vp, _vp],
     "rc_eval_fold": [_vp, _i32, _i32, _vp, _vp, _vp],
 }

@@ -10,6 +10,10 @@
 // Above 512 channels (CLIP ViT-L/14: 768, ViT-H/14: 1024) the tile no longer fits next to the text ring: the streamed-X form
 // (kStreamX) turns the same 128 KB into a ring of eight 64-channel chunks that is refilled for every text block, so X is
 // re-read from the L2 once per block of 256 text rows.
+// The scores form (eval_topk_scores_umma*_kernel, rc_eval_topk_scores_bf16): the same scan also writes, per ranked row, the
+// cosine and the softmax probability over all K rows at a temperature read from device memory -- open-vocabulary inference
+// without a ground truth.  Each scan thread keeps a log-sum-exp of its columns next to its list (one ex2 and two FMA-pipe
+// instructions per logit); a bf16 x gets its pixel norm from the X chunks while the first text block's MMA has them staged.
 #include "common.cuh"
 #include "umma.cuh"
 #include "eval_metrics.cuh"
@@ -44,12 +48,14 @@ struct __align__(8) Bars {
   uint64_t x_full[kMaxChunks], x_empty[kMaxChunks];   // per 64-channel chunk of the resident X tile / per slot of the X ring
   uint64_t s_full[2], s_empty[2];
   uint32_t tmem_base, pad;
+  uint64_t x_seen[kMaxChunks];           // scores form: the first text block's MMA has read this X slot (it is in both CTAs)
 };
 constexpr int kOffRing = kXBytes;
 constexpr int kOffThr = kOffRing + kStages * kStageBytes;      // k-th best of every scan thread, read by its partner [256] f32
 constexpr int kOffBars = kOffThr + 256 * 4;
 static_assert(kPairStages * kPairStageBytes == kStages * kStageBytes, "both forms use the same ring bytes");
-constexpr int kSmemBytes = kOffBars + (int)sizeof(Bars);
+constexpr int kOffNorm = (kOffBars + (int)sizeof(Bars) + 15) / 16 * 16;   // scores form: |x_p|^2 of the tile [2 tiles][128] f32
+constexpr int kSmemBytes = kOffNorm + 2 * kTilePx * 4;
 static_assert(kSmemBytes <= 232448, "shared-memory budget of one SM (227 KB)");
 
 struct Params {
@@ -68,6 +74,34 @@ struct Params {
   unsigned long long* counters;          // [3]
   int w;                                 // R = 4: width of the half-resolution rows (HW = h * w); out / gt are [2h][2w]
 };
+// scores form (kScores): cosine and softmax probability of every ranked row next to its id, same layout as `out` (a type of
+// its own: the ids-only kernels keep their parameter block)
+struct ScoreParams : Params {
+  const float* log_tau;                  // device float: log of the softmax temperature
+  const float* inv_norm;                 // nullable: 1 / max(|x_p|, 1e-12) of the fp32 pre-pass; NULL: taken from the staged X
+  float* cosine;
+  float* prob;
+};
+
+template <bool kScores, class Prm>
+__device__ __forceinline__ bool norm_from_x(const Prm& prm) {
+  if constexpr (kScores) return prm.inv_norm == nullptr;
+  else return false;
+}
+
+// 32 lanes x 2 columns between registers and TMEM (the scores form parks a pixel's (m, s) next to its list)
+__device__ __forceinline__ void tmem_st_32x2(uint32_t taddr, uint32_t a, uint32_t b) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};" ::"r"(taddr), "r"(a), "r"(b) : "memory");
+}
+__device__ __forceinline__ void tmem_ld_32x2(uint32_t taddr, uint32_t& a, uint32_t& b) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "r"(taddr) : "memory");
+}
+
+__device__ __forceinline__ float ex2f(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
 
 // KT > 0: compile-time k (the insertion network has exactly k stages); KT == 0: run-time k <= kMaxK
 template <int KT>
@@ -173,8 +207,13 @@ __device__ __forceinline__ uint32_t push_gt(uint32_t m, float v, float kth) {
 // block's four pixels and scores each of them against its own full-resolution ground truth.
 // kStreamX: X chunk c goes through the ring slot of the chunk's running count (not slot c) for EVERY text block; the producer
 // loads it and the MMA issuer waits for it and releases it per (block, chunk), in the order both walk the text ring.
-template <int KT, bool kPair, int P, int R, bool kStreamX>
-__device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const CUtensorMap& map_t, const Params& prm) {
+// kScores: the epilogue also writes the cosine and the softmax probability (over all K rows, at the temperature read from
+// log_tau) of every ranked row.  The scan threads keep a running log-sum-exp next to their top-k lists, and for a bf16 x
+// they take each pixel's norm from the X chunks of the tile's first text block while those sit in shared memory: the MMA
+// issuer signals x_seen once it has read a chunk, and a slot is refilled only when the eight scan warps have released it
+// too (x_empty counts 1 + 8 arrivals; the producer stands in for them on the later blocks' chunks of the streamed ring).
+template <int KT, bool kPair, int P, int R, bool kStreamX, bool kScores = false, class Prm = Params>
+__device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const CUtensorMap& map_t, const Prm& prm) {
   extern __shared__ __align__(1024) uint8_t smem[];
   Bars* bars = reinterpret_cast<Bars*>(smem + kOffBars);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -191,10 +230,18 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
   // the candidate set may have been built on the device (rc_contrast_build): its size is read here, by every role alike
   const int Kv = prm.k_dev != nullptr ? max(1, min(__ldg(prm.k_dev), prm.K)) : prm.K;
   const int n_blocks = prm.k_dev != nullptr ? (Kv + kNB - 1) / kNB : prm.n_blocks;
+  static_assert(!kScores || P == 2, "the scores form's norm pass is laid out for eight scan warps");
+  const bool norm_x = norm_from_x<kScores>(prm);      // pixel norms from the staged X (bf16 x)
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&map_x); tma_prefetch_desc(&map_t);
     for (int i = 0; i < kMaxStages; ++i) { mbar_init(&bars->full[i], 1); mbar_init(&bars->empty[i], 1); }
-    for (int i = 0; i < kMaxChunks; ++i) { mbar_init(&bars->x_full[i], 1); mbar_init(&bars->x_empty[i], 1); }
+    if constexpr (kScores) {
+      for (int i = 0; i < kMaxChunks; ++i) {
+        mbar_init(&bars->x_full[i], 1); mbar_init(&bars->x_empty[i], norm_x ? 1 + 4 * P : 1); mbar_init(&bars->x_seen[i], 1);
+      }
+    } else {
+      for (int i = 0; i < kMaxChunks; ++i) { mbar_init(&bars->x_full[i], 1); mbar_init(&bars->x_empty[i], 1); }
+    }
     // S buffers: released by ONE arrival per scan warp (of both CTAs in the pair form)
     for (int i = 0; i < 2; ++i) { mbar_init(&bars->s_full[i], 1); mbar_init(&bars->s_empty[i], (kPair ? 2 : 1) * 4 * P); }
     fence_barrier_init();
@@ -238,6 +285,8 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
               tma_load_3d(smem + xs * 16384, &map_x, &bars->x_full[xs], px0, c * 64, b);
               tma_load_3d(smem + xs * 16384 + 8192, &map_x, &bars->x_full[xs], px0 + 64, c * 64, b);
             }
+            if constexpr (kScores && kStreamX)
+              if (norm_x && nb != 0) mbar_arrive_n(&bars->x_empty[xs], 4 * P);   // no norm pass reads this fill
             if (kStreamX) ++xit;
           }
           const int st = it % kRingStages;
@@ -280,12 +329,16 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
                 mma_bf16_ss_2sm(tmem + sbuf * kNB, xa + ((ks * 2048) >> 4), tb + ((ks * 32) >> 4), idesc, (c | ks) != 0);
               mma_commit_2sm(&bars->empty[st]);
               if (kStreamX || last) mma_commit_2sm(&bars->x_empty[xs]);
+              if constexpr (kScores)
+                if (norm_x && nb == 0) mma_commit_2sm(&bars->x_seen[xs]);
             } else {
 #pragma unroll
               for (int ks = 0; ks < 4; ++ks)
                 mma_bf16_ss(tmem + sbuf * kNB, xa + ((ks * 2048) >> 4), tb + ((ks * 32) >> 4), idesc, (c | ks) != 0);
               mma_commit(&bars->empty[st]);
               if (kStreamX || last) mma_commit(&bars->x_empty[xs]);       // this X chunk has been read for the last time (by this block)
+              if constexpr (kScores)
+                if (norm_x && nb == 0) mma_commit(&bars->x_seen[xs]);
             }
           }
           __syncwarp();
@@ -319,6 +372,10 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
     volatile float* thr_peer = reinterpret_cast<volatile float*>(smem + kOffThr) + ((threadIdx.x - 128) ^ 128);
     *thr_mine = -FLT_MAX;
     named_bar_sync(4 + quarter, 64);
+    // scores form: log2(e) / tau, this CTA's tile count and the parity bits of the x_seen slots
+    [[maybe_unused]] float c_tau = 0.f;
+    if constexpr (kScores) c_tau = expf(-__ldg(prm.log_tau)) * 1.4426950408889634f;
+    [[maybe_unused]] uint32_t lt = 0, seen = 0;
     for (int u = unit0; u < n_units; u += unit_step) {
       const int tile = tile_of(u);
       const bool tile_ok = tile < prm.n_tiles;         // (a pair's second tile past the end: scanned, never written)
@@ -329,6 +386,54 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
 #pragma unroll
       for (int j = 0; j < kMaxK; ++j) { bv[j] = -FLT_MAX; bi[j] = -1; }
       float kth = -FLT_MAX;              // current k-th best: cheap reject before the insertion network
+      // scores form: 1 / |x_p|, the scale c of 2^(v c) = e^(cos / tau), and the running log-sum-exp of this thread's columns
+      // as s = sum 2^((v - m) c) against a reference m that never decreases
+      [[maybe_unused]] float inv_n = 0.f, cs = 0.f, m_run = -FLT_MAX, s_run = 0.f;
+      if constexpr (kScores) {
+        if (norm_x) {
+          // |x_p|^2 from the first text block's X chunks: lanes 16 h + r of scan warp w take the 8 pixels of group
+          // g = 2 w + h and the channels d = r (mod 16) of every chunk; the group's 16 partial sums meet in a butterfly
+          const int g = 2 * (warp - 4) + (lane >> 4), sr = lane & 15;
+          const uint32_t xit0 = kStreamX ? lt * (uint32_t)(n_blocks * n_dchunks) : 0u;
+          float ss[8];
+#pragma unroll
+          for (int j = 0; j < 8; ++j) ss[j] = 0.f;
+#pragma unroll 1
+          for (int c = 0; c < n_dchunks; ++c) {
+            const int xs = kStreamX ? (int)((xit0 + c) % kMaxChunks) : c;
+            mbar_wait(&bars->x_seen[xs], (seen >> xs) & 1u, 7);
+            seen ^= 1u << xs;
+            // [64 d][64 px] per 8 KB half, 128-byte rows, 16-byte granule q of row d stored at q ^ (d & 7)
+            const uint8_t* base = smem + xs * 16384 + (g >> 3) * 8192 + sr * 128 + (((g & 7) ^ (sr & 7)) << 4);
+#pragma unroll
+            for (int rr = 0; rr < 4; ++rr) {
+              const uint4 v = *reinterpret_cast<const uint4*>(base + rr * 2048);
+              const uint32_t w4[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+              for (int j = 0; j < 4; ++j) {
+                ss[2 * j] = sqacc_bf16x2_lo(ss[2 * j], w4[j]);
+                ss[2 * j + 1] = sqacc_bf16x2_hi(ss[2 * j + 1], w4[j]);
+              }
+            }
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&bars->x_empty[xs]);
+          }
+#pragma unroll
+          for (int o = 8; o >= 1; o >>= 1)
+#pragma unroll
+            for (int j = 0; j < 8; ++j) ss[j] += __shfl_xor_sync(0xffffffffu, ss[j], o);
+          float* nrm = reinterpret_cast<float*>(smem + kOffNorm) + (lt & 1) * kTilePx;    // two tiles: no reader is overtaken
+          if (sr == 0) {
+            reinterpret_cast<float4*>(nrm + 8 * g)[0] = make_float4(ss[0], ss[1], ss[2], ss[3]);
+            reinterpret_cast<float4*>(nrm + 8 * g)[1] = make_float4(ss[4], ss[5], ss[6], ss[7]);
+          }
+          named_bar_sync(8, 128 * P);
+          inv_n = 1.f / fmaxf(sqrtf(nrm[row]), 1e-12f);
+        } else {
+          inv_n = tile_ok && px < prm.HW ? __ldg(prm.inv_norm + (int64_t)b * prm.HW + px) : 0.f;
+        }
+        cs = inv_n * c_tau;
+      }
       for (int nb = 0; nb < n_blocks; ++nb, ++nbc) {
         const int sbuf = nbc & 1;
         mbar_wait(&bars->s_full[sbuf], (nbc >> 1) & 1, 6);
@@ -421,6 +526,38 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
             if (P == 2) *thr_mine = kth;
           }
         };
+        // scores form: s += sum over the chunk's valid columns of 2^((v - m) c).  The reference m must not depend on the
+        // partner's bound (read at whatever moment it is read) for the result to be reproducible, so it is the list's best after
+        // the tile's first chunk (whose columns all enter the list), and moves only when a chunk's sum leaves [0, 2^64]:
+        // then to the chunk's maximum, with s <- s 2^((m_old - m) c).
+        [[maybe_unused]] auto lse_chunk = [&](const uint32_t (&r)[32], int c) {
+          const int nvalid = Kv - (kbase + c * 32);
+          if (nb == 0 && c == 0) m_run = bv[0];
+          auto chunk_sum = [&]() {
+            const float mc = m_run * cs;
+            float a[4] = {0.f, 0.f, 0.f, 0.f};
+            if (nvalid >= 32) {
+#pragma unroll
+              for (int i = 0; i < 32; ++i) a[i & 3] += ex2f(fmaf(__uint_as_float(r[i]), cs, -mc));
+            } else {
+#pragma unroll
+              for (int i = 0; i < 32; ++i)
+                if (i < nvalid) a[i & 3] += ex2f(fmaf(__uint_as_float(r[i]), cs, -mc));
+            }
+            return (a[0] + a[1]) + (a[2] + a[3]);
+          };
+          float sum = chunk_sum();
+          if (!(sum <= 0x1p64f)) {
+            float mx = m_run;
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (i < nvalid) mx = fmaxf(mx, __uint_as_float(r[i]));
+            s_run *= ex2f((m_run - mx) * cs);
+            m_run = mx;
+            sum = chunk_sum();
+          }
+          s_run += sum;
+        };
         if (P == 2) {
           uint32_t ra[32], rb[32];
           if (n_chunks > 0) tmem_ld_32x32(trow + sbuf * kNB, ra);
@@ -429,10 +566,12 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
             tmem_ld_wait32(ra);
             if (c + 1 < n_chunks) tmem_ld_32x32(trow + sbuf * kNB + (c + 1) * 32, rb);
             scan_chunk(ra, c);
+            if constexpr (kScores) lse_chunk(ra, c);
             if (c + 1 < n_chunks) {
               tmem_ld_wait32(rb);
               if (c + 2 < n_chunks) tmem_ld_32x32(trow + sbuf * kNB + (c + 2) * 32, ra);
               scan_chunk(rb, c + 1);
+              if constexpr (kScores) lse_chunk(rb, c + 1);
             }
           }
         } else {
@@ -446,7 +585,8 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
         }
         if (nb + 1 == n_blocks) {
           // merge the P lists of a pixel: parts 1.. park theirs in 16 TMEM columns of their own, already scanned range of
-          // this buffer; part 0 folds them into its list (explicit index tie-break: the ranges interleave across blocks)
+          // this buffer (scores form: 18, with m and s); part 0 folds them into its list (explicit index tie-break: the ranges
+          // interleave across blocks)
           const uint32_t tq = tmem + ((uint32_t)(quarter * 32) << 16) + sbuf * kNB;
           *thr_mine = -FLT_MAX;            // the bound belongs to this tile's pixel: reset before the barrier both partners pass
           if (half != 0) {
@@ -454,6 +594,7 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
 #pragma unroll
             for (int j = 0; j < kMaxK; ++j) { pkd[j] = __float_as_uint(bv[j]); pkd[8 + j] = (uint32_t)bi[j]; }
             tmem_st_32x16(tq + half * kCols, pkd);
+            if constexpr (kScores) tmem_st_32x2(tq + half * kCols + 16, __float_as_uint(m_run), __float_as_uint(s_run));
             tmem_st_wait();
             tc_fence_before();
             named_bar_sync(4 + quarter, 32 * P);
@@ -464,7 +605,14 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
             for (int part = 1; part < P; ++part) {
               uint32_t pkd[16];
               tmem_ld_32x16(tq + part * kCols, pkd);
+              [[maybe_unused]] uint32_t pm, ps;
+              if constexpr (kScores) tmem_ld_32x2(tq + part * kCols + 16, pm, ps);
               tmem_ld_wait();
+              if constexpr (kScores) {
+                const float m1 = __uint_as_float(pm), m = fmaxf(m_run, m1);
+                s_run = s_run * ex2f((m_run - m) * cs) + __uint_as_float(ps) * ex2f((m1 - m) * cs);
+                m_run = m;
+              }
 #pragma unroll
               for (int j = 0; j < kMaxK; ++j)
                 if (j < prm.k && (int)pkd[8 + j] >= 0) topk_insert_tie<KT>(bv, bi, prm.k, __uint_as_float(pkd[j]), (int)pkd[8 + j]);
@@ -502,11 +650,25 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
           warp_agg_add(prm.hist + 3 * (int64_t)prm.C, m.orc, m.ok);
           warp_agg_add(prm.hist + 4 * (int64_t)prm.C, m.ge, m.ok && m.orc_same);
         };
+        // scores form: cosine v / |x_p| and probability 2^((v - m) c) / s of rank j (m, s: the merged log-sum-exp)
+        [[maybe_unused]] const float rs = kScores ? 1.f / s_run : 0.f;
+        [[maybe_unused]] auto cos_of = [&](int j) { return bv[j] * inv_n; };
+        [[maybe_unused]] auto prob_of = [&](int j) { return ex2f((bv[j] - m_run) * cs) * rs; };
         if (R == 1) {
           if (inb && prm.out != nullptr) {
 #pragma unroll
             for (int j = 0; j < kMaxK; ++j)
               if (j < prm.k) prm.out[((int64_t)b * prm.k + j) * prm.HW + px] = ids[j];
+          }
+          if constexpr (kScores) {
+            if (inb) {
+#pragma unroll
+              for (int j = 0; j < kMaxK; ++j)
+                if (j < prm.k) {
+                  prm.cosine[((int64_t)b * prm.k + j) * prm.HW + px] = cos_of(j);
+                  prm.prob[((int64_t)b * prm.k + j) * prm.HW + px] = prob_of(j);
+                }
+            }
           }
           if (prm.hist != nullptr) count(inb ? __ldg(prm.gt + (int64_t)b * prm.HW + px) : 0);
         } else {
@@ -525,6 +687,21 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
                 o[W2 / 2] = v;
               }
           }
+          if constexpr (kScores) {     // 8-byte stores: the pixel pair of each image row
+            if (inb) {
+#pragma unroll
+              for (int j = 0; j < kMaxK; ++j)
+                if (j < prm.k) {
+                  float2* oc = reinterpret_cast<float2*>(prm.cosine + ((int64_t)b * prm.k + j) * HW4 + p00);
+                  float2* op = reinterpret_cast<float2*>(prm.prob + ((int64_t)b * prm.k + j) * HW4 + p00);
+                  const float2 vc = make_float2(cos_of(j), cos_of(j)), vp = make_float2(prob_of(j), prob_of(j));
+                  oc[0] = vc;
+                  oc[W2 / 2] = vc;
+                  op[0] = vp;
+                  op[W2 / 2] = vp;
+                }
+            }
+          }
           if (prm.hist != nullptr) {
             longlong2 g0 = make_longlong2(0, 0), g1 = g0;
             if (inb) {
@@ -538,6 +715,7 @@ __device__ __forceinline__ void eval_topk_body(const CUtensorMap& map_x, const C
           }
         }
       }
+      if constexpr (kScores) ++lt;
     }
     if (half == 0 && prm.hist != nullptr) {
       for (int o = 16; o > 0; o >>= 1) {
@@ -578,6 +756,20 @@ eval_topk_umma_xs_kernel(const __grid_constant__ CUtensorMap map_x, const __grid
   eval_topk_body<KT, kPair, P, R, true>(map_x, map_t, prm);
 }
 
+// The scores forms of the two kernels above (ids, cosine and softmax probability per rank): same scan, own names
+template <int KT, bool kPair, int P, int R = 1>
+__global__ void __launch_bounds__(128 + 128 * P, 1)
+eval_topk_scores_umma_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_t,
+                             const ScoreParams prm) {
+  eval_topk_body<KT, kPair, P, R, false, true>(map_x, map_t, prm);
+}
+template <int KT, bool kPair, int P, int R = 1>
+__global__ void __launch_bounds__(128 + 128 * P, 1)
+eval_topk_scores_umma_xs_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_t,
+                                const ScoreParams prm) {
+  eval_topk_body<KT, kPair, P, R, true, true>(map_x, map_t, prm);
+}
+
 }  // namespace topk
 }  // namespace rc
 
@@ -585,11 +777,14 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
                                const int64_t* index_map, int k, int64_t* out, const int64_t* gt, const uint8_t* E,
                                const int64_t* cmap, int C, int64_t* hist, int64_t* counters, void* workspace,
                                int64_t workspace_bytes, void* stream, const char* who, const int32_t* k_dev = nullptr,
-                               int rep_w = 0) {
+                               int rep_w = 0, const float* log_tau = nullptr, float* cosine = nullptr, float* prob = nullptr) {
   // rep_w = 0: one target per row (x is [B][D][HW], out / gt [B][HW]); rep_w = w > 0: x holds the half-resolution rows
-  // [B][D][h*w] (HW = h*w) and out / gt are the full-resolution [B][2h][2w] maps (four targets per row)
+  // [B][D][h*w] (HW = h*w) and out / gt are the full-resolution [B][2h][2w] maps (four targets per row).
+  // cosine != NULL: the scores form (log_tau, cosine and prob given together, laid out as out)
   using namespace rc;
+  const bool scores = cosine != nullptr;
   RC_REQUIRE(x && t_bf16 && index_map && (out || hist), "%s: null pointer", who);
+  if (scores) RC_REQUIRE(out && log_tau && prob, "%s: null pointer", who);
   RC_REQUIRE(B >= 0 && HW >= 0 && K >= 1 && k >= 1 && k <= topk::kMaxK && k <= K, "%s: bad shape (k=%d K=%d)", who, k, K);
   if (hist != nullptr) RC_REQUIRE(gt && E && cmap && counters && C >= 1, "%s: the fused metrics need gt, E, cmap, counters and C >= 1", who);
   if (D < 64 || D > topk::kMaxStreamD || D % 64 != 0)
@@ -598,6 +793,9 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   if (rep_w > 0)             // 16-byte stores of the ids / loads of the gt words (pixel pairs from an even index)
     RC_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0 && (reinterpret_cast<uintptr_t>(gt) & 15) == 0,
                "%s: out and gt must be 16-byte aligned", who);
+  if (rep_w > 0 && scores)   // 8-byte stores of the pixel pairs' scores
+    RC_REQUIRE(((reinterpret_cast<uintptr_t>(cosine) | reinterpret_cast<uintptr_t>(prob)) & 7) == 0,
+               "%s: cosine and prob must be 8-byte aligned", who);
   RC_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(t_bf16) & 15) == 0,
              "%s: x and t must be 16-byte aligned", who);
   if (B == 0 || HW == 0) return RC_OK;
@@ -605,6 +803,7 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   if (rcode) return rcode;
   cudaStream_t s = (cudaStream_t)stream;
   const void* xsrc = x;
+  const float* inv_norm_ws = nullptr;
   if (x_dtype == RC_F32) {
     const int64_t M = (int64_t)B * HW;
     RC_REQUIRE(workspace && workspace_bytes >= rc_infonce_workspace_bytes(B, D, HW, K, RC_F32), "%s: workspace too small for the bf16 copy", who);
@@ -613,6 +812,7 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
     __nv_bfloat16* xb = reinterpret_cast<__nv_bfloat16*>(ws + ((M * 4 + 255) / 256) * 256);
     if ((rcode = launch_rownorm_f32((const float*)x, B, D, HW, xb, inv_norm, s))) return rcode;
     xsrc = xb;
+    inv_norm_ws = inv_norm;
   }
   const int Kp = (K + 63) / 64 * 64;
   CUtensorMap m_x, m_t;
@@ -625,7 +825,7 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
     const uint32_t tbox[2] = {64, (uint32_t)topk::kNB};
     if ((rcode = make_tmap_bf16(&m_t, t_bf16, 2, tdims, tstr, tbox, "topk map_t"))) return rcode;
   }
-  topk::Params prm;
+  topk::ScoreParams prm;           // the ids-only kernels take its Params part
   prm.B = B; prm.D = D; prm.K = K; prm.k = k; prm.HW = HW;
   prm.tiles_per_img = (int)((HW + topk::kTilePx - 1) / topk::kTilePx);
   if ((int64_t)B * prm.tiles_per_img > 0x7fffffff) return fail(RC_ERR_UNSUPPORTED, "%s: too many tiles", who);
@@ -635,6 +835,7 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   prm.gt = gt; prm.E = E; prm.cmap = cmap; prm.C = C;
   prm.hist = reinterpret_cast<unsigned long long*>(hist); prm.counters = reinterpret_cast<unsigned long long*>(counters);
   prm.w = rep_w;
+  prm.log_tau = log_tau; prm.inv_norm = inv_norm_ws; prm.cosine = cosine; prm.prob = prob;
   // CTA pairs (two tiles per cluster, text chunks shared between the two SMs) whenever there is more than one tile
   const bool pair = prm.n_tiles >= 2 && (prm.n_blocks >= 2 || k == 1);       // one text block per tile: nothing to share, the coupling costs 5 %
   CUtensorMap m_tp = m_t;
@@ -675,6 +876,26 @@ static int eval_topk_bf16_impl(const void* x, rc_dtype x_dtype, int B, int D, in
   const bool stream_x = D > topk::kMaxChunks * 64;       // the tile does not fit the 128 KB X region
   auto dispatch = [&](auto r) -> int {
     constexpr int R = decltype(r)::value;
+    if (scores) {
+      if (stream_x) {
+        if (pair) {
+          if (k == 1) return launch(topk::eval_topk_scores_umma_xs_kernel<1, true, 2, R>, true, 384);
+          if (k == 5) return launch(topk::eval_topk_scores_umma_xs_kernel<5, true, 2, R>, true, 384);
+          return launch(topk::eval_topk_scores_umma_xs_kernel<0, true, 2, R>, true, 384);
+        }
+        if (k == 1) return launch(topk::eval_topk_scores_umma_xs_kernel<1, false, 2, R>, false, 384);
+        if (k == 5) return launch(topk::eval_topk_scores_umma_xs_kernel<5, false, 2, R>, false, 384);
+        return launch(topk::eval_topk_scores_umma_xs_kernel<0, false, 2, R>, false, 384);
+      }
+      if (pair) {
+        if (k == 1) return launch(topk::eval_topk_scores_umma_kernel<1, true, 2, R>, true, 384);
+        if (k == 5) return launch(topk::eval_topk_scores_umma_kernel<5, true, 2, R>, true, 384);
+        return launch(topk::eval_topk_scores_umma_kernel<0, true, 2, R>, true, 384);
+      }
+      if (k == 1) return launch(topk::eval_topk_scores_umma_kernel<1, false, 2, R>, false, 384);
+      if (k == 5) return launch(topk::eval_topk_scores_umma_kernel<5, false, 2, R>, false, 384);
+      return launch(topk::eval_topk_scores_umma_kernel<0, false, 2, R>, false, 384);
+    }
     if (stream_x) {
       if (pair) {
         if (k == 1) return launch(topk::eval_topk_umma_xs_kernel<1, true, 2, R>, true, 384);
@@ -735,4 +956,25 @@ extern "C" int rc_eval_topk_bf16_rep4(const void* x, rc_dtype x_dtype, int B, in
   RC_REQUIRE(h >= 1 && w >= 1, "rc_eval_topk_bf16_rep4: bad shape (h=%d w=%d)", h, w);
   return eval_topk_bf16_impl(x, x_dtype, B, D, (int64_t)h * w, t_bf16, K, index_map, k, out, gt, E, cmap, C, hist, counters,
                              workspace, workspace_bytes, stream, "rc_eval_topk_bf16_rep4", k_dev, w);
+}
+
+/* Open-vocabulary scores: the ids of rc_eval_topk_bf16 (same ranking, bit for bit) with the cosine of each ranked row and its
+ * softmax probability over all K rows at the temperature exp(*log_tau) (a device float: no host synchronisation). */
+extern "C" int rc_eval_topk_scores_bf16(const void* x, rc_dtype x_dtype, int B, int D, int64_t HW, const void* t_bf16, int K,
+                                        const int64_t* index_map, int k, const float* log_tau, int64_t* ids, float* cosine,
+                                        float* prob, void* workspace, int64_t workspace_bytes, void* stream) {
+  RC_REQUIRE(ids && cosine && prob && log_tau, "rc_eval_topk_scores_bf16: null pointer");
+  return eval_topk_bf16_impl(x, x_dtype, B, D, HW, t_bf16, K, index_map, k, ids, nullptr, nullptr, nullptr, 0, nullptr, nullptr,
+                             workspace, workspace_bytes, stream, "rc_eval_topk_scores_bf16", nullptr, 0, log_tau, cosine, prob);
+}
+
+/* The same on the decoder's half-resolution rows x [B][D][h*w]: ids, cosine and prob are full resolution [B][k][2h][2w]. */
+extern "C" int rc_eval_topk_scores_bf16_rep4(const void* x, rc_dtype x_dtype, int B, int D, int h, int w, const void* t_bf16,
+                                             int K, const int64_t* index_map, int k, const float* log_tau, int64_t* ids,
+                                             float* cosine, float* prob, void* workspace, int64_t workspace_bytes, void* stream) {
+  RC_REQUIRE(x && t_bf16 && index_map && ids && cosine && prob && log_tau, "rc_eval_topk_scores_bf16_rep4: null pointer");
+  RC_REQUIRE(h >= 1 && w >= 1, "rc_eval_topk_scores_bf16_rep4: bad shape (h=%d w=%d)", h, w);
+  return eval_topk_bf16_impl(x, x_dtype, B, D, (int64_t)h * w, t_bf16, K, index_map, k, ids, nullptr, nullptr, nullptr, 0, nullptr,
+                             nullptr, workspace, workspace_bytes, stream, "rc_eval_topk_scores_bf16_rep4", nullptr, w, log_tau,
+                             cosine, prob);
 }

@@ -99,6 +99,36 @@ def predict_from_embeddings(pixel_embeddings, candidate_text_embeddings, segment
     return topk, F.normalize(pixel_embeddings, dim=1)
 
 
+def segment_from_embeddings(pixel_embeddings, text_embeddings, log_temperature, top_k=1, candidates=None, shared2x2=False):
+    """Open-vocabulary segmentation of a decoder output against a vocabulary of the caller's choosing -- no ground truth,
+    no RNG, no host synchronisation.  ``text_embeddings`` [V,D] (normalised here, as ``F.normalize``); ``candidates``: an
+    optional 1-D tensor of vocabulary rows to rank (default: all V); ``log_temperature``: a 0-d tensor (e.g.
+    ``model.log_temperature_text``) or a float.  Returns (ids [B,k,H,W] int64 in the vocabulary's index space, cosine
+    [B,k,H,W] fp32, prob [B,k,H,W] fp32): the top ``k = min(top_k, K)`` rows of every pixel by cosine similarity, their
+    cosines, and their softmax probabilities over all K candidate rows at the temperature -- CLIP-style confidences; the
+    cosine is the score to reject "none of these" with.  One tensor-core launch (rc_eval_topk_scores_bf16); the [B,K,HW]
+    logits are never materialised.  ``shared2x2=True``: ``pixel_embeddings`` is the decoder's ``output_conv`` result
+    [B,D,H/2,W/2] (see ``predict_from_embeddings``) and the outputs are full resolution.  Shapes outside the kernel
+    (top_k > 8, D % 64 != 0, D > 1024, H*W % 8 != 0) raise."""
+    if shared2x2 and pixel_embeddings.dim() != 4:
+        raise RuntimeError("segment_from_embeddings: shared2x2=True takes the output_conv result [B, D, h, w]")
+    if not (pixel_embeddings.is_cuda and text_embeddings.is_cuda):
+        raise RuntimeError("segment_from_embeddings: needs CUDA tensors (no CPU fallback exists)")
+    dev = pixel_embeddings.device
+    if candidates is not None:
+        if candidates.dim() != 1:
+            raise RuntimeError("segment_from_embeddings: candidates must be a 1-D tensor of vocabulary rows")
+        index_map = candidates.to(device=dev, dtype=torch.int64)
+    else:
+        index_map = torch.arange(text_embeddings.shape[0], device=dev)
+    _, tb, _ = ops.text_prepare(text_embeddings, index_map if candidates is not None else None, want_f32=False, want_bf16=True)
+    if isinstance(log_temperature, torch.Tensor):
+        log_tau = log_temperature.detach().to(device=dev, dtype=torch.float32).reshape(1)
+    else:
+        log_tau = torch.full((1,), float(log_temperature), device=dev, dtype=torch.float32)
+    return torch.ops.rangeclip.eval_topk_scores(pixel_embeddings, tb, index_map, int(top_k), log_tau, bool(shared2x2))
+
+
 def predict_and_accumulate(pixel_embeddings, candidate_text_embeddings, segmentation, accumulator, num_negatives=300, top_k=5,
                            batch_index=None, want_ids=True, candidate_builder="reference", shared2x2=False):
     """``predict_from_embeddings`` + ``MetricAccumulator.update`` as one fused kernel per batch: same reduced candidate

@@ -807,6 +807,52 @@ def eval_topk_rep4(x: torch.Tensor, t_bf16: torch.Tensor, index_map: torch.Tenso
     return out
 
 
+def eval_topk_scores(x: torch.Tensor, t_bf16: torch.Tensor, index_map: torch.Tensor, k: int, log_tau: torch.Tensor,
+                     shared2x2: bool = False):
+    """Top-k over a vocabulary with scores (rc_eval_topk_scores_bf16 / _rep4): ``t_bf16`` [Kp,D] holds the L2-normalised rows
+    of ``index_map`` [K] (``text_prepare``), ``log_tau`` (device float, one element) the log of the softmax temperature.
+    Returns (ids int64, cosine fp32, prob fp32), each [B,k,H,W]: the ids of ``eval_topk`` mapped through ``index_map``, the
+    cosine of every ranked row and its softmax probability over all K rows at tau.  ``shared2x2``: ``x`` [B,D,h,w] is the
+    decoder's ``output_conv`` result and the outputs are [B,k,2h,2w].  Nothing is read back to the host."""
+    _need_cuda(x, t_bf16, index_map, log_tau)
+    if shared2x2:
+        if x.dim() != 4:
+            raise RuntimeError("eval_topk_scores: shared2x2 needs x [B, D, h, w]")
+        x = x.contiguous()
+        B, D, h, w = x.shape
+        HW, out_hw = h * w, (2 * h, 2 * w)
+    else:
+        x, B, D, HW = _emb3(x)
+        out_hw = tuple(x.shape[2:])
+    if not topk_bf16_supported(D, HW):
+        raise RuntimeError(f"eval_topk_scores: the tensor-core kernel does not cover D={D}, HW={HW}")
+    K = int(index_map.numel())
+    if K < 1 or t_bf16.dtype != torch.bfloat16 or t_bf16.dim() != 2 or t_bf16.shape[1] != D or t_bf16.shape[0] < (K + 63) // 64 * 64:
+        raise RuntimeError(f"eval_topk_scores: t_bf16 must be bf16 [round_up(K, 64), D] = [{(K + 63) // 64 * 64}, {D}]")
+    if log_tau.numel() != 1:
+        raise RuntimeError("eval_topk_scores: log_tau must hold one value")
+    k = min(int(k), K)
+    index_map = index_map.to(torch.int64).contiguous()
+    lt = log_tau.detach().reshape(1).to(torch.float32).contiguous()
+    ids = torch.empty((B, k) + out_hw, device=x.device, dtype=torch.int64)
+    cos = torch.empty((B, k) + out_hw, device=x.device, dtype=torch.float32)
+    prob = torch.empty((B, k) + out_hw, device=x.device, dtype=torch.float32)
+    L = _lib.lib()
+    xdt = _dt(x)
+    ws, ws_bytes = None, 0
+    if xdt == RC_F32:
+        ws_bytes = int(L.rc_infonce_workspace_bytes(B, D, HW, K, xdt))
+        ws = torch.empty(ws_bytes, device=x.device, dtype=torch.uint8)
+    tb = t_bf16.contiguous()
+    if shared2x2:
+        check(L.rc_eval_topk_scores_bf16_rep4(_p(x), xdt, B, D, h, w, _p(tb), K, _p(index_map), k, _p(lt), _p(ids), _p(cos),
+                                              _p(prob), _p(ws), ws_bytes, _stream(x)), "rc_eval_topk_scores_bf16_rep4")
+    else:
+        check(L.rc_eval_topk_scores_bf16(_p(x), xdt, B, D, HW, _p(tb), K, _p(index_map), k, _p(lt), _p(ids), _p(cos), _p(prob),
+                                         _p(ws), ws_bytes, _stream(x)), "rc_eval_topk_scores_bf16")
+    return ids, cos, prob
+
+
 def eval_hist(gt: torch.Tensor, topk: torch.Tensor, E_u8: torch.Tensor, cmap: torch.Tensor,
               hist: Optional[torch.Tensor] = None, counters: Optional[torch.Tensor] = None):
     """One batch of validate.py:88-139 as five class histograms + three counters (int64, added to)."""
@@ -1267,6 +1313,21 @@ def _op_eval_topk(x: torch.Tensor, t_norm: torch.Tensor, index_map: torch.Tensor
 def _(x, t_norm, index_map, k, precision, t_bf16):
     k = min(k, t_norm.shape[0])
     return torch.empty((x.shape[0], k) + tuple(x.shape[2:]), device=x.device, dtype=torch.int64)
+
+
+@_op("rangeclip::eval_topk_scores", mutates_args=(), device_types="cuda")
+def _op_eval_topk_scores(x: torch.Tensor, t_bf16: torch.Tensor, index_map: torch.Tensor, k: int, log_tau: torch.Tensor,
+                         shared2x2: bool) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    return eval_topk_scores(x, t_bf16, index_map, k, log_tau, shared2x2)
+
+
+@_op_eval_topk_scores.register_fake
+def _(x, t_bf16, index_map, k, log_tau, shared2x2):
+    k = min(k, index_map.numel())
+    hw = (2 * x.shape[2], 2 * x.shape[3]) if shared2x2 else tuple(x.shape[2:])
+    shape = (x.shape[0], k) + hw
+    return (torch.empty(shape, device=x.device, dtype=torch.int64), torch.empty(shape, device=x.device, dtype=torch.float32),
+            torch.empty(shape, device=x.device, dtype=torch.float32))
 
 
 @_op("rangeclip::eval_hist", mutates_args=("hist", "counters"), device_types="cuda")
